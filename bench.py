@@ -25,6 +25,9 @@ incidence, adjacency, connected components -- everything GeneMerGraph.__init__ c
            C4), each with its own parity check
 
 One JSON line on stdout (rank 0).  Everything else goes to stderr.
+
+--dump-outputs DIR writes the graph arrays of the last timed build (rank 0's, as a caller of DeviceGraph.arrays()
+receives them) to DIR/<name>.npy; the workload is seeded, so two builds of the project can be compared array by array.
 """
 from __future__ import annotations
 
@@ -134,6 +137,30 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_ROWS = 1 << 17
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """every array as float64 (exact for these integer arrays); one with more than DUMP_ROWS rows is replaced by the
+    rows at a fixed seeded sample of indices, which go to <name>_rows.npy, so that the dump stays within DUMP_BYTES"""
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, a in sorted(arrays.items()):
+        if not isinstance(a, np.ndarray) or a.ndim == 0:
+            continue
+        if len(a) > DUMP_ROWS:
+            rows = np.sort(np.random.default_rng(0).choice(len(a), DUMP_ROWS, replace=False)).astype(np.float64)
+            np.save(os.path.join(path, name + "_rows.npy"), rows)
+            total += rows.nbytes
+            a = a[rows.astype(np.int64)]
+        a = a.astype(np.float64)
+        np.save(os.path.join(path, name + ".npy"), a)
+        total += a.nbytes
+    assert total <= DUMP_BYTES, total
+    log("dumped the last timed build's arrays to %s (%.1f MB)" % (path, total / 2**20))
 
 
 def pinned(arr):
@@ -401,6 +428,8 @@ def run_gpu(args):
         dist.all_reduce(w_all)
     W_all = int(w_all.item())
     value = W_all * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dg.arrays())
 
     # per-phase times and the dominant kernel's duration: CUDA events on the handle's streams, separate untimed builds
     dg.set_profiling(True)
@@ -684,7 +713,10 @@ def main():
     ap.add_argument("--no-c2", action="store_true", help="alias of --no-extras")
     ap.add_argument("--no-c4", action="store_true")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end arm (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays of the last timed build to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.no_extras = args.no_extras or args.no_c2
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":

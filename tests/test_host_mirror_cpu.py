@@ -15,7 +15,7 @@ from amira_b200.construct_gene_mer import GeneMer
 from amira_b200.construct_read import Read
 from tests.fake_device import OracleBackedDevice
 from tests.graph_snapshot import check_small_cases, snapshot
-from tests.helpers import ROOT
+from tests.helpers import ROOT, check_postbuild
 
 
 @pytest.fixture()
@@ -100,13 +100,13 @@ def test_materialised_graph_matches_upstream_small_cases(fake_device, golden_sma
     check_small_cases(amira_b200.GeneMerGraph, golden_small, pytest)
 
 
-def test_host_mutators_and_gml(fake_device):
+def test_host_mutators_and_gml(fake_device, tmp_path):
     g = amira_b200.GeneMerGraph({"read1": ["+gene1", "-gene2", "+gene3", "-gene4"],
                                  "read2": ["+gene1", "-gene2", "+gene3", "-gene6"]}, 3)
     assert g.get_total_number_of_nodes() == 3 and g.get_total_number_of_edges() == 4
     first = next(g.all_nodes())
     assert g.get_degree(first) == 2 and len(g.get_all_neighbors(first)) == 2
-    gml = g.generate_gml(os.path.join("/tmp", "amira_b200_test_gml"), 3, 1, 1)
+    gml = g.generate_gml(str(tmp_path / "test_gml"), 3, 1, 1)
     assert gml[0] == "graph\t[" and gml[1] == "multigraph 1" and gml[-1] == "]"
     assert sum(e.startswith("\tnode") for e in gml) == 3 and sum(e.startswith("\tedge") for e in gml) == 4
     # single-object removal on the host, then the GPU filter must refuse the stale device copy
@@ -196,34 +196,35 @@ def test_bulk_keys_equal_hashlib_pickle():
             assert out[i].tobytes() == hashlib.sha256(pickle.dumps(t, protocol=4)).digest(), (arity, t)
 
 
-def test_post_build_statistics_match_upstream(fake_device):
-    """graph_utils.get_overall_mean_node_coverages / remove_junk_reads / get_valid_reads_only (the scans callers run
-    right after a build) against upstream's own implementations on upstream's own graph"""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip("upstream checkout not present (only in the build container)")
-    cg = ref_harness.load()
-    import amira.graph_utils as up_gu
+def statistics_values(G=None):
+    """-> label -> result of graph_utils.get_overall_mean_node_coverages / remove_junk_reads / get_valid_reads_only
+    (the scans callers run right after a build) on a C3 sample; the coverages both from the exported incidence
+    array and from the objects"""
     from amira_b200 import synth
     cfg = synth.CONFIGS["c3"]
     ids, off = synth.generate(cfg, 0, 400)
     reads = synth.to_read_dict(ids, off, synth.vocabulary_names(cfg.vocab))
     positions = {r: [(10 * i, 10 * i + 9) for i in range(len(v))] for r, v in reads.items()}
-    theirs = cg.GeneMerGraph(reads, 3, positions)
-    want = up_gu.get_overall_mean_node_coverages(theirs)
-    for G in (amira_b200.GeneMerGraph, amira_b200.bind_upstream(cg)):
-        g = G(reads, 3, positions)
-        got = amira_b200.get_overall_mean_node_coverages(g)            # from the exported incidence array
-        assert got == want and [type(v) for v in got.values()] == [type(v) for v in want.values()]
-        g._incidence_arrays = None                                      # ... and from the objects
-        assert amira_b200.get_overall_mean_node_coverages(g) == want
-    theirs.filter_graph(3, 1)
+    g = (G or amira_b200.GeneMerGraph)(reads, 3, positions)
+    v = {"mean_node_coverages": amira_b200.get_overall_mean_node_coverages(g)}
+    g._incidence_arrays = None
+    v["mean_node_coverages_from_objects"] = amira_b200.get_overall_mean_node_coverages(g)
     g = amira_b200.GeneMerGraph(reads, 3, positions)
     g.filter_graph(3, 1)
     for rate in (0.8, 0.5, 0.99):
-        assert g.remove_junk_reads(rate) == theirs.remove_junk_reads(rate)
-    assert g.get_valid_reads_only() == theirs.get_valid_reads_only()
-    assert amira_b200.get_overall_mean_node_coverages(g) == up_gu.get_overall_mean_node_coverages(theirs)
+        v["junk_reads_%s" % rate] = g.remove_junk_reads(rate)
+    v["valid_reads_only"] = g.get_valid_reads_only()
+    v["filtered_mean_node_coverages"] = amira_b200.get_overall_mean_node_coverages(g)
+    return v
+
+
+def test_post_build_statistics_match_upstream(fake_device):
+    """against the results of upstream's own implementations on upstream's own graph, stored as digests (see
+    tests/test_postbuild.py); with the upstream package at hand, also through the class bound to it"""
+    from oracle import ref_harness
+    check_postbuild("statistics/c3_400", statistics_values())
+    if ref_harness.available():
+        check_postbuild("statistics/c3_400", statistics_values(amira_b200.bind_upstream(ref_harness.load())))
 
 
 def test_encoded_reads_round_trip_and_incremental_update(tmp_path):

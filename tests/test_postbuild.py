@@ -1,38 +1,22 @@
 """The scans and edits Amira runs right after a build (SURVEY.md 8f): coverage statistics, junk / valid read
-selection, gene look-ups, linear paths, dead-end removal, AMR-node pruning, GML -- the drop-in class against
-UPSTREAM'S OWN functions on upstream's own graph of the same reads.
+selection, gene look-ups, linear paths, dead-end removal, AMR-node pruning, GML.
 
-Upstream comes from /root/reference (build container) or baseline/_ref (the git-ignored install that travels to
-the GPU box); without either the comparisons are skipped.  On CPU the device is the oracle-backed test double
-(read-only scans, paths, GML); with `-m gpu` everything runs on the real device, including the node removals."""
+The expected results are digests in tests/golden/postbuild.json (tests/record_postbuild.py writes them).  They were
+recorded from the drop-in class of the commit at which these tests last compared it, live, with upstream's own
+functions on upstream's own graph of the same reads; upstream's package is not part of this repository.  On CPU the
+device is the oracle-backed test double (read-only scans, paths, GML); with `-m gpu` everything runs on the real
+device, including the node removals."""
 import os
 
-import numpy as np
 import pytest
 
 import amira_b200
 from amira_b200 import construct_graph, graph_utils
-from oracle import ref_harness
 from tests.fake_device import OracleBackedDevice
 from tests.graph_snapshot import snapshot
-from tests.helpers import load_input, read_dict
-
-pytestmark = pytest.mark.skipif(not ref_harness.available(), reason="upstream package not present (baseline/_ref)")
+from tests.helpers import check_postbuild, load_input, read_dict
 
 CASES = [("fixture_eight", 3), ("fixture_seven", 3), ("fixture_four", 5), ("synth_c2_2000", 3)]
-
-
-def upstream_graph(name, k):
-    cg = ref_harness.load()
-    vocab, ids, off, ps, pe = load_input(name)
-    reads, pos = read_dict(vocab, ids, off, ps, pe)
-    return cg, cg.GeneMerGraph({r: list(v) for r, v in reads.items()}, k, pos), reads, pos, vocab
-
-
-def upstream_graph_utils():
-    ref_harness.load()
-    import importlib
-    return importlib.import_module("amira.graph_utils")
 
 
 def genes_of_interest(vocab):
@@ -40,40 +24,77 @@ def genes_of_interest(vocab):
     return [names[i] for i in range(0, len(names), max(1, len(names) // 7))][:6] + ["not_a_gene_in_this_sample"]
 
 
-def check_readonly(name, k):
-    cg, up, reads, pos, vocab = upstream_graph(name, k)
+def readonly_values(name, k, tmp):
+    """-> (graph, vocabulary, label -> result of every read-only scan)"""
+    vocab, ids, off, ps, pe = load_input(name)
+    reads, pos = read_dict(vocab, ids, off, ps, pe)
     ours = amira_b200.GeneMerGraph({r: list(v) for r, v in reads.items()}, k, pos)
-    gu = upstream_graph_utils()
+    v = {}
     # statistics straight from the device arrays (nothing materialised yet)
     assert ours.__dict__["_lazy"]
-    assert graph_utils.get_overall_mean_node_coverages(ours) == gu.get_overall_mean_node_coverages(up)
-    assert ours.get_mean_node_coverage() == up.get_mean_node_coverage()
-    assert ours.get_all_node_coverages() == up.get_all_node_coverages()
-    assert ours.get_total_number_of_nodes() == up.get_total_number_of_nodes()
-    assert ours.components() == up.components()
+    v["overall_mean_node_coverages"] = graph_utils.get_overall_mean_node_coverages(ours)
+    v["mean_node_coverage"] = ours.get_mean_node_coverage()
+    v["all_node_coverages"] = ours.get_all_node_coverages()
+    v["total_number_of_nodes"] = ours.get_total_number_of_nodes()
+    v["components"] = ours.components()
     assert ours.__dict__["_lazy"], "the statistics must not need the host objects"
     # GML from the arrays
-    out = os.path.join("/tmp", "amira_b200_gml_%s_%d" % (name, k))
-    assert ours.generate_gml(out, k, 1, 1) == up.generate_gml(out + "_up", k, 1, 1)
+    out = os.path.join(str(tmp), "gml_%s_%d" % (name, k))
+    v["gml_1_1"] = ours.generate_gml(out, k, 1, 1)
     assert ours.__dict__["_lazy"]
     # filters on the device, then the read selections (still no host objects)
     ours.filter_graph(3, 1)
-    up.filter_graph(3, 1)
     for er in (0.0, 0.2, 0.5, 0.93):
-        assert ours.remove_junk_reads(er) == up.remove_junk_reads(er), er
-    assert ours.get_valid_reads_only() == up.get_valid_reads_only()
-    assert ours.generate_gml(out, k, 3, 1) == up.generate_gml(out + "_up", k, 3, 1)
+        v["junk_reads_%s" % er] = ours.remove_junk_reads(er)
+    v["valid_reads_only"] = ours.get_valid_reads_only()
+    v["gml_3_1"] = ours.generate_gml(out, k, 3, 1)
     assert ours.__dict__["_lazy"]
-    assert snapshot(ours) == snapshot(up)            # materialises from the filtered device graph
+    v["snapshot_filtered"] = snapshot(ours)            # materialises from the filtered device graph
     # gene look-ups and linear paths
     for g in genes_of_interest(vocab):
-        assert [n.__hash__() for n in ours.get_nodes_containing(g)] == [n.__hash__() for n in up.get_nodes_containing(g)], g
-    goi = genes_of_interest(vocab)
-    assert list(ours.get_AMR_nodes(goi)) == list(up.get_AMR_nodes(goi))
+        v["nodes_containing_" + g] = [n.__hash__() for n in ours.get_nodes_containing(g)]
+    v["AMR_nodes"] = list(ours.get_AMR_nodes(genes_of_interest(vocab)))
     for want in (False, True):
-        for no, nu in zip(ours.all_nodes(), up.all_nodes()):
-            assert ours.get_linear_path_for_node(no, want) == up.get_linear_path_for_node(nu, want)
-    return ours, up, vocab
+        v["linear_paths_%s" % want] = [ours.get_linear_path_for_node(n, want) for n in ours.all_nodes()]
+    return ours, vocab, v
+
+
+def edit_values(ours, vocab):
+    """dead ends: remove_short_linear_paths (construct_graph.py:679-720) with and without genes of interest, then
+    pruning to the reads of the genes of interest"""
+    v = {}
+    v["short_paths_4"] = sorted(ours.remove_short_linear_paths(4, genes_of_interest(vocab)[:2]))
+    v["snapshot_short_paths_4"] = snapshot(ours)
+    v["short_paths_6"] = sorted(ours.remove_short_linear_paths(6))
+    v["snapshot_short_paths_6"] = snapshot(ours)
+    ours.remove_non_AMR_associated_nodes(genes_of_interest(vocab))
+    v["snapshot_non_AMR_removed"] = snapshot(ours)
+    return v
+
+
+def k_sweep_values():
+    """choose_kmer_size's sweep (graph_utils.py:258-296): one encoding, resident CSR, one build per k"""
+    vocab, ids, off, ps, pe = load_input("fixture_four")
+    reads, pos = read_dict(vocab, ids, off, ps, pe)
+    v = {}
+    for k, g in graph_utils.build_k_sweep(reads, range(3, 10, 2), pos).items():
+        assert g.__dict__["_lazy"]
+        v["k%d_mean_node_coverage" % k] = g.get_mean_node_coverage()
+        v["k%d_snapshot" % k] = snapshot(g)
+    return v
+
+
+def lazy_rebuild_values():
+    """a graph whose device copy was overwritten by a later build (one handle per device) rebuilds and replays its
+    device operations before answering"""
+    vocab, ids, off, ps, pe = load_input("fixture_eight")
+    reads, pos = read_dict(vocab, ids, off, ps, pe)
+    g1 = amira_b200.GeneMerGraph(reads, 3)
+    g1.remove_low_coverage_components(5)
+    g1.filter_graph(3, 1)
+    g2 = amira_b200.GeneMerGraph(reads, 5)
+    return {"g1_mean_node_coverage": g1.get_mean_node_coverage(), "g1_snapshot": snapshot(g1),
+            "g2_total_number_of_nodes": g2.get_total_number_of_nodes()}
 
 
 @pytest.fixture()
@@ -83,56 +104,23 @@ def fake_device(monkeypatch):
 
 
 @pytest.mark.parametrize("name,k", CASES[:2])
-def test_postbuild_scans_cpu_double(fake_device, name, k):
-    check_readonly(name, k)
+def test_postbuild_scans_cpu_double(fake_device, tmp_path, name, k):
+    check_postbuild("scans/%s_k%d" % (name, k), readonly_values(name, k, tmp_path)[2])
 
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name,k", CASES)
-def test_postbuild_scans_gpu(name, k):
-    ours, up, vocab = check_readonly(name, k)
-    # dead ends: remove_short_linear_paths (construct_graph.py:679-720) with and without genes of interest
-    goi = genes_of_interest(vocab)[:2]
-    removed_o = ours.remove_short_linear_paths(4, goi)
-    removed_u = up.remove_short_linear_paths(4, goi)
-    assert sorted(removed_o) == sorted(removed_u)
-    assert snapshot(ours) == snapshot(up)
-    # a second round on the edited graph, then pruning to the reads of the genes of interest
-    assert sorted(ours.remove_short_linear_paths(6)) == sorted(up.remove_short_linear_paths(6))
-    assert snapshot(ours) == snapshot(up)
-    ours.remove_non_AMR_associated_nodes(genes_of_interest(vocab))
-    up.remove_non_AMR_associated_nodes(genes_of_interest(vocab))
-    assert snapshot(ours) == snapshot(up)
+def test_postbuild_scans_gpu(tmp_path, name, k):
+    ours, vocab, v = readonly_values(name, k, tmp_path)
+    check_postbuild("scans/%s_k%d" % (name, k), v)
+    check_postbuild("edits/%s_k%d" % (name, k), edit_values(ours, vocab))
 
 
 @pytest.mark.gpu
 def test_k_sweep_on_resident_reads_gpu():
-    """choose_kmer_size's sweep (graph_utils.py:258-296): one encoding, resident CSR, one build per k"""
-    vocab, ids, off, ps, pe = load_input("fixture_four")
-    reads, pos = read_dict(vocab, ids, off, ps, pe)
-    sweep = graph_utils.build_k_sweep(reads, range(3, 10, 2), pos)
-    cg = ref_harness.load()
-    for k, g in sweep.items():
-        assert g.__dict__["_lazy"]
-        up = cg.GeneMerGraph({r: list(v) for r, v in reads.items()}, k, pos)
-        assert g.get_mean_node_coverage() == up.get_mean_node_coverage()
-        assert snapshot(g) == snapshot(up), k
+    check_postbuild("k_sweep/fixture_four", k_sweep_values())
 
 
 @pytest.mark.gpu
 def test_lazy_graph_survives_another_build_gpu():
-    """a graph whose device copy was overwritten by a later build (one handle per device) rebuilds and replays its
-    device operations before answering"""
-    vocab, ids, off, ps, pe = load_input("fixture_eight")
-    reads, pos = read_dict(vocab, ids, off, ps, pe)
-    cg = ref_harness.load()
-    g1 = amira_b200.GeneMerGraph(reads, 3)
-    g1.remove_low_coverage_components(5)
-    g1.filter_graph(3, 1)
-    g2 = amira_b200.GeneMerGraph(reads, 5)
-    up = cg.GeneMerGraph({r: list(v) for r, v in reads.items()}, 3)
-    up.remove_low_coverage_components(5)
-    up.filter_graph(3, 1)
-    assert g1.get_mean_node_coverage() == up.get_mean_node_coverage()
-    assert snapshot(g1) == snapshot(up)
-    assert g2.get_total_number_of_nodes() == cg.GeneMerGraph({r: list(v) for r, v in reads.items()}, 5).get_total_number_of_nodes()
+    check_postbuild("lazy_rebuild/fixture_eight", lazy_rebuild_values())
