@@ -7,6 +7,7 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <atomic>
 #include <string>
 
 #include "../../include/amira_gmg.h"
@@ -31,12 +32,20 @@ void set_error(const char *fmt, ...);
         if (_s != AMIRA_OK) return _s; \
     } while (0)
 
+// Bumped whenever a device buffer is reallocated or two buffers trade places.  A captured CUDA graph holds raw
+// pointers: it may only be replayed while the generation it was captured at is still current.
+inline std::atomic<uint64_t> &buffer_generation() {
+    static std::atomic<uint64_t> g{0};
+    return g;
+}
+
 // grow-only device allocation, reused across builds (Amira rebuilds the graph ~10-100x per sample)
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
     int reserve(size_t bytes) {
         if (bytes <= cap) return AMIRA_OK;
+        buffer_generation()++;
         if (p) cudaFree(p);
         p = nullptr;
         cap = 0;

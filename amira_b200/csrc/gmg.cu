@@ -120,9 +120,11 @@ struct amira_gmg {
         int64_t R, G, cap_nodes, cap_edges;
         unsigned int ncap, ecap;
         int k, key_bits, layout;
+        uint64_t buffers;  // buffer_generation() (common.cuh): the device buffers the graph was captured with
         bool operator==(const GraphKey &o) const {
             return ids == o.ids && off == o.off && ps == o.ps && pe == o.pe && R == o.R && G == o.G && cap_nodes == o.cap_nodes &&
-                   cap_edges == o.cap_edges && ncap == o.ncap && ecap == o.ecap && k == o.k && key_bits == o.key_bits && layout == o.layout;
+                   cap_edges == o.cap_edges && ncap == o.ncap && ecap == o.ecap && k == o.k && key_bits == o.key_bits && layout == o.layout &&
+                   buffers == o.buffers;
         }
     };
     GraphKey graph_key = {}, last_key = {};
@@ -734,7 +736,7 @@ int do_build(amira_gmg *h) {
         AMIRA_TRY(plan_build(h));
         AMIRA_TRY(reserve_graph(h, h->ncap, 2 * (int64_t)h->ecap));
         const amira_gmg::GraphKey key{h->ids, h->off, h->ps, h->pe, h->R, h->G, h->cap_nodes, h->cap_edges, h->ncap, h->ecap,
-                                      h->k, h->key_bits, (h->n16 ? 1 : 0) | (h->e16 ? 2 : 0)};
+                                      h->k, h->key_bits, (h->n16 ? 1 : 0) | (h->e16 ? 2 : 0), buffer_generation().load()};
         static const bool no_graph = getenv("AMIRA_NO_GRAPH") != nullptr;
         const bool can_graph = h->input_on_device && !h->profiling && h->n_pieces == 0 && h->G <= (64ll << 20) && !no_graph;
         auto after_launch = [&]() -> int {
@@ -912,7 +914,8 @@ int finish(amira_gmg *h, bool early) {
         h->n_inc = z[SZ_INC];
         h->n_fw = z[SZ_FW];
         h->n_bw = h->n_edges - h->n_fw;
-        h->n_comps = h->n_nodes;  // upper bound on component ids (ids are <= number of nodes)
+        // upper bound on component ids: ids are <= the number of nodes of the BUILD, and filters keep the ids
+        if (h->pending_is_build) h->n_comps = h->n_nodes;
         h->pending = 0;
         if (h->pending_is_build) {
             if (h->world == 1) {
@@ -988,6 +991,7 @@ int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
         AMIRA_CUDA(cudaMemcpyAsync(h->h_status, h->d_status.p, sizeof(int) * ST_COUNT, cudaMemcpyDeviceToHost, st));
         AMIRA_CUDA(cudaStreamSynchronize(st));
         if (h->h_status[ST_ERR] == AMIRA_E_MULTI_EDGE) {
+            h->filt_N = h->filt_E = -1;  // the graph is unchanged, and keep_n no longer holds the last filter's flags
             set_error("unhashable type: 'list'");
             return AMIRA_E_MULTI_EDGE;
         }
@@ -1032,11 +1036,19 @@ int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
         std::swap(h->e_td, h->e_td2);
         std::swap(h->e_cov, h->e_cov2);
     }
+    buffer_generation()++;  // a build captured before this filter would write into the old buffers
     AMIRA_TRY(build_adjacency(h, false));
     AMIRA_TRY(enqueue_report(h, 1));
     h->pending = 2;
     h->pending_is_build = false;
     return AMIRA_OK;
+}
+
+// the status a filter / removal leaves for the calls after it.  One refused for a multi-edge changed nothing, so the
+// graph stays usable and keeps the status it had (upstream's graph also survives the TypeError).
+int filter_status(amira_gmg *h, int rc) {
+    if (rc != AMIRA_E_MULTI_EDGE) h->last_status = rc;
+    return rc;
 }
 
 // ---- multi-GPU: merge the local tables of all ranks into the global node / edge arrays ----------
@@ -1852,12 +1864,12 @@ int amira_gmg_export_reads(amira_gmg *h, int64_t *win_off, int32_t *node_idx, in
 
 int amira_gmg_remove_low_coverage_components(amira_gmg *h, uint32_t min_component_cov) {
     AMIRA_TRY(check_handle(h));
-    return h->last_status = do_filter(h, 1, min_component_cov, 0);
+    return filter_status(h, do_filter(h, 1, min_component_cov, 0));
 }
 
 int amira_gmg_filter(amira_gmg *h, uint32_t min_node_cov, uint32_t min_edge_cov) {
     AMIRA_TRY(check_handle(h));
-    return h->last_status = do_filter(h, 0, min_node_cov, min_edge_cov);
+    return filter_status(h, do_filter(h, 0, min_node_cov, min_edge_cov));
 }
 
 int amira_gmg_filter_mask_sizes(amira_gmg *h, int64_t *n_nodes_before, int64_t *n_edges_before) {
@@ -1946,7 +1958,10 @@ int amira_gmg_node_coverage_stats(amira_gmg *h, int64_t *sum_cov, uint32_t *max_
 int amira_gmg_junk_read_mask(amira_gmg *h, double error_rate, uint8_t *mask) {
     AMIRA_TRY(stats_ready(h));
     if (h->R == 0) return AMIRA_OK;
-    if (!mask) return AMIRA_E_ARG;
+    if (!mask) {
+        set_error("junk_read_mask: no output buffer");
+        return AMIRA_E_ARG;
+    }
     AMIRA_TRY(h->scratch_off.reserve((size_t)h->R + 8));
     LAUNCH(h, k_junk_read_mask, grid_for(h->R, 256), 256, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
            h->is_short.as<uint8_t>(), (long long)h->R, error_rate, h->scratch_off.as<uint8_t>());
@@ -1958,7 +1973,10 @@ int amira_gmg_junk_read_mask(amira_gmg *h, double error_rate, uint8_t *mask) {
 namespace {
 // flags[i] = node i holds one of the genes; left on the device in scratch_off (N bytes), ranks in comp_max
 int flag_nodes_containing(amira_gmg *h, const int32_t *ranks, int32_t n) {
-    if (n < 0 || (n > 0 && !ranks)) return AMIRA_E_ARG;
+    if (n < 0 || (n > 0 && !ranks)) {
+        set_error("bad gene ranks (n = %d)", n);
+        return AMIRA_E_ARG;
+    }
     const int64_t N = h->n_nodes;
     AMIRA_TRY(h->scratch_off.reserve((size_t)std::max<int64_t>(N, h->R) + 8));
     AMIRA_TRY(h->comp_max.reserve(sizeof(int32_t) * (size_t)std::max(n, 1) + sizeof(uint32_t) * (size_t)(h->n_comps + 2)));
@@ -1985,21 +2003,27 @@ int amira_gmg_remove_nodes(amira_gmg *h, const uint8_t *remove_flags) {
     AMIRA_TRY(check_handle(h));
     AMIRA_TRY(filter_reserve(h));
     const int64_t N = h->n_nodes;
-    if (N == 0) return h->last_status = AMIRA_OK;
-    if (!remove_flags) return AMIRA_E_ARG;
-    std::vector<int> keep((size_t)N + 1);
-    for (int64_t i = 0; i < N; ++i) keep[i] = remove_flags[i] ? 0 : 1;
-    keep[N] = 0;
-    AMIRA_CUDA(cudaMemcpyAsync(h->keep_n.p, keep.data(), sizeof(int) * (N + 1), cudaMemcpyHostToDevice, h->stream));
-    AMIRA_CUDA(cudaStreamSynchronize(h->stream));  // `keep` goes out of scope
-    return h->last_status = do_filter(h, 2, 0, 0);
+    // an empty graph still goes through do_filter: the filter masks must then describe this call (zero nodes),
+    // not the previous one
+    if (N > 0) {
+        if (!remove_flags) {
+            set_error("remove_nodes: no flags for %lld nodes", (long long)N);
+            return AMIRA_E_ARG;
+        }
+        std::vector<int> keep((size_t)N + 1);
+        for (int64_t i = 0; i < N; ++i) keep[i] = remove_flags[i] ? 0 : 1;
+        keep[N] = 0;
+        AMIRA_CUDA(cudaMemcpyAsync(h->keep_n.p, keep.data(), sizeof(int) * (N + 1), cudaMemcpyHostToDevice, h->stream));
+        AMIRA_CUDA(cudaStreamSynchronize(h->stream));  // `keep` goes out of scope
+    }
+    return filter_status(h, do_filter(h, 2, 0, 0));
 }
 
 int amira_gmg_remove_nodes_without_reads_of(amira_gmg *h, const int32_t *ranks, int32_t n) {
     AMIRA_TRY(check_handle(h));
     AMIRA_TRY(filter_reserve(h));
     const int64_t N = h->n_nodes, R = h->R;
-    if (N == 0) return h->last_status = AMIRA_OK;
+    if (N == 0) return filter_status(h, do_filter(h, 2, 0, 0));  // as in amira_gmg_remove_nodes
     AMIRA_TRY(flag_nodes_containing(h, ranks, n));
     // reads of the flagged nodes (byte flags behind the node flags), then the nodes that touch none of them
     AMIRA_TRY(h->dups.reserve((size_t)R + 8));
@@ -2009,13 +2033,14 @@ int amira_gmg_remove_nodes_without_reads_of(amira_gmg *h, const int32_t *ranks, 
            h->reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, read_flag);
     LAUNCH(h, k_nodes_with_marked_reads, grid_for((N + 1) * 32, 256), 256, read_flag, h->reads_off.as<int64_t>(),
            h->reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, h->keep_n.as<int>());
-    return h->last_status = do_filter(h, 2, 0, 0);
+    return filter_status(h, do_filter(h, 2, 0, 0));
 }
 
 int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int8_t *fw_dir, uint8_t *fw_ext, int32_t *bw_next,
                            int8_t *bw_dir, uint8_t *bw_ext) {
     AMIRA_TRY(stats_ready(h));
     const int64_t N = h->n_nodes;
+    h->filt_N = h->filt_E = -1;  // the steps are computed in keep_e, the edge mask of the last filter
     if (N == 0) return AMIRA_OK;
     // [degree u32][next fw i32][next bw i32][dir fw i8][dir bw i8][ext fw u8][ext bw u8] per node
     AMIRA_TRY(h->keep_e.reserve((size_t)N * 16 + 64));
@@ -2038,7 +2063,6 @@ int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int
     AMIRA_TRY(d2h(h, fw_ext, S.ext[0], N));
     AMIRA_TRY(d2h(h, bw_ext, S.ext[1], N));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
-    h->filt_N = h->filt_E = -1;  // keep_e was the edge mask of the last filter
     return AMIRA_OK;
 }
 

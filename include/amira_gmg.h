@@ -163,7 +163,11 @@ int amira_gmg_export_filter_masks(amira_gmg *h, int32_t *node_keep, int32_t *edg
  * linear_steps: the building block of get_linear_path_for_node / remove_short_linear_paths / get_unitigs_in_graph
  *   (construct_graph.py:722-861, 679-720, 2961-2975): Node degree and, per node and side (forward / backward),
  *   upstream's one step along a linear path: next node (-1 none), direction in which it is entered, and whether
- *   the walk continues (target of degree 1 or 2, not the node itself). */
+ *   the walk continues (target of degree 1 or 2, not the node itself).  It reuses the memory of the filter masks:
+ *   after it, amira_gmg_filter_mask_sizes / amira_gmg_export_filter_masks fail with AMIRA_E_STATE until the next
+ *   filter or removal.
+ * A filter or removal that fails with AMIRA_E_MULTI_EDGE leaves the graph unchanged and usable, without filter masks;
+ * after one on a graph without nodes the masks describe zero nodes and zero edges. */
 int amira_gmg_read_length_coverages(amira_gmg *h, const int32_t *min_len, int32_t n, int64_t *sums);
 int amira_gmg_node_coverage_stats(amira_gmg *h, int64_t *sum_cov, uint32_t *max_cov);
 int amira_gmg_junk_read_mask(amira_gmg *h, double error_rate, uint8_t *mask);

@@ -34,6 +34,7 @@ def lib():
         _lib.oracle_build.restype = C.c_int
         _lib.oracle_filter.restype = C.c_int
         _lib.oracle_remove_low_coverage_components.restype = C.c_int
+        _lib.oracle_remove_nodes.restype = C.c_int
     return _lib
 
 
@@ -67,6 +68,16 @@ class COracleGraph:
     def remove_low_coverage_components(self, c):
         rc = lib().oracle_remove_low_coverage_components(self._h, C.c_uint32(c))
         if rc == E_MULTIEDGE:
+            raise TypeError("unhashable type: 'list'")
+
+    def remove_nodes(self, flags):
+        """remove_node for every node whose flag is set (flags[n_nodes], current node order); TypeError and no
+        change when one of them has two edges to the same neighbour"""
+        f = np.ascontiguousarray(flags, np.uint8)
+        n = C.c_int64()
+        lib().oracle_sizes(self._h, C.byref(n), *[C.byref(C.c_int64()) for _ in range(5)])
+        assert f.shape == (n.value,), (f.shape, n.value)
+        if lib().oracle_remove_nodes(self._h, _p(f)) == E_MULTIEDGE:
             raise TypeError("unhashable type: 'list'")
 
     def arrays(self) -> dict:

@@ -13,6 +13,7 @@
  *   - node read list (unique, first touch)     amira/construct_node.py:64-67
  *   - component numbering                      amira/construct_graph.py:911-927
  *   - filter_graph / remove_low_coverage_components   amira/construct_graph.py:409-540, 929-958
+ *   - remove_node for a set of nodes           amira/construct_graph.py:463-484
  *
  * It follows the reference's *event order* literally (forward edge then reverse edge per adjacent
  * pair, each one insert-or-get followed by a coverage increment) rather than any derived shortcut,
@@ -351,6 +352,30 @@ int oracle_filter(oracle_graph *g, uint32_t min_node_cov, uint32_t min_edge_cov)
     return ORACLE_OK;
 }
 
+/* remove_node -> get_edge_hashes_between_nodes returns lists when a doomed node has two edges
+   to the same neighbour; upstream then raises TypeError.  Only possible for k = 1 / even k.
+   Two edges between the same ordered pair always differ in relative orientation (sd * td). */
+static int has_multi_edge(oracle_graph *g, const uint8_t *node_rm) {
+    if (!g->emap) {  /* dropped by an earlier removal: rebuild it at its final size (a full table never ends a probe) */
+        int64_t cap = 4096;
+        while (cap < 2 * g->n_edges + 2) cap *= 2;
+        g->emap_cap = cap / 2;
+        rehash_edges(g);
+    }
+    for (int64_t e = 0; e < g->n_edges; ++e) {
+        if (!node_rm[g->edge_src[e]]) continue;
+        int rel = -(g->edge_sd[e] * g->edge_td[e]);
+        uint64_t s = edge_hash(g->edge_src[e], g->edge_tgt[e], rel) & (uint64_t)(g->emap_cap - 1);
+        while (g->emap[s] >= 0) {
+            int32_t f = g->emap[s];
+            if (g->edge_src[f] == g->edge_src[e] && g->edge_tgt[f] == g->edge_tgt[e] &&
+                g->edge_sd[f] * g->edge_td[f] == rel) return 1;
+            s = (s + 1) & (uint64_t)(g->emap_cap - 1);
+        }
+    }
+    return 0;
+}
+
 int oracle_remove_low_coverage_components(oracle_graph *g, uint32_t min_component_cov) {
     uint32_t maxc = 0;
     for (int64_t i = 0; i < g->n_nodes; ++i) if (g->node_comp[i] > maxc) maxc = g->node_comp[i];
@@ -360,22 +385,17 @@ int oracle_remove_low_coverage_components(oracle_graph *g, uint32_t min_componen
     uint8_t *nrm = calloc(g->n_nodes + 1, 1), *erm = calloc(g->n_edges + 1, 1);
     for (int64_t i = 0; i < g->n_nodes; ++i) nrm[i] = best[g->node_comp[i]] < min_component_cov;
     free(best);
-    /* remove_node -> get_edge_hashes_between_nodes returns lists when a doomed node has two edges
-       to the same neighbour; upstream then raises TypeError.  Only possible for k = 1 / even k. */
-    int multi = 0;
-    if (!g->emap) { g->emap_cap = 0; rehash_edges(g); while (g->emap_cap < 2 * g->n_edges + 2) rehash_edges(g); }
-    for (int64_t e = 0; e < g->n_edges && !multi; ++e) {
-        if (!nrm[g->edge_src[e]]) continue;
-        int rel = -(g->edge_sd[e] * g->edge_td[e]);
-        uint64_t s = edge_hash(g->edge_src[e], g->edge_tgt[e], rel) & (uint64_t)(g->emap_cap - 1);
-        while (g->emap[s] >= 0) {
-            int32_t f = g->emap[s];
-            if (g->edge_src[f] == g->edge_src[e] && g->edge_tgt[f] == g->edge_tgt[e] &&
-                g->edge_sd[f] * g->edge_td[f] == rel) { multi = 1; break; }
-            s = (s + 1) & (uint64_t)(g->emap_cap - 1);
-        }
-    }
-    if (multi) { free(nrm); free(erm); return ORACLE_E_MULTIEDGE; }
+    if (has_multi_edge(g, nrm)) { free(nrm); free(erm); return ORACLE_E_MULTIEDGE; }
+    apply_removal(g, nrm, erm);
+    free(nrm); free(erm);
+    return ORACLE_OK;
+}
+
+/* remove_node (construct_graph.py:463-484) for every node whose flag is set; nothing changes on a multi-edge */
+int oracle_remove_nodes(oracle_graph *g, const uint8_t *flags) {
+    uint8_t *nrm = calloc(g->n_nodes + 1, 1), *erm = calloc(g->n_edges + 1, 1);
+    for (int64_t i = 0; i < g->n_nodes; ++i) nrm[i] = flags[i] != 0;
+    if (has_multi_edge(g, nrm)) { free(nrm); free(erm); return ORACLE_E_MULTIEDGE; }
     apply_removal(g, nrm, erm);
     free(nrm); free(erm);
     return ORACLE_OK;

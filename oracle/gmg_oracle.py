@@ -28,6 +28,7 @@ independent, keyed by signed SHA-rank gene ids, in the reference's insertion ord
 """
 from __future__ import annotations
 
+import copy
 import hashlib
 import pickle
 
@@ -251,6 +252,20 @@ class OracleGraph:
             if all(n.cov < min_component_cov for n in members):
                 for n in members:
                     self._remove_node(n)
+
+    def remove_nodes(self, indices):
+        """remove_node, one at a time, for the nodes at these positions of the current node order (upstream's loop
+        in remove_short_linear_paths / remove_non_AMR_associated_nodes).  Upstream raises TypeError half way through
+        and leaves the graph partly edited; here the graph is restored, as the library leaves it unchanged."""
+        nodes = list(self.nodes.values())
+        doomed = [nodes[i] for i in sorted(set(int(i) for i in indices))]
+        saved = copy.deepcopy(self.__dict__)
+        try:
+            for n in doomed:
+                self._remove_node(n)
+        except TypeError:
+            self.__dict__ = saved
+            raise
 
     # ---- array view -------------------------------------------------------------
     def vocabulary(self):

@@ -304,11 +304,9 @@ def test_gpu_segmented_sort_all_size_classes(dg, out_of_place, vmax):
     assert np.array_equal(dups, want_dups) and total == int(want_dups.sum())
 
 
-def test_gpu_repeated_genemers_and_heavy_nodes(dg):
-    """a gene-mer twice on one read (duplicate incidences are removed, coverage counts both) and nodes that lie
-    on more reads than a CTA sorts in shared memory"""
-    from oracle import c_oracle
-    from oracle import gmg_oracle as O
+def heavy_node_reads():
+    """20000 reads that all carry the core genes 1, 2, 3, 4 (every 7th twice, around gene 9) beside a random tail of
+    genes 5..399 -> (ids, off)"""
     rng = np.random.default_rng(3)
     reads = []
     for i in range(20000):                                   # every read carries (1,2,3[,4]) -> nodes on 20000 reads
@@ -321,6 +319,15 @@ def test_gpu_repeated_genemers_and_heavy_nodes(dg):
         reads.append(core + tail if i % 3 else tail + core)
     off = np.concatenate([[0], np.cumsum([len(r) for r in reads])]).astype(np.int64)
     ids = np.concatenate([np.asarray(r, np.int32) for r in reads])
+    return ids, off
+
+
+def test_gpu_repeated_genemers_and_heavy_nodes(dg):
+    """a gene-mer twice on one read (duplicate incidences are removed, coverage counts both) and nodes that lie
+    on more reads than a CTA sorts in shared memory"""
+    from oracle import c_oracle
+    from oracle import gmg_oracle as O
+    ids, off = heavy_node_reads()
     for k in (3, 5):
         ref = c_oracle.COracleGraph(ids, off, k)
         dg.build(ids, off, k)

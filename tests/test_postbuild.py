@@ -4,8 +4,8 @@ selection, gene look-ups, linear paths, dead-end removal, AMR-node pruning, GML.
 The expected results are digests in tests/golden/postbuild.json (tests/record_postbuild.py writes them).  They were
 recorded from the drop-in class of the commit at which these tests last compared it, live, with upstream's own
 functions on upstream's own graph of the same reads; upstream's package is not part of this repository.  On CPU the
-device is the oracle-backed test double (read-only scans, paths, GML); with `-m gpu` everything runs on the real
-device, including the node removals."""
+device is the oracle-backed test double (scans, paths, GML and the node removals); with `-m gpu` everything runs on
+the real device."""
 import os
 
 import pytest
@@ -106,6 +106,15 @@ def fake_device(monkeypatch):
 @pytest.mark.parametrize("name,k", CASES[:2])
 def test_postbuild_scans_cpu_double(fake_device, tmp_path, name, k):
     check_postbuild("scans/%s_k%d" % (name, k), readonly_values(name, k, tmp_path)[2])
+
+
+@pytest.mark.parametrize("name,k", CASES[:2])
+def test_postbuild_edits_cpu_double(fake_device, tmp_path, name, k):
+    """the node removals (linear-path pruning, AMR pruning) through the test double's remove_nodes /
+    remove_nodes_without_reads_of, against the digests the device recorded"""
+    ours, vocab, v = readonly_values(name, k, tmp_path)
+    check_postbuild("scans/%s_k%d" % (name, k), v)
+    check_postbuild("edits/%s_k%d" % (name, k), edit_values(ours, vocab))
 
 
 @pytest.mark.gpu
