@@ -8,7 +8,7 @@
 #include <string.h>
 
 #include <atomic>
-#include <string>
+#include <utility>
 
 #include "../../include/amira_gmg.h"
 
@@ -39,16 +39,25 @@ inline std::atomic<uint64_t> &buffer_generation() {
     return g;
 }
 
-// grow-only device allocation, reused across builds (Amira rebuilds the graph ~10-100x per sample)
+// grow-only device allocation, reused across builds (Amira rebuilds the graph ~10-100x per sample).  The owner frees
+// it; it must be destroyed while its device is current.
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept { swap(o); }
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        swap(o);
+        o.release();
+        return *this;
+    }
+    ~DevBuf() { release(); }
     int reserve(size_t bytes) {
         if (bytes <= cap) return AMIRA_OK;
         buffer_generation()++;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        release();
         size_t want = bytes + bytes / 8 + 256;
         cudaError_t e = cudaMalloc(&p, want);
         if (e != cudaSuccess) {
@@ -62,6 +71,12 @@ struct DevBuf {
         }
         cap = want;
         return AMIRA_OK;
+    }
+    // two buffers trading places: a graph captured before holds the other one's pointer
+    void swap(DevBuf &o) {
+        std::swap(p, o.p);
+        std::swap(cap, o.cap);
+        buffer_generation()++;
     }
     void release() {
         if (p) cudaFree(p);

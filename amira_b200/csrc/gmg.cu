@@ -21,6 +21,36 @@ void set_error(const char *fmt, ...) {
     va_end(ap);
 }
 
+// per node, in node order: the gene-mer (k ids), coverage, first direction, component, and the reads (CSR)
+struct NodeArrays {
+    DevBuf key, cov, dir, comp, reads_off, reads;
+    // n nodes of k genes with n_inc (node, read) incidences between them
+    int reserve(int64_t n, int k, int64_t n_inc) {
+        AMIRA_TRY(key.reserve(sizeof(int32_t) * std::max<int64_t>(1, n * k)));
+        AMIRA_TRY(cov.reserve(sizeof(uint32_t) * (n + 1)));
+        AMIRA_TRY(dir.reserve(n + 1));
+        AMIRA_TRY(comp.reserve(sizeof(uint32_t) * (n + 1)));
+        AMIRA_TRY(reads_off.reserve(sizeof(int64_t) * (n + 2)));
+        return reads.reserve(sizeof(uint32_t) * std::max<int64_t>(1, n_inc));
+    }
+    void swap(NodeArrays &o) {
+        key.swap(o.key); cov.swap(o.cov); dir.swap(o.dir); comp.swap(o.comp); reads_off.swap(o.reads_off); reads.swap(o.reads);
+    }
+};
+
+// per directed edge: source and target node, their directions, coverage
+struct EdgeArrays {
+    DevBuf src, tgt, sd, td, cov;
+    int reserve(int64_t n) {
+        AMIRA_TRY(src.reserve(sizeof(int32_t) * (n + 2)));
+        AMIRA_TRY(tgt.reserve(sizeof(int32_t) * (n + 2)));
+        AMIRA_TRY(sd.reserve(n + 2));
+        AMIRA_TRY(td.reserve(n + 2));
+        return cov.reserve(sizeof(uint32_t) * (n + 2));
+    }
+    void swap(EdgeArrays &o) { src.swap(o.src); tgt.swap(o.tgt); sd.swap(o.sd); td.swap(o.td); cov.swap(o.cov); }
+};
+
 }  // namespace amira
 
 using namespace amira;
@@ -84,13 +114,10 @@ struct amira_gmg {
     int64_t filt_N = -1, filt_E = -1;  // node / edge counts before the last filter (keep flags are retained)
     int64_t prev_G = 0, prev_nodes = 0, prev_und_edges = 0;  // sizes of the previous build on this handle
     int64_t cap_nodes = 0, cap_edges = 0;  // capacities of the node / edge arrays of the current build
-    // nodes (cur) and compaction targets (alt)
-    DevBuf node_key, node_cov, node_dir, node_comp, reads_off, reads;
-    DevBuf node_key2, node_cov2, node_dir2, node_comp2, reads_off2, reads2;
+    // nodes and edges of the graph, and the targets a filter compacts them into (the two sets then trade places)
+    NodeArrays nodes, nodes_alt;
+    EdgeArrays edges, edges_alt;
     DevBuf parent, is_root, cc_min, link, run_id, run_pairs;  // link: node i is joined to node i - 1; run_id: run of linked nodes
-    // edges
-    DevBuf e_src, e_tgt, e_sd, e_td, e_cov;
-    DevBuf e_src2, e_tgt2, e_sd2, e_td2, e_cov2;
     // adjacency: adj_off[2N+1] (forward lists of all nodes, then backward lists), adj_edges[E]
     DevBuf adj_off, adj_edges, adj_cursor, adj_tmp, reads_tmp;
     // scratch
@@ -168,20 +195,19 @@ struct Phase {
     }
 };
 
-#define LAUNCH(h, kern, grid, block, ...)                              \
+// every hand-written kernel is launched through these, on the current stream
+#define LAUNCH_SMEM(h, kern, grid, block, smem, ...)                   \
     do {                                                               \
-        kern<<<(grid), (block), 0, (h)->cur>>>(__VA_ARGS__);           \
+        kern<<<(grid), (block), (smem), (h)->cur>>>(__VA_ARGS__);      \
         (h)->launches++;                                               \
         AMIRA_CUDA(cudaGetLastError());                                \
     } while (0)
+#define LAUNCH(h, kern, grid, block, ...) LAUNCH_SMEM(h, kern, grid, block, 0, __VA_ARGS__)
 
 // launches inside this scope go to the second stream
 struct SideStream {
     amira_gmg *h;
-    explicit SideStream(amira_gmg *h_) : h(h_) {
-        static const bool one_stream = getenv("AMIRA_ONE_STREAM") != nullptr;  // developer experiments: clean per-phase times
-        h->cur = one_stream ? h->stream : h->stream2;
-    }
+    explicit SideStream(amira_gmg *h_) : h(h_) { h->cur = h->stream2; }
     ~SideStream() { h->cur = h->stream; }
 };
 
@@ -207,9 +233,7 @@ int run_scan(amira_gmg *h, L load, S store, const long long *n_ptr, long long n_
         h->lib_launches++;
         state = ws.as<unsigned long long>();
     }
-    k_exscan<<<(unsigned int)(tiles - 1), SCAN_THREADS, 0, h->cur>>>(load, store, n_ptr, n_mul, n_imm, state);
-    h->launches++;
-    AMIRA_CUDA(cudaGetLastError());
+    LAUNCH(h, k_exscan, (unsigned int)(tiles - 1), SCAN_THREADS, load, store, n_ptr, n_mul, n_imm, state);
     return AMIRA_OK;
 }
 
@@ -237,38 +261,50 @@ void reset_graph(amira_gmg *h) {
 int sharded_merge_nodes(amira_gmg *h);
 int sharded_merge_edges(amira_gmg *h);
 
+// ---- segmented sort (segsort.cuh) ----------------------------------------------------------------------
+// radix passes and digit width for keys below max_value: the last pass must land in the destination, so an even
+// number of passes in place and an odd one out of place
+void segsort_passes(SegJob &J, int64_t max_value, bool out_of_place) {
+    const int bits = bits_for64(std::max<int64_t>(max_value, 2));
+    if (out_of_place) J.passes = bits <= 3 * SEG_MAX_DIGIT_BITS ? 3 : 5;
+    else J.passes = bits <= 2 * SEG_MAX_DIGIT_BITS ? 2 : 4;
+    J.digit_bits = std::max(5, (bits + J.passes - 1) / J.passes);
+}
+
+// the work lists of a sort over at most elem_max keys, cleared on the current stream
+int segsort_work(amira_gmg *h, int64_t elem_max, SegWork &work) {
+    DevBuf &wb = h->seg_work[h->cur == h->stream2 ? 1 : 0];
+    const int64_t cap = elem_max / SEG_BITONIC_MAX + 64;
+    AMIRA_TRY(wb.reserve(sizeof(long long) * (size_t)(cap + 2)));  // reserved by reserve_graph; grows otherwise
+    work = SegWork{wb.as<unsigned int>(), wb.as<long long>() + 1, cap};
+    AMIRA_CUDA(cudaMemsetAsync(wb.p, 0, sizeof(long long), h->cur));
+    h->lib_launches++;
+    return AMIRA_OK;
+}
+
+// the segments the first pass left on the work lists: warp-sized ones, then the larger ones, one CTA each (its
+// shared memory holds the digit counters of its warps; kcap 0: what fits shared memory went to k_segsort_warp)
+int segsort_tail(amira_gmg *h, const SegJob &J, const SegWork &work) {
+    LAUNCH(h, k_segsort_warp, (int)std::min<int64_t>((work.cap + 3) / 4, (int64_t)h->n_sm * 4), 128, J, work);
+    const size_t cnt_bytes = sizeof(unsigned int) * SEG_RADIX_WARPS * ((size_t)1 << J.digit_bits);
+    LAUNCH_SMEM(h, k_segsort_radix, (int)std::min<int64_t>(work.cap, (int64_t)h->n_sm * 3), SEG_RADIX_THREADS, cnt_bytes, J, work, 0);
+    return AMIRA_OK;
+}
+
 // segmented sort on the current stream: segment s < *n_seg_ptr * mul has off[s+1] - off[s] keys below `max_value`;
 // in place (a_start == nullptr, out_of_place == false: `a` sorted, `b` is scratch) or from a (segment starts
 // a_start[s], or off[s]) into b
 int run_segsort(amira_gmg *h, uint32_t *a, uint32_t *b, const int64_t *off, const uint32_t *a_start, bool out_of_place,
                 const long long *n_seg_ptr, int mul, int64_t seg_max, int64_t elem_max, int64_t max_value, uint32_t *dups,
                 unsigned long long *total_dups) {
-    DevBuf &wb = h->seg_work[h->cur == h->stream2 ? 1 : 0];
-    const int64_t cap = elem_max / SEG_BITONIC_MAX + 64;
-    AMIRA_TRY(wb.reserve(sizeof(long long) * (size_t)(cap + 2)));  // reserved by reserve_graph; grows otherwise
-    SegWork work{wb.as<unsigned int>(), wb.as<long long>() + 1, cap};
-    AMIRA_CUDA(cudaMemsetAsync(wb.p, 0, sizeof(long long), h->cur));
-    h->lib_launches++;
-    const int bits = bits_for64(std::max<int64_t>(max_value, 2));
+    SegWork work;
+    AMIRA_TRY(segsort_work(h, elem_max, work));
     SegJob J;
     J.a = a; J.b = b; J.off = off; J.a_start = a_start; J.n_seg_ptr = n_seg_ptr; J.seg_mul = mul;
     J.dups = dups; J.total_dups = total_dups;
-    // the last pass must land in the destination: an even number of passes in place, an odd one out of place
-    if (out_of_place) J.passes = bits <= 3 * 8 ? 3 : (bits <= 3 * SEG_MAX_DIGIT_BITS ? 3 : 5);
-    else J.passes = bits <= 2 * SEG_MAX_DIGIT_BITS ? 2 : 4;
-    J.digit_bits = std::max(5, (bits + J.passes - 1) / J.passes);
-    const int grid_main = (int)std::min<int64_t>(grid_for(seg_max, 256), (int64_t)h->n_sm * 8);
-    LAUNCH(h, k_segsort_main, grid_main, 256, J, work);
-    LAUNCH(h, k_segsort_warp, (int)std::min<int64_t>((cap + 3) / 4, (int64_t)h->n_sm * 4), 128, J, work);
-    // shared memory: the digit counters of 8 warps + two key buffers (8192 keys each when they fit ~72 KB)
-    const size_t cnt_bytes = sizeof(unsigned int) * SEG_RADIX_WARPS * ((size_t)1 << J.digit_bits);
-    const int kcap = 0;  // everything that fits shared memory is sorted by k_segsort_warp
-    const size_t smem = cnt_bytes + 2 * sizeof(uint32_t) * (size_t)kcap;
-    const int grid_rad = (int)std::min<int64_t>(cap, (int64_t)h->n_sm * 3);
-    k_segsort_radix<<<grid_rad, SEG_RADIX_THREADS, smem, h->cur>>>(J, work, kcap);
-    h->launches++;
-    AMIRA_CUDA(cudaGetLastError());
-    return AMIRA_OK;
+    segsort_passes(J, max_value, out_of_place);
+    LAUNCH(h, k_segsort_main, (int)std::min<int64_t>(grid_for(seg_max, 256), (int64_t)h->n_sm * 8), 256, J, work);
+    return segsort_tail(h, J, work);
 }
 
 // node -> forward/backward edge CSR from the current edge arrays (degrees already counted in adj_off
@@ -279,12 +315,12 @@ int build_adjacency(amira_gmg *h, bool counted) {
     unsigned long long *deg = h->adj_off.as<unsigned long long>();
     if (!counted) {
         LAUNCH(h, k_fill_u64, h->n_sm * 4, 256, deg, N, 2, 2, 0ull);
-        LAUNCH(h, k_adj_count, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 32), 256, h->e_src.as<int32_t>(), h->e_sd.as<int8_t>(), E, N, deg);
+        LAUNCH(h, k_adj_count, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 32), 256, h->edges.src.as<int32_t>(), h->edges.sd.as<int8_t>(), E, N, deg);
     }
     // number of segments = 2N, on the device: the scan runs over 2N + 1 items
     AMIRA_TRY(run_scan(h, DegLoad{deg}, DegStore{h->adj_off.as<int64_t>(), h->adj_cursor.as<unsigned long long>(), N, dsz(h, 0)},
                        dsz(h, SZ_NODES), 2, 0, 2 * h->cap_nodes + 1));
-    LAUNCH(h, k_adj_scatter, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 32), 256, h->e_src.as<int32_t>(), h->e_sd.as<int8_t>(), E, N,
+    LAUNCH(h, k_adj_scatter, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 32), 256, h->edges.src.as<int32_t>(), h->edges.sd.as<int8_t>(), E, N,
            h->adj_cursor.as<unsigned long long>(), h->adj_edges.as<uint32_t>());
     AMIRA_TRY(run_segsort(h, h->adj_edges.as<uint32_t>(), h->adj_tmp.as<uint32_t>(), h->adj_off.as<int64_t>(), nullptr, false,
                           dsz(h, SZ_NODES), 2, 2 * h->cap_nodes, h->cap_edges, h->cap_edges + 1, nullptr, nullptr));
@@ -324,9 +360,7 @@ int plan_build(amira_gmg *h) {
     const bool n16 = T <= KEY16_BITS && h->id_bits > 0 && h->id_bits < 32 && !(h->force_layout & 1);
     h->key_bits = (T <= 124 && h->id_bits > 0 && h->id_bits < 32 && !(h->force_layout & 4)) ? h->id_bits : 0;
     const bool e16 = G < (1ll << ORD32_P_BITS) && !(h->force_layout & 2);
-    double nslack = n16 ? 2.4 : 2.0, eslack = 2.0;
-    if (const char *e = getenv("AMIRA_NODE_SLACK")) nslack = atof(e);  // developer experiments
-    if (const char *e = getenv("AMIRA_EDGE_SLACK")) eslack = atof(e);
+    const double nslack = n16 ? 2.4 : 2.0, eslack = 2.0;
     if (h->hint_nodes > 0) ncap = h->hint_nodes * 2 + 1024;
     else if (h->prev_G > 0 && G <= 4 * h->prev_G)
         ncap = (int64_t)((double)h->prev_nodes * ((double)G / (double)h->prev_G) * nslack) + 4096;
@@ -380,24 +414,15 @@ int reserve_graph(amira_gmg *h, int64_t capN, int64_t capE) {
     const int k = h->k;
     h->cap_nodes = capN;
     h->cap_edges = capE;
-    AMIRA_TRY(h->node_key.reserve(sizeof(int32_t) * std::max<int64_t>(1, capN * k)));
-    AMIRA_TRY(h->node_cov.reserve(sizeof(uint32_t) * (capN + 1)));
-    AMIRA_TRY(h->node_dir.reserve(capN + 1));
-    AMIRA_TRY(h->node_comp.reserve(sizeof(uint32_t) * (capN + 1)));
+    AMIRA_TRY(h->nodes.reserve(capN, k, G));
+    AMIRA_TRY(h->edges.reserve(capE));
     AMIRA_TRY(h->parent.reserve(sizeof(int32_t) * (capN + 1)));
     AMIRA_TRY(h->link.reserve(capN + 2));
     if (h->prev_nodes > 0 && h->prev_nodes <= UF_SMALL_RUNS) AMIRA_TRY(h->run_pairs.reserve(sizeof(unsigned long long) * (size_t)(capE / 2 + 4)));
     AMIRA_TRY(h->run_id.reserve(sizeof(int32_t) * (capN + 2)));
     AMIRA_TRY(h->is_root.reserve(sizeof(int) * (capN + 2)));
     AMIRA_TRY(h->cc_min.reserve(sizeof(unsigned int) * (capN + 1)));
-    AMIRA_TRY(h->reads_off.reserve(sizeof(int64_t) * (capN + 2)));
     AMIRA_TRY(h->dups.reserve(sizeof(uint32_t) * (capN + 1)));
-    AMIRA_TRY(h->reads.reserve(sizeof(uint32_t) * G));
-    AMIRA_TRY(h->e_src.reserve(sizeof(int32_t) * (capE + 2)));
-    AMIRA_TRY(h->e_tgt.reserve(sizeof(int32_t) * (capE + 2)));
-    AMIRA_TRY(h->e_sd.reserve(capE + 2));
-    AMIRA_TRY(h->e_td.reserve(capE + 2));
-    AMIRA_TRY(h->e_cov.reserve(sizeof(uint32_t) * (capE + 2)));
     AMIRA_TRY(h->adj_off.reserve(sizeof(int64_t) * (2 * capN + 3)));
     AMIRA_TRY(h->adj_cursor.reserve(sizeof(unsigned long long) * (2 * capN + 3)));
     AMIRA_TRY(h->adj_edges.reserve(sizeof(uint32_t) * (capE + 1)));
@@ -554,8 +579,8 @@ int enqueue_order(amira_gmg *h) {
         LAUNCH(h, k_rank_nodes, std::min<int>(grid_for(h->ncap, 256), h->n_sm * 16), 256, h->nview, bm_node, h->cnt_node.as<int>(),
                h->is_root.as<uint32_t>());
         LAUNCH(h, k_emit_nodes, (int)std::min<int64_t>(grid_for(h->cap_nodes, 256), (int64_t)h->n_sm * 16), 256, h->nview, h->ids, h->k,
-               dcnt(h, SZ_NODES), h->is_root.as<uint32_t>(), h->node_key.as<int32_t>(), h->node_cov.as<uint32_t>(),
-               h->node_dir.as<int8_t>(), h->link.as<uint8_t>(),
+               dcnt(h, SZ_NODES), h->is_root.as<uint32_t>(), h->nodes.key.as<int32_t>(), h->nodes.cov.as<uint32_t>(),
+               h->nodes.dir.as<int8_t>(), h->link.as<uint8_t>(),
                (h->n16 && h->key_bits > 0) ? h->ntab.as<NodeSlot16>() : (const NodeSlot16 *)nullptr, h->key_bits);
     }
     return AMIRA_OK;
@@ -581,8 +606,8 @@ int enqueue_tail_side(amira_gmg *h) {
             LAUNCH(h, k_rank_edges, std::min<int>(grid_for(h->ecap, 256), h->n_sm * 16), 256, h->eview, bm_ea, bm_eb,
                    h->cnt_edge.as<int>(), h->adj_tmp.as<uint32_t>(), h->d_status.as<int>());
             LAUNCH(h, k_emit_edges, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 16), 256, h->eview, h->nview,
-                   h->adj_tmp.as<uint32_t>(), E, N, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(), h->e_sd.as<int8_t>(),
-                   h->e_td.as<int8_t>(), h->e_cov.as<uint32_t>(), deg, h->link.as<uint8_t>());
+                   h->adj_tmp.as<uint32_t>(), E, N, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(), h->edges.sd.as<int8_t>(),
+                   h->edges.td.as<int8_t>(), h->edges.cov.as<uint32_t>(), deg, h->link.as<uint8_t>());
             counted = true;
             // runs of consecutive first-seen nodes joined by an edge (a prefix count, no pointer chasing), then
             // union-find over the runs with the edges that leave a run, in first-seen edge order
@@ -599,106 +624,86 @@ int enqueue_tail_side(amira_gmg *h) {
                 unsigned long long *pairs = h->run_pairs.as<unsigned long long>();
                 AMIRA_CUDA(cudaMemsetAsync(pairs, 0, 2 * sizeof(unsigned long long), h->cur));
                 h->lib_launches++;
-                LAUNCH(h, k_collect_run_edges, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 16), 256, h->e_src.as<int32_t>(),
-                       h->e_tgt.as<int32_t>(), E, N, run_ids, pairs + 2, pairs);
-                k_union_small<<<1, UF_SMALL_THREADS, sizeof(int32_t) * UF_SMALL_RUNS, h->cur>>>(pairs + 2, pairs, N, run_ids, h->parent.as<int32_t>(), pairs + 1);
-                h->launches++;
-                AMIRA_CUDA(cudaGetLastError());
+                LAUNCH(h, k_collect_run_edges, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 16), 256, h->edges.src.as<int32_t>(),
+                       h->edges.tgt.as<int32_t>(), E, N, run_ids, pairs + 2, pairs);
+                LAUNCH_SMEM(h, k_union_small, 1, UF_SMALL_THREADS, sizeof(int32_t) * UF_SMALL_RUNS, pairs + 2, pairs, N, run_ids,
+                            h->parent.as<int32_t>(), pairs + 1);
                 done = pairs + 1;
             }
-            LAUNCH(h, k_union_edges, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 64), 256, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(), E, h->parent.as<int32_t>(), run_ids, done);
+            LAUNCH(h, k_union_edges, (int)std::min<int64_t>(grid_for(h->cap_edges, 256), (int64_t)h->n_sm * 64), 256, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(), E, h->parent.as<int32_t>(), run_ids, done);
         } else if (h->sh_Eg > 0) {
             Phase ph(h, AMIRA_PH_EMIT);
             LAUNCH(h, k_emit_edges_sorted, grid_for(h->sh_Eg, 256), 256, h->x_sorti2.as<unsigned int>(), h->sh_gedge,
-                   h->x_fan.as<int>(), (long long)h->sh_Eg, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(),
-                   h->e_sd.as<int8_t>(), h->e_td.as<int8_t>(), h->e_cov.as<uint32_t>(), h->link.as<uint8_t>());
+                   h->x_fan.as<int>(), (long long)h->sh_Eg, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(),
+                   h->edges.sd.as<int8_t>(), h->edges.td.as<int8_t>(), h->edges.cov.as<uint32_t>(), h->link.as<uint8_t>());
         }
         if (h->world > 1) {
             run_ids = h->run_id.as<int32_t>();
             AMIRA_TRY(run_scan(h, RunLoad{h->link.as<uint8_t>()}, RunStore{h->run_id.as<int32_t>(), h->parent.as<int32_t>(), N},
                                dsz(h, SZ_NODES), 1, 0, h->cap_nodes));
-            LAUNCH(h, k_union_edges, (int)std::min<int64_t>(grid_for(std::max<int64_t>(h->cap_edges, 1), 256), (int64_t)h->n_sm * 64), 256, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(), E, h->parent.as<int32_t>(), run_ids, nullptr);
+            LAUNCH(h, k_union_edges, (int)std::min<int64_t>(grid_for(std::max<int64_t>(h->cap_edges, 1), 256), (int64_t)h->n_sm * 64), 256, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(), E, h->parent.as<int32_t>(), run_ids, nullptr);
         }
         AMIRA_TRY(build_adjacency(h, counted));
         {
             Phase ph(h, AMIRA_PH_COMPONENTS);
             LAUNCH(h, k_fill_u32, h->n_sm * 4, 256, h->cc_min.as<uint32_t>(), N, 1, 1, 0xFFFFFFFFu);
             LAUNCH(h, k_cc_flatten, (int)std::min<int64_t>(grid_for(h->cap_nodes, 256), (int64_t)h->n_sm * 64), 256, h->parent.as<int32_t>(), N, h->cc_min.as<unsigned int>(),
-                   h->node_comp.as<uint32_t>(), run_ids);
-            AMIRA_TRY(run_scan(h, FirstLoad{h->node_comp.as<uint32_t>(), h->cc_min.as<unsigned int>()},
+                   h->nodes.comp.as<uint32_t>(), run_ids);
+            AMIRA_TRY(run_scan(h, FirstLoad{h->nodes.comp.as<uint32_t>(), h->cc_min.as<unsigned int>()},
                                FirstStore{h->is_root.as<int>(), N, dsz(h, 0)}, dsz(h, SZ_NODES), 1, 0, h->cap_nodes));
             LAUNCH(h, k_cc_number, (int)std::min<int64_t>(grid_for(h->cap_nodes, 256), (int64_t)h->n_sm * 64), 256, h->cc_min.as<unsigned int>(), h->is_root.as<int>(), N,
-                   h->node_comp.as<uint32_t>());
+                   h->nodes.comp.as<uint32_t>());
         }
         AMIRA_CUDA(cudaEventRecord(h->ev_join, h->cur));
     }
     return AMIRA_OK;
 }
 
+// node -> reads records dealt into buckets (incidence.cuh), in the shape P
+template <class P>
+int launch_partition(amira_gmg *h, unsigned int *bcur) {
+    const int grid = (int)std::min<int64_t>(std::max<int64_t>(1, (h->G + P::TILE - 1) / P::TILE), (int64_t)h->n_sm * P::CTAS);
+    LAUNCH_SMEM(h, k_partition<P>, grid, P::THREADS, P::SMEM, h->slot_info.as<uint2>(), h->win_slot.as<int32_t>(), h->win_read.as<int32_t>(),
+                h->win_node.as<int32_t>(), (const long long *)h->d_sizes.p, bcur + INC_NB_BIG, h->unit_plan, bcur, h->inc_rec.as<uint2>());
+    return AMIRA_OK;
+}
+
 // branch A, on the main stream
 int enqueue_tail_main(amira_gmg *h) {
-    const int64_t G = h->G;
-    cudaStream_t st = h->stream;
     const Cnt N = dcnt(h, SZ_NODES);
     {
         // node -> reads (incidence.cuh): coverage per node (counted by the insert kernel) -> offsets, units,
         // records dealt into buckets (the same pass writes the per-read node lists), one CTA per unit
-        const uint32_t *cov = h->world > 1 ? h->cov_local.as<uint32_t>() : h->node_cov.as<uint32_t>();
+        const uint32_t *cov = h->world > 1 ? h->cov_local.as<uint32_t>() : h->nodes.cov.as<uint32_t>();
         const UnitPlan &u = h->unit_plan;
         {
             Phase ph(h, AMIRA_PH_REMAP);
-            AMIRA_TRY(run_scan(h, CovLoad{cov}, CovStore{h->reads_off.as<int64_t>(), N, dsz(h, 0)}, dsz(h, SZ_NODES), 1, 0,
+            AMIRA_TRY(run_scan(h, CovLoad{cov}, CovStore{h->nodes.reads_off.as<int64_t>(), N, dsz(h, 0)}, dsz(h, SZ_NODES), 1, 0,
                                h->cap_nodes));
             LAUNCH(h, k_unit_table, (int)std::min<int64_t>(grid_for(std::max<int64_t>(h->ncap, h->cap_nodes + 1), 256), (int64_t)h->n_sm * 16), 256,
-                   h->nview, h->reads_off.as<int64_t>(), dsz(h, SZ_NODES), u, h->unit_lo.as<int>(), h->d_status.as<int>());
+                   h->nview, h->nodes.reads_off.as<int64_t>(), dsz(h, SZ_NODES), u, h->unit_lo.as<int>(), h->d_status.as<int>());
             unsigned int *bcur = h->bucket_cursor.as<unsigned int>();
-            LAUNCH(h, k_bucket_base, u.nb_max / 256, 256, h->unit_lo.as<int>(), h->reads_off.as<int64_t>(), u, bcur + INC_NB_BIG, bcur);
+            LAUNCH(h, k_bucket_base, u.nb_max / 256, 256, h->unit_lo.as<int>(), h->nodes.reads_off.as<int64_t>(), u, bcur + INC_NB_BIG, bcur);
             // low coverage (by the previous build on this handle): large tiles, see incidence.cuh
             const bool wide = h->prev_nodes > 0 && h->prev_G < (int64_t)PART_WIDE_BELOW * h->prev_nodes;
-            if (u.nb_max == INC_NB_MAX && !wide) {
-                const int pgrid = (int)std::min<int64_t>(std::max<int64_t>(1, (G + PartSmall::TILE - 1) / PartSmall::TILE), (int64_t)h->n_sm * PartSmall::CTAS);
-                k_partition<PartSmall><<<pgrid, PartSmall::THREADS, PartSmall::SMEM, st>>>(
-                    h->slot_info.as<uint2>(), h->win_slot.as<int32_t>(), h->win_read.as<int32_t>(), h->win_node.as<int32_t>(),
-                    (const long long *)h->d_sizes.p, bcur + INC_NB_BIG, u, bcur, h->inc_rec.as<uint2>());
-            } else if (u.nb_max == INC_NB_MAX) {
-                const int pgrid = (int)std::min<int64_t>(std::max<int64_t>(1, (G + PartWide::TILE - 1) / PartWide::TILE), (int64_t)h->n_sm * PartWide::CTAS);
-                k_partition<PartWide><<<pgrid, PartWide::THREADS, PartWide::SMEM, st>>>(
-                    h->slot_info.as<uint2>(), h->win_slot.as<int32_t>(), h->win_read.as<int32_t>(), h->win_node.as<int32_t>(),
-                    (const long long *)h->d_sizes.p, bcur + INC_NB_BIG, u, bcur, h->inc_rec.as<uint2>());
-            } else {
-                const int pgrid = (int)std::min<int64_t>(std::max<int64_t>(1, (G + PartBig::TILE - 1) / PartBig::TILE), (int64_t)h->n_sm * PartBig::CTAS);
-                k_partition<PartBig><<<pgrid, PartBig::THREADS, PartBig::SMEM, st>>>(
-                    h->slot_info.as<uint2>(), h->win_slot.as<int32_t>(), h->win_read.as<int32_t>(), h->win_node.as<int32_t>(),
-                    (const long long *)h->d_sizes.p, bcur + INC_NB_BIG, u, bcur, h->inc_rec.as<uint2>());
-            }
-            h->launches++;
-            AMIRA_CUDA(cudaGetLastError());
+            if (u.nb_max != INC_NB_MAX) AMIRA_TRY(launch_partition<PartBig>(h, bcur));
+            else if (wide) AMIRA_TRY(launch_partition<PartWide>(h, bcur));
+            else AMIRA_TRY(launch_partition<PartSmall>(h, bcur));
         }
-        if (!h->capturing) AMIRA_CUDA(cudaEventRecord(h->ev_reads_ready, st));
+        if (!h->capturing) AMIRA_CUDA(cudaEventRecord(h->ev_reads_ready, h->stream));
         Phase ph(h, AMIRA_PH_INCIDENCE);
         // in-place job over `reads` for the units that outgrow shared memory (and the lists they leave to the
         // work-list kernels of segsort.cuh)
-        DevBuf &wb = h->seg_work[0];
-        const int64_t wcap = std::max<int64_t>(G, 1) / SEG_BITONIC_MAX + 64;
-        SegWork work{wb.as<unsigned int>(), wb.as<long long>() + 1, wcap};
-        AMIRA_CUDA(cudaMemsetAsync(wb.p, 0, sizeof(long long), st));
-        h->lib_launches++;
-        const int64_t reads_global = h->world > 1 ? 0x7FFFFFF0ll : h->R;
-        const int bits = bits_for64(std::max<int64_t>(reads_global + 1, 2));
+        SegWork work;
+        AMIRA_TRY(segsort_work(h, std::max<int64_t>(h->G, 1), work));
         SegJob J;
-        J.a = h->reads.as<uint32_t>(); J.b = h->reads_tmp.as<uint32_t>(); J.off = h->reads_off.as<int64_t>(); J.a_start = nullptr;
+        J.a = h->nodes.reads.as<uint32_t>(); J.b = h->reads_tmp.as<uint32_t>(); J.off = h->nodes.reads_off.as<int64_t>(); J.a_start = nullptr;
         J.n_seg_ptr = dsz(h, SZ_NODES); J.seg_mul = 1;
         J.dups = h->dups.as<uint32_t>(); J.total_dups = (unsigned long long *)dsz(h, SZ_DUPS);
-        J.passes = bits <= 2 * SEG_MAX_DIGIT_BITS ? 2 : 4;
-        J.digit_bits = std::max(5, (bits + J.passes - 1) / J.passes);
-        k_unit_lists<<<u.n_units, INC_THREADS, INC_SMEM, st>>>(h->inc_rec.as<uint2>(), h->unit_lo.as<int>(), u, J, work);
-        h->launches++;
-        AMIRA_CUDA(cudaGetLastError());
-        LAUNCH(h, k_segsort_warp, (int)std::min<int64_t>((wcap + 3) / 4, (int64_t)h->n_sm * 4), 128, J, work);
-        const size_t cnt_bytes = sizeof(unsigned int) * SEG_RADIX_WARPS * ((size_t)1 << J.digit_bits);
-        k_segsort_radix<<<(int)std::min<int64_t>(wcap, (int64_t)h->n_sm * 3), SEG_RADIX_THREADS, cnt_bytes, st>>>(J, work, 0);
-        h->launches++;
-        AMIRA_CUDA(cudaGetLastError());
+        const int64_t reads_global = h->world > 1 ? 0x7FFFFFF0ll : h->R;
+        segsort_passes(J, reads_global + 1, false);
+        LAUNCH_SMEM(h, k_unit_lists, u.n_units, INC_THREADS, INC_SMEM, h->inc_rec.as<uint2>(), h->unit_lo.as<int>(), u, J, work);
+        AMIRA_TRY(segsort_tail(h, J, work));
     }
     return AMIRA_OK;
 }
@@ -730,6 +735,38 @@ __global__ void k_set_sizes(long long *sizes, long long n_nodes, long long n_edg
     }
 }
 
+// an error the device reported in ST_ERR
+int device_error(int e) {
+    set_error("%s", e == AMIRA_E_PALINDROME ? "Gene-mer and reverse complement gene-mer are identical" : "invalid read offsets");
+    return e;
+}
+
+// What the status block of a build (one GPU: the whole build; multi-GPU: the local tables) asks for: AMIRA_OK, the
+// build stands; BUILD_REDO, enqueue it again with grown tables or a re-measured key width (at most 6 times per
+// amira_gmg_build); else an error, with its message set.
+constexpr int BUILD_REDO = -1;
+int build_verdict(amira_gmg *h, const int *s) {
+    if (s[ST_ERR]) {
+        h->grow_n = h->grow_e = 1;
+        return device_error(s[ST_ERR]);
+    }
+    const bool unpack = s[ST_UNPACK] && h->key_bits > 0;
+    if (s[ST_OVERFLOW_N] || s[ST_OVERFLOW_E] || unpack) {
+        if (++h->attempts > 6) {
+            set_error("hash tables overflowed after %d attempts (ncap=%u ecap=%u)", h->attempts, h->ncap, h->ecap);
+            return AMIRA_E_NOMEM;
+        }
+        if (unpack) h->id_bits = 0;  // an id outgrew the remembered width: measure again
+        if (s[ST_OVERFLOW_N]) h->grow_n *= 4;
+        if (s[ST_OVERFLOW_E]) h->grow_e *= 4;
+        return BUILD_REDO;
+    }
+    h->grow_n = h->grow_e = 1;
+    // the key width follows the data in both directions
+    if (h->id_bits != 0 && (unsigned int)s[ST_MAXABS] > 0) h->id_bits = bits_for_ids((unsigned int)s[ST_MAXABS]);
+    return AMIRA_OK;
+}
+
 int do_build(amira_gmg *h) {
     cudaStream_t st = h->stream;
     if (h->world == 1) {
@@ -737,8 +774,7 @@ int do_build(amira_gmg *h) {
         AMIRA_TRY(reserve_graph(h, h->ncap, 2 * (int64_t)h->ecap));
         const amira_gmg::GraphKey key{h->ids, h->off, h->ps, h->pe, h->R, h->G, h->cap_nodes, h->cap_edges, h->ncap, h->ecap,
                                       h->k, h->key_bits, (h->n16 ? 1 : 0) | (h->e16 ? 2 : 0), buffer_generation().load()};
-        static const bool no_graph = getenv("AMIRA_NO_GRAPH") != nullptr;
-        const bool can_graph = h->input_on_device && !h->profiling && h->n_pieces == 0 && h->G <= (64ll << 20) && !no_graph;
+        const bool can_graph = h->input_on_device && !h->profiling && h->n_pieces == 0 && h->G <= (64ll << 20);
         auto after_launch = [&]() -> int {
             AMIRA_CUDA(cudaEventRecord(h->ev_reads_ready, st));
             AMIRA_CUDA(cudaEventRecord(h->ev_early, st));
@@ -785,36 +821,23 @@ int do_build(amira_gmg *h) {
         AMIRA_TRY(enqueue_order(h));
         return enqueue_tail(h);
     }
-    // multi-GPU: the exchange needs host-side counts, so the local tables are finished synchronously
-    for (int attempt = 0;; ++attempt) {
+    // multi-GPU: the exchange needs host-side counts, so the local tables are finished synchronously.  (ST_STALE is
+    // not looked at here: re-reading the call count after the ranks have exchanged their global offsets would
+    // desynchronise them, so a stale cached count goes unnoticed on this path.)
+    int rc;
+    do {
         AMIRA_TRY(plan_build(h));
         AMIRA_TRY(enqueue_insert(h));
         AMIRA_TRY(enqueue_report(h, 0));
         AMIRA_CUDA(cudaStreamSynchronize(st));
-        const int *s = h->h_status;
-        if (s[ST_ERR]) break;
-        const bool unpack = s[ST_UNPACK] && h->key_bits > 0;
-        if (unpack) h->id_bits = 0;
-        if (!s[ST_OVERFLOW_N] && !s[ST_OVERFLOW_E] && !unpack) break;
-        if (attempt >= 6) {
-            set_error("hash tables overflowed after %d attempts (ncap=%u ecap=%u)", attempt + 1, h->ncap, h->ecap);
-            return AMIRA_E_NOMEM;
-        }
-        if (s[ST_OVERFLOW_N]) h->grow_n *= 4;
-        if (s[ST_OVERFLOW_E]) h->grow_e *= 4;
-    }
-    h->grow_n = h->grow_e = 1;
-    if ((unsigned int)h->h_status[ST_MAXABS] > 0 && h->id_bits != 0) h->id_bits = bits_for_ids((unsigned int)h->h_status[ST_MAXABS]);
+        rc = build_verdict(h, h->h_status);
+    } while (rc == BUILD_REDO);
+    if (rc == AMIRA_E_NOMEM) return rc;  // out of attempts (an error the device found is agreed on first)
     // every rank must leave the build together: agree on the error status before any exchange
     AMIRA_TRY(comm_allreduce_max_i32(h->comm, h->d_status.as<int>(), 4, st));
     AMIRA_CUDA(cudaMemcpyAsync(h->h_status, h->d_status.p, sizeof(int) * ST_COUNT, cudaMemcpyDeviceToHost, st));
     AMIRA_CUDA(cudaStreamSynchronize(st));
-    if (h->h_status[ST_ERR]) {
-        const int e = h->h_status[ST_ERR];
-        if (e == AMIRA_E_PALINDROME) set_error("Gene-mer and reverse complement gene-mer are identical");
-        else set_error("invalid read offsets");
-        return e;
-    }
+    if (h->h_status[ST_ERR]) return device_error(h->h_status[ST_ERR]);
     h->W = h->h_sizes[SZ_W];
     h->n_short = h->h_sizes[SZ_SHORT];
     h->prev_G = h->G;
@@ -838,17 +861,17 @@ int do_build(amira_gmg *h) {
 int finalize_incidence(amira_gmg *h) {
     const int64_t N = h->n_nodes;
     const Cnt cn{nullptr, N};
-    AMIRA_TRY(h->reads_off2.reserve(sizeof(int64_t) * (N + 2)));
-    AMIRA_TRY(h->reads2.reserve(sizeof(uint32_t) * std::max<int64_t>(1, h->n_inc)));
-    AMIRA_TRY(run_scan(h, UniqLoad{h->reads_off.as<int64_t>(), h->dups.as<uint32_t>()},
-                       OffStore{h->reads_off2.as<int64_t>(), cn, dsz(h, SZ_INC)}, nullptr, 1, N, N));
+    AMIRA_TRY(h->nodes_alt.reads_off.reserve(sizeof(int64_t) * (N + 2)));
+    AMIRA_TRY(h->nodes_alt.reads.reserve(sizeof(uint32_t) * std::max<int64_t>(1, h->n_inc)));
+    AMIRA_TRY(run_scan(h, UniqLoad{h->nodes.reads_off.as<int64_t>(), h->dups.as<uint32_t>()},
+                       OffStore{h->nodes_alt.reads_off.as<int64_t>(), cn, dsz(h, SZ_INC)}, nullptr, 1, N, N));
     LAUNCH(h, k_compact_unique, (int)std::min<int64_t>(grid_for(N * 32, 256), (int64_t)h->n_sm * 8), 256,
-           h->reads_off.as<int64_t>(), h->reads.as<uint32_t>(), h->reads_off2.as<int64_t>(), h->reads2.as<uint32_t>(), cn);
+           h->nodes.reads_off.as<int64_t>(), h->nodes.reads.as<uint32_t>(), h->nodes_alt.reads_off.as<int64_t>(), h->nodes_alt.reads.as<uint32_t>(), cn);
     long long n_inc = 0;
     AMIRA_CUDA(cudaMemcpyAsync(&n_inc, dsz(h, SZ_INC), sizeof(long long), cudaMemcpyDeviceToHost, h->stream));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
-    std::swap(h->reads_off, h->reads_off2);
-    std::swap(h->reads, h->reads2);
+    h->nodes.reads_off.swap(h->nodes_alt.reads_off);
+    h->nodes.reads.swap(h->nodes_alt.reads);
     h->n_inc = n_inc;
     return AMIRA_OK;
 }
@@ -863,9 +886,10 @@ int finish(amira_gmg *h, bool early) {
         const int *s = h->h_status + which * ST_COUNT;
         const long long *z = h->h_sizes + which * SZ_COUNT;
         if (h->pending_is_build && h->world == 1) {
-            // problems the device found: redo the build (synchronously from here on)
-            const bool unpack = s[ST_UNPACK] && h->key_bits > 0;
-            if (s[ST_ERR] || s[ST_STALE] || s[ST_OVERFLOW_N] || s[ST_OVERFLOW_E] || unpack) {
+            // problems the device found: redo the build (synchronously from here on).  A stale call count comes
+            // first: the other flags of a build over the wrong count mean nothing.
+            int rc = s[ST_STALE] ? BUILD_REDO : build_verdict(h, s);
+            if (rc != AMIRA_OK) {
                 AMIRA_CUDA(cudaEventSynchronize(h->ev_done));
                 h->pending = 0;
                 if (s[ST_STALE]) {
@@ -874,28 +898,12 @@ int finish(amira_gmg *h, bool early) {
                     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
                     if (G < 0 || G >= MAX_CALLS) {
                         set_error("bad call count %lld", (long long)G);
-                        h->built = false;
-                        return h->last_status = AMIRA_E_ARG;
+                        rc = AMIRA_E_ARG;
+                    } else {
+                        h->G = h->cache_G = G;
                     }
-                    h->G = h->cache_G = G;
-                } else if (s[ST_ERR]) {
-                    const int e = s[ST_ERR];
-                    if (e == AMIRA_E_PALINDROME) set_error("Gene-mer and reverse complement gene-mer are identical");
-                    else set_error("invalid read offsets");
-                    h->built = false;
-                    h->grow_n = h->grow_e = 1;
-                    return h->last_status = e;
-                } else {
-                    if (++h->attempts > 6) {
-                        set_error("hash tables overflowed after %d attempts (ncap=%u ecap=%u)", h->attempts, h->ncap, h->ecap);
-                        h->built = false;
-                        return h->last_status = AMIRA_E_NOMEM;
-                    }
-                    if (unpack) h->id_bits = 0;  // an id outgrew the remembered width: measure again
-                    if (s[ST_OVERFLOW_N]) h->grow_n *= 4;
-                    if (s[ST_OVERFLOW_E]) h->grow_e *= 4;
                 }
-                const int rc = do_build(h);
+                if (rc == BUILD_REDO) rc = do_build(h);
                 if (rc != AMIRA_OK) {
                     h->built = false;
                     return h->last_status = rc;
@@ -922,10 +930,6 @@ int finish(amira_gmg *h, bool early) {
                 h->prev_G = h->G;
                 h->prev_nodes = h->n_nodes;
                 h->prev_und_edges = (h->n_edges + 1) / 2 + 1;  // directed edges come in pairs, self-edges alone
-                h->grow_n = h->grow_e = 1;
-                h->attempts = 0;
-                // the key width follows the data in both directions
-                if (h->id_bits != 0 && (unsigned int)s[ST_MAXABS] > 0) h->id_bits = bits_for_ids((unsigned int)s[ST_MAXABS]);
             }
             if (z[SZ_DUPS] > 0) AMIRA_TRY(finalize_incidence(h));
         }
@@ -942,20 +946,10 @@ int filter_reserve(amira_gmg *h) {
     AMIRA_TRY(finish(h, false));
     if (!h->built) return h->last_status;
     const int64_t N = h->n_nodes, E = h->n_edges;
-    const int k = h->k;
     AMIRA_TRY(h->keep_n.reserve(sizeof(int) * 2 * (N + 2)));
     AMIRA_TRY(h->keep_e.reserve(sizeof(int) * 2 * (E + 2)));
-    AMIRA_TRY(h->node_key2.reserve(sizeof(int32_t) * std::max<int64_t>(1, N * k)));
-    AMIRA_TRY(h->node_cov2.reserve(sizeof(uint32_t) * (N + 1)));
-    AMIRA_TRY(h->node_dir2.reserve(N + 1));
-    AMIRA_TRY(h->node_comp2.reserve(sizeof(uint32_t) * (N + 1)));
-    AMIRA_TRY(h->reads_off2.reserve(sizeof(int64_t) * (N + 2)));
-    AMIRA_TRY(h->reads2.reserve(sizeof(uint32_t) * std::max<int64_t>(1, h->n_inc)));
-    AMIRA_TRY(h->e_src2.reserve(sizeof(int32_t) * (E + 2)));
-    AMIRA_TRY(h->e_tgt2.reserve(sizeof(int32_t) * (E + 2)));
-    AMIRA_TRY(h->e_sd2.reserve(E + 2));
-    AMIRA_TRY(h->e_td2.reserve(E + 2));
-    AMIRA_TRY(h->e_cov2.reserve(sizeof(uint32_t) * (E + 2)));
+    AMIRA_TRY(h->nodes_alt.reserve(N, h->k, h->n_inc));
+    AMIRA_TRY(h->edges_alt.reserve(E));
     AMIRA_TRY(h->comp_max.reserve(sizeof(uint32_t) * (h->n_comps + 2)));
     // the graph only shrinks: the capacities of the build (or of the previous filter) still hold
     h->cap_nodes = std::max<int64_t>(h->cap_nodes, N);
@@ -978,15 +972,15 @@ int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
     int *keep_e = h->keep_e.as<int>(), *new_e = keep_e + (E + 2);
     if (mode == 1) {
         AMIRA_CUDA(cudaMemsetAsync(h->comp_max.p, 0, sizeof(uint32_t) * (h->n_comps + 2), st));
-        LAUNCH(h, k_component_max, grid_for(N, 256), 256, h->node_cov.as<uint32_t>(), h->node_comp.as<uint32_t>(), N,
+        LAUNCH(h, k_component_max, grid_for(N, 256), 256, h->nodes.cov.as<uint32_t>(), h->nodes.comp.as<uint32_t>(), N,
                h->comp_max.as<uint32_t>());
     }
     if (mode != 2)
-        LAUNCH(h, k_node_keep, grid_for(N + 1, 256), 256, h->node_cov.as<uint32_t>(), h->node_comp.as<uint32_t>(),
+        LAUNCH(h, k_node_keep, grid_for(N + 1, 256), 256, h->nodes.cov.as<uint32_t>(), h->nodes.comp.as<uint32_t>(),
                h->comp_max.as<uint32_t>(), N, thr_node, mode, keep_n);
     if (mode != 0 && E > 0) {
         AMIRA_CUDA(cudaMemsetAsync(h->d_status.p, 0, sizeof(int) * ST_COUNT, st));
-        LAUNCH(h, k_multi_edge_check, grid_for(N, 256), 256, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(),
+        LAUNCH(h, k_multi_edge_check, grid_for(N, 256), 256, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(),
                h->adj_edges.as<uint32_t>(), h->adj_off.as<int64_t>(), keep_n, N, h->d_status.as<int>());
         AMIRA_CUDA(cudaMemcpyAsync(h->h_status, h->d_status.p, sizeof(int) * ST_COUNT, cudaMemcpyDeviceToHost, st));
         AMIRA_CUDA(cudaStreamSynchronize(st));
@@ -996,25 +990,25 @@ int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
             return AMIRA_E_MULTI_EDGE;
         }
     }
-    LAUNCH(h, k_edge_keep, grid_for(E + 1, 256), 256, h->e_src.as<int32_t>(), h->e_tgt.as<int32_t>(),
-           h->e_cov.as<uint32_t>(), keep_n, E, thr_edge, keep_e);
+    LAUNCH(h, k_edge_keep, grid_for(E + 1, 256), 256, h->edges.src.as<int32_t>(), h->edges.tgt.as<int32_t>(),
+           h->edges.cov.as<uint32_t>(), keep_n, E, thr_edge, keep_e);
     // new indices; the sizes of the filtered graph stay on the device
     AMIRA_TRY(run_scan(h, KeepLoad{keep_n}, KeepStore{new_n, N, dsz(h, SZ_NODES)}, nullptr, 1, N, N));
     AMIRA_TRY(run_scan(h, KeepLoad{keep_e}, KeepStore{new_e, E, dsz(h, SZ_EDGES)}, nullptr, 1, E, E));
-    LAUNCH(h, k_compact_nodes, grid_for(N, 256), 256, keep_n, new_n, N, k, h->node_key.as<int32_t>(),
-           h->node_cov.as<uint32_t>(), h->node_dir.as<int8_t>(), h->node_comp.as<uint32_t>(), h->reads_off.as<int64_t>(),
-           h->node_key2.as<int32_t>(), h->node_cov2.as<uint32_t>(), h->node_dir2.as<int8_t>(),
-           h->node_comp2.as<uint32_t>(), h->reads_off2.as<int64_t>());
+    LAUNCH(h, k_compact_nodes, grid_for(N, 256), 256, keep_n, new_n, N, k, h->nodes.key.as<int32_t>(),
+           h->nodes.cov.as<uint32_t>(), h->nodes.dir.as<int8_t>(), h->nodes.comp.as<uint32_t>(), h->nodes.reads_off.as<int64_t>(),
+           h->nodes_alt.key.as<int32_t>(), h->nodes_alt.cov.as<uint32_t>(), h->nodes_alt.dir.as<int8_t>(),
+           h->nodes_alt.comp.as<uint32_t>(), h->nodes_alt.reads_off.as<int64_t>());
     // read counts of the survivors -> offsets (in place), over the new node count
-    AMIRA_TRY(run_scan(h, CountLoad{h->reads_off2.as<int64_t>()},
-                       OffStore{h->reads_off2.as<int64_t>(), dcnt(h, SZ_NODES), dsz(h, SZ_INC)}, dsz(h, SZ_NODES), 1, 0, N));
-    LAUNCH(h, k_compact_incidence, grid_for(N * 32, 256), 256, keep_n, new_n, N, h->reads_off.as<int64_t>(),
-           h->reads.as<uint32_t>(), h->reads_off2.as<int64_t>(), h->reads2.as<uint32_t>());
+    AMIRA_TRY(run_scan(h, CountLoad{h->nodes_alt.reads_off.as<int64_t>()},
+                       OffStore{h->nodes_alt.reads_off.as<int64_t>(), dcnt(h, SZ_NODES), dsz(h, SZ_INC)}, dsz(h, SZ_NODES), 1, 0, N));
+    LAUNCH(h, k_compact_incidence, grid_for(N * 32, 256), 256, keep_n, new_n, N, h->nodes.reads_off.as<int64_t>(),
+           h->nodes.reads.as<uint32_t>(), h->nodes_alt.reads_off.as<int64_t>(), h->nodes_alt.reads.as<uint32_t>());
     if (E > 0) {
-        LAUNCH(h, k_compact_edges, grid_for(E, 256), 256, keep_e, new_e, new_n, E, h->e_src.as<int32_t>(),
-               h->e_tgt.as<int32_t>(), h->e_sd.as<int8_t>(), h->e_td.as<int8_t>(), h->e_cov.as<uint32_t>(),
-               h->e_src2.as<int32_t>(), h->e_tgt2.as<int32_t>(), h->e_sd2.as<int8_t>(), h->e_td2.as<int8_t>(),
-               h->e_cov2.as<uint32_t>());
+        LAUNCH(h, k_compact_edges, grid_for(E, 256), 256, keep_e, new_e, new_n, E, h->edges.src.as<int32_t>(),
+               h->edges.tgt.as<int32_t>(), h->edges.sd.as<int8_t>(), h->edges.td.as<int8_t>(), h->edges.cov.as<uint32_t>(),
+               h->edges_alt.src.as<int32_t>(), h->edges_alt.tgt.as<int32_t>(), h->edges_alt.sd.as<int8_t>(), h->edges_alt.td.as<int8_t>(),
+               h->edges_alt.cov.as<uint32_t>());
     }
     if (W > 0) {
         LAUNCH(h, k_mask_windows, (int)std::min<int64_t>(grid_for(W, 256), (int64_t)h->n_sm * 32), 256, keep_n, new_n,
@@ -1023,20 +1017,8 @@ int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
                (long long)W, h->to_correct.as<uint8_t>());
     }
     AMIRA_CUDA(cudaEventRecord(h->ev_reads_ready, h->stream));
-    std::swap(h->node_key, h->node_key2);
-    std::swap(h->node_cov, h->node_cov2);
-    std::swap(h->node_dir, h->node_dir2);
-    std::swap(h->node_comp, h->node_comp2);
-    std::swap(h->reads_off, h->reads_off2);
-    std::swap(h->reads, h->reads2);
-    if (E > 0) {
-        std::swap(h->e_src, h->e_src2);
-        std::swap(h->e_tgt, h->e_tgt2);
-        std::swap(h->e_sd, h->e_sd2);
-        std::swap(h->e_td, h->e_td2);
-        std::swap(h->e_cov, h->e_cov2);
-    }
-    buffer_generation()++;  // a build captured before this filter would write into the old buffers
+    h->nodes.swap(h->nodes_alt);
+    if (E > 0) h->edges.swap(h->edges_alt);
     AMIRA_TRY(build_adjacency(h, false));
     AMIRA_TRY(enqueue_report(h, 1));
     h->pending = 2;
@@ -1133,40 +1115,10 @@ int publish_to_all(amira_gmg *h, bool p2p, const void *mine, int64_t n_mine, siz
     return comm_allgatherv(h->comm, mine, n_mine, fallback_recv, g_off.data(), elem, h->cur);
 }
 
-// AMIRA_SHARD_TRACE=1: per-step device times of the merge on stderr (developer aid)
-struct MergeTrace {
-    amira_gmg *h;
-    bool on;
-    std::vector<std::pair<const char *, cudaEvent_t>> marks;
-    explicit MergeTrace(amira_gmg *h_) : h(h_), on(getenv("AMIRA_SHARD_TRACE") != nullptr) { mark("start"); }
-    void mark(const char *name) {
-        if (!on) return;
-        cudaEvent_t e;
-        cudaEventCreate(&e);
-        cudaEventRecord(e, h->cur);
-        marks.push_back({name, e});
-    }
-    ~MergeTrace() {
-        if (!on) return;
-        cudaStreamSynchronize(h->cur);
-        std::string line = "[merge rank " + std::to_string(h->rank) + "]";
-        for (size_t i = 1; i < marks.size(); ++i) {
-            float ms = 0;
-            cudaEventElapsedTime(&ms, marks[i - 1].second, marks[i].second);
-            char buf[96];
-            snprintf(buf, sizeof(buf), " %s=%.3f", marks[i].first, ms);
-            line += buf;
-        }
-        fprintf(stderr, "%s\n", line.c_str());
-        for (auto &m : marks) cudaEventDestroy(m.second);
-    }
-};
-
 // node half, on the main stream: afterwards every local slot knows its global node index and the global node
 // arrays are final, so the per-read passes can start while the edges are still being exchanged
 int sharded_merge_nodes(amira_gmg *h) {
     Phase ph(h, AMIRA_PH_EXCHANGE);
-    MergeTrace tr(h);
     const int world = h->world, k = h->k, me = h->rank;
     cudaStream_t st = h->cur;
     const int tgrid_n = std::min<int>(grid_for(h->ncap, 256), h->n_sm * 16);
@@ -1183,7 +1135,6 @@ int sharded_merge_nodes(amira_gmg *h) {
     memset(&ndst, 0, sizeof(ndst));
     LAUNCH(h, k_node_route<false>, tgrid_n, 256, h->nview, h->ids, k, world, call_base, d_cnt, ndst);
     AMIRA_TRY(exchange_counts(h, send_off, recv_off));
-    tr.mark("n_count");
     const int64_t Nl = send_off[world], Nr = recv_off[world];
     int64_t nr_max = 0, nl_sum = 0;
     for (int d = 0; d < world; ++d) {
@@ -1231,7 +1182,6 @@ int sharded_merge_nodes(amira_gmg *h) {
         r_key = h->x_rkey.as<int32_t>();
         r_meta = h->x_rmeta.as<NodeRec>();
     }
-    tr.mark("n_a2a");
 
     // ---- owner merge: records in first-position order into a table (sum of counts, earliest record)
     int64_t mcap = std::min<int64_t>(2 * Nr + 1024, 0x7FFFFFF0ll);
@@ -1257,7 +1207,6 @@ int sharded_merge_nodes(amira_gmg *h) {
                h->x_mmeta.as<NodeRec>());
     }
     AMIRA_TRY(gather_counts(h, g_off));
-    tr.mark("n_merge");
     const int64_t Nm = g_off[h->rank + 1] - g_off[h->rank], Ng = g_off[world];
     if (Ng >= 0x7FFFFFF0ll) {
         set_error("too many nodes for int32 node indices");
@@ -1279,7 +1228,6 @@ int sharded_merge_nodes(amira_gmg *h) {
         g_key = h->x_gkey.as<int32_t>();
         g_meta = h->x_gmeta.as<NodeRec>();
     }
-    tr.mark("n_allgather");
 
     // ---- global node arrays in upstream's insertion order (= first global position)
     AMIRA_TRY(reserve_graph(h, Ng, 0));
@@ -1288,15 +1236,14 @@ int sharded_merge_nodes(amira_gmg *h) {
     if (Ng > 0) {
         AMIRA_TRY(h->x_sorti2.reserve(sizeof(unsigned int) * Ng));
         AMIRA_TRY(rank_by_position(h, NodePos{g_meta}, (long long)Ng, h->x_sorti2.as<unsigned int>()));
-        LAUNCH(h, k_finalize_nodes, grid_for(Ng, 256), 256, h->x_sorti2.as<unsigned int>(), g_key, g_meta, k, (long long)Ng, h->node_key.as<int32_t>(), h->node_cov.as<uint32_t>(),
-               h->node_dir.as<int8_t>(), h->link.as<uint8_t>());
+        LAUNCH(h, k_finalize_nodes, grid_for(Ng, 256), 256, h->x_sorti2.as<unsigned int>(), g_key, g_meta, k, (long long)Ng, h->nodes.key.as<int32_t>(), h->nodes.cov.as<uint32_t>(),
+               h->nodes.dir.as<int8_t>(), h->link.as<uint8_t>());
         // local slots -> global node indices: probe the rank's own node table with every global gene-mer
         if (h->G > 0)
             LAUNCH(h, k_global_to_local, grid_for(Ng, 256), 256, h->local_P, h->n16 ? 1 : 0, h->nview,
-                   h->node_key.as<int32_t>(), (long long)Ng, h->cov_local.as<uint32_t>());
+                   h->nodes.key.as<int32_t>(), (long long)Ng, h->cov_local.as<uint32_t>());
     }
 
-    tr.mark("n_global");
     h->n_nodes = Ng;
     h->prev_nodes = Nl;
     return AMIRA_OK;
@@ -1305,7 +1252,6 @@ int sharded_merge_nodes(amira_gmg *h) {
 // edge half, on the CURRENT stream (the second one: it runs beside the per-read passes of the main stream)
 int sharded_merge_edges(amira_gmg *h) {
     Phase ph(h, AMIRA_PH_EXCHANGE_EDGES);
-    MergeTrace tr(h);
     const int world = h->world, me = h->rank;
     cudaStream_t st = h->cur;
     const int tgrid_e = std::min<int>(grid_for(h->ecap, 256), h->n_sm * 16);
@@ -1320,7 +1266,6 @@ int sharded_merge_edges(amira_gmg *h) {
     memset(&edst, 0, sizeof(edst));
     LAUNCH(h, k_edge_route<false>, tgrid_e, 256, h->eview, h->nview, world, call_base, d_cnt, edst);
     AMIRA_TRY(exchange_counts(h, send_off, recv_off));
-    tr.mark("e_count");
     const int64_t El = send_off[world], Er = recv_off[world];
     int64_t er_max = 0, el_sum = 0;
     for (int d = 0; d < world; ++d) {
@@ -1356,7 +1301,6 @@ int sharded_merge_edges(amira_gmg *h) {
         AMIRA_TRY(comm_alltoallv(h->comm, h->x_sedge.p, send_off.data(), h->x_redge.p, recv_off.data(), sizeof(EdgeSlot), st));
         r_edge = h->x_redge.as<EdgeSlot>();
     }
-    tr.mark("e_a2a");
     AMIRA_TRY(h->x_medge.reserve(sizeof(EdgeSlot) * std::max<int64_t>(Er, 1)));
     const int64_t mecap = std::min<int64_t>(2 * Er + 1024, 0x7FFFFFF0ll);
     AMIRA_TRY(h->x_etab.reserve(sizeof(EdgeSlot) * mecap));
@@ -1369,7 +1313,6 @@ int sharded_merge_edges(amira_gmg *h) {
                (unsigned int)mecap, d_cnt, h->x_medge.as<EdgeSlot>());
     }
     AMIRA_TRY(gather_counts(h, g_off));
-    tr.mark("e_merge");
     const int64_t Em = g_off[h->rank + 1] - g_off[h->rank], Eg = g_off[world];
     const EdgeSlot *g_edge;
     if (p2p) {
@@ -1381,7 +1324,6 @@ int sharded_merge_edges(amira_gmg *h) {
         AMIRA_TRY(publish_to_all(h, false, h->x_medge.p, Em, sizeof(EdgeSlot), 0, g_off, h->x_gedge.p));
         g_edge = h->x_gedge.as<EdgeSlot>();
     }
-    tr.mark("e_allgather");
     int64_t E_dir = 0;
     AMIRA_TRY(h->x_fan.reserve(sizeof(int) * (Eg + 2)));
     if (Eg > 0) {
@@ -1403,7 +1345,6 @@ int sharded_merge_edges(amira_gmg *h) {
     // the directed edge arrays (+ union-find) are emitted on the second stream, beside the per-read passes
     h->sh_Eg = Eg;
     h->sh_gedge = g_edge;
-    tr.mark("e_global");
     h->n_edges = E_dir;
     h->prev_und_edges = El + 1;
     return AMIRA_OK;
@@ -1470,8 +1411,7 @@ int amira_gmg_create(amira_gmg **out, int device, void *cuda_stream) {
         // between the waves of the bandwidth-bound sort on the main stream
         int prio_lo = 0, prio_hi = 0;
         AMIRA_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
-        const bool side_low = getenv("AMIRA_SIDE_LOW") != nullptr;  // developer experiments
-        AMIRA_CUDA(cudaStreamCreateWithPriority(&h->stream2, cudaStreamNonBlocking, side_low ? prio_lo : prio_hi));
+        AMIRA_CUDA(cudaStreamCreateWithPriority(&h->stream2, cudaStreamNonBlocking, prio_hi));
     }
     AMIRA_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     AMIRA_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
@@ -1522,19 +1462,6 @@ void amira_gmg_destroy(amira_gmg *h) {
         if (h->ev_h2d[i]) cudaEventDestroy(h->ev_h2d[i]);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_join) cudaEventDestroy(h->ev_join);
-    DevBuf *bufs[] = {&h->d_ids, &h->d_off, &h->d_ps, &h->d_pe, &h->win_off, &h->is_short, &h->to_correct, &h->tile_r0,
-                      &h->win_node, &h->win_dir, &h->win_read, &h->win_start, &h->win_end, &h->ntab, &h->etab,
-                      &h->bitmaps, &h->cnt_node, &h->cnt_edge, &h->node_key, &h->node_cov, &h->node_dir, &h->node_comp,
-                      &h->reads_off, &h->reads, &h->node_key2, &h->node_cov2, &h->node_dir2, &h->node_comp2,
-                      &h->reads_off2, &h->reads2, &h->parent, &h->link, &h->run_id, &h->run_pairs, &h->is_root, &h->e_src, &h->e_tgt, &h->e_sd, &h->e_td,
-                      &h->e_cov, &h->e_src2, &h->e_tgt2, &h->e_sd2, &h->e_td2, &h->e_cov2, &h->adj_off, &h->adj_edges,
-                      &h->adj_cursor, &h->adj_tmp, &h->reads_tmp, &h->slot_info, &h->inc_rec, &h->unit_lo, &h->bucket_cursor, &h->win_slot, &h->seg_work[0], &h->seg_work[1], &h->scan_state[0], &h->scan_state[1], &h->scan_pool, &h->dups,
-                      &h->keep_n, &h->keep_e, &h->comp_max, &h->scratch_off, &h->d_status, &h->d_sizes,
-                      &h->x_cnt, &h->x_skey, &h->x_smeta, &h->x_rkey, &h->x_rmeta, &h->x_rmeta2,
-                      &h->x_mkey, &h->x_mmeta, &h->x_gkey, &h->x_gmeta, &h->x_tab, &h->x_bm, &h->x_pref,
-                      &h->x_sorti2, &h->x_sedge, &h->x_redge, &h->x_medge, &h->x_gedge, &h->x_etab, &h->x_fan,
-                      &h->cov_local, &h->cc_min, &h->d_maxabs};
-    for (DevBuf *b : bufs) b->release();
     if (h->comm) comm_destroy(h->comm);
     if (h->h_cnt) cudaFreeHost(h->h_cnt);
     if (h->graph_exec) cudaGraphExecDestroy(h->graph_exec);
@@ -1546,7 +1473,7 @@ void amira_gmg_destroy(amira_gmg *h) {
         for (int j = 0; j < 2; ++j)
             if (h->ev[i][j]) cudaEventDestroy(h->ev[i][j]);
     if (h->own_stream) cudaStreamDestroy(h->stream);
-    delete h;
+    delete h;  // the device buffers free themselves, on the device set above
 }
 
 int amira_gmg_reserve(amira_gmg *h, int64_t n_nodes_hint, int64_t n_edges_hint) {
@@ -1786,12 +1713,12 @@ int amira_gmg_export_nodes(amira_gmg *h, int32_t *key, uint32_t *cov, int8_t *fi
         if (bw_off) bw_off[0] = 0;
         return AMIRA_OK;
     }
-    AMIRA_TRY(d2h(h, key, h->node_key.p, sizeof(int32_t) * N * h->k));
-    AMIRA_TRY(d2h(h, cov, h->node_cov.p, sizeof(uint32_t) * N));
-    AMIRA_TRY(d2h(h, first_dir, h->node_dir.p, N));
-    AMIRA_TRY(d2h(h, component, h->node_comp.p, sizeof(uint32_t) * N));
-    AMIRA_TRY(d2h(h, reads_off, h->reads_off.p, sizeof(int64_t) * (N + 1)));
-    AMIRA_TRY(d2h(h, reads, h->reads.p, sizeof(int32_t) * h->n_inc));
+    AMIRA_TRY(d2h(h, key, h->nodes.key.p, sizeof(int32_t) * N * h->k));
+    AMIRA_TRY(d2h(h, cov, h->nodes.cov.p, sizeof(uint32_t) * N));
+    AMIRA_TRY(d2h(h, first_dir, h->nodes.dir.p, N));
+    AMIRA_TRY(d2h(h, component, h->nodes.comp.p, sizeof(uint32_t) * N));
+    AMIRA_TRY(d2h(h, reads_off, h->nodes.reads_off.p, sizeof(int64_t) * (N + 1)));
+    AMIRA_TRY(d2h(h, reads, h->nodes.reads.p, sizeof(int32_t) * h->n_inc));
     AMIRA_TRY(d2h(h, fw_off, h->adj_off.p, sizeof(int64_t) * (N + 1)));
     AMIRA_TRY(d2h(h, fw_edges, h->adj_edges.p, sizeof(int32_t) * h->n_fw));
     if (bw_off) {
@@ -1815,11 +1742,11 @@ int amira_gmg_export_edges(amira_gmg *h, int32_t *src, int32_t *tgt, int8_t *sd,
     if (!h->built) return h->last_status;
     const int64_t E = h->n_edges;
     if (E == 0) return AMIRA_OK;
-    AMIRA_TRY(d2h(h, src, h->e_src.p, sizeof(int32_t) * E));
-    AMIRA_TRY(d2h(h, tgt, h->e_tgt.p, sizeof(int32_t) * E));
-    AMIRA_TRY(d2h(h, sd, h->e_sd.p, E));
-    AMIRA_TRY(d2h(h, td, h->e_td.p, E));
-    AMIRA_TRY(d2h(h, cov, h->e_cov.p, sizeof(uint32_t) * E));
+    AMIRA_TRY(d2h(h, src, h->edges.src.p, sizeof(int32_t) * E));
+    AMIRA_TRY(d2h(h, tgt, h->edges.tgt.p, sizeof(int32_t) * E));
+    AMIRA_TRY(d2h(h, sd, h->edges.sd.p, E));
+    AMIRA_TRY(d2h(h, td, h->edges.td.p, E));
+    AMIRA_TRY(d2h(h, cov, h->edges.cov.p, sizeof(uint32_t) * E));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
     return AMIRA_OK;
 }
@@ -1930,7 +1857,7 @@ int amira_gmg_read_length_coverages(amira_gmg *h, const int32_t *min_len, int32_
     AMIRA_CUDA(cudaMemsetAsync(d_sums, 0, sizeof(unsigned long long) * STAT_MAX_THRESHOLDS, h->stream));
     if (h->n_inc > 0 && n > 0)
         LAUNCH(h, k_read_length_coverages, (int)std::min<int64_t>(grid_for(h->n_inc, 256), (int64_t)h->n_sm * 16), 256,
-               h->reads_off.as<int64_t>(), h->reads.as<uint32_t>(), h->off, (long long)h->n_inc, (int32_t)h->first_read_global, T,
+               h->nodes.reads_off.as<int64_t>(), h->nodes.reads.as<uint32_t>(), h->off, (long long)h->n_inc, (int32_t)h->first_read_global, T,
                d_sums);
     unsigned long long out[STAT_MAX_THRESHOLDS];
     AMIRA_CUDA(cudaMemcpyAsync(out, d_sums, sizeof(out), cudaMemcpyDeviceToHost, h->stream));
@@ -1946,7 +1873,7 @@ int amira_gmg_node_coverage_stats(amira_gmg *h, int64_t *sum_cov, uint32_t *max_
     AMIRA_CUDA(cudaMemsetAsync(d, 0, sizeof(unsigned long long) * 2, h->stream));
     if (h->n_nodes > 0)
         LAUNCH(h, k_coverage_sum, (int)std::min<int64_t>(grid_for(h->n_nodes, 256), (int64_t)h->n_sm * 8), 256,
-               h->node_cov.as<uint32_t>(), (long long)h->n_nodes, d);
+               h->nodes.cov.as<uint32_t>(), (long long)h->n_nodes, d);
     unsigned long long out[2];
     AMIRA_CUDA(cudaMemcpyAsync(out, d, sizeof(out), cudaMemcpyDeviceToHost, h->stream));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
@@ -1982,7 +1909,7 @@ int flag_nodes_containing(amira_gmg *h, const int32_t *ranks, int32_t n) {
     AMIRA_TRY(h->comp_max.reserve(sizeof(int32_t) * (size_t)std::max(n, 1) + sizeof(uint32_t) * (size_t)(h->n_comps + 2)));
     if (n > 0) AMIRA_CUDA(cudaMemcpyAsync(h->comp_max.p, ranks, sizeof(int32_t) * n, cudaMemcpyHostToDevice, h->stream));
     if (N > 0)
-        LAUNCH(h, k_nodes_containing, grid_for(N, 256), 256, h->node_key.as<int32_t>(), (long long)N, h->k, h->comp_max.as<int32_t>(),
+        LAUNCH(h, k_nodes_containing, grid_for(N, 256), 256, h->nodes.key.as<int32_t>(), (long long)N, h->k, h->comp_max.as<int32_t>(),
                n, h->scratch_off.as<uint8_t>());
     return AMIRA_OK;
 }
@@ -2029,10 +1956,10 @@ int amira_gmg_remove_nodes_without_reads_of(amira_gmg *h, const int32_t *ranks, 
     AMIRA_TRY(h->dups.reserve((size_t)R + 8));
     uint8_t *read_flag = h->dups.as<uint8_t>();
     AMIRA_CUDA(cudaMemsetAsync(read_flag, 0, (size_t)R + 1, h->stream));
-    LAUNCH(h, k_mark_reads_of_nodes, grid_for(N * 32, 256), 256, h->scratch_off.as<uint8_t>(), h->reads_off.as<int64_t>(),
-           h->reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, read_flag);
-    LAUNCH(h, k_nodes_with_marked_reads, grid_for((N + 1) * 32, 256), 256, read_flag, h->reads_off.as<int64_t>(),
-           h->reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, h->keep_n.as<int>());
+    LAUNCH(h, k_mark_reads_of_nodes, grid_for(N * 32, 256), 256, h->scratch_off.as<uint8_t>(), h->nodes.reads_off.as<int64_t>(),
+           h->nodes.reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, read_flag);
+    LAUNCH(h, k_nodes_with_marked_reads, grid_for((N + 1) * 32, 256), 256, read_flag, h->nodes.reads_off.as<int64_t>(),
+           h->nodes.reads.as<uint32_t>(), (long long)N, (int32_t)h->first_read_global, h->keep_n.as<int>());
     return filter_status(h, do_filter(h, 2, 0, 0));
 }
 
@@ -2053,8 +1980,8 @@ int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int
     S.dir[1] = (int8_t *)(base + 13 * N);
     S.ext[0] = (uint8_t *)(base + 14 * N);
     S.ext[1] = (uint8_t *)(base + 15 * N);
-    LAUNCH(h, k_linear_steps, grid_for(N, 256), 256, h->adj_off.as<int64_t>(), h->adj_edges.as<uint32_t>(), h->e_tgt.as<int32_t>(),
-           h->e_td.as<int8_t>(), (long long)N, S);
+    LAUNCH(h, k_linear_steps, grid_for(N, 256), 256, h->adj_off.as<int64_t>(), h->adj_edges.as<uint32_t>(), h->edges.tgt.as<int32_t>(),
+           h->edges.td.as<int8_t>(), (long long)N, S);
     AMIRA_TRY(d2h(h, degree, S.degree, sizeof(uint32_t) * N));
     AMIRA_TRY(d2h(h, fw_next, S.next[0], sizeof(int32_t) * N));
     AMIRA_TRY(d2h(h, bw_next, S.next[1], sizeof(int32_t) * N));
@@ -2106,7 +2033,6 @@ int amira_gmg_debug_segsort(amira_gmg *h, uint32_t *data, const int64_t *off, in
         AMIRA_CUDA(cudaStreamSynchronize(st));
         if (total_dups) *total_dups = cnt[1];
     }
-    for (DevBuf *x : {&d_a, &d_b, &d_off, &d_dups, &d_cnt, &d_start}) x->release();
     return rc;
 }
 
@@ -2169,7 +2095,6 @@ int amira_gmg_atomic_peak(amira_gmg *h, int64_t table_bytes, int64_t n_ops, doub
     }
     cudaEventDestroy(a);
     cudaEventDestroy(b);
-    t.release();
     return AMIRA_OK;
 }
 

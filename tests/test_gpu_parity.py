@@ -405,3 +405,12 @@ def test_gpu_repeated_resident_builds_replay_a_graph(dg):
     for rep in range(3):                      # back-to-back replays without looking at the results in between
         dg.build(d[0], d[1], 3, on_device=True, wait=False)
     assert O.diff_arrays(dg.arrays(), ref[3]) == []
+    # duplicate incidences: reading the results of each build removes them by swapping the read lists into the
+    # second buffer pair, so a graph captured before that swap would write into the wrong buffers
+    ids3, off3 = heavy_node_reads()
+    d3 = [torch.from_numpy(x).cuda() for x in (ids3, off3)]
+    torch.cuda.synchronize()
+    ref3 = c_oracle.COracleGraph(ids3, off3, 3).arrays()
+    for rep in range(5):
+        dg.build(d3[0], d3[1], 3, on_device=True, wait=False)
+        assert O.diff_arrays(dg.arrays(), ref3) == [], rep
