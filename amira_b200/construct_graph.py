@@ -129,7 +129,7 @@ class GeneMerGraph:
         self._read_ids = []
         self._win_off = None
         self._device_ops = ()
-        self._steps_cache = None
+        self._index_cache = None         # node hash -> device index of a materialised device graph
         self.timings = {}
         _lib.load()                      # fail loudly if the CUDA library is missing
         if len(readDict) > 0:
@@ -293,7 +293,7 @@ class GeneMerGraph:
 
     def _apply_device_removal(self, h):
         """mirror the device's last removal on the host objects (same deletions upstream performs)"""
-        self._steps_cache = None
+        self._index_cache = None
         if self.__dict__.get("_lazy"):
             return                       # nothing materialised yet: the arrays are the graph
         node_keep, edge_keep = h.filter_masks()
@@ -474,18 +474,10 @@ class GeneMerGraph:
 
     # ------------------------------------------------------------------ linear paths (upstream :722-861, 679-720)
     def _linear_steps(self) -> dict:
-        """per node and side: upstream's one step of a linear-path walk (next node index, entry direction, extend flag)
-        and the node degrees -- from the device adjacency CSR (k_linear_steps), or from the host objects when the
-        graph was edited on the host since"""
-        if self._steps_cache is not None and self._on_device():
-            return self._steps_cache
+        """per node and side of a graph edited on the host: upstream's one step of a linear-path walk (next node index,
+        entry direction, extend flag) and the node degrees, from the host objects (device graphs walk on the device:
+        amira_gmg_linear_walks)"""
         nodes = self._nodes
-        if self._on_device():
-            st = {k: v.tolist() for k, v in self._require_device_state().linear_steps().items()}
-            st["index"] = {h: i for i, h in enumerate(self._node_order)}
-            st["hash"] = self._node_order
-            self._steps_cache = st
-            return st
         order = list(nodes)
         index = {h: i for i, h in enumerate(order)}
         st = {"index": index, "hash": order, "degree": [self.get_degree(n) for n in nodes.values()]}
@@ -525,15 +517,47 @@ class GeneMerGraph:
                 path.append(nx)
         return path
 
+    def _walks_over(self, st, states, want_branched: bool) -> tuple:
+        """_walk from every state 2 * node + side (0 = forward list, 1 = backward list) of the step table `st`, without
+        the start node -> (offsets, nodes), as amira_gmg_linear_walks returns them"""
+        off, out = [0], []
+        for s in np.asarray(states, np.int64).tolist():
+            out.extend(self._walk(st, s >> 1, "bw" if s & 1 else "fw", False, want_branched)[1:])
+            off.append(len(out))
+        return np.asarray(off, np.int64), np.asarray(out, np.int64)
+
+    def _device_walks(self, h, states, want_branched: bool) -> tuple:
+        """linear walks on the device graph (amira_gmg_linear_walks).  A handle without them -- the oracle-backed test
+        double the CPU tests build with -- is walked with _walk over its step table."""
+        if hasattr(h, "linear_walks"):
+            return h.linear_walks(states, want_branched)
+        return self._walks_over({f: v.tolist() for f, v in h.linear_steps().items()}, states, want_branched)
+
+    def _device_walk(self, node, side: int, want_branched: bool) -> list:
+        """node hashes of the device walk from one side (0 = forward list, 1 = backward list) of a node, the node first"""
+        self._nodes                                     # the arguments are node objects: materialised, in device order
+        if self._index_cache is None:
+            self._index_cache = {h: i for i, h in enumerate(self._node_order)}
+        i = self._index_cache[node.__hash__()]
+        _, walk = self._device_walks(self._require_device_state(), [2 * i + side], want_branched)
+        order = self._node_order
+        return [order[i]] + [order[j] for j in walk.tolist()]
+
     def get_forward_path_from_node(self, node, startDirection, wantBranchedNode=False) -> list:
+        side = 0 if startDirection == 1 else 1
+        if self._on_device():
+            return self._device_walk(node, side, wantBranchedNode)
         st = self._linear_steps()
         i = st["index"][node.__hash__()]
-        return [st["hash"][j] for j in self._walk(st, i, "fw" if startDirection == 1 else "bw", False, wantBranchedNode)]
+        return [st["hash"][j] for j in self._walk(st, i, ("fw", "bw")[side], False, wantBranchedNode)]
 
     def get_backward_path_from_node(self, node, startDirection, wantBranchedNode=False) -> list:
+        side = 1 if startDirection == -1 else 0
+        if self._on_device():
+            return self._device_walk(node, side, wantBranchedNode)[::-1]
         st = self._linear_steps()
         i = st["index"][node.__hash__()]
-        return [st["hash"][j] for j in self._walk(st, i, "bw" if startDirection == -1 else "fw", True, wantBranchedNode)]
+        return [st["hash"][j] for j in self._walk(st, i, ("fw", "bw")[side], True, wantBranchedNode)]
 
     def get_linear_path_for_node(self, node, wantBranchedNode=False) -> list:
         """upstream construct_graph.py:849-861"""
@@ -546,47 +570,92 @@ class GeneMerGraph:
 
     def remove_short_linear_paths(self, min_length, sample_genesOfInterest={}):
         """upstream construct_graph.py:679-720: dead ends (degree-1 nodes) whose linear path is shorter than min_length
-        are removed unless the whole path is well covered, holds an AMR gene or is its whole component.  The paths
-        come from the device step table; the removal is one device pass (amira_gmg_remove_nodes)."""
-        st = self._linear_steps()
-        nodes = self._nodes
-        mean15 = self.get_mean_node_coverage() * 1.5 if len(nodes) else 0
-        paths_to_remove = {}
-        for i, node in enumerate(list(nodes.values())):
-            if st["degree"][st["index"][node.__hash__()]] != 1:
-                continue
-            path = self.get_linear_path_for_node(node)
-            if 0 < len(path) < min_length:
-                if all(nodes[n].get_node_coverage() > mean15 for n in path):
-                    continue
-                paths_to_remove.setdefault(node.get_component(), []).append(path)
-        AMR_nodes = self.get_AMR_nodes(sample_genesOfInterest)
-        removed = []
-        seen = set()
-        for component, paths in paths_to_remove.items():
-            in_comp = {n.__hash__() for n in self.get_nodes_in_component(component)} if component is not None else set()
-            for path in paths:
-                if component is not None and len(in_comp.intersection(path)) == len(in_comp):
-                    continue
-                for nh in path:
-                    if nh in AMR_nodes or nh in seen:
-                        continue
-                    seen.add(nh)
-                    removed.append(nh)
-        if not removed:
-            return []
+        are removed unless the whole path is well covered, holds an AMR gene or is its whole component.  A device graph
+        is walked on the device (amira_gmg_linear_walks) and trimmed in one device pass (amira_gmg_remove_nodes)
+        without creating host objects; a graph edited on the host is walked over its objects."""
         if self._on_device():
+            if self.get_total_number_of_nodes() == 0:
+                return []
             h = self._require_device_state()
-            flags = np.zeros(len(self._node_order), np.uint8)
-            index = st["index"]
-            flags[[index[nh] for nh in removed]] = 1
+            degree = h.linear_steps()["degree"]
+            cov, comp, ndir, key = self._arrays("node_cov", "node_comp", "node_dir", "node_key")
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            amr = h.nodes_containing(ranks) if ranks else np.zeros(len(cov), bool)
+            removed = self._short_path_nodes(min_length, degree, cov, comp.astype(np.int64), ndir, amr,
+                                             lambda states: self._device_walks(h, states, False))
+            if not len(removed):
+                return []
+            hashes = _keys.node_keys(key[removed].astype(np.int64), self._vocab)[0]
+            flags = np.zeros(len(cov), np.uint8)
+            flags[removed] = 1
             h.remove_nodes(flags)
             self._device_ops = self._device_ops + (("remove_nodes", (flags,)),)
             self._apply_device_removal(h)
-        else:
-            for nh in removed:
-                self.remove_node(nodes[nh])
-        return removed
+            return hashes
+        st = self._linear_steps()
+        nodes = self._nodes
+        if not nodes:
+            return []
+        objs = list(nodes.values())
+        codes = {}                                      # component ids (None: no component) -> 0, 1, ...
+        comp = np.asarray([-1 if n.get_component() is None else codes.setdefault(n.get_component(), len(codes))
+                           for n in objs], np.int64)
+        AMR_nodes = self.get_AMR_nodes(sample_genesOfInterest)
+        amr = np.asarray([nh in AMR_nodes for nh in st["hash"]], bool)
+        removed = self._short_path_nodes(min_length, np.asarray(st["degree"]), np.asarray([n.get_node_coverage() for n in objs]),
+                                         comp, np.asarray([n.get_geneMer().get_geneMerDirection() for n in objs]), amr,
+                                         lambda states: self._walks_over(st, states, False))
+        hashes = [st["hash"][i] for i in removed.tolist()]
+        for nh in hashes:
+            self.remove_node(nodes[nh])
+        return hashes
+
+    def _short_path_nodes(self, min_length, degree, cov, comp, ndir, amr, walks) -> np.ndarray:
+        """the trimming policy of remove_short_linear_paths over node indices.  walks(states) -> (offsets, nodes) gives
+        the linear walks from the states 2 * node + side; comp[i] = -1: node i has no component.  Returns the nodes to
+        remove in upstream's order: component first seen, then path, then node along the path, each node once."""
+        none = np.zeros(0, np.int64)
+        tips = np.flatnonzero(degree == 1)
+        if not len(tips):
+            return none
+        # get_linear_path_for_node: the backward walk (reversed), the node, the forward walk
+        back = (ndir[tips] == 1).astype(np.int64)
+        off, w = walks(np.stack([2 * tips + back, 2 * tips + 1 - back], 1).ravel())
+        off, w = np.asarray(off, np.int64), np.asarray(w, np.int64)
+        nb, nf = off[1::2] - off[0:-1:2], off[2::2] - off[1::2]
+        q = np.flatnonzero(nb + 1 + nf < min_length)     # short paths, by tip
+        if not len(q):
+            return none
+        plen = nb[q] + 1 + nf[q]
+        start = np.concatenate([[0], np.cumsum(plen)[:-1]])
+        pid = np.repeat(np.arange(len(q)), plen)          # path of every element, elements in path order
+        p = np.arange(len(pid)) - start[pid]
+        b = nb[q][pid]
+        w_end = np.append(w, -1)
+        bi = np.where(p < b, off[2 * q][pid] + b - 1 - p, len(w))
+        fi = np.where(p > b, off[2 * q + 1][pid] + p - b - 1, len(w))
+        node = np.where(p == b, tips[q][pid], np.where(p < b, w_end[bi], w_end[fi]))
+        # paths whose every node is covered above 1.5 x the mean stay
+        mean15 = self.get_mean_node_coverage() * 1.5
+        kept = np.add.reduceat((cov[node] <= mean15).astype(np.int64), start) > 0
+        # components in the order their first kept path was seen
+        c = comp[tips[q]]
+        kq = np.flatnonzero(kept)
+        _, first, inv = np.unique(c[kq], return_index=True, return_inverse=True)
+        rank = np.full(len(q), len(q), np.int64)
+        rank[kq] = first[inv.ravel()]
+        # a path that is its whole component stays
+        n_nodes = len(degree)
+        sizes = np.bincount(comp[comp >= 0], minlength=n_nodes)
+        u = np.unique(pid * n_nodes + node)
+        upid, unode = u // n_nodes, u % n_nodes
+        in_comp = np.bincount(upid[comp[unode] == c[upid]], minlength=len(q))
+        whole = (c >= 0) & (in_comp == sizes[np.maximum(c, 0)])
+        go = kept & ~whole
+        sel = np.flatnonzero(go[pid] & ~amr[node])
+        seq = node[sel[np.argsort(rank[pid[sel]], kind="stable")]]
+        _, first_at = np.unique(seq, return_index=True)
+        return seq[np.sort(first_at)]
 
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
@@ -692,7 +761,7 @@ class GeneMerGraph:
     def _touch(self):
         self._nodes                          # host edits need the host objects (materialise before going stale)
         self._device_synced = False
-        self._steps_cache = None
+        self._index_cache = None
 
     def add_node_to_read(self, node, readId: str, node_direction: int, node_position=None):
         self._touch()
@@ -988,7 +1057,7 @@ def bind_upstream(upstream_construct_graph):
                    "_touch", "remove_junk_reads", "get_valid_reads_only", "get_total_number_of_nodes",
                    "get_total_number_of_edges", "get_all_node_coverages", "get_mean_node_coverage", "components",
                    "get_nodes_containing", "_gene_ranks", "get_AMR_nodes", "remove_non_AMR_associated_nodes", "_linear_steps",
-                   "_walk", "get_forward_path_from_node", "get_backward_path_from_node", "get_linear_path_for_node",
+                   "_walk", "_walks_over", "_device_walks", "_device_walk", "_short_path_nodes", "get_forward_path_from_node", "get_backward_path_from_node", "get_linear_path_for_node",
                    "remove_short_linear_paths", "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

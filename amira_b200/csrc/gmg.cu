@@ -8,6 +8,7 @@
 
 #include "post_kernels.cuh"
 #include "stats.cuh"
+#include "paths.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -175,6 +176,17 @@ struct amira_gmg {
     DevBuf x_cnt, x_skey, x_smeta, x_rkey, x_rmeta, x_rmeta2, x_mkey, x_mmeta, x_gkey, x_gmeta, x_tab,
         x_bm, x_pref, x_sorti2, x_sedge, x_redge, x_medge, x_gedge, x_etab, x_fan, cov_local;
     long long *h_cnt = nullptr;  // pinned, world*world + 4
+
+    // linear walks (paths.cuh): the jump table and the forest ranks of the walk states, valid while the graph they
+    // were computed from is (graph_version: bumped by every build and every filter / removal)
+    uint64_t graph_version = 0;
+    struct {
+        DevBuf jump, nxt, root[2], dist[2], is_label;
+        DevBuf q_states, q_steps, q_len, q_off, q_bad, out;
+        int L = 0, fin = 0;  // levels; which root / dist buffer holds the final ranks
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+    } walks;
 };
 
 namespace {
@@ -254,6 +266,7 @@ int bits_for_ids(unsigned int max_abs) {
 }
 
 void reset_graph(amira_gmg *h) {
+    h->graph_version++;
     h->n_nodes = h->n_edges = h->W = h->n_inc = h->n_short = h->n_fw = h->n_bw = h->n_comps = 0;
     h->pending = 0;
 }
@@ -961,6 +974,7 @@ int filter_reserve(amira_gmg *h) {
 // already in keep_n (remove_node for every node whose flag is 0)
 int do_filter(amira_gmg *h, int mode, uint32_t thr_node, uint32_t thr_edge) {
     AMIRA_TRY(filter_reserve(h));
+    h->graph_version++;
     const int64_t N = h->n_nodes, E = h->n_edges, W = h->W;
     const int k = h->k;
     cudaStream_t st = h->stream;
@@ -1990,6 +2004,116 @@ int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int
     AMIRA_TRY(d2h(h, fw_ext, S.ext[0], N));
     AMIRA_TRY(d2h(h, bw_ext, S.ext[1], N));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+namespace {
+// jump table and forest ranks of the 2N walk states (paths.cuh), reused while neither the graph nor any device buffer
+// has changed since they were computed
+int walk_table(amira_gmg *h, WalkTable &T) {
+    auto &w = h->walks;
+    const long long S = 2 * h->n_nodes;
+    if (!(w.valid && w.version == h->graph_version && w.generation == buffer_generation())) {
+        w.valid = false;
+        int L = 1;
+        while ((1ll << L) <= S) ++L;
+        AMIRA_TRY(w.jump.reserve(sizeof(int32_t) * (size_t)S * L));
+        AMIRA_TRY(w.nxt.reserve(sizeof(int32_t) * (size_t)S));
+        AMIRA_TRY(w.is_label.reserve((size_t)S));
+        for (int i = 0; i < 2; ++i) {
+            AMIRA_TRY(w.root[i].reserve(sizeof(int32_t) * (size_t)S));
+            AMIRA_TRY(w.dist[i].reserve(sizeof(int32_t) * (size_t)S));
+        }
+        int32_t *J = w.jump.as<int32_t>();
+        const int grid = grid_for(S, 256);
+        LAUNCH(h, k_walk_succ, grid, 256, h->adj_off.as<int64_t>(), h->adj_edges.as<uint32_t>(), h->edges.tgt.as<int32_t>(),
+               h->edges.td.as<int8_t>(), (long long)h->n_nodes, J, w.nxt.as<int32_t>());
+        for (int l = 1; l < L; ++l) LAUNCH(h, k_walk_jump_level, grid, 256, J + (l - 1) * S, J + l * S, S);
+        // cycle labels: window minima over 2^L states (root[] as scratch), then the minimum seen from each cycle
+        int32_t *m[2] = {w.root[0].as<int32_t>(), w.root[1].as<int32_t>()};
+        for (int l = 0; l < L; ++l) LAUNCH(h, k_walk_cycle_min, grid, 256, J + l * S, l ? m[(l - 1) & 1] : nullptr, m[l & 1], S);
+        AMIRA_CUDA(cudaMemsetAsync(w.is_label.p, 0, (size_t)S, h->stream));
+        h->lib_launches++;
+        LAUNCH(h, k_walk_cycle_labels, grid, 256, J + (L - 1) * S, m[(L - 1) & 1], w.is_label.as<uint8_t>(), S);
+        // rank the forest left by cutting every cycle at its label
+        int32_t *r[2] = {w.root[0].as<int32_t>(), w.root[1].as<int32_t>()}, *d[2] = {w.dist[0].as<int32_t>(), w.dist[1].as<int32_t>()};
+        LAUNCH(h, k_walk_rank_init, grid, 256, J, w.is_label.as<uint8_t>(), r[0], d[0], S);
+        for (int l = 0; l < L; ++l) LAUNCH(h, k_walk_rank_round, grid, 256, r[l & 1], d[l & 1], r[(l + 1) & 1], d[(l + 1) & 1], S);
+        w.L = L;
+        w.fin = L & 1;
+        w.version = h->graph_version;
+        w.generation = buffer_generation();
+        w.valid = true;
+    }
+    T.J = w.jump.as<int32_t>();
+    T.nxt = w.nxt.as<int32_t>();
+    T.root = w.root[w.fin].as<int32_t>();
+    T.dist = w.dist[w.fin].as<int32_t>();
+    T.S = S;
+    T.L = w.L;
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int want_branched, int64_t *walk_off,
+                           int32_t *walk_nodes) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("linear_walks: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    if (n < 0 || (n > 0 && !states) || !walk_off) {
+        set_error("linear_walks: bad arguments (n = %lld)", (long long)n);
+        return AMIRA_E_ARG;
+    }
+    const long long S = 2 * h->n_nodes;
+    for (int64_t i = 0; i < n; ++i) {
+        if (states[i] < 0 || states[i] >= S) {
+            set_error("linear_walks: state %d (query %lld) is out of range: the graph has %lld states", states[i], (long long)i, S);
+            return AMIRA_E_ARG;
+        }
+    }
+    const int64_t room = walk_nodes ? walk_off[n] : 0;  // the size pass told the caller how much to allocate
+    if (n == 0) {
+        walk_off[0] = 0;
+        return AMIRA_OK;
+    }
+    auto &w = h->walks;
+    AMIRA_TRY(w.q_states.reserve(sizeof(int32_t) * (size_t)n));
+    AMIRA_TRY(w.q_steps.reserve(sizeof(int32_t) * (size_t)n));
+    AMIRA_TRY(w.q_len.reserve(sizeof(unsigned long long) * (size_t)n));
+    AMIRA_TRY(w.q_off.reserve(sizeof(int64_t) * (size_t)(n + 1)));
+    AMIRA_TRY(w.q_bad.reserve(sizeof(int)));
+    WalkTable T;
+    AMIRA_TRY(walk_table(h, T));
+    cudaStream_t st = h->stream;
+    int bad = WALK_NEVER_ENDS;
+    AMIRA_CUDA(cudaMemcpyAsync(w.q_states.p, states, sizeof(int32_t) * n, cudaMemcpyHostToDevice, st));
+    AMIRA_CUDA(cudaMemcpyAsync(w.q_bad.p, &bad, sizeof(int), cudaMemcpyHostToDevice, st));
+    h->lib_launches += 2;
+    LAUNCH(h, k_walk_lengths, grid_for(n, 256), 256, T, w.q_states.as<int32_t>(), (long long)n, want_branched ? 1 : 0,
+           w.q_steps.as<int32_t>(), w.q_len.as<unsigned long long>(), w.q_bad.as<int>());
+    AMIRA_TRY(run_scan(h, WalkLenLoad{w.q_len.as<unsigned long long>()}, WalkOffStore{w.q_off.as<int64_t>()}, nullptr, 1, n, n));
+    AMIRA_TRY(d2h(h, &bad, w.q_bad.p, sizeof(int)));
+    AMIRA_TRY(d2h(h, walk_off, w.q_off.p, sizeof(int64_t) * (n + 1)));
+    AMIRA_CUDA(cudaStreamSynchronize(st));
+    if (bad != WALK_NEVER_ENDS) {
+        set_error("linear_walks: the walk from state %d (query %d) never ends: it runs into a cycle without its start node",
+                  states[bad], bad);
+        return AMIRA_E_STATE;
+    }
+    if (!walk_nodes) return AMIRA_OK;
+    const int64_t total = walk_off[n];
+    if (total != room) {
+        set_error("linear_walks: the walks take %lld nodes, walk_off[n] said %lld", (long long)total, (long long)room);
+        return AMIRA_E_ARG;
+    }
+    if (total == 0) return AMIRA_OK;
+    AMIRA_TRY(w.out.reserve(sizeof(int32_t) * (size_t)total));
+    LAUNCH(h, k_walk_fill, (int)std::min<int64_t>(grid_for(total, 256), (int64_t)h->n_sm * 32), 256, T, w.q_states.as<int32_t>(),
+           (long long)n, w.q_off.as<int64_t>(), w.q_steps.as<int32_t>(), w.out.as<int32_t>());
+    AMIRA_TRY(d2h(h, walk_nodes, w.out.p, sizeof(int32_t) * total));
+    AMIRA_CUDA(cudaStreamSynchronize(st));
     return AMIRA_OK;
 }
 

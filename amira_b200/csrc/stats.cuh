@@ -133,26 +133,34 @@ struct LinearSteps {
     uint32_t *degree;
 };
 
+__device__ __forceinline__ void linear_step(const int64_t *__restrict__ adj_off, const uint32_t *__restrict__ adj_edges,
+                                            const int32_t *__restrict__ e_tgt, const int8_t *__restrict__ e_td, const long long N,
+                                            const long long n, const int side, int32_t &nx, int8_t &d, uint8_t &ex) {
+    const long long a0 = adj_off[side * N + n], a1 = adj_off[side * N + n + 1];
+    const bool take = side ? (a1 > a0) : (a1 - a0 == 1);
+    nx = -1;
+    d = 0;
+    ex = 0;
+    if (take) {
+        const uint32_t e = adj_edges[a0];
+        nx = e_tgt[e];
+        d = e_td[e];
+        const long long deg = (adj_off[nx + 1] - adj_off[nx]) + (adj_off[N + nx + 1] - adj_off[N + nx]);
+        ex = (deg == 1 || deg == 2) && nx != (int32_t)n;
+    }
+}
+
 __global__ void k_linear_steps(const int64_t *__restrict__ adj_off, const uint32_t *__restrict__ adj_edges,
                                const int32_t *__restrict__ e_tgt, const int8_t *__restrict__ e_td, const long long N,
                                const LinearSteps S) {
     const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (n >= N) return;
-    const long long f0 = adj_off[n], f1 = adj_off[n + 1], b0 = adj_off[N + n], b1 = adj_off[N + n + 1];
-    S.degree[n] = (uint32_t)((f1 - f0) + (b1 - b0));
+    S.degree[n] = (uint32_t)((adj_off[n + 1] - adj_off[n]) + (adj_off[N + n + 1] - adj_off[N + n]));
     for (int side = 0; side < 2; ++side) {
-        const long long a0 = side ? b0 : f0, a1 = side ? b1 : f1;
-        const bool take = side ? (a1 > a0) : (a1 - a0 == 1);
-        int32_t nx = -1;
-        int8_t d = 0;
-        uint8_t ex = 0;
-        if (take) {
-            const uint32_t e = adj_edges[a0];
-            nx = e_tgt[e];
-            d = e_td[e];
-            const long long deg = (adj_off[nx + 1] - adj_off[nx]) + (adj_off[N + nx + 1] - adj_off[N + nx]);
-            ex = (deg == 1 || deg == 2) && nx != (int32_t)n;
-        }
+        int32_t nx;
+        int8_t d;
+        uint8_t ex;
+        linear_step(adj_off, adj_edges, e_tgt, e_td, N, n, side, nx, d, ex);
         S.next[side][n] = nx;
         S.dir[side][n] = d;
         S.ext[side][n] = ex;

@@ -129,6 +129,21 @@ class DeviceGraph:
                                                                                      "bw_next", "bw_dir", "bw_ext")]))
         return a
 
+    def linear_walks(self, states, want_branched: bool = False):
+        """walks from the states 2 * node + side (0 = forward list, 1 = backward list), without the start node, plus the
+        branching node when want_branched -> (off[n + 1] int64, nodes int32): walk i is nodes[off[i]:off[i + 1]]"""
+        s = np.asarray(states, np.int64).ravel()
+        if len(s) and (s.min() < -2**31 or s.max() >= 2**31):
+            raise ValueError("linear_walks: state out of range")
+        s = np.ascontiguousarray(s, np.int32)
+        off = np.zeros(len(s) + 1, np.int64)
+        _lib.check(self._lib.amira_gmg_linear_walks(self._h, _ptr(s), len(s), int(bool(want_branched)), _ptr(off), None))
+        nodes = np.empty(int(off[-1]), np.int32)
+        if len(nodes):
+            _lib.check(self._lib.amira_gmg_linear_walks(self._h, _ptr(s), len(s), int(bool(want_branched)), _ptr(off),
+                                                        _ptr(nodes)))
+        return off, nodes
+
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""
         a, b = C.c_int64(), C.c_int64()

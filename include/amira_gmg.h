@@ -177,6 +177,16 @@ int amira_gmg_remove_nodes_without_reads_of(amira_gmg *h, const int32_t *ranks, 
 int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int8_t *fw_dir, uint8_t *fw_ext,
                            int32_t *bw_next, int8_t *bw_dir, uint8_t *bw_ext);
 
+/* Linear walks (get_forward_path_from_node / get_backward_path_from_node, construct_graph.py:722-848) from n start
+ * states (2*node + side, side 0 = forward list, 1 = backward list), without the start node, in walk order, plus the
+ * branching node when want_branched.  walk_nodes == NULL: only walk_off[n+1] is written (sizes); then call again with
+ * walk_nodes[walk_off[n]].  Leaves the filter masks alone.  AMIRA_E_STATE for a walk that never ends.
+ * The walk from s0 (node n0) follows succ(s) = 2*next[s] + (dir[s] == 1 ? 0 : 1) while ext[s] is set (linear_steps),
+ * and stops before a state of n0; the branching node is next[s] of the state it stopped on, when there is one.
+ * Not available on a sharded handle (AMIRA_E_STATE). */
+int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int want_branched, int64_t *walk_off,
+                           int32_t *walk_nodes);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
