@@ -657,6 +657,99 @@ class GeneMerGraph:
         _, first_at = np.unique(seq, return_index=True)
         return seq[np.sort(first_at)]
 
+    # ------------------------------------------------------------------ compacted graph (no upstream counterpart)
+    def compacted_unitigs(self) -> dict:
+        """every maximal non-branching path as one unitig (include/amira_gmg.h, amira_gmg_unitigs), as numpy arrays:
+        node_unitig / node_pos / node_orient per node in `_nodes` order; unitig_off / unitig_nodes (node indices in
+        listed order), circular, cov_sum / cov_min / cov_max per unitig; edge_internal per edge in `_edges` order (1:
+        the edge joins consecutive nodes of one unitig, 0: a junction).  A device graph is compacted on the device and
+        stays lazy; a graph edited on the host is compacted from its objects."""
+        if self._on_device():
+            h = self._require_device_state()
+            if hasattr(h, "unitigs"):
+                return h.unitigs()
+            return self._unitigs_over(h.arrays())
+        return self._unitigs_over(self._unitig_index_arrays())
+
+    def _unitig_index_arrays(self) -> dict:
+        """the index arrays _unitigs_over reads, from the host objects: nodes in `_nodes` order, edges in `_edges`
+        order, each node's forward / backward list as a CSR over edge indices"""
+        nodes, edges = self._nodes, self._edges
+        index = {nh: i for i, nh in enumerate(nodes)}
+        eindex = {eh: j for j, eh in enumerate(edges)}
+        es = list(edges.values())
+        a = {"node_cov": np.asarray([n.get_node_coverage() for n in nodes.values()], np.int64),
+             "edge_src": np.asarray([index[e.get_sourceNode().__hash__()] for e in es], np.int64),
+             "edge_tgt": np.asarray([index[e.get_targetNode().__hash__()] for e in es], np.int64),
+             "edge_sd": np.asarray([e.get_sourceNodeDirection() for e in es], np.int64),
+             "edge_td": np.asarray([e.get_targetNodeDirection() for e in es], np.int64)}
+        for side, getter in (("fw", "get_forward_edge_hashes"), ("bw", "get_backward_edge_hashes")):
+            lists = [getattr(n, getter)() for n in nodes.values()]
+            a[side + "_off"] = np.concatenate([[0], np.cumsum([len(x) for x in lists], dtype=np.int64)]).astype(np.int64)
+            a[side + "_edges"] = np.asarray([eindex[eh] for x in lists for eh in x], np.int64)
+        return a
+
+    def _unitigs_over(self, a) -> dict:
+        """amira_gmg_unitigs over index arrays (node_cov, edge_src / tgt / sd / td, fw_off / fw_edges, bw_off /
+        bw_edges), by the same list ranking as csrc/unitigs.cuh: states s = 2 * node + side, succ(s), distances to
+        the tail and running minima by pointer jumping, cycles cut at their smallest state"""
+        N = len(a["node_cov"])
+        S = 2 * N
+        out = {"node_unitig": np.zeros(N, np.int32), "node_pos": np.zeros(N, np.int32), "node_orient": np.zeros(N, np.int8),
+               "unitig_off": np.zeros(1, np.int64), "unitig_nodes": np.zeros(N, np.int32), "circular": np.zeros(0, np.uint8),
+               "cov_sum": np.zeros(0, np.int64), "cov_min": np.zeros(0, np.uint32), "cov_max": np.zeros(0, np.uint32),
+               "edge_internal": np.zeros(len(a["edge_src"]), np.uint8)}
+        if N == 0:
+            return out
+        tgt, td = np.asarray(a["edge_tgt"], np.int64), np.asarray(a["edge_td"], np.int64)
+        size = np.stack([np.diff(a["fw_off"]), np.diff(a["bw_off"])], 1).ravel()   # size[s]: edges in the list of s
+        one = np.full(S, -1, np.int64)                                              # the edge of a one-edge list
+        for side, f in enumerate(("fw", "bw")):
+            sel = np.flatnonzero(np.diff(a[f + "_off"]) == 1)
+            one[2 * sel + side] = np.asarray(a[f + "_edges"], np.int64)[np.asarray(a[f + "_off"], np.int64)[sel]]
+        st = np.flatnonzero(one >= 0)
+        v, leave = tgt[one[st]], (td[one[st]] != 1).astype(np.int64)
+        ok = (v != st >> 1) & (size[2 * v + (1 - leave)] == 1)
+        succ = np.full(S, -1, np.int64)
+        succ[st[ok]] = 2 * v[ok] + leave[ok]
+        idx = np.arange(S, dtype=np.int64)
+        rounds = int(S - 1).bit_length() + 1                                         # ceil(log2 S) + 1
+
+        def rank(cut, mn=None):
+            ptr, dist = np.where(cut, idx, succ), (~cut).astype(np.int64)
+            for _ in range(rounds):
+                if mn is not None:
+                    mn = np.minimum(mn, mn[ptr])
+                dist = np.minimum(dist + dist[ptr], S)
+                ptr = ptr[ptr]
+            return ptr, dist, mn
+
+        ptr, dist, mn = rank(succ < 0, idx)
+        cyc = succ[ptr] >= 0
+        if cyc.any():
+            dist = rank((succ < 0) | (cyc & (mn == idx)))[1]
+        nodes = np.arange(N, dtype=np.int64)
+        cm = np.minimum(mn[0::2], mn[1::2] ^ 1)          # the smallest state of the chain of 2n
+        m, s = cm >> 1, 2 * nodes + (cm & 1)              # the unitig's smallest node, the state n is listed through
+        heads = np.flatnonzero(m == nodes)
+        uid = np.zeros(N, np.int64)
+        uid[heads] = np.arange(len(heads))
+        circ = cyc[2 * heads]
+        length = np.where(circ, dist[np.maximum(succ[2 * heads], 0)] + 1, dist[2 * heads] + dist[2 * heads + 1] + 1)
+        off = np.concatenate([[0], np.cumsum(length)]).astype(np.int64)
+        unit, pos = uid[m], dist[s ^ 1]
+        order = np.zeros(N, np.int64)
+        order[off[unit] + pos] = nodes
+        cov = np.asarray(a["node_cov"], np.int64)[order]
+        src = np.asarray(a["edge_src"], np.int64)
+        out.update(node_unitig=unit.astype(np.int32), node_pos=pos.astype(np.int32),
+                   node_orient=np.where(s & 1, -1, 1).astype(np.int8), unitig_off=off, unitig_nodes=order.astype(np.int32),
+                   circular=circ.astype(np.uint8), cov_sum=np.add.reduceat(cov, off[:-1]),
+                   cov_min=np.minimum.reduceat(cov, off[:-1]).astype(np.uint32),
+                   cov_max=np.maximum.reduceat(cov, off[:-1]).astype(np.uint32),
+                   edge_internal=(succ[2 * src + (np.asarray(a["edge_sd"]) < 0)] >= 0).astype(np.uint8))
+        return out
+
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
         return bool(self._device_synced) and len(self._reads) > 0
@@ -1058,7 +1151,8 @@ def bind_upstream(upstream_construct_graph):
                    "get_total_number_of_edges", "get_all_node_coverages", "get_mean_node_coverage", "components",
                    "get_nodes_containing", "_gene_ranks", "get_AMR_nodes", "remove_non_AMR_associated_nodes", "_linear_steps",
                    "_walk", "_walks_over", "_device_walks", "_device_walk", "_short_path_nodes", "get_forward_path_from_node", "get_backward_path_from_node", "get_linear_path_for_node",
-                   "remove_short_linear_paths", "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
+                   "remove_short_linear_paths", "compacted_unitigs", "_unitig_index_arrays", "_unitigs_over",
+                   "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up
     # host mutators must mark the device copy stale

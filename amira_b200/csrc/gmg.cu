@@ -9,6 +9,7 @@
 #include "post_kernels.cuh"
 #include "stats.cuh"
 #include "paths.cuh"
+#include "unitigs.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -187,6 +188,14 @@ struct amira_gmg {
         bool valid = false;
         uint64_t version = 0, generation = 0;
     } walks;
+    // unitigs (unitigs.cuh): the ranking arrays of the 2N states and the compacted graph, valid under the same rule
+    struct {
+        DevBuf succ, ptr[2], dist[2], mn[2], circ, any_cycle, uid, len, n_unitigs;
+        DevBuf node_unitig, node_pos, node_orient, off, nodes, circular, cov_sum, cov_min, cov_max, edge_internal;
+        int64_t U = 0;
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+    } unitigs;
 };
 
 namespace {
@@ -2114,6 +2123,123 @@ int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int w
            (long long)n, w.q_off.as<int64_t>(), w.q_steps.as<int32_t>(), w.out.as<int32_t>());
     AMIRA_TRY(d2h(h, walk_nodes, w.out.p, sizeof(int32_t) * total));
     AMIRA_CUDA(cudaStreamSynchronize(st));
+    return AMIRA_OK;
+}
+
+namespace {
+// the compacted graph (unitigs.cuh), reused while neither the graph nor any device buffer has changed since it was
+// computed
+int unitig_table(amira_gmg *h) {
+    auto &u = h->unitigs;
+    if (u.valid && u.version == h->graph_version && u.generation == buffer_generation()) return AMIRA_OK;
+    u.valid = false;
+    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
+    if (S >= (1ll << 31)) {
+        set_error("unitigs: %lld nodes, the states 2 * node + side must fit in 31 bits", N);
+        return AMIRA_E_ARG;
+    }
+    u.U = 0;
+    if (N > 0) {
+        const size_t s4 = sizeof(int32_t) * (size_t)S, n4 = sizeof(int32_t) * (size_t)N;
+        AMIRA_TRY(u.succ.reserve(s4));
+        for (int i = 0; i < 2; ++i) {
+            AMIRA_TRY(u.ptr[i].reserve(s4));
+            AMIRA_TRY(u.dist[i].reserve(s4));
+            AMIRA_TRY(u.mn[i].reserve(s4));
+        }
+        AMIRA_TRY(u.circ.reserve((size_t)N));
+        AMIRA_TRY(u.any_cycle.reserve(sizeof(int)));
+        AMIRA_TRY(u.uid.reserve(n4));
+        AMIRA_TRY(u.len.reserve(n4));
+        AMIRA_TRY(u.n_unitigs.reserve(sizeof(long long)));
+        AMIRA_TRY(u.node_unitig.reserve(n4));
+        AMIRA_TRY(u.node_pos.reserve(n4));
+        AMIRA_TRY(u.node_orient.reserve((size_t)N));
+        AMIRA_TRY(u.off.reserve(sizeof(int64_t) * (size_t)(N + 1)));
+        AMIRA_TRY(u.nodes.reserve(n4));
+        AMIRA_TRY(u.circular.reserve((size_t)N));
+        AMIRA_TRY(u.cov_sum.reserve(sizeof(unsigned long long) * (size_t)N));
+        AMIRA_TRY(u.cov_min.reserve(n4));
+        AMIRA_TRY(u.cov_max.reserve(n4));
+        AMIRA_TRY(u.edge_internal.reserve((size_t)std::max<long long>(E, 1)));
+        int32_t *succ = u.succ.as<int32_t>();
+        int32_t *p[2] = {u.ptr[0].as<int32_t>(), u.ptr[1].as<int32_t>()}, *m[2] = {u.mn[0].as<int32_t>(), u.mn[1].as<int32_t>()};
+        uint32_t *d[2] = {u.dist[0].as<uint32_t>(), u.dist[1].as<uint32_t>()};
+        int rounds = 1;  // ceil(log2 S) + 1: 2^rounds >= 2S steps cover every path and every cycle
+        while ((1ll << (rounds - 1)) < S) ++rounds;
+        const int grid = grid_for(S, 256);
+        cudaStream_t st = h->stream;
+        LAUNCH(h, k_unitig_succ, grid, 256, h->adj_off.as<int64_t>(), h->adj_edges.as<uint32_t>(), h->edges.tgt.as<int32_t>(),
+               h->edges.td.as<int8_t>(), N, succ, p[0], d[0], m[0]);
+        for (int r = 0; r < rounds; ++r)
+            LAUNCH(h, k_unitig_rank_round, grid, 256, p[r & 1], d[r & 1], m[r & 1], p[(r + 1) & 1], d[(r + 1) & 1], m[(r + 1) & 1], S);
+        const int f = rounds & 1;  // the buffers of the first ranking
+        int any_cycle = 0;
+        AMIRA_CUDA(cudaMemsetAsync(u.any_cycle.p, 0, sizeof(int), st));
+        h->lib_launches++;
+        LAUNCH(h, k_unitig_cycle_cut, grid, 256, succ, p[f], m[f], p[f ^ 1], d[f ^ 1], u.circ.as<uint8_t>(), u.any_cycle.as<int>(), S);
+        AMIRA_TRY(d2h(h, &any_cycle, u.any_cycle.p, sizeof(int)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        int fd = f;  // the distances the results are read from
+        if (any_cycle) {
+            fd = f ^ 1;
+            for (int r = 0; r < rounds; ++r, fd ^= 1)
+                LAUNCH(h, k_unitig_rank_round, grid, 256, p[fd], d[fd], (const int32_t *)nullptr, p[fd ^ 1], d[fd ^ 1], (int32_t *)nullptr, S);
+        }
+        const UnitigRanks R{succ, m[f], d[fd], u.circ.as<uint8_t>()};
+        long long *d_U = u.n_unitigs.as<long long>();
+        unsigned long long *cov_sum = u.cov_sum.as<unsigned long long>();
+        uint32_t *cov_min = u.cov_min.as<uint32_t>(), *cov_max = u.cov_max.as<uint32_t>();
+        AMIRA_TRY(run_scan(h, UnitigHeadLoad{R},
+                           UnitigHeadStore{R, u.uid.as<int32_t>(), u.len.as<uint32_t>(), u.circular.as<uint8_t>(), cov_sum, cov_min,
+                                           cov_max, N, d_U},
+                           nullptr, 1, N, N));
+        AMIRA_TRY(run_scan(h, UnitigLenLoad{u.len.as<uint32_t>()}, UnitigOffStore{u.off.as<int64_t>()}, d_U, 1, 0, N));
+        LAUNCH(h, k_unitig_scatter, grid_for(N, 256), 256, R, u.uid.as<int32_t>(), u.off.as<int64_t>(), h->nodes.cov.as<uint32_t>(), N,
+               u.node_unitig.as<int32_t>(), u.node_pos.as<int32_t>(), u.node_orient.as<int8_t>(), u.nodes.as<int32_t>(), cov_sum,
+               cov_min, cov_max);
+        if (E > 0)
+            LAUNCH(h, k_unitig_edges, grid_for(E, 256), 256, succ, h->edges.src.as<int32_t>(), h->edges.sd.as<int8_t>(), E,
+                   u.edge_internal.as<uint8_t>());
+        long long U = 0;
+        AMIRA_TRY(d2h(h, &U, d_U, sizeof(long long)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        u.U = U;
+    }
+    u.version = h->graph_version;
+    u.generation = buffer_generation();
+    u.valid = true;
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, int32_t *node_pos, int8_t *node_orient,
+                      int64_t *unitig_off, int32_t *unitig_nodes, uint8_t *circular, int64_t *cov_sum, uint32_t *cov_min,
+                      uint32_t *cov_max, uint8_t *edge_internal) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("unitigs: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    AMIRA_TRY(unitig_table(h));
+    const auto &u = h->unitigs;
+    const int64_t N = h->n_nodes, E = h->n_edges, U = u.U;
+    if (n_unitigs) *n_unitigs = U;
+    if (N == 0) {
+        if (unitig_off) unitig_off[0] = 0;
+        return AMIRA_OK;
+    }
+    AMIRA_TRY(d2h(h, node_unitig, u.node_unitig.p, sizeof(int32_t) * N));
+    AMIRA_TRY(d2h(h, node_pos, u.node_pos.p, sizeof(int32_t) * N));
+    AMIRA_TRY(d2h(h, node_orient, u.node_orient.p, (size_t)N));
+    AMIRA_TRY(d2h(h, unitig_off, u.off.p, sizeof(int64_t) * (U + 1)));
+    AMIRA_TRY(d2h(h, unitig_nodes, u.nodes.p, sizeof(int32_t) * N));
+    AMIRA_TRY(d2h(h, circular, u.circular.p, (size_t)U));
+    AMIRA_TRY(d2h(h, cov_sum, u.cov_sum.p, sizeof(int64_t) * U));
+    AMIRA_TRY(d2h(h, cov_min, u.cov_min.p, sizeof(uint32_t) * U));
+    AMIRA_TRY(d2h(h, cov_max, u.cov_max.p, sizeof(uint32_t) * U));
+    AMIRA_TRY(d2h(h, edge_internal, u.edge_internal.p, (size_t)E));
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
     return AMIRA_OK;
 }
 

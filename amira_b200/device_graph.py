@@ -11,6 +11,11 @@ import numpy as np
 from . import _lib
 
 
+# the arrays of amira_gmg_unitigs, in its argument order
+UNITIG_FIELDS = ("node_unitig", "node_pos", "node_orient", "unitig_off", "unitig_nodes", "circular", "cov_sum", "cov_min",
+                 "cov_max", "edge_internal")
+
+
 def _ptr(a):
     if a is None:
         return None
@@ -143,6 +148,21 @@ class DeviceGraph:
             _lib.check(self._lib.amira_gmg_linear_walks(self._h, _ptr(s), len(s), int(bool(want_branched)), _ptr(off),
                                                         _ptr(nodes)))
         return off, nodes
+
+    def unitigs(self) -> dict:
+        """the compacted graph (amira_gmg_unitigs): per node its unitig, position and orientation; per unitig its
+        nodes (unitig_nodes[unitig_off[u]:unitig_off[u + 1]]), circular flag and coverage sum / min / max; per directed
+        edge whether it joins consecutive nodes of one unitig"""
+        U = C.c_int64()
+        _lib.check(self._lib.amira_gmg_unitigs(self._h, C.byref(U), *[None] * 10))
+        s = self.sizes_early()
+        n, m, U = s["nodes"], s["edges"], U.value
+        a = {"node_unitig": np.empty(n, np.int32), "node_pos": np.empty(n, np.int32), "node_orient": np.empty(n, np.int8),
+             "unitig_off": np.empty(U + 1, np.int64), "unitig_nodes": np.empty(n, np.int32),
+             "circular": np.empty(U, np.uint8), "cov_sum": np.empty(U, np.int64), "cov_min": np.empty(U, np.uint32),
+             "cov_max": np.empty(U, np.uint32), "edge_internal": np.empty(m, np.uint8)}
+        _lib.check(self._lib.amira_gmg_unitigs(self._h, None, *[_ptr(a[f]) for f in UNITIG_FIELDS]))
+        return a
 
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""

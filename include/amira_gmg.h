@@ -187,6 +187,25 @@ int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int
 int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int want_branched, int64_t *walk_off,
                            int32_t *walk_nodes);
 
+/* The compacted graph: every maximal non-branching path as one unitig (no upstream counterpart).  With states
+ * s = 2*node + side as above, succ(2u + a) = 2v + (td == 1 ? 0 : 1) when list a of u holds exactly one edge
+ * (u -> v, td), v != u, and v's entering list (backward if td == +1, forward if td == -1) holds exactly one edge.
+ * The states form disjoint paths and cycles; a chain with its mirror (every state ^ 1) is one unitig, and every node
+ * lies in exactly one.  A unitig is listed in the orientation whose chain holds 2m, m its smallest node: a linear one
+ * from its head (the state without predecessor) to its tail, a circular one from m.  Unitig ids follow m ascending.
+ *   per node [N]: node_unitig, node_pos (position in the listed order), node_orient (+1: left through its forward
+ *     list in that order, -1: through its backward list);
+ *   per unitig [U]: unitig_off[U+1] into unitig_nodes[N] (node indices in listed order), circular, cov_sum /
+ *     cov_min / cov_max of the node coverages;
+ *   per directed edge [E]: edge_internal = 1 when the edge joins consecutive nodes of one unitig (in either
+ *     direction); the others are the junctions.  There are 2 * (N - linear unitigs) internal edges.
+ * Every pointer may be NULL.  Call with n_unitigs only to size the per-unitig arrays, then again for the arrays: the
+ * result is kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.
+ * Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
+int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, int32_t *node_pos, int8_t *node_orient,
+                      int64_t *unitig_off, int32_t *unitig_nodes, uint8_t *circular, int64_t *cov_sum, uint32_t *cov_min,
+                      uint32_t *cov_max, uint8_t *edge_internal);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
