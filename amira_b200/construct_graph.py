@@ -672,8 +672,8 @@ class GeneMerGraph:
         return self._unitigs_over(self._unitig_index_arrays())
 
     def _unitig_index_arrays(self) -> dict:
-        """the index arrays _unitigs_over reads, from the host objects: nodes in `_nodes` order, edges in `_edges`
-        order, each node's forward / backward list as a CSR over edge indices"""
+        """the index arrays _unitigs_over and _links_over read, from the host objects: nodes in `_nodes` order, edges
+        in `_edges` order, each node's forward / backward list as a CSR over edge indices"""
         nodes, edges = self._nodes, self._edges
         index = {nh: i for i, nh in enumerate(nodes)}
         eindex = {eh: j for j, eh in enumerate(edges)}
@@ -682,7 +682,8 @@ class GeneMerGraph:
              "edge_src": np.asarray([index[e.get_sourceNode().__hash__()] for e in es], np.int64),
              "edge_tgt": np.asarray([index[e.get_targetNode().__hash__()] for e in es], np.int64),
              "edge_sd": np.asarray([e.get_sourceNodeDirection() for e in es], np.int64),
-             "edge_td": np.asarray([e.get_targetNodeDirection() for e in es], np.int64)}
+             "edge_td": np.asarray([e.get_targetNodeDirection() for e in es], np.int64),
+             "edge_cov": np.asarray([e.get_edge_coverage() for e in es], np.int64)}
         for side, getter in (("fw", "get_forward_edge_hashes"), ("bw", "get_backward_edge_hashes")):
             lists = [getattr(n, getter)() for n in nodes.values()]
             a[side + "_off"] = np.concatenate([[0], np.cumsum([len(x) for x in lists], dtype=np.int64)]).astype(np.int64)
@@ -701,17 +702,7 @@ class GeneMerGraph:
                "edge_internal": np.zeros(len(a["edge_src"]), np.uint8)}
         if N == 0:
             return out
-        tgt, td = np.asarray(a["edge_tgt"], np.int64), np.asarray(a["edge_td"], np.int64)
-        size = np.stack([np.diff(a["fw_off"]), np.diff(a["bw_off"])], 1).ravel()   # size[s]: edges in the list of s
-        one = np.full(S, -1, np.int64)                                              # the edge of a one-edge list
-        for side, f in enumerate(("fw", "bw")):
-            sel = np.flatnonzero(np.diff(a[f + "_off"]) == 1)
-            one[2 * sel + side] = np.asarray(a[f + "_edges"], np.int64)[np.asarray(a[f + "_off"], np.int64)[sel]]
-        st = np.flatnonzero(one >= 0)
-        v, leave = tgt[one[st]], (td[one[st]] != 1).astype(np.int64)
-        ok = (v != st >> 1) & (size[2 * v + (1 - leave)] == 1)
-        succ = np.full(S, -1, np.int64)
-        succ[st[ok]] = 2 * v[ok] + leave[ok]
+        succ = self._unitig_succ(a)
         idx = np.arange(S, dtype=np.int64)
         rounds = int(S - 1).bit_length() + 1                                         # ceil(log2 S) + 1
 
@@ -749,6 +740,99 @@ class GeneMerGraph:
                    cov_max=np.maximum.reduceat(cov, off[:-1]).astype(np.uint32),
                    edge_internal=(succ[2 * src + (np.asarray(a["edge_sd"]) < 0)] >= 0).astype(np.uint8))
         return out
+
+    @staticmethod
+    def _unitig_succ(a) -> np.ndarray:
+        """succ of every state s = 2 * node + side over index arrays (csrc/unitigs.cuh), -1 where there is none: list
+        `side` of the node holds one edge (-> v, td), v is another node, and v's entering list holds one edge"""
+        S = 2 * len(a["node_cov"])
+        tgt, td = np.asarray(a["edge_tgt"], np.int64), np.asarray(a["edge_td"], np.int64)
+        size = np.stack([np.diff(a["fw_off"]), np.diff(a["bw_off"])], 1).ravel()   # size[s]: edges in the list of s
+        one = np.full(S, -1, np.int64)                                              # the edge of a one-edge list
+        for side, f in enumerate(("fw", "bw")):
+            sel = np.flatnonzero(np.diff(a[f + "_off"]) == 1)
+            one[2 * sel + side] = np.asarray(a[f + "_edges"], np.int64)[np.asarray(a[f + "_off"], np.int64)[sel]]
+        st = np.flatnonzero(one >= 0)
+        v, leave = tgt[one[st]], (td[one[st]] != 1).astype(np.int64)
+        ok = (v != st >> 1) & (size[2 * v + (1 - leave)] == 1)
+        succ = np.full(S, -1, np.int64)
+        succ[st[ok]] = 2 * v[ok] + leave[ok]
+        return succ
+
+    def compacted_links(self) -> dict:
+        """the junction edges of the compacted graph (include/amira_gmg.h, amira_gmg_unitig_links), one link per edge
+        with edge_internal == 0 in `_edges` order, as numpy arrays: edge (its index), from_unitig / from_orient (the
+        unitig end it leaves: +1 its last node in listed order, -1 its first), to_unitig / to_orient (the end it
+        enters: +1 the first node, -1 the last), cov.  A device graph is served by the device and stays lazy."""
+        if self._on_device():
+            h = self._require_device_state()
+            if hasattr(h, "unitig_links"):
+                return h.unitig_links()
+            return self._links_over(h.arrays())
+        return self._links_over(self._unitig_index_arrays())
+
+    def read_unitig_paths(self) -> dict:
+        """every read of get_reads(), in that order, as steps along the unitigs of compacted_unitigs()
+        (amira_gmg_read_unitig_paths): read r's steps are path_off[r]:path_off[r + 1]; a step is a maximal run of
+        consecutive windows of the read that follow one unitig, with its unitig, orient (+1: in listed order), pos
+        (of its first window's node), win (that window's index in _readNodes[read]) and length (windows).  None
+        windows belong to no step; short reads have empty paths.  A device graph is served by the device and stays
+        lazy."""
+        if self._on_device():
+            h = self._require_device_state()
+            if hasattr(h, "read_unitig_paths"):
+                return h.read_unitig_paths()
+            a = h.arrays()
+            return self._read_paths_over(a, a)
+        return self._read_paths_over(self._unitig_index_arrays(), self._read_index_arrays())
+
+    def _read_index_arrays(self) -> dict:
+        """the per-read window arrays _read_paths_over reads, from _readNodes / _readNodeDirections in get_reads()
+        order: win_off, win_node (index in `_nodes` order, -1 for None), win_dir (0 for None); a read without an entry
+        has no windows"""
+        index = {nh: i for i, nh in enumerate(self._nodes)}
+        rn, rd = self._readNodes, self._readNodeDirections
+        nodes = [rn.get(r, []) for r in self._reads]
+        dirs = [rd.get(r, []) for r in self._reads]
+        node = np.asarray([index.get(x, -1) if x is not None else -1 for row in nodes for x in row], np.int64)
+        return {"win_off": np.concatenate([[0], np.cumsum([len(x) for x in nodes], dtype=np.int64)]).astype(np.int64),
+                "win_node": node,
+                "win_dir": np.where(node >= 0, np.asarray([d or 0 for row in dirs for d in row], np.int64), 0)}
+
+    def _links_over(self, a) -> dict:
+        """amira_gmg_unitig_links over index arrays (those of _unitigs_over, and edge_cov)"""
+        u = self._unitigs_over(a)
+        j = np.flatnonzero(u["edge_internal"] == 0)
+        src, tgt = np.asarray(a["edge_src"], np.int64)[j], np.asarray(a["edge_tgt"], np.int64)[j]
+        sd, td = np.asarray(a["edge_sd"], np.int64)[j], np.asarray(a["edge_td"], np.int64)[j]
+        return {"edge": j.astype(np.int32), "from_unitig": u["node_unitig"][src],
+                "from_orient": (sd * u["node_orient"][src]).astype(np.int8), "to_unitig": u["node_unitig"][tgt],
+                "to_orient": (td * u["node_orient"][tgt]).astype(np.int8),
+                "cov": np.asarray(a["edge_cov"], np.int64)[j].astype(np.uint32)}
+
+    def _read_paths_over(self, a, w) -> dict:
+        """amira_gmg_read_unitig_paths over index arrays: the graph `a` (as _unitigs_over) and the windows `w`
+        (win_off, win_node with -1 for None, win_dir).  A window continues the one before it when both are live, in
+        one read, and succ(state before) == its state, a window's state being 2 * node + (dir < 0)"""
+        u = self._unitigs_over(a)
+        woff = np.asarray(w["win_off"], np.int64)
+        node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
+        R, W = len(woff) - 1, len(node)
+        live = node >= 0
+        state = np.where(live, 2 * node + (d < 0), 0)
+        cont = np.zeros(W, bool)
+        if W and len(u["node_unitig"]):
+            succ = self._unitig_succ(a)
+            cont[1:] = live[1:] & live[:-1] & (succ[state[:-1]] == state[1:])
+            cont[woff[:-1][woff[:-1] < W]] = False                # a read's first window continues nothing
+        start = np.flatnonzero(live & ~cont)
+        end = np.flatnonzero(live & ~np.append(cont[1:], False))
+        read = np.repeat(np.arange(R, dtype=np.int64), np.diff(woff))[start]
+        n = node[start]
+        return {"path_off": np.concatenate([[0], np.cumsum(np.bincount(read, minlength=R))]).astype(np.int64),
+                "unitig": u["node_unitig"][n], "orient": (np.where(d[start] < 0, -1, 1) * u["node_orient"][n]).astype(np.int8),
+                "pos": u["node_pos"][n], "win": (start - woff[read]).astype(np.int32),
+                "length": (end - start + 1).astype(np.int32)}
 
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
@@ -1152,6 +1236,8 @@ def bind_upstream(upstream_construct_graph):
                    "get_nodes_containing", "_gene_ranks", "get_AMR_nodes", "remove_non_AMR_associated_nodes", "_linear_steps",
                    "_walk", "_walks_over", "_device_walks", "_device_walk", "_short_path_nodes", "get_forward_path_from_node", "get_backward_path_from_node", "get_linear_path_for_node",
                    "remove_short_linear_paths", "compacted_unitigs", "_unitig_index_arrays", "_unitigs_over",
+                   "_unitig_succ", "compacted_links", "read_unitig_paths", "_read_index_arrays", "_links_over",
+                   "_read_paths_over",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

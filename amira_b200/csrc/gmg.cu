@@ -196,6 +196,21 @@ struct amira_gmg {
         bool valid = false;
         uint64_t version = 0, generation = 0;
     } unitigs;
+    // the junction edges as links between unitig ends, and the reads as steps along unitigs (unitigs.cuh), valid under
+    // the same rule
+    struct {
+        DevBuf n_links, edge, from_unitig, from_orient, to_unitig, to_orient, cov;
+        int64_t L = 0;
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+    } links;
+    struct {
+        DevBuf flags, n_steps, path_off, unitig, orient, pos, win, length;
+        int64_t T = 0;
+        bool on_device = false;  // path_off was computed (else every read's path is empty)
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+    } paths;
 };
 
 namespace {
@@ -2239,6 +2254,152 @@ int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, in
     AMIRA_TRY(d2h(h, cov_min, u.cov_min.p, sizeof(uint32_t) * U));
     AMIRA_TRY(d2h(h, cov_max, u.cov_max.p, sizeof(uint32_t) * U));
     AMIRA_TRY(d2h(h, edge_internal, u.edge_internal.p, (size_t)E));
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+namespace {
+// the scan tile states of a scan over n items, reserved ahead (a buffer that grows bumps the buffer generation)
+int reserve_scan(amira_gmg *h, int64_t n) {
+    return h->scan_state[0].reserve(sizeof(unsigned long long) * (size_t)scan_tiles(n));
+}
+
+// the links of the compacted graph, cached under the rule of unitig_table.  Every buffer is reserved before
+// unitig_table runs: a reservation that grows bumps the buffer generation and would drop the unitigs just computed.
+int unitig_links_table(amira_gmg *h) {
+    auto &l = h->links;
+    if (l.valid && l.version == h->graph_version && l.generation == buffer_generation()) return AMIRA_OK;
+    l.valid = false;
+    const long long E = h->n_edges;
+    if (E > 0) {
+        const size_t e4 = sizeof(int32_t) * (size_t)E;
+        AMIRA_TRY(l.n_links.reserve(sizeof(long long)));
+        AMIRA_TRY(l.edge.reserve(e4));
+        AMIRA_TRY(l.from_unitig.reserve(e4));
+        AMIRA_TRY(l.from_orient.reserve((size_t)E));
+        AMIRA_TRY(l.to_unitig.reserve(e4));
+        AMIRA_TRY(l.to_orient.reserve((size_t)E));
+        AMIRA_TRY(l.cov.reserve(e4));
+        AMIRA_TRY(reserve_scan(h, E));
+    }
+    AMIRA_TRY(unitig_table(h));
+    l.L = 0;
+    if (E > 0) {
+        const auto &u = h->unitigs;
+        cudaStream_t st = h->stream;
+        long long *d_L = l.n_links.as<long long>();
+        AMIRA_TRY(run_scan(h, JunctionLoad{u.edge_internal.as<uint8_t>()}, JunctionStore{l.edge.as<int32_t>(), E, d_L}, nullptr, 1,
+                           E, E));
+        long long L = 0;
+        AMIRA_TRY(d2h(h, &L, d_L, sizeof(long long)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        if (L > 0)
+            LAUNCH(h, k_unitig_links, grid_for(L, 256), 256, l.edge.as<int32_t>(), L, h->edges.src.as<int32_t>(),
+                   h->edges.tgt.as<int32_t>(), h->edges.sd.as<int8_t>(), h->edges.td.as<int8_t>(), h->edges.cov.as<uint32_t>(),
+                   u.node_unitig.as<int32_t>(), u.node_orient.as<int8_t>(), l.from_unitig.as<int32_t>(), l.from_orient.as<int8_t>(),
+                   l.to_unitig.as<int32_t>(), l.to_orient.as<int8_t>(), l.cov.as<uint32_t>());
+        l.L = L;
+    }
+    l.version = h->graph_version;
+    l.generation = buffer_generation();
+    l.valid = true;
+    return AMIRA_OK;
+}
+
+// the reads as steps along the unitigs, cached under the same rule; reserved ahead for the same reason, with W as
+// the bound on the number of steps
+int read_path_table(amira_gmg *h) {
+    auto &p = h->paths;
+    if (p.valid && p.version == h->graph_version && p.generation == buffer_generation()) return AMIRA_OK;
+    p.valid = false;
+    const long long R = h->R, W = h->W, N = h->n_nodes;
+    // without a node every window is None, and without a window every read is short: all paths are empty
+    const bool steps = W > 0 && N > 0;
+    if (steps) {
+        const size_t w4 = sizeof(int32_t) * (size_t)W;
+        AMIRA_TRY(p.flags.reserve((size_t)W));
+        AMIRA_TRY(p.n_steps.reserve(sizeof(long long)));
+        AMIRA_TRY(p.path_off.reserve(sizeof(int64_t) * (size_t)(R + 1)));
+        AMIRA_TRY(p.unitig.reserve(w4));
+        AMIRA_TRY(p.orient.reserve((size_t)W));
+        AMIRA_TRY(p.pos.reserve(w4));
+        AMIRA_TRY(p.win.reserve(w4));
+        AMIRA_TRY(p.length.reserve(w4));
+        AMIRA_TRY(reserve_scan(h, W));
+    }
+    AMIRA_TRY(unitig_table(h));
+    p.T = 0;
+    p.on_device = steps;
+    if (steps) {
+        const auto &u = h->unitigs;
+        cudaStream_t st = h->stream;
+        const int32_t *win_node = h->win_node.as<int32_t>(), *win_read = h->win_read.as<int32_t>();
+        const int8_t *win_dir = h->win_dir.as<int8_t>();
+        uint8_t *flags = p.flags.as<uint8_t>();
+        long long *d_T = p.n_steps.as<long long>();
+        LAUNCH(h, k_read_step_flags, grid_for(W, 256), 256, win_node, win_dir, win_read, W, u.succ.as<int32_t>(), flags);
+        AMIRA_TRY(run_scan(h, StepLoad{flags},
+                           StepStore{flags, win_node, win_read, win_dir, h->win_off.as<int64_t>(), u.node_unitig.as<int32_t>(),
+                                     u.node_pos.as<int32_t>(), u.node_orient.as<int8_t>(), W, R, p.path_off.as<int64_t>(),
+                                     p.unitig.as<int32_t>(), p.pos.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+                                     p.orient.as<int8_t>(), d_T},
+                           nullptr, 1, W, W));
+        long long T = 0;
+        AMIRA_TRY(d2h(h, &T, d_T, sizeof(long long)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        if (T > 0) LAUNCH(h, k_read_step_lengths, grid_for(T, 256), 256, p.win.as<int32_t>(), T, p.length.as<int32_t>());
+        p.T = T;
+    }
+    p.version = h->graph_version;
+    p.generation = buffer_generation();
+    p.valid = true;
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_t *from_unitig, int8_t *from_orient,
+                           int32_t *to_unitig, int8_t *to_orient, uint32_t *cov) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("unitig_links: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    AMIRA_TRY(unitig_links_table(h));
+    const auto &l = h->links;
+    const int64_t L = l.L;
+    if (n_links) *n_links = L;
+    if (L == 0) return AMIRA_OK;
+    AMIRA_TRY(d2h(h, edge, l.edge.p, sizeof(int32_t) * L));
+    AMIRA_TRY(d2h(h, from_unitig, l.from_unitig.p, sizeof(int32_t) * L));
+    AMIRA_TRY(d2h(h, from_orient, l.from_orient.p, (size_t)L));
+    AMIRA_TRY(d2h(h, to_unitig, l.to_unitig.p, sizeof(int32_t) * L));
+    AMIRA_TRY(d2h(h, to_orient, l.to_orient.p, (size_t)L));
+    AMIRA_TRY(d2h(h, cov, l.cov.p, sizeof(uint32_t) * L));
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig, int8_t *orient, int32_t *pos,
+                                int32_t *win, int32_t *length) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("read_unitig_paths: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    AMIRA_TRY(read_path_table(h));
+    const auto &p = h->paths;
+    const int64_t R = h->R, T = p.T;
+    if (path_off) {
+        if (p.on_device) AMIRA_TRY(d2h(h, path_off, p.path_off.p, sizeof(int64_t) * (size_t)(R + 1)));
+        else std::fill(path_off, path_off + R + 1, (int64_t)0);
+    }
+    if (T > 0) {
+        AMIRA_TRY(d2h(h, unitig, p.unitig.p, sizeof(int32_t) * T));
+        AMIRA_TRY(d2h(h, orient, p.orient.p, (size_t)T));
+        AMIRA_TRY(d2h(h, pos, p.pos.p, sizeof(int32_t) * T));
+        AMIRA_TRY(d2h(h, win, p.win.p, sizeof(int32_t) * T));
+        AMIRA_TRY(d2h(h, length, p.length.p, sizeof(int32_t) * T));
+    }
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
     return AMIRA_OK;
 }

@@ -24,6 +24,8 @@
 //   segsort.cuh        segmented sorts (adjacency lists; read lists beyond one CTA's shared memory)
 //   scan.cuh           single-pass look-back scans with device-side element counts
 //   stats.cuh          the post-build scans of the callers
+//   unitigs.cuh        the compacted graph by list ranking; its junction edges as links between unitig ends, and
+//                      the reads as steps along unitigs (one scan over the windows)
 //   sharded.cuh        the multi-GPU exchange and merge
 #pragma once
 

@@ -26,6 +26,21 @@
 //  - edges: a directed edge of list a of node u joins consecutive nodes of one unitig iff succ(2u + a) exists.
 // The jump table of paths.cuh (S x L x 4 bytes) is not needed here: memory is 7 x S x 4 bytes for the ranking plus
 // O(N + E) for the results.  The cycle kernels of paths.cuh work on that table's levels and do not apply.
+//
+// The edges and the reads of the compacted graph, over the cached succ / node_unitig / node_pos / node_orient:
+//  - links: a scan over the directed edges flagged "edge_internal == 0" compacts the junction edges in edge order;
+//    one thread per link (k_unitig_links) then writes its unitig ends: from (node_unitig[u], sd * node_orient[u])
+//    to (node_unitig[v], td * node_orient[v]), and the edge's coverage.
+//  - read paths: a window on node n with direction d leaves n through the state 2n + (d < 0), as the edge the
+//    build made from it and the next window does.  A window continues the window before it when both are live
+//    (not None), in one read, and succ(state of the one before) == its state.  One thread per window
+//    (k_read_step_flags) flags "starts a step" (live, does not continue) and "ends a step" (live, the next window
+//    does not continue it); one scan over the W windows numbers the steps and, at a start, writes the step's
+//    unitig, orientation, position and window index, at an end the step's last window + 1; at each read's first
+//    window it writes path_off (also for the short reads before it, which have no windows).  A None window starts
+//    and ends nothing, so a step's length comes from its own end, not from the next step's start:
+//    k_read_step_lengths subtracts.  Window and step numbers are 64-bit; a window's index within its read and a
+//    step's length are 32-bit.
 #pragma once
 
 #include "stats.cuh"
@@ -177,6 +192,111 @@ __global__ void k_unitig_edges(const int32_t *__restrict__ succ, const int32_t *
     const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= E) return;
     internal[j] = succ[2 * (long long)e_src[j] + (e_sd[j] < 0 ? 1 : 0)] >= 0 ? 1 : 0;
+}
+
+// ---- links: the junction edges, in edge order --------------------------------------------------------------------
+struct JunctionLoad {
+    const uint8_t *internal;
+    __device__ __forceinline__ unsigned long long operator()(long long j) const { return internal[j] ? 0ull : 1ull; }
+};
+// ... -> link_edge[excl] = j for a junction; *n_links = L
+struct JunctionStore {
+    int32_t *link_edge;
+    long long E;
+    long long *n_links;
+    __device__ __forceinline__ void operator()(long long j, unsigned long long excl, unsigned long long junction) const {
+        if (j == E) *n_links = (long long)excl;
+        else if (junction) link_edge[excl] = (int32_t)j;
+    }
+};
+
+__global__ void k_unitig_links(const int32_t *__restrict__ link_edge, const long long L, const int32_t *__restrict__ e_src,
+                               const int32_t *__restrict__ e_tgt, const int8_t *__restrict__ e_sd, const int8_t *__restrict__ e_td,
+                               const uint32_t *__restrict__ e_cov, const int32_t *__restrict__ node_unitig,
+                               const int8_t *__restrict__ node_orient, int32_t *__restrict__ from_unitig,
+                               int8_t *__restrict__ from_orient, int32_t *__restrict__ to_unitig, int8_t *__restrict__ to_orient,
+                               uint32_t *__restrict__ cov) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= L) return;
+    const int32_t j = link_edge[t], u = e_src[j], v = e_tgt[j];
+    from_unitig[t] = node_unitig[u];
+    from_orient[t] = (int8_t)(e_sd[j] * node_orient[u]);
+    to_unitig[t] = node_unitig[v];
+    to_orient[t] = (int8_t)(e_td[j] * node_orient[v]);
+    cov[t] = e_cov[j];
+}
+
+// ---- read paths: maximal runs of windows that follow succ ---------------------------------------------------------
+constexpr uint8_t STEP_START = 1, STEP_END = 2;
+
+// the state a live window leaves its node through
+__device__ __forceinline__ int32_t window_state(const int32_t n, const int8_t d) { return 2 * n + (d < 0 ? 1 : 0); }
+
+__global__ void k_read_step_flags(const int32_t *__restrict__ win_node, const int8_t *__restrict__ win_dir,
+                                  const int32_t *__restrict__ win_read, const long long W, const int32_t *__restrict__ succ,
+                                  uint8_t *__restrict__ flags) {
+    const long long w = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= W) return;
+    const int32_t n = win_node[w];
+    if (n < 0) {
+        flags[w] = 0;
+        return;
+    }
+    const int32_t s = window_state(n, win_dir[w]), r = win_read[w];
+    bool in = false, out = false;  // w continues w - 1; w + 1 continues w
+    if (w > 0 && win_read[w - 1] == r) {
+        const int32_t p = win_node[w - 1];
+        in = p >= 0 && succ[window_state(p, win_dir[w - 1])] == s;
+    }
+    if (w + 1 < W && win_read[w + 1] == r) {
+        const int32_t q = win_node[w + 1];
+        out = q >= 0 && succ[s] == window_state(q, win_dir[w + 1]);
+    }
+    flags[w] = (in ? 0 : STEP_START) | (out ? 0 : STEP_END);
+}
+
+struct StepLoad {
+    const uint8_t *flags;
+    __device__ __forceinline__ unsigned long long operator()(long long w) const { return flags[w] & STEP_START; }
+};
+// ... -> path_off of the reads whose windows begin at w; at a start the step's fields (length = the end of the step
+// within its read, until k_read_step_lengths); *n_steps = T
+struct StepStore {
+    const uint8_t *flags;
+    const int32_t *win_node, *win_read;
+    const int8_t *win_dir;
+    const int64_t *win_off;
+    const int32_t *node_unitig, *node_pos;
+    const int8_t *node_orient;
+    long long W, R;
+    int64_t *path_off;
+    int32_t *unitig, *pos, *win, *length;
+    int8_t *orient;
+    long long *n_steps;
+    __device__ __forceinline__ void operator()(long long w, unsigned long long excl, unsigned long long start) const {
+        const long long r = w < W ? (long long)win_read[w] : R;
+        for (long long q = w > 0 ? (long long)win_read[w - 1] + 1 : 0; q <= r; ++q) path_off[q] = (int64_t)excl;
+        if (w == W) {
+            *n_steps = (long long)excl;
+            return;
+        }
+        const uint8_t f = flags[w];
+        if (!f) return;
+        const long long first = win_off[r];
+        if (start) {
+            const int32_t n = win_node[w];
+            unitig[excl] = node_unitig[n];
+            orient[excl] = (int8_t)((win_dir[w] < 0 ? -1 : 1) * node_orient[n]);
+            pos[excl] = node_pos[n];
+            win[excl] = (int32_t)(w - first);
+        }
+        if (f & STEP_END) length[excl + start - 1] = (int32_t)(w + 1 - first);
+    }
+};
+
+__global__ void k_read_step_lengths(const int32_t *__restrict__ win, const long long T, int32_t *__restrict__ length) {
+    const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t < T) length[t] -= win[t];
 }
 
 }  // namespace amira

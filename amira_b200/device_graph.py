@@ -14,6 +14,9 @@ from . import _lib
 # the arrays of amira_gmg_unitigs, in its argument order
 UNITIG_FIELDS = ("node_unitig", "node_pos", "node_orient", "unitig_off", "unitig_nodes", "circular", "cov_sum", "cov_min",
                  "cov_max", "edge_internal")
+# the arrays of amira_gmg_unitig_links and amira_gmg_read_unitig_paths, in their argument order
+LINK_FIELDS = ("edge", "from_unitig", "from_orient", "to_unitig", "to_orient", "cov")
+PATH_FIELDS = ("path_off", "unitig", "orient", "pos", "win", "length")
 
 
 def _ptr(a):
@@ -162,6 +165,29 @@ class DeviceGraph:
              "circular": np.empty(U, np.uint8), "cov_sum": np.empty(U, np.int64), "cov_min": np.empty(U, np.uint32),
              "cov_max": np.empty(U, np.uint32), "edge_internal": np.empty(m, np.uint8)}
         _lib.check(self._lib.amira_gmg_unitigs(self._h, None, *[_ptr(a[f]) for f in UNITIG_FIELDS]))
+        return a
+
+    def unitig_links(self) -> dict:
+        """the junction edges of the compacted graph (amira_gmg_unitig_links), in edge order: per link its edge index,
+        the unitig and orientation it leaves and enters (+1: in the unitig's listed order), and the edge's coverage"""
+        L = C.c_int64()
+        _lib.check(self._lib.amira_gmg_unitig_links(self._h, C.byref(L), *[None] * 6))
+        L = L.value
+        a = {"edge": np.empty(L, np.int32), "from_unitig": np.empty(L, np.int32), "from_orient": np.empty(L, np.int8),
+             "to_unitig": np.empty(L, np.int32), "to_orient": np.empty(L, np.int8), "cov": np.empty(L, np.uint32)}
+        _lib.check(self._lib.amira_gmg_unitig_links(self._h, None, *[_ptr(a[f]) for f in LINK_FIELDS]))
+        return a
+
+    def read_unitig_paths(self) -> dict:
+        """every read as steps along the unitigs (amira_gmg_read_unitig_paths): read r's steps are
+        path_off[r]:path_off[r + 1]; per step its unitig, orientation, position of its first window, that window's
+        index within the read, and its number of windows"""
+        off = np.zeros(self.R + 1, np.int64)
+        _lib.check(self._lib.amira_gmg_read_unitig_paths(self._h, _ptr(off), *[None] * 5))
+        T = int(off[-1])
+        a = {"path_off": off, "unitig": np.empty(T, np.int32), "orient": np.empty(T, np.int8), "pos": np.empty(T, np.int32),
+             "win": np.empty(T, np.int32), "length": np.empty(T, np.int32)}
+        _lib.check(self._lib.amira_gmg_read_unitig_paths(self._h, *[_ptr(a[f]) for f in PATH_FIELDS]))
         return a
 
     def filter_masks(self):

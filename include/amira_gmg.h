@@ -206,6 +206,37 @@ int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, in
                       int64_t *unitig_off, int32_t *unitig_nodes, uint8_t *circular, int64_t *cov_sum, uint32_t *cov_min,
                       uint32_t *cov_max, uint8_t *edge_internal);
 
+/* The edges and the reads of the compacted graph (no upstream counterpart), over the unitigs of amira_gmg_unitigs
+ * (node_unitig, node_pos, node_orient and succ as above; reused while cached, not ranked again).  A directed edge
+ * j = (u -> v, sd, td) leaves u through the state 2u + (sd < 0); a read window on node n with direction d leaves n
+ * through 2n + (d < 0) (the build makes the edge between two windows with the first one's direction as sd).
+ * An orientation of +1 means in the unitig's listed order.
+ *
+ * Links: one per junction edge (edge_internal == 0), in edge order, E - sum(edge_internal) of them:
+ *   edge = j, from_unitig = node_unitig[u], from_orient = sd * node_orient[u], to_unitig = node_unitig[v],
+ *   to_orient = td * node_orient[v], cov = the edge's coverage.
+ *   With from_orient = +1, u is the last node of its unitig, with -1 the first; likewise v at the entering end
+ *   (+1: first, -1: last).  No link touches a circular unitig.  Every link (a, oa) -> (b, ob) has its twin
+ *   (b, -ob) -> (a, -oa) from the reverse edge (a self edge may be its own twin).
+ *
+ * Read paths: per read, in read order, its steps.  A step is a maximal run of consecutive windows i..j of one read,
+ * all live (not None), each continuing the one before: succ(state(i')) == state(i' + 1).  Equivalently: one unitig,
+ * one orientation, and the position moves by one in the direction of travel (modulo the length of a circular
+ * unitig, which a read may go round more than once: a step may be longer than its unitig).  A None window belongs
+ * to no step and ends the current one.  Per step:
+ *   unitig, orient = d * node_orient[n] of its first window (constant along the step), pos = node_pos of the first
+ *   window's node, win = the first window's index within the read (as in _readNodes[read]), length = its windows.
+ *   path_off[R+1] delimits each read's steps (path_off[R] = the number of steps); short reads and reads whose
+ *   windows are all None have empty paths.
+ *
+ * Both calls: every pointer may be NULL.  Call with n_links only, or path_off only, to size the outputs, then again
+ * for the arrays: the results are kept on the device until the graph or a device buffer changes.  Leave the filter
+ * masks alone.  Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
+int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_t *from_unitig, int8_t *from_orient,
+                           int32_t *to_unitig, int8_t *to_orient, uint32_t *cov);
+int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig, int8_t *orient, int32_t *pos,
+                                int32_t *win, int32_t *length);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
