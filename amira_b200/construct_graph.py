@@ -747,17 +747,24 @@ class GeneMerGraph:
         `side` of the node holds one edge (-> v, td), v is another node, and v's entering list holds one edge"""
         S = 2 * len(a["node_cov"])
         tgt, td = np.asarray(a["edge_tgt"], np.int64), np.asarray(a["edge_td"], np.int64)
-        size = np.stack([np.diff(a["fw_off"]), np.diff(a["bw_off"])], 1).ravel()   # size[s]: edges in the list of s
-        one = np.full(S, -1, np.int64)                                              # the edge of a one-edge list
-        for side, f in enumerate(("fw", "bw")):
-            sel = np.flatnonzero(np.diff(a[f + "_off"]) == 1)
-            one[2 * sel + side] = np.asarray(a[f + "_edges"], np.int64)[np.asarray(a[f + "_off"], np.int64)[sel]]
+        size, one = GeneMerGraph._list_sizes(a)
         st = np.flatnonzero(one >= 0)
         v, leave = tgt[one[st]], (td[one[st]] != 1).astype(np.int64)
         ok = (v != st >> 1) & (size[2 * v + (1 - leave)] == 1)
         succ = np.full(S, -1, np.int64)
         succ[st[ok]] = 2 * v[ok] + leave[ok]
         return succ
+
+    @staticmethod
+    def _list_sizes(a) -> tuple:
+        """over index arrays: size[s], the number of edges in the list of state s, and one[s], the edge of a one-edge
+        list (-1 for the others)"""
+        size = np.stack([np.diff(a["fw_off"]), np.diff(a["bw_off"])], 1).ravel()
+        one = np.full(len(size), -1, np.int64)
+        for side, f in enumerate(("fw", "bw")):
+            sel = np.flatnonzero(np.diff(a[f + "_off"]) == 1)
+            one[2 * sel + side] = np.asarray(a[f + "_edges"], np.int64)[np.asarray(a[f + "_off"], np.int64)[sel]]
+        return size, one
 
     def compacted_links(self) -> dict:
         """the junction edges of the compacted graph (include/amira_gmg.h, amira_gmg_unitig_links), one link per edge
@@ -833,6 +840,142 @@ class GeneMerGraph:
                 "unitig": u["node_unitig"][n], "orient": (np.where(d[start] < 0, -1, 1) * u["node_orient"][n]).astype(np.int8),
                 "pos": u["node_pos"][n], "win": (start - woff[read]).astype(np.int32),
                 "length": (end - start + 1).astype(np.int32)}
+
+    def compacted_bubbles(self) -> dict:
+        """the simple bubbles of the compacted graph (include/amira_gmg.h, amira_gmg_bubbles) as numpy arrays: per
+        bubble its source and sink states (2 * node + side, node indices in `_nodes` order), its branches
+        branch_off[b]:branch_off[b + 1]; per branch its unitig (of compacted_unitigs()), orientation (+1: entered at the
+        unitig's first node) and branch_reads (the reads that run the whole branch).  A device graph is served by the
+        device and stays lazy."""
+        if self._on_device():
+            h = self._require_device_state()
+            if hasattr(h, "bubbles"):
+                return h.bubbles()
+            a = h.arrays()
+            return self._bubbles_over(a, a)
+        return self._bubbles_over(self._unitig_index_arrays(), self._read_index_arrays())
+
+    def _bubbles_over(self, a, w) -> dict:
+        """amira_gmg_bubbles over index arrays: the graph `a` (as _unitigs_over) and the windows `w` (as
+        _read_paths_over).  Every directed edge is tested as a branch entry at once; the entries of the lists, in state
+        order and list order, are grouped by (sigma, tau)"""
+        out = {"source": np.zeros(0, np.int32), "sink": np.zeros(0, np.int32), "branch_off": np.zeros(1, np.int64),
+               "branch_unitig": np.zeros(0, np.int32), "branch_orient": np.zeros(0, np.int8),
+               "branch_reads": np.zeros(0, np.uint32)}
+        N, E = len(a["node_cov"]), len(a["edge_src"])
+        if E == 0:
+            return out
+        u = self._unitigs_over(a)
+        src, tgt = np.asarray(a["edge_src"], np.int64), np.asarray(a["edge_tgt"], np.int64)
+        sd, td = np.asarray(a["edge_sd"], np.int64), np.asarray(a["edge_td"], np.int64)
+        fo, bo = np.asarray(a["fw_off"], np.int64), np.asarray(a["bw_off"], np.int64)
+        size, one = self._list_sizes(a)
+        nu, uoff = u["node_unitig"].astype(np.int64), u["unitig_off"]
+        unodes = u["unitig_nodes"].astype(np.int64)
+        listed = 2 * np.arange(N, dtype=np.int64) + (u["node_orient"] < 0)          # the state a node is listed through
+        sigma, c = 2 * src + (sd < 0), 2 * tgt + (td < 0)
+        b = nu[tgt]
+        along = c == listed[tgt]                                                    # the walk follows b's listed order
+        t = np.where(along, unodes[uoff[b + 1] - 1], unodes[uoff[b]])
+        e2 = one[listed[t] ^ ~along]
+        ok = (size[c ^ 1] == 1) & (u["circular"][b] == 0) & (e2 >= 0)
+        e2 = np.maximum(e2, 0)
+        y = tgt[e2]
+        tau = 2 * y + (td[e2] < 0)
+        ok &= (nu[src] != b) & (nu[y] != b) & (sigma < (tau ^ 1))
+        # the list entries in state order, then list order; the branch entries grouped by (sigma, tau)
+        state = np.concatenate([2 * np.repeat(np.arange(N, dtype=np.int64), np.diff(fo)),
+                                2 * np.repeat(np.arange(N, dtype=np.int64), np.diff(bo)) + 1])
+        ent = np.concatenate([np.asarray(a["fw_edges"], np.int64), np.asarray(a["bw_edges"], np.int64)])
+        ent = ent[np.argsort(state, kind="stable")]
+        ent = ent[ok[ent]]
+        _, first, inv, cnt = np.unique(sigma[ent] * (2 * N) + tau[ent], return_index=True, return_inverse=True,
+                                       return_counts=True)
+        inv = inv.ravel()
+        g = first[inv]                                                              # the entry of its group's first
+        sel = np.flatnonzero(cnt[inv] >= 2)
+        sel = sel[np.argsort(g[sel], kind="stable")]                                # bubble by bubble, in list order
+        starts = np.flatnonzero(g[sel] == sel)
+        br, heads = ent[sel], ent[sel[starts]]
+        bu = nu[tgt[br]]
+        p = self._read_paths_over(a, w)
+        ulen = np.diff(uoff)
+        branch_of = np.full(len(ulen), -1, np.int64)
+        branch_of[bu] = np.arange(len(bu))
+        hit = branch_of[p["unitig"]]
+        full = (hit >= 0) & (p["length"] == ulen[p["unitig"]])
+        out.update(source=sigma[heads].astype(np.int32), sink=tau[heads].astype(np.int32),
+                   branch_off=np.append(starts, len(sel)).astype(np.int64), branch_unitig=bu.astype(np.int32),
+                   branch_orient=np.where(unodes[uoff[bu]] == tgt[br], 1, -1).astype(np.int8),
+                   branch_reads=np.bincount(hit[full], minlength=len(bu)).astype(np.uint32))
+        return out
+
+    def pop_compacted_bubbles(self, sample_genesOfInterest={}):
+        """pop the simple bubbles of compacted_bubbles(): in each bubble keep the branch with the largest mean node
+        coverage (cov_sum / length, compared exactly; ties to the most branch_reads, then to the first branch) and
+        remove every other branch whole, unless one of its nodes holds a gene of sample_genesOfInterest.  Returns the
+        removed node hashes in bubble order, branch order and the unitig's listed order.  Reads through a removed
+        branch get None windows and are marked for correction, as with any removal.  A device graph is popped on the
+        device (amira_gmg_bubbles, amira_gmg_remove_nodes) and stays lazy; a graph edited on the host is popped over
+        its objects.  One call pops the bubbles present now: call again for those that popping makes."""
+        if self._on_device():
+            if self.get_total_number_of_nodes() == 0:
+                return []
+            h = self._require_device_state()
+            bub, u = self.compacted_bubbles(), self.compacted_unitigs()
+            (key,) = self._arrays("node_key")
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            amr = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(key), bool)
+            removed = self._bubble_pop_nodes(bub, u, amr)
+            if not len(removed):
+                return []
+            hashes = _keys.node_keys(key[removed].astype(np.int64), self._vocab)[0]
+            flags = np.zeros(len(key), np.uint8)
+            flags[removed] = 1
+            h.remove_nodes(flags)
+            self._device_ops = self._device_ops + (("remove_nodes", (flags,)),)
+            self._apply_device_removal(h)
+            return hashes
+        nodes = self._nodes
+        if not nodes:
+            return []
+        a = self._unitig_index_arrays()
+        bub, u = self._bubbles_over(a, self._read_index_arrays()), self._unitigs_over(a)
+        AMR_nodes = self.get_AMR_nodes(sample_genesOfInterest)
+        order = list(nodes)
+        removed = self._bubble_pop_nodes(bub, u, np.asarray([nh in AMR_nodes for nh in order], bool))
+        hashes = [order[i] for i in removed.tolist()]
+        for nh in hashes:
+            self.remove_node(nodes[nh])
+        return hashes
+
+    @staticmethod
+    def _bubble_pop_nodes(bub, u, amr) -> np.ndarray:
+        """the popping policy of pop_compacted_bubbles over index arrays: bub as compacted_bubbles, u as
+        compacted_unitigs, amr[n]: node n holds a gene of interest.  Returns the node indices to remove, in bubble
+        order, branch order and listed order."""
+        off = np.asarray(bub["branch_off"], np.int64)
+        d = np.diff(off)
+        if not len(d):
+            return np.zeros(0, np.int64)
+        bu = np.asarray(bub["branch_unitig"], np.int64)
+        uoff = np.asarray(u["unitig_off"], np.int64)
+        ln, cs = np.diff(uoff)[bu], np.asarray(u["cov_sum"], np.int64)[bu]
+        rd = np.asarray(bub["branch_reads"], np.int64)
+        # every ordered pair (i, j) of branches of one bubble; i beats j on the mean coverage cs / ln (cross-multiplied),
+        # then on the reads, then on the position.  The branch that beats all the others of its bubble is kept.
+        pb = np.repeat(np.arange(len(d)), d * d)
+        k = np.arange(len(pb)) - np.repeat(np.cumsum(d * d) - d * d, d * d)
+        i, j = off[pb] + k // d[pb], off[pb] + k % d[pb]
+        lhs, rhs = cs[i] * ln[j], cs[j] * ln[i]
+        beats = (lhs > rhs) | ((lhs == rhs) & ((rd[i] > rd[j]) | ((rd[i] == rd[j]) & (i < j))))
+        keep = np.bincount(i[beats], minlength=len(bu)) == np.repeat(d, d) - 1
+        gene = np.zeros(len(uoff) - 1, bool)
+        gene[np.asarray(u["node_unitig"], np.int64)[np.flatnonzero(amr)]] = True
+        go = bu[~keep & ~gene[bu]]
+        n = np.diff(uoff)[go]
+        idx = np.repeat(uoff[go] - np.cumsum(n) + n, n) + np.arange(int(n.sum()))
+        return np.asarray(u["unitig_nodes"], np.int64)[idx]
 
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
@@ -1237,7 +1380,8 @@ def bind_upstream(upstream_construct_graph):
                    "_walk", "_walks_over", "_device_walks", "_device_walk", "_short_path_nodes", "get_forward_path_from_node", "get_backward_path_from_node", "get_linear_path_for_node",
                    "remove_short_linear_paths", "compacted_unitigs", "_unitig_index_arrays", "_unitigs_over",
                    "_unitig_succ", "compacted_links", "read_unitig_paths", "_read_index_arrays", "_links_over",
-                   "_read_paths_over",
+                   "_read_paths_over", "_list_sizes", "compacted_bubbles", "_bubbles_over", "pop_compacted_bubbles",
+                   "_bubble_pop_nodes",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

@@ -10,6 +10,7 @@
 #include "stats.cuh"
 #include "paths.cuh"
 #include "unitigs.cuh"
+#include "bubbles.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -211,6 +212,14 @@ struct amira_gmg {
         bool valid = false;
         uint64_t version = 0, generation = 0;
     } paths;
+    // the simple bubbles of the compacted graph (bubbles.cuh), valid under the same rule
+    struct {
+        DevBuf edge_tau, ebr, ebub, ehead, counts, first, n_out;
+        DevBuf source, sink, branch_off, branch_unitig, branch_orient, branch_reads, unitig_branch;
+        int64_t B = 0, NB = 0;
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+    } bubbles;
 };
 
 namespace {
@@ -2400,6 +2409,111 @@ int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig
         AMIRA_TRY(d2h(h, win, p.win.p, sizeof(int32_t) * T));
         AMIRA_TRY(d2h(h, length, p.length.p, sizeof(int32_t) * T));
     }
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+namespace {
+// the simple bubbles, cached under the rule of unitig_table.  Every buffer and the scan's tile states are reserved
+// before read_path_table (and through it unitig_table) runs, for the reason given at unitig_links_table.  A bubble
+// has two branches or more and a branch is one edge of its list, so E bounds the branches and E / 2 the bubbles.
+int bubble_table(amira_gmg *h) {
+    auto &q = h->bubbles;
+    if (q.valid && q.version == h->graph_version && q.generation == buffer_generation()) return AMIRA_OK;
+    q.valid = false;
+    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
+    if (S >= (1ll << 31)) {
+        set_error("bubbles: %lld nodes, the states 2 * node + side must fit in 31 bits", N);
+        return AMIRA_E_ARG;
+    }
+    const bool any = E > 0;  // without an edge there is no branch
+    if (any) {
+        const size_t e4 = sizeof(int32_t) * (size_t)E;
+        AMIRA_TRY(q.edge_tau.reserve(e4));
+        AMIRA_TRY(q.ebr.reserve(e4));
+        AMIRA_TRY(q.ebub.reserve(e4));
+        AMIRA_TRY(q.ehead.reserve(e4));
+        AMIRA_TRY(q.counts.reserve(sizeof(unsigned long long) * (size_t)S));
+        AMIRA_TRY(q.first.reserve(sizeof(unsigned long long) * (size_t)S));
+        AMIRA_TRY(q.n_out.reserve(sizeof(unsigned long long)));
+        AMIRA_TRY(q.source.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.sink.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.branch_off.reserve(sizeof(int64_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.branch_unitig.reserve(e4));
+        AMIRA_TRY(q.branch_orient.reserve((size_t)E));
+        AMIRA_TRY(q.branch_reads.reserve(e4));
+        AMIRA_TRY(q.unitig_branch.reserve(sizeof(int32_t) * (size_t)N));
+        AMIRA_TRY(reserve_scan(h, S));
+    }
+    AMIRA_TRY(read_path_table(h));
+    q.B = q.NB = 0;
+    if (any) {
+        const auto &u = h->unitigs;
+        const auto &p = h->paths;
+        cudaStream_t st = h->stream;
+        const int64_t *adj_off = h->adj_off.as<int64_t>();
+        const uint32_t *adj_edges = h->adj_edges.as<uint32_t>();
+        const int32_t *e_src = h->edges.src.as<int32_t>(), *e_tgt = h->edges.tgt.as<int32_t>();
+        const int8_t *e_sd = h->edges.sd.as<int8_t>();
+        int32_t *edge_tau = q.edge_tau.as<int32_t>(), *ebr = q.ebr.as<int32_t>(), *ebub = q.ebub.as<int32_t>();
+        unsigned long long *d_n = q.n_out.as<unsigned long long>();
+        LAUNCH(h, k_bubble_branches, grid_for(E, 256), 256, adj_off, adj_edges, N, e_src, e_tgt, e_sd, h->edges.td.as<int8_t>(), E,
+               u.node_unitig.as<int32_t>(), u.node_orient.as<int8_t>(), u.off.as<int64_t>(), u.nodes.as<int32_t>(),
+               u.circular.as<uint8_t>(), edge_tau);
+        LAUNCH(h, k_bubble_group, grid_for(S, 256), 256, adj_off, adj_edges, N, edge_tau, ebr, ebub, q.ehead.as<int32_t>(),
+               q.counts.as<unsigned long long>());
+        AMIRA_TRY(run_scan(h, BubbleCountLoad{q.counts.as<unsigned long long>()},
+                           BubbleCountStore{q.first.as<unsigned long long>(), S, d_n, q.branch_off.as<int64_t>()}, nullptr, 1, S,
+                           S));
+        unsigned long long packed = 0;
+        AMIRA_TRY(d2h(h, &packed, d_n, sizeof(packed)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        q.B = (int64_t)(packed >> 32);
+        q.NB = (int64_t)(packed & 0xffffffffull);
+        if (q.NB > 0) {
+            int32_t *unitig_branch = q.unitig_branch.as<int32_t>();
+            uint32_t *branch_reads = q.branch_reads.as<uint32_t>();
+            AMIRA_CUDA(cudaMemsetAsync(unitig_branch, 0xff, sizeof(int32_t) * (size_t)u.U, st));
+            AMIRA_CUDA(cudaMemsetAsync(branch_reads, 0, sizeof(uint32_t) * (size_t)q.NB, st));
+            h->lib_launches += 2;
+            LAUNCH(h, k_bubble_fill, grid_for(E, 256), 256, ebr, ebub, edge_tau, E, e_src, e_tgt, e_sd,
+                   q.first.as<unsigned long long>(), u.node_unitig.as<int32_t>(), u.off.as<int64_t>(), u.nodes.as<int32_t>(),
+                   q.source.as<int32_t>(), q.sink.as<int32_t>(), q.branch_off.as<int64_t>(), q.branch_unitig.as<int32_t>(),
+                   q.branch_orient.as<int8_t>(), unitig_branch);
+            if (p.T > 0)
+                LAUNCH(h, k_bubble_reads, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.length.as<int32_t>(), (long long)p.T,
+                       unitig_branch, u.off.as<int64_t>(), branch_reads);
+        }
+    }
+    q.version = h->graph_version;
+    q.generation = buffer_generation();
+    q.valid = true;
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int32_t *source, int32_t *sink,
+                      int64_t *branch_off, int32_t *branch_unitig, int8_t *branch_orient, uint32_t *branch_reads) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("bubbles: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    AMIRA_TRY(bubble_table(h));
+    const auto &q = h->bubbles;
+    const int64_t B = q.B, NB = q.NB;
+    if (n_bubbles) *n_bubbles = B;
+    if (n_branches) *n_branches = NB;
+    if (B == 0) {
+        if (branch_off) branch_off[0] = 0;
+        return AMIRA_OK;
+    }
+    AMIRA_TRY(d2h(h, source, q.source.p, sizeof(int32_t) * B));
+    AMIRA_TRY(d2h(h, sink, q.sink.p, sizeof(int32_t) * B));
+    AMIRA_TRY(d2h(h, branch_off, q.branch_off.p, sizeof(int64_t) * (B + 1)));
+    AMIRA_TRY(d2h(h, branch_unitig, q.branch_unitig.p, sizeof(int32_t) * NB));
+    AMIRA_TRY(d2h(h, branch_orient, q.branch_orient.p, (size_t)NB));
+    AMIRA_TRY(d2h(h, branch_reads, q.branch_reads.p, sizeof(uint32_t) * NB));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
     return AMIRA_OK;
 }

@@ -26,6 +26,7 @@
 //   stats.cuh          the post-build scans of the callers
 //   unitigs.cuh        the compacted graph by list ranking; its junction edges as links between unitig ends, and
 //                      the reads as steps along unitigs (one scan over the windows)
+//   bubbles.cuh        the simple bubbles of the compacted graph (branches per edge, grouping per list by warp)
 //   sharded.cuh        the multi-GPU exchange and merge
 #pragma once
 

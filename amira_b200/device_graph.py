@@ -17,6 +17,8 @@ UNITIG_FIELDS = ("node_unitig", "node_pos", "node_orient", "unitig_off", "unitig
 # the arrays of amira_gmg_unitig_links and amira_gmg_read_unitig_paths, in their argument order
 LINK_FIELDS = ("edge", "from_unitig", "from_orient", "to_unitig", "to_orient", "cov")
 PATH_FIELDS = ("path_off", "unitig", "orient", "pos", "win", "length")
+# the arrays of amira_gmg_bubbles, in its argument order
+BUBBLE_FIELDS = ("source", "sink", "branch_off", "branch_unitig", "branch_orient", "branch_reads")
 
 
 def _ptr(a):
@@ -188,6 +190,19 @@ class DeviceGraph:
         a = {"path_off": off, "unitig": np.empty(T, np.int32), "orient": np.empty(T, np.int8), "pos": np.empty(T, np.int32),
              "win": np.empty(T, np.int32), "length": np.empty(T, np.int32)}
         _lib.check(self._lib.amira_gmg_read_unitig_paths(self._h, *[_ptr(a[f]) for f in PATH_FIELDS]))
+        return a
+
+    def bubbles(self) -> dict:
+        """the simple bubbles of the compacted graph (amira_gmg_bubbles): per bubble its source and sink states, its
+        branches branch_off[b]:branch_off[b + 1]; per branch its unitig, orientation (+1: entered at the unitig's first
+        node) and the number of reads that run the whole branch"""
+        B, NB = C.c_int64(), C.c_int64()
+        _lib.check(self._lib.amira_gmg_bubbles(self._h, C.byref(B), C.byref(NB), *[None] * 6))
+        B, NB = B.value, NB.value
+        a = {"source": np.empty(B, np.int32), "sink": np.empty(B, np.int32), "branch_off": np.zeros(B + 1, np.int64),
+             "branch_unitig": np.empty(NB, np.int32), "branch_orient": np.empty(NB, np.int8),
+             "branch_reads": np.empty(NB, np.uint32)}
+        _lib.check(self._lib.amira_gmg_bubbles(self._h, None, None, *[_ptr(a[f]) for f in BUBBLE_FIELDS]))
         return a
 
     def filter_masks(self):

@@ -237,6 +237,46 @@ int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_
 int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig, int8_t *orient, int32_t *pos,
                                 int32_t *win, int32_t *length);
 
+/* The simple bubbles of the compacted graph (no upstream counterpart): two or more unitigs that leave one junction
+ * and rejoin the graph at another, as one wrong gene call in one read makes (a run of about k wrong gene-mers beside
+ * the true path).  Over the unitigs of amira_gmg_unitigs and the read paths of amira_gmg_read_unitig_paths (reused
+ * while cached, not ranked again).
+ *
+ * A state is s = 2 * node + side; list(s) is that node's forward (side 0) or backward (side 1) list.  A directed
+ * edge e = (u -> v, sd, td) lies in list(2u + (sd < 0)); it continues through cont(e) = 2v + (td < 0), the state a
+ * walk leaves v through, and v's entering list for e is list(cont(e) ^ 1).
+ *
+ * Branch: an edge e in list(sigma), x = sigma >> 1, with target h, enters the branch b = the unitig of h when
+ *   1. list(cont(e) ^ 1) holds exactly one edge;
+ *   2. b is not circular;
+ *   3. the walk through b from h in the direction of cont(e) reaches b's other end node t, t is left through s_t,
+ *      and list(s_t) holds exactly one edge e', with target y;
+ *   4. neither x nor y is a node of b.
+ * (With 1. and x not in b, h has no predecessor in b: it is b's end on the entering side, and the branch is all of b.)
+ * The branch runs from sigma to tau = cont(e').  Its orientation is +1 when h is the first node of b in listed
+ * order (always for a one-node b), -1 otherwise.
+ * Bubble: the branches of list(sigma) grouped by tau; a group of two or more with sigma < (tau ^ 1) is one bubble.
+ * With sigma > (tau ^ 1) the same bubble is reported from tau ^ 1 (its mirror); with sigma == (tau ^ 1) the branches
+ * only turn back into the end they left, and there is no bubble.  So every bubble is reported once, and a unitig is
+ * a branch of at most one bubble.
+ *
+ * Outputs, in an order that does not depend on thread timing: bubbles by sigma ascending, then by the list(sigma)
+ * position of their first branch; branches in list(sigma) order (upstream's forward / backward list order).
+ *   per bubble: source = sigma, sink = tau (states); branch_off[B+1] delimits its branches;
+ *   per branch: branch_unitig, branch_orient, branch_reads = the read steps (amira_gmg_read_unitig_paths) on the
+ *   unitig whose length equals its node count: the reads that run the whole branch, in either direction.
+ * Lengths and coverages are those of amira_gmg_unitigs (unitig_off, cov_sum, ...), not copied here.
+ *
+ * Out of scope: bubbles whose branches are not single unitigs (nested or overlapping errors, superbubbles), and
+ * branches without a node (an edge joining the two junction nodes directly, as a deletion makes at k = 1).
+ *
+ * Every pointer may be NULL.  Call with n_bubbles / n_branches only to size the outputs, then again for the arrays:
+ * the result is kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.  Not
+ * available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31.  Grouping a list of d edges takes
+ * O(d^2 / 32) warp steps. */
+int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int32_t *source, int32_t *sink,
+                      int64_t *branch_off, int32_t *branch_unitig, int8_t *branch_orient, uint32_t *branch_reads);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
