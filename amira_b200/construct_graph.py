@@ -950,10 +950,10 @@ class GeneMerGraph:
         return hashes
 
     @staticmethod
-    def _bubble_pop_nodes(bub, u, amr) -> np.ndarray:
+    def _bubble_winners(bub, u, amr) -> np.ndarray:
         """the popping policy of pop_compacted_bubbles over index arrays: bub as compacted_bubbles, u as
-        compacted_unitigs, amr[n]: node n holds a gene of interest.  Returns the node indices to remove, in bubble
-        order, branch order and listed order."""
+        compacted_unitigs, amr[n]: node n holds a gene of interest.  Returns per branch the branch of its bubble that
+        is kept, or -1 for the branches that stay (the kept ones, and those with a node holding a gene of interest)."""
         off = np.asarray(bub["branch_off"], np.int64)
         d = np.diff(off)
         if not len(d):
@@ -972,10 +972,134 @@ class GeneMerGraph:
         keep = np.bincount(i[beats], minlength=len(bu)) == np.repeat(d, d) - 1
         gene = np.zeros(len(uoff) - 1, bool)
         gene[np.asarray(u["node_unitig"], np.int64)[np.flatnonzero(amr)]] = True
-        go = bu[~keep & ~gene[bu]]
+        return np.where(~keep & ~gene[bu], np.repeat(np.flatnonzero(keep), d), -1)
+
+    @staticmethod
+    def _bubble_pop_nodes(bub, u, amr) -> np.ndarray:
+        """the node indices pop_compacted_bubbles removes (the branches _bubble_winners replaces), in bubble order,
+        branch order and listed order"""
+        go = np.asarray(bub["branch_unitig"], np.int64)[GeneMerGraph._bubble_winners(bub, u, amr) >= 0]
+        uoff = np.asarray(u["unitig_off"], np.int64)
         n = np.diff(uoff)[go]
         idx = np.repeat(uoff[go] - np.cumsum(n) + n, n) + np.arange(int(n.sum()))
         return np.asarray(u["unitig_nodes"], np.int64)[idx]
+
+    def correct_compacted_bubbles(self, sample_genesOfInterest={}):
+        """the reads rewritten through the bubbles pop_compacted_bubbles would pop (the same kept branch, the same
+        branches spared for a gene of sample_genesOfInterest), as a new encode.EncodedReads to rebuild from
+        (include/amira_gmg.h, amira_gmg_correct_bubble_reads): a read that runs a replaced branch whole, between the
+        bubble's two junction nodes, spells the kept branch there instead; every other call is unchanged.  It shares
+        the vocabulary and read ids of this graph's reads, its dicts are shallow copies with only the changed reads
+        decoded, and it carries `changed` (per read) and `branch_rewritten` (per branch of compacted_bubbles()).  The
+        graph and its reads are left as they are.  A device graph is corrected on the device, which writes the new CSR
+        that a rebuild from the result reads without uploading it again."""
+        src = self._source_encoded()
+        if self._on_device():
+            h = self._require_device_state()
+            bub, u = self.compacted_bubbles(), self.compacted_unitigs()
+            (key,) = self._arrays("node_key")
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            amr = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(key), bool)
+            rw = self._bubble_winners(bub, u, amr)
+            if hasattr(h, "correct_bubble_reads"):
+                return src.corrected(h.correct_bubble_reads(rw, on_device=True), self._device)
+            a = h.arrays()
+            return src.corrected(self._corrected_reads_over(u, self._read_paths_over(a, a), bub, a, key, rw, src))
+        a, w = self._unitig_index_arrays(), self._read_index_arrays()
+        u, bub = self._unitigs_over(a), self._bubbles_over(a, w)
+        amr_nodes = self.get_AMR_nodes(sample_genesOfInterest)
+        rank = {n: i + 1 for i, n in enumerate(src.vocab.names)}
+        key = np.asarray([[g.get_strand() * rank[g.get_name()] for g in n.get_canonical_geneMer()] for n in self._nodes.values()],
+                         np.int64).reshape(len(self._nodes), int(self._kmerSize))
+        rw = self._bubble_winners(bub, u, np.asarray([nh in amr_nodes for nh in self._nodes], bool))
+        return src.corrected(self._corrected_reads_over(u, self._read_paths_over(a, w), bub, w, key, rw, src))
+
+    def _source_encoded(self):
+        """this graph's reads as an encode.EncodedReads: the one it was built from, or the reads encoded as the build
+        encoded them"""
+        if self._encoded is not None:
+            return self._encoded
+        e = encode.EncodedReads.__new__(encode.EncodedReads)
+        e.vocab, e.ids, e.off, e.pos_start, e.pos_end = self._encode()
+        e.reads, e.positions, e.read_ids, e._device = self._reads, self._genePositions or None, list(self._reads), None
+        return e
+
+    @staticmethod
+    def _corrected_reads_over(u, p, bub, w, key, replace_with, src) -> dict:
+        """amira_gmg_correct_bubble_reads over index arrays: u as compacted_unitigs, p as read_unitig_paths, bub as
+        compacted_bubbles, the windows w (win_off, win_node with -1 for None, win_dir), node keys key[N, k], and the
+        encoded reads src (ids, off, pos_start, pos_end).  Every step is tested at once; the edits (which never
+        overlap) set per call its number of output calls, whose prefix sums place every call"""
+        rw = np.asarray(replace_with, np.int64)
+        ids, off = np.asarray(src.ids, np.int32), np.asarray(src.off, np.int64)
+        ps, pe = src.pos_start, src.pos_end
+        R, NB = len(off) - 1, len(rw)
+        if NB:
+            boff = np.asarray(bub["branch_off"], np.int64)
+            of = np.repeat(np.arange(len(boff) - 1), np.diff(boff))
+            bad = (rw < -1) | (rw >= NB) | (rw == np.arange(NB))
+            if (bad | ((rw >= 0) & (of[np.clip(rw, 0, NB - 1)] != of))).any():
+                raise ValueError("correct_bubble_reads: replace_with must hold -1 or another branch of the same bubble")
+        t = np.zeros(0, np.int64)
+        if NB and len(p["unitig"]):
+            uoff = np.asarray(u["unitig_off"], np.int64)
+            ulen = np.diff(uoff)
+            bu = np.asarray(bub["branch_unitig"], np.int64)
+            branch_of = np.full(len(ulen), -1, np.int64)
+            branch_of[bu] = np.arange(NB)
+            sun = np.asarray(p["unitig"], np.int64)
+            g, m = branch_of[sun], ulen[sun]
+            read = np.repeat(np.arange(R, dtype=np.int64), np.diff(p["path_off"]))
+            woff = np.asarray(w["win_off"], np.int64)
+            win = np.asarray(p["win"], np.int64)
+            t = np.flatnonzero((g >= 0) & (rw[np.maximum(g, 0)] >= 0) & (p["length"] == m) & (win >= 1)
+                               & (win + m < np.diff(woff)[read]))
+            node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
+            before = woff[read[t]] + win[t] - 1
+            after = before + m[t] + 1
+            sp, sn = 2 * node[before] + (d[before] < 0), 2 * node[after] + (d[after] < 0)
+            q = of[g[t]]
+            sigma, tau = np.asarray(bub["source"], np.int64)[q], np.asarray(bub["sink"], np.int64)[q]
+            fwd = (sp == sigma) & (sn == tau)
+            ok = (node[before] >= 0) & (node[after] >= 0) & (fwd | ((sp == tau ^ 1) & (sn == sigma ^ 1)))
+            t, fwd = t[ok], fwd[ok]
+        changed = np.zeros(R, np.uint8)
+        rewritten = np.zeros(NB, np.uint32)
+        count = np.ones(len(ids), np.int64)
+        touched = np.zeros(len(ids), bool)
+        if len(t):
+            r, gt, mt = read[t], g[t], m[t]
+            keep = rw[gt]
+            kb = bu[keep]
+            m2 = ulen[kb]
+            c0 = off[r] + win[t]
+            rep = np.repeat(c0 - np.cumsum(mt) + mt, mt) + np.arange(int(mt.sum()))
+            touched[rep] = True
+            count[rep] = 0
+            count[c0] = m2
+            changed[r] = 1
+            rewritten = np.bincount(gt, minlength=NB).astype(np.uint32)
+        idx = np.concatenate([[0], np.cumsum(count)]).astype(np.int64)
+        total = int(idx[-1])
+        out = {"ids": np.empty(total, np.int32), "off": idx[off],
+               "pos_start": None if ps is None else np.empty(total, np.int32),
+               "pos_end": None if pe is None else np.empty(total, np.int32), "changed": changed, "branch_rewritten": rewritten}
+        keep_calls = np.flatnonzero(~touched)
+        out["ids"][idx[keep_calls]] = ids[keep_calls]
+        for f, x in (("pos_start", ps), ("pos_end", pe)):
+            if x is not None:
+                out[f][idx[keep_calls]] = x[keep_calls]
+        if len(t):
+            e = np.repeat(np.arange(len(t)), m2)
+            j = np.arange(int(m2.sum())) - np.repeat(np.cumsum(m2) - m2, m2)
+            walk = np.where(fwd, 1, -1)[e] * np.asarray(bub["branch_orient"], np.int64)[keep[e]]
+            n = np.asarray(u["unitig_nodes"], np.int64)[np.where(walk > 0, uoff[kb[e]] + j, uoff[kb[e]] + m2[e] - 1 - j)]
+            key = np.asarray(key, np.int64)
+            out["ids"][idx[c0[e]] + j] = np.where(walk * np.asarray(u["node_orient"], np.int64)[n] > 0, key[n, 0], -key[n, -1])
+            for f, x in (("pos_start", ps), ("pos_end", pe)):
+                if x is not None:
+                    out[f][idx[c0[e]] + j] = x[c0[e] + np.minimum(j, mt[e] - 1)]
+        return out
 
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
@@ -1381,7 +1505,8 @@ def bind_upstream(upstream_construct_graph):
                    "remove_short_linear_paths", "compacted_unitigs", "_unitig_index_arrays", "_unitigs_over",
                    "_unitig_succ", "compacted_links", "read_unitig_paths", "_read_index_arrays", "_links_over",
                    "_read_paths_over", "_list_sizes", "compacted_bubbles", "_bubbles_over", "pop_compacted_bubbles",
-                   "_bubble_pop_nodes",
+                   "_bubble_pop_nodes", "_bubble_winners", "correct_compacted_bubbles", "_source_encoded",
+                   "_corrected_reads_over",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

@@ -11,6 +11,7 @@
 #include "paths.cuh"
 #include "unitigs.cuh"
 #include "bubbles.cuh"
+#include "correct.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -220,6 +221,10 @@ struct amira_gmg {
         bool valid = false;
         uint64_t version = 0, generation = 0;
     } bubbles;
+    // the scratch of amira_gmg_correct_bubble_reads (correct.cuh): recomputed by every call, nothing cached
+    struct {
+        DevBuf replace, cnt, idx, step_new, changed, rewritten, n_out;
+    } correct;
 };
 
 namespace {
@@ -2515,6 +2520,148 @@ int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int
     AMIRA_TRY(d2h(h, branch_orient, q.branch_orient.p, (size_t)NB));
     AMIRA_TRY(d2h(h, branch_reads, q.branch_reads.p, sizeof(uint32_t) * NB));
     AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+namespace {
+// a device allocation for the length of one call (the staging of host outputs).  It is not a handle buffer, so it
+// leaves the buffer generation, and with it the cached unitigs, read paths and bubbles, alone.
+struct CallBuf {
+    void *p = nullptr;
+    cudaStream_t st = nullptr;
+    ~CallBuf() {
+        if (p) cudaFreeAsync(p, st);
+    }
+};
+}  // namespace
+
+int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
+                                   int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
+                                   int out_on_device) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("correct_bubble_reads: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    auto &c = h->correct;
+    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
+    // every buffer before the bubbles: a reservation that grows bumps the buffer generation and would drop them
+    if (R > 0) {
+        const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
+        AMIRA_TRY(c.replace.reserve(e4));
+        AMIRA_TRY(c.rewritten.reserve(e4));
+        AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
+        AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
+        AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
+        AMIRA_TRY(c.changed.reserve((size_t)R));
+        AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
+        AMIRA_TRY(reserve_scan(h, G));
+    }
+    AMIRA_TRY(bubble_table(h));
+    const auto &q = h->bubbles;
+    const int64_t B = q.B, NB = q.NB;
+    cudaStream_t st = h->stream;
+    if (NB > 0) {
+        if (!replace_with) {
+            set_error("correct_bubble_reads: no replace_with for %lld branches", (long long)NB);
+            return AMIRA_E_ARG;
+        }
+        std::vector<int64_t> boff((size_t)B + 1);
+        AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        for (int64_t b = 0; b < B; ++b)
+            for (int64_t g = boff[b]; g < boff[b + 1]; ++g) {
+                const int64_t x = replace_with[g];
+                if (x != -1 && (x < boff[b] || x >= boff[b + 1] || x == g)) {
+                    set_error("correct_bubble_reads: replace_with[%lld] = %lld is not -1 or another branch of bubble %lld",
+                              (long long)g, (long long)x, (long long)b);
+                    return AMIRA_E_ARG;
+                }
+            }
+    }
+    if (R == 0) {  // no read, no node, no bubble
+        if (n_calls) *n_calls = 0;
+        if (read_off) {
+            if (out_on_device) AMIRA_CUDA(cudaMemsetAsync(read_off, 0, sizeof(int64_t), st));
+            else read_off[0] = 0;
+        }
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        return AMIRA_OK;
+    }
+    const auto &u = h->unitigs;
+    const auto &p = h->paths;
+    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
+    int64_t *idx = c.idx.as<int64_t>();
+    int32_t *step_new = c.step_new.as<int32_t>(), *replace = c.replace.as<int32_t>();
+    uint8_t *d_changed = c.changed.as<uint8_t>();
+    AMIRA_CUDA(cudaMemsetAsync(d_changed, 0, (size_t)R, st));
+    AMIRA_CUDA(cudaMemsetAsync(idx, 0, sizeof(int64_t), st));  // idx[0] when there is no call
+    h->lib_launches += 2;
+    if (G > 0) {
+        AMIRA_CUDA(cudaMemsetAsync(cnt, 0, sizeof(uint32_t) * (size_t)G, st));
+        h->lib_launches++;
+    }
+    if (NB > 0) {
+        AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
+        AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
+        h->lib_launches += 2;
+        if (p.T > 0)
+            LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
+                   h->win_dir.as<int8_t>(), h->off, u.off.as<int64_t>(), q.unitig_branch.as<int32_t>(), q.branch_off.as<int64_t>(),
+                   (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(), q.branch_unitig.as<int32_t>(), replace, cnt,
+                   step_new, d_changed, rewritten);
+    }
+    long long total = 0;
+    if (G > 0) {
+        unsigned long long *d_n = c.n_out.as<unsigned long long>();
+        AMIRA_TRY(run_scan(h, CorrectCountLoad{cnt, step_new}, CorrectIndexStore{idx, G, d_n}, nullptr, 1, G, G));
+        AMIRA_TRY(d2h(h, &total, d_n, sizeof(total)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+    }
+    if (n_calls) *n_calls = total;
+
+    // the outputs: the caller's device arrays, or one staging allocation copied to the caller's host arrays
+    int32_t *o_ps = h->has_pos ? pos_start : nullptr, *o_pe = h->has_pos ? pos_end : nullptr, *o_ids = ids;
+    int64_t *o_off = read_off;
+    CallBuf stage;
+    if (!out_on_device && (read_off || ids || o_ps || o_pe)) {
+        const size_t b_off = read_off ? sizeof(int64_t) * (size_t)(R + 1) : 0, b_call = sizeof(int32_t) * (size_t)total;
+        const size_t bytes = b_off + b_call * ((ids ? 1 : 0) + (o_ps ? 1 : 0) + (o_pe ? 1 : 0));
+        stage.st = st;
+        AMIRA_CUDA(cudaMallocAsync(&stage.p, std::max<size_t>(bytes, 1), st));
+        char *at = static_cast<char *>(stage.p);
+        o_off = read_off ? reinterpret_cast<int64_t *>(at) : nullptr;
+        at += b_off;
+        for (int32_t **o : {&o_ids, &o_ps, &o_pe})
+            if (*o) {
+                *o = reinterpret_cast<int32_t *>(at);
+                at += b_call;
+            }
+    }
+    if (o_off) LAUNCH(h, k_correct_offsets, grid_for(R + 1, 256), 256, h->off, R, idx, o_off);
+    if (G > 0 && (o_ids || o_ps || o_pe))
+        LAUNCH(h, k_correct_fill, grid_for(G, 256), 256, cnt, idx, G, h->ids, h->ps, h->pe, step_new, p.unitig.as<int32_t>(),
+               p.length.as<int32_t>(), q.unitig_branch.as<int32_t>(), replace, q.branch_unitig.as<int32_t>(),
+               q.branch_orient.as<int8_t>(), u.off.as<int64_t>(), u.nodes.as<int32_t>(), u.node_orient.as<int8_t>(),
+               h->nodes.key.as<int32_t>(), h->k, o_ids, o_ps, o_pe);
+    const cudaMemcpyKind kind = out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+    struct {
+        void *dst;
+        const void *src;
+        size_t bytes;
+    } jobs[] = {{changed, d_changed, (size_t)R},
+                {branch_rewritten, rewritten, sizeof(uint32_t) * (size_t)NB},
+                {out_on_device ? nullptr : read_off, o_off, sizeof(int64_t) * (size_t)(R + 1)},
+                {out_on_device ? nullptr : ids, o_ids, sizeof(int32_t) * (size_t)total},
+                {out_on_device ? nullptr : o_ps ? pos_start : nullptr, o_ps, sizeof(int32_t) * (size_t)total},
+                {out_on_device ? nullptr : o_pe ? pos_end : nullptr, o_pe, sizeof(int32_t) * (size_t)total}};
+    for (const auto &j : jobs)
+        if (j.dst && j.bytes) {
+            AMIRA_CUDA(cudaMemcpyAsync(j.dst, j.src, j.bytes, kind, st));
+            h->lib_launches++;
+        }
+    AMIRA_CUDA(cudaStreamSynchronize(st));
     return AMIRA_OK;
 }
 

@@ -27,6 +27,8 @@
 //   unitigs.cuh        the compacted graph by list ranking; its junction edges as links between unitig ends, and
 //                      the reads as steps along unitigs (one scan over the windows)
 //   bubbles.cuh        the simple bubbles of the compacted graph (branches per edge, grouping per list by warp)
+//   correct.cuh        the reads through the bubbles rewritten along a kept branch (edits per step, one scan
+//                      over the calls)
 //   sharded.cuh        the multi-GPU exchange and merge
 #pragma once
 

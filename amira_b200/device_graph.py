@@ -205,6 +205,43 @@ class DeviceGraph:
         _lib.check(self._lib.amira_gmg_bubbles(self._h, None, None, *[_ptr(a[f]) for f in BUBBLE_FIELDS]))
         return a
 
+    def correct_bubble_reads(self, replace_with, on_device: bool = False) -> dict:
+        """the reads through the bubbles of bubbles() rewritten along a kept branch (amira_gmg_correct_bubble_reads):
+        replace_with[g] = -1 leaves branch g's reads alone, otherwise it is the branch of the same bubble whose genes
+        replace g's calls.  Returns the corrected CSR ids / off / pos_start / pos_end (None without positions) as numpy
+        arrays, or as torch tensors on this handle's device written by the device when on_device; and as numpy arrays
+        changed (per read: 1 when rewritten) and branch_rewritten (per branch: its reads rewritten)"""
+        NB = C.c_int64()
+        _lib.check(self._lib.amira_gmg_bubbles(self._h, None, C.byref(NB), *[None] * 6))
+        rw = np.asarray(replace_with, np.int64).ravel()
+        if len(rw) != NB.value or (len(rw) and (rw.min() < -1 or rw.max() >= NB.value)):
+            raise ValueError("correct_bubble_reads: replace_with must hold -1 or a branch index for each of %d branches"
+                             % NB.value)
+        rw = np.ascontiguousarray(rw, np.int32)
+        n = C.c_int64()
+        _lib.check(self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), C.byref(n), *[None] * 6, 0))
+        G, R = n.value, self.R
+        if on_device:
+            import torch
+            dev = torch.device("cuda", self.device)
+            new = lambda size, dt: torch.empty(size, dtype=getattr(torch, dt), device=dev)
+        else:
+            new = lambda size, dt: np.empty(size, dt)
+        a = {"ids": new(G, "int32"), "off": new(R + 1, "int64"),
+             "pos_start": new(G, "int32") if self.has_pos else None, "pos_end": new(G, "int32") if self.has_pos else None,
+             "changed": np.empty(R, np.uint8), "branch_rewritten": np.empty(NB.value, np.uint32)}
+        if on_device:
+            changed, rewritten = new(R, "uint8"), new(NB.value, "int32")     # per branch counts < 2^31, as uint32
+        else:
+            changed, rewritten = a["changed"], a["branch_rewritten"]
+        _lib.check(self._lib.amira_gmg_correct_bubble_reads(
+            self._h, _ptr(rw), None, _ptr(a["off"]), _ptr(a["ids"]), _ptr(a["pos_start"]), _ptr(a["pos_end"]),
+            _ptr(changed), _ptr(rewritten), int(bool(on_device))))
+        if on_device:
+            a["changed"][:] = changed.cpu().numpy()
+            a["branch_rewritten"][:] = rewritten.cpu().numpy().view(np.uint32)
+        return a
+
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""
         a, b = C.c_int64(), C.c_int64()

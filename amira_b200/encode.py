@@ -188,6 +188,32 @@ class EncodedReads:
                               for i, r in enumerate(self.read_ids)}
         return self
 
+    def corrected(self, out: dict, device: int | None = None):
+        """a new EncodedReads over the corrected CSR `out` (GeneMerGraph.correct_compacted_bubbles: ids, off,
+        pos_start, pos_end, changed per read, branch_rewritten per branch) of these reads.  It shares the vocabulary
+        and the read ids; its read / position dicts are shallow copies of these with only the changed reads decoded.
+        With torch tensors in `out` (written on GPU `device`) they become its device CSR, and the host CSR is one copy
+        of them.  This object is left as it is."""
+        new = EncodedReads.__new__(EncodedReads)
+        new.vocab, new.read_ids, new._device = self.vocab, self.read_ids, None
+        csr = [out[f] for f in ("ids", "off", "pos_start", "pos_end")]
+        if not isinstance(csr[0], np.ndarray):
+            new._device = (device, *csr)
+            csr = [None if x is None else x.cpu().numpy() for x in csr]
+        new.ids, new.off, new.pos_start, new.pos_end = csr
+        new.changed = np.asarray(out["changed"], np.uint8)
+        new.branch_rewritten = np.asarray(out["branch_rewritten"], np.uint32)
+        new.reads = dict(self.reads)
+        new.positions = dict(self.positions) if self.positions is not None else None
+        names = self.vocab.names
+        for i in np.flatnonzero(new.changed).tolist():
+            lo, hi = int(new.off[i]), int(new.off[i + 1])
+            rid = self.read_ids[i]
+            new.reads[rid] = [("+" if g > 0 else "-") + names[abs(g) - 1] for g in new.ids[lo:hi].tolist()]
+            if new.positions is not None and new.positions.get(rid):
+                new.positions[rid] = list(zip(new.pos_start[lo:hi].tolist(), new.pos_end[lo:hi].tolist()))
+        return new
+
     def update(self, changed: dict, positions: dict | None = None):
         """Re-encode only the reads in `changed` ({read_id: new gene calls}; the rebuild-after-correction loop of
         iterative_bubble_popping, amira/graph_utils.py:127-181, rewrites a few reads per iteration): the other reads

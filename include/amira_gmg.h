@@ -277,6 +277,40 @@ int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig
 int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int32_t *source, int32_t *sink,
                       int64_t *branch_off, int32_t *branch_unitig, int8_t *branch_orient, uint32_t *branch_reads);
 
+/* The reads through the simple bubbles of amira_gmg_bubbles rewritten along a kept branch (no upstream counterpart,
+ * like the popping policy): the correction step of a "pop, correct, rebuild" cleaning loop, computed from the build's
+ * input CSR (kept or borrowed by amira_gmg_build), the cached read paths and bubbles, and the node keys.
+ *
+ * replace_with[n_branches] (host): per branch g of amira_gmg_bubbles, -1 leaves g's reads alone; otherwise it is
+ * another branch of the same bubble, whose genes replace g's calls.
+ * Edit: a read step (amira_gmg_read_unitig_paths) on branch g = unitig b of m nodes in bubble (sigma, tau), with
+ * replace_with[g] >= 0, length m, the windows win - 1 and win + m present in its read and live, and their states
+ * (2 * node + (dir < 0)) either (sigma, tau) -- the read runs sigma -> b -> tau -- or (tau ^ 1, sigma ^ 1) -- the
+ * mirror.  (The state check matters: a filter with min_edge_cov > 1 can delete the edge between two live windows.)
+ * Rewrite: window i of a read starts at its call i.  An edit replaces the m calls [win, win + m) by m' calls, m' the
+ * kept branch's node count; call j is the first gene of the j-th kept node in the direction of travel: the kept
+ * branch is walked in listed order when (+1 for sigma -> tau, -1 for the mirror) * its branch_orient is +1, a node
+ * n's direction along the walk is node_orient[n] in listed order and -node_orient[n] against it, and its first gene
+ * is key[n * k] in direction +1, -key[n * k + k - 1] in direction -1.  The read then spells source, kept branch,
+ * sink.  Edits never overlap, and two edits of one read have an untouched call between them: every node of a branch
+ * has one-edge lists on both sides, a junction node a list of two edges or more.
+ * Positions (without positions pos_start / pos_end are ignored): untouched calls keep theirs; new call j < m takes
+ * those of replaced call j, new call j >= m those of the last replaced call.
+ * Everything else is unchanged: steps that do not qualify (a full-length step without both flanks, as a read that
+ * starts or ends on the branch, counts in branch_reads but is not rewritten), short reads, reads without an edit.
+ *
+ * Outputs: n_calls = the new call count; read_off[R + 1], ids / pos_start / pos_end [n_calls] the corrected CSR in
+ * read order (read_off[r] = the output index of the input's call read_off_in[r]); changed[R] = 1 for a read with an
+ * edit; branch_rewritten[n_branches] = the edits per branch.  Call with n_calls only to size the outputs, then again
+ * for the arrays; every output may be NULL.  out_on_device != 0: the array outputs are device pointers on the handle's
+ * device; either way the call returns with the work complete, and the library keeps no pointer.  Leaves the graph,
+ * the cached unitigs / paths / bubbles and the filter masks as they were.  AMIRA_E_ARG when replace_with points out
+ * of range, into another bubble or at the branch itself; AMIRA_E_STATE on a sharded handle.  Out of scope: reads that
+ * end inside a branch, nested bubbles and superbubbles. */
+int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off,
+                                   int32_t *ids, int32_t *pos_start, int32_t *pos_end, uint8_t *changed,
+                                   uint32_t *branch_rewritten, int out_on_device);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
