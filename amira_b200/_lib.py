@@ -23,7 +23,7 @@ EXPORTED = (
     "amira_gmg_read_length_coverages", "amira_gmg_node_coverage_stats", "amira_gmg_junk_read_mask", "amira_gmg_nodes_containing",
     "amira_gmg_remove_nodes", "amira_gmg_remove_nodes_without_reads_of", "amira_gmg_linear_steps", "amira_gmg_linear_walks",
     "amira_gmg_unitigs", "amira_gmg_unitig_links", "amira_gmg_read_unitig_paths", "amira_gmg_bubbles",
-    "amira_gmg_correct_bubble_reads",
+    "amira_gmg_correct_bubble_reads", "amira_gmg_bubble_policy", "amira_gmg_input_calls",
 )
 
 _lib = None
@@ -80,6 +80,8 @@ def load():
     lib.amira_gmg_read_unitig_paths.argtypes = [vp] * 7
     lib.amira_gmg_bubbles.argtypes = [vp] * 9
     lib.amira_gmg_correct_bubble_reads.argtypes = [vp] * 9 + [C.c_int]
+    lib.amira_gmg_bubble_policy.argtypes = [vp, vp, i32, vp, vp]
+    lib.amira_gmg_input_calls.argtypes = [vp, vp, i64, i64]
     lib.amira_gmg_debug_layout.argtypes = [vp, C.c_int]
     lib.amira_gmg_debug_segsort.argtypes = [vp, vp, vp, i64, vp, C.POINTER(i64), C.c_int, i64]
     lib.amira_gmg_atomic_peak.argtypes = [vp, i64, i64] + [C.POINTER(C.c_double)] * 3

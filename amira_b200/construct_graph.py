@@ -52,6 +52,19 @@ def _handle(device: int) -> DeviceGraph:
     return h
 
 
+def _host(x) -> np.ndarray:
+    """a numpy array, or a device tensor copied to one"""
+    return x if isinstance(x, np.ndarray) else x.cpu().numpy()
+
+
+def _union(a, b):
+    """a | b for per-read flags, on b's device when b is a device tensor"""
+    if isinstance(a, np.ndarray) and not isinstance(b, np.ndarray):
+        import torch
+        a = torch.from_numpy(a).to(b.device)
+    return a | b
+
+
 class _Classes:
     """the element classes a graph is materialised with (ours, or upstream's when bound)"""
     Gene, GeneMer, Node, Edge = Gene, GeneMer, Node, Edge
@@ -148,15 +161,19 @@ class GeneMerGraph:
 
     def _build_on_device(self):
         vocab, ids, off, ps, pe = self._encode()
-        self._vocab = vocab
-        self._csr_fingerprint = (len(ids), int(off[-1]) if len(off) else 0, zlib.crc32(np.ascontiguousarray(ids).tobytes()))
-        self._read_len = np.diff(off)
         h = _handle(self._device)
         h.owner = None
         if self._encoded is not None and hasattr(h, "build_resident"):
             h.build_resident(self._encoded, int(self._kmerSize), self._device)
         else:
             h.build(ids, off, int(self._kmerSize), ps, pe)
+        self._adopt_build(h, vocab, ids, off)
+
+    def _adopt_build(self, h, vocab, ids, off):
+        """make the build the handle holds, of this graph's reads (vocab, host ids / off), this graph's lazy device copy"""
+        self._vocab = vocab
+        self._csr_fingerprint = (len(ids), int(off[-1]) if len(off) else 0, zlib.crc32(np.ascontiguousarray(ids).tobytes()))
+        self._read_len = np.diff(off)
         h.owner = weakref.ref(self)
         self._read_ids = list(self._reads)
         self._device_synced = True
@@ -993,18 +1010,28 @@ class GeneMerGraph:
         decoded, and it carries `changed` (per read) and `branch_rewritten` (per branch of compacted_bubbles()).  The
         graph and its reads are left as they are.  A device graph is corrected on the device, which writes the new CSR
         that a rebuild from the result reads without uploading it again."""
+        return self._source_encoded().corrected(self._bubble_correction(sample_genesOfInterest)[0], self._device)
+
+    def _bubble_correction(self, sample_genesOfInterest, flags_on_device=False) -> tuple:
+        """correct_compacted_bubbles before it becomes an EncodedReads: (the outputs of DeviceGraph.correct_bubble_reads,
+        the bubble count, the branches replaced).  A device graph whose handle has the policy is corrected on the handle
+        alone (_handle_correction)."""
         src = self._source_encoded()
         if self._on_device():
             h = self._require_device_state()
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            if hasattr(h, "bubble_policy"):
+                return self._handle_correction(h, ranks, flags_on_device)
             bub, u = self.compacted_bubbles(), self.compacted_unitigs()
             (key,) = self._arrays("node_key")
-            ranks = self._gene_ranks(list(sample_genesOfInterest))
             amr = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(key), bool)
             rw = self._bubble_winners(bub, u, amr)
             if hasattr(h, "correct_bubble_reads"):
-                return src.corrected(h.correct_bubble_reads(rw, on_device=True), self._device)
-            a = h.arrays()
-            return src.corrected(self._corrected_reads_over(u, self._read_paths_over(a, a), bub, a, key, rw, src))
+                out = h.correct_bubble_reads(rw, on_device=True)
+            else:
+                a = h.arrays()
+                out = self._corrected_reads_over(u, self._read_paths_over(a, a), bub, a, key, rw, src)
+            return out, len(bub["source"]), int((rw >= 0).sum())
         a, w = self._unitig_index_arrays(), self._read_index_arrays()
         u, bub = self._unitigs_over(a), self._bubbles_over(a, w)
         amr_nodes = self.get_AMR_nodes(sample_genesOfInterest)
@@ -1012,7 +1039,84 @@ class GeneMerGraph:
         key = np.asarray([[g.get_strand() * rank[g.get_name()] for g in n.get_canonical_geneMer()] for n in self._nodes.values()],
                          np.int64).reshape(len(self._nodes), int(self._kmerSize))
         rw = self._bubble_winners(bub, u, np.asarray([nh in amr_nodes for nh in self._nodes], bool))
-        return src.corrected(self._corrected_reads_over(u, self._read_paths_over(a, w), bub, w, key, rw, src))
+        return (self._corrected_reads_over(u, self._read_paths_over(a, w), bub, w, key, rw, src), len(bub["source"]),
+                int((rw >= 0).sum()))
+
+    @staticmethod
+    def _handle_correction(h, ranks, flags_on_device) -> tuple:
+        """one correction of the graph the handle holds, with the device's popping policy: the corrected CSR written on
+        the device, the bubble count, the branches replaced"""
+        n_replaced = h.bubble_policy(ranks)
+        out = h.correct_bubble_reads(None, on_device=True, flags_on_device=flags_on_device)
+        return out, h.bubble_counts()[0], n_replaced
+
+    def correct_bubbles_until_stable(self, max_rounds=30, sample_genesOfInterest={}, filter_graph=None):
+        """rounds of correct_compacted_bubbles and a rebuild from the corrected reads, until a round rewrites no read
+        step or max_rounds rounds have run -> (graph, reads).  It gives exactly what this loop gives:
+
+            cur, e = self, reads of self
+            for _ in range(max_rounds):
+                e2 = cur.correct_compacted_bubbles(sample_genesOfInterest)
+                if not e2.branch_rewritten.any(): break
+                e = e2; cur = GeneMerGraph(e, k); filter_graph and cur.filter_graph(*filter_graph)
+            return cur, e
+
+        Round 1 corrects this graph as it is (filtered, trimmed or edited on the host); every later round corrects the
+        rebuild of the previous round's reads, filtered first when filter_graph = (minNodeCoverage, minEdgeCoverage).
+        `graph` is lazy and owns the device handle, or is this graph when round 1 rewrites nothing.  `reads` is an
+        encode.EncodedReads: `changed` is the union over the rounds, `branch_rewritten` that of the last round that
+        rewrote a step, and `rounds` holds per round run (the last one included) its bubbles, branches, branches
+        replaced, steps rewritten, reads rewritten and the call count after it.  This graph and its reads are left as
+        they were; a device graph rebuilds its device copy when next asked for it.
+
+        Rounds after the first run on the device handle alone: the policy, the correction and the rebuild stay on the
+        GPU and only counts come back; the corrected reads are copied to the host and decoded once, at the end."""
+        src = self._source_encoded()
+        k = int(self._kmerSize)
+        filt = None if filter_graph is None else (max(int(filter_graph[0]), 0), max(int(filter_graph[1]), 0))
+        rounds, out, last, changed, filtered, h = [], None, None, None, False, None
+        for r in range(max_rounds):
+            if r == 0:
+                x, n_bubbles, n_replaced = self._bubble_correction(sample_genesOfInterest, flags_on_device=True)
+            else:
+                x, n_bubbles, n_replaced = self._handle_correction(h, ranks, True)
+            steps = int(x["branch_rewritten"].sum())
+            rounds.append({"bubbles": n_bubbles, "branches": len(x["branch_rewritten"]), "replaced": n_replaced,
+                           "steps": steps, "reads": int(x["changed"].sum()), "calls": len(x["ids"])})
+            last = x
+            if steps == 0:
+                break
+            out = x                      # the previous CSR is dropped only now, after this round's correction
+            changed = x["changed"] if changed is None else _union(changed, x["changed"])
+            if h is None:
+                h, ranks = _handle(self._device), self._gene_ranks(list(sample_genesOfInterest))
+            h.owner = None               # the graph that held the handle rebuilds on demand
+            if isinstance(x["ids"], np.ndarray):
+                h.build(x["ids"], x["off"], k, x["pos_start"], x["pos_end"])
+            else:                        # the correction's device CSR, whose call count is known exactly
+                h.build(x["ids"], x["off"], k, x["pos_start"], x["pos_end"], on_device=True, n_calls=len(x["ids"]))
+            filtered = bool(filt) and h.sizes_early()["nodes"] > 0
+            if filtered:
+                h.filter_graph(*filt)
+        if out is None:
+            R = len(src.read_ids)
+            reads = src.corrected({"ids": src.ids, "off": src.off, "pos_start": src.pos_start, "pos_end": src.pos_end,
+                                   "changed": np.zeros(R, np.uint8),
+                                   "branch_rewritten": _host(last["branch_rewritten"]) if last else np.zeros(0, np.uint32)})
+            reads.rounds = rounds
+            return self, reads
+        reads = src.corrected({**out, "changed": _host(changed), "branch_rewritten": _host(out["branch_rewritten"])},
+                              self._device)
+        reads.rounds = rounds
+        g = type(self)({}, self._kmerSize, device=self._device)
+        g._encoded, g._reads, g._genePositions = reads, reads.reads, reads.positions
+        g._adopt_build(h, reads.vocab, reads.ids, reads.off)
+        if filter_graph is not None:
+            g.set_minNodeCoverage(filter_graph[0])
+            g.set_minEdgeCoverage(filter_graph[1])
+            if filtered:
+                g._device_ops = (("filter_graph", filt),)
+        return g, reads
 
     def _source_encoded(self):
         """this graph's reads as an encode.EncodedReads: the one it was built from, or the reads encoded as the build
@@ -1506,7 +1610,8 @@ def bind_upstream(upstream_construct_graph):
                    "_unitig_succ", "compacted_links", "read_unitig_paths", "_read_index_arrays", "_links_over",
                    "_read_paths_over", "_list_sizes", "compacted_bubbles", "_bubbles_over", "pop_compacted_bubbles",
                    "_bubble_pop_nodes", "_bubble_winners", "correct_compacted_bubbles", "_source_encoded",
-                   "_corrected_reads_over",
+                   "_corrected_reads_over", "_adopt_build", "_bubble_correction", "_handle_correction",
+                   "correct_bubbles_until_stable",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

@@ -28,6 +28,11 @@
 //    as long as the unitig.
 // Ordering comes from the list positions alone, never from thread timing: bubbles by sigma, then by the list
 // position of their first branch; branches by list position.
+//
+// The popping policy (amira_gmg_bubble_policy) over the cached bubbles and unitigs:
+//  - k_bubble_spare: one thread per node flagged as holding a gene of interest marks the branch of its unitig spared.
+//  - k_bubble_policy: one warp per bubble finds the kept branch (largest mean node coverage, compared exactly; then
+//    most branch_reads; then lowest index) and writes replace_with for every branch of the bubble.
 #pragma once
 
 #include "unitigs.cuh"
@@ -205,6 +210,73 @@ __global__ void k_bubble_reads(const int32_t *__restrict__ step_unitig, const in
     if (t >= T) return;
     const int32_t b = step_unitig[t], g = unitig_branch[b];
     if (g >= 0 && (int64_t)step_length[t] == unitig_off[b + 1] - unitig_off[b]) atomicAdd(&branch_reads[g], 1u);
+}
+
+// ---- the popping policy (amira_gmg_bubble_policy) ----------------------------------------------------------------
+
+// one thread per node: a node flagged by k_nodes_containing spares the branch its unitig is (plain stores of 1)
+__global__ void k_bubble_spare(const uint8_t *__restrict__ flags, const long long N, const int32_t *__restrict__ node_unitig,
+                               const int32_t *__restrict__ unitig_branch, uint8_t *__restrict__ spared) {
+    const long long n = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (n >= N || !flags[n]) return;
+    const int32_t g = unitig_branch[node_unitig[n]];
+    if (g >= 0) spared[g] = 1;
+}
+
+// a branch's rank key: mean node coverage cs / ln, then reads, then (lower first) its index
+struct BranchRank {
+    unsigned long long cs, ln;
+    uint32_t rd;
+    int32_t g;  // -1: no branch
+};
+
+// a beats b.  The means are compared as cs_a * ln_b against cs_b * ln_a, exactly, in 128 bits: cs is a sum of 32-bit
+// coverages over up to 2^30 nodes (< 2^62) and ln < 2^31, so the products need up to 93 bits.
+__device__ __forceinline__ bool branch_beats(const BranchRank &a, const BranchRank &b) {
+    if (b.g < 0) return a.g >= 0;
+    if (a.g < 0) return false;
+    const unsigned long long lh = __umul64hi(a.cs, b.ln), rh = __umul64hi(b.cs, a.ln);
+    if (lh != rh) return lh > rh;
+    const unsigned long long ll = a.cs * b.ln, rl = b.cs * a.ln;
+    if (ll != rl) return ll > rl;
+    if (a.rd != b.rd) return a.rd > b.rd;
+    return a.g < b.g;
+}
+
+// one warp per bubble, strided over its branches (a bubble may have any number): each lane keeps the best of its
+// branches, a butterfly of shuffles leaves the bubble's winner in every lane, then every branch that is not the winner
+// and not spared gets replace[g] = winner, others -1.  The replaced branches are counted with a ballot per stride and
+// one atomic per warp.
+__global__ void k_bubble_policy(const int64_t *__restrict__ branch_off, const long long B, const int32_t *__restrict__ branch_unitig,
+                                const uint32_t *__restrict__ branch_reads, const int64_t *__restrict__ unitig_off,
+                                const unsigned long long *__restrict__ cov_sum, const uint8_t *__restrict__ spared,
+                                int32_t *__restrict__ replace, unsigned long long *__restrict__ n_replaced) {
+    const long long q = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (q >= B) return;  // whole warps: B is per warp
+    const long long lo = branch_off[q], hi = branch_off[q + 1];
+    BranchRank best{0, 0, 0, -1};
+    for (long long g = lo + lane; g < hi; g += 32) {
+        const int32_t b = branch_unitig[g];
+        const BranchRank x{cov_sum[b], (unsigned long long)(unitig_off[b + 1] - unitig_off[b]), branch_reads[g], (int32_t)g};
+        if (branch_beats(x, best)) best = x;
+    }
+    for (int d = 16; d > 0; d >>= 1) {
+        BranchRank o;
+        o.cs = __shfl_xor_sync(0xffffffffu, best.cs, d);
+        o.ln = __shfl_xor_sync(0xffffffffu, best.ln, d);
+        o.rd = __shfl_xor_sync(0xffffffffu, best.rd, d);
+        o.g = __shfl_xor_sync(0xffffffffu, best.g, d);
+        if (branch_beats(o, best)) best = o;
+    }
+    unsigned int count = 0;
+    for (long long base = lo; base < hi; base += 32) {
+        const long long g = base + lane;
+        const bool rep = g < hi && g != best.g && !spared[g];
+        if (g < hi) replace[g] = rep ? best.g : -1;
+        count += __popc(__ballot_sync(0xffffffffu, rep));
+    }
+    if (lane == 0 && count) atomicAdd(n_replaced, (unsigned long long)count);
 }
 
 }  // namespace amira

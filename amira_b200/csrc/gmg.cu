@@ -101,6 +101,10 @@ struct amira_gmg {
     // array is passed again (the per-read kernel verifies it on the device: ST_STALE)
     const int64_t *cache_off = nullptr;
     int64_t cache_R = -1, cache_G = 0;
+    // the call count the caller gave for the next build from a device CSR (amira_gmg_input_calls), used by that build
+    // only: an entry that outlived its array could name an address the allocator has since handed to another CSR
+    const int64_t *hint_off = nullptr;
+    int64_t hint_R = -1, hint_G = 0;
 
     // per read / per tile
     DevBuf win_off, is_short, to_correct, tile_r0;
@@ -221,9 +225,12 @@ struct amira_gmg {
         bool valid = false;
         uint64_t version = 0, generation = 0;
     } bubbles;
-    // the scratch of amira_gmg_correct_bubble_reads (correct.cuh): recomputed by every call, nothing cached
+    // the scratch of amira_gmg_correct_bubble_reads (correct.cuh), recomputed by every call, and the replace_with of
+    // the last amira_gmg_bubble_policy, valid for the bubble cache (version, generation) it was computed on
     struct {
-        DevBuf replace, cnt, idx, step_new, changed, rewritten, n_out;
+        DevBuf replace, spared, cnt, idx, step_new, changed, rewritten, n_out;
+        bool policy = false;
+        uint64_t policy_version = 0, policy_generation = 0;
     } correct;
 };
 
@@ -1562,6 +1569,8 @@ int amira_gmg_kernel_launches(const amira_gmg *h, int64_t *n) {
 int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read_off, int64_t R, int32_t k,
                     const int32_t *pos_start, const int32_t *pos_end, int input_on_device) {
     AMIRA_TRY(check_handle(h));
+    const int64_t *hint_off = h->hint_off, hint_R = h->hint_R, hint_G = h->hint_G;
+    h->hint_off = nullptr;  // for this build only
     // a previous build nobody looked at: keep what it learned (table sizes, id width) if it has finished
     if (h->pending && h->pending_is_build && h->world == 1 && cudaEventQuery(h->ev_done) == cudaSuccess) finish(h, false);
     cudaGetLastError();
@@ -1589,7 +1598,12 @@ int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read
     h->input_on_device = input_on_device != 0;
     if (arg_status == AMIRA_OK && R > 0) {
         if (input_on_device) {
-            if (read_off == h->cache_off && R == h->cache_R) {
+            if (read_off == hint_off && R == hint_R) {
+                G = hint_G;  // the caller's count, verified on the device like a cached one
+                h->cache_off = read_off;
+                h->cache_R = R;
+                h->cache_G = G;
+            } else if (read_off == h->cache_off && R == h->cache_R) {
                 G = h->cache_G;  // verified on the device by the per-read pass (ST_STALE)
             } else {
                 AMIRA_CUDA(cudaMemcpyAsync(&G, read_off + R, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
@@ -1719,6 +1733,18 @@ int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read
     h->last_status = rc;
     h->built = (rc == AMIRA_OK);
     return rc;
+}
+
+int amira_gmg_input_calls(amira_gmg *h, const int64_t *read_off, int64_t R, int64_t n_calls) {
+    AMIRA_TRY(check_handle(h));
+    if (!read_off || R <= 0 || n_calls < 0 || n_calls >= MAX_CALLS) {
+        set_error("input_calls: bad arguments (R = %lld, n_calls = %lld)", (long long)R, (long long)n_calls);
+        return AMIRA_E_ARG;
+    }
+    h->hint_off = read_off;
+    h->hint_R = R;
+    h->hint_G = n_calls;
+    return AMIRA_OK;
 }
 
 int amira_gmg_sync(amira_gmg *h) {
@@ -2535,6 +2561,70 @@ struct CallBuf {
 };
 }  // namespace
 
+namespace {
+// the buffers of amira_gmg_bubble_policy and amira_gmg_correct_bubble_reads, reserved by both before the bubbles: a
+// reservation that grows bumps the buffer generation and would drop them.  Reserving the correction's buffers in the
+// policy too lets a correction that follows the policy find the bubble cache the policy was computed on.
+int reserve_correct(amira_gmg *h) {
+    auto &c = h->correct;
+    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
+    if (R == 0) return AMIRA_OK;
+    const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
+    AMIRA_TRY(c.replace.reserve(e4));
+    AMIRA_TRY(c.spared.reserve((size_t)std::max<long long>(E, 1)));
+    AMIRA_TRY(c.rewritten.reserve(e4));
+    AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
+    AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
+    AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
+    AMIRA_TRY(c.changed.reserve((size_t)R));
+    AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
+    return reserve_scan(h, G);
+}
+}  // namespace
+
+int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_replaced, int32_t *replace_with) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("bubble_policy: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    if (n_ranks < 0 || (n_ranks > 0 && !spare_ranks)) {
+        set_error("bubble_policy: bad gene ranks (n = %d)", n_ranks);
+        return AMIRA_E_ARG;
+    }
+    auto &c = h->correct;
+    c.policy = false;
+    // every reservation before the bubbles, the gene flags' (scratch_off, comp_max) included
+    AMIRA_TRY(reserve_correct(h));
+    if (n_ranks > 0) AMIRA_TRY(flag_nodes_containing(h, spare_ranks, n_ranks));
+    AMIRA_TRY(bubble_table(h));
+    const auto &q = h->bubbles;
+    const int64_t B = q.B, NB = q.NB, N = h->n_nodes;
+    cudaStream_t st = h->stream;
+    unsigned long long total = 0;
+    if (NB > 0) {
+        uint8_t *spared = c.spared.as<uint8_t>();
+        unsigned long long *d_n = c.n_out.as<unsigned long long>();
+        AMIRA_CUDA(cudaMemsetAsync(spared, 0, (size_t)NB, st));
+        AMIRA_CUDA(cudaMemsetAsync(d_n, 0, sizeof(unsigned long long), st));
+        h->lib_launches += 2;
+        if (n_ranks > 0)
+            LAUNCH(h, k_bubble_spare, grid_for(N, 256), 256, h->scratch_off.as<uint8_t>(), (long long)N,
+                   h->unitigs.node_unitig.as<int32_t>(), q.unitig_branch.as<int32_t>(), spared);
+        LAUNCH(h, k_bubble_policy, grid_for(B * 32, 256), 256, q.branch_off.as<int64_t>(), (long long)B,
+               q.branch_unitig.as<int32_t>(), q.branch_reads.as<uint32_t>(), h->unitigs.off.as<int64_t>(),
+               h->unitigs.cov_sum.as<unsigned long long>(), spared, c.replace.as<int32_t>(), d_n);
+        AMIRA_TRY(d2h(h, &total, d_n, sizeof(total)));
+        AMIRA_TRY(d2h(h, replace_with, c.replace.p, sizeof(int32_t) * (size_t)NB));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+    }
+    if (n_replaced) *n_replaced = (int64_t)total;
+    c.policy = true;
+    c.policy_version = q.version;
+    c.policy_generation = q.generation;
+    return AMIRA_OK;
+}
+
 int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                                    int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
                                    int out_on_device) {
@@ -2544,28 +2634,20 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
         return AMIRA_E_STATE;
     }
     auto &c = h->correct;
-    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
-    // every buffer before the bubbles: a reservation that grows bumps the buffer generation and would drop them
-    if (R > 0) {
-        const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
-        AMIRA_TRY(c.replace.reserve(e4));
-        AMIRA_TRY(c.rewritten.reserve(e4));
-        AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
-        AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
-        AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
-        AMIRA_TRY(c.changed.reserve((size_t)R));
-        AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
-        AMIRA_TRY(reserve_scan(h, G));
-    }
+    const long long R = h->R, G = R > 0 ? h->G : 0;
+    AMIRA_TRY(reserve_correct(h));
     AMIRA_TRY(bubble_table(h));
     const auto &q = h->bubbles;
     const int64_t B = q.B, NB = q.NB;
     cudaStream_t st = h->stream;
-    if (NB > 0) {
-        if (!replace_with) {
-            set_error("correct_bubble_reads: no replace_with for %lld branches", (long long)NB);
-            return AMIRA_E_ARG;
-        }
+    // NULL: the replace_with of the last policy, which the device holds, valid by construction
+    const bool held = NB > 0 && !replace_with;
+    if (held && !(c.policy && c.policy_version == q.version && c.policy_generation == q.generation)) {
+        set_error("correct_bubble_reads: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles",
+                  (long long)NB);
+        return AMIRA_E_STATE;
+    }
+    if (NB > 0 && !held) {
         std::vector<int64_t> boff((size_t)B + 1);
         AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
         AMIRA_CUDA(cudaStreamSynchronize(st));
@@ -2603,8 +2685,12 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
     }
     if (NB > 0) {
         AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
-        AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
-        h->lib_launches += 2;
+        h->lib_launches++;
+        if (!held) {
+            c.policy = false;  // the policy's replace_with is overwritten
+            AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
+            h->lib_launches++;
+        }
         if (p.T > 0)
             LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
                    (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),

@@ -26,7 +26,8 @@
 //   stats.cuh          the post-build scans of the callers
 //   unitigs.cuh        the compacted graph by list ranking; its junction edges as links between unitig ends, and
 //                      the reads as steps along unitigs (one scan over the windows)
-//   bubbles.cuh        the simple bubbles of the compacted graph (branches per edge, grouping per list by warp)
+//   bubbles.cuh        the simple bubbles of the compacted graph (branches per edge, grouping per list by warp),
+//                      and the popping policy (one warp per bubble)
 //   correct.cuh        the reads through the bubbles rewritten along a kept branch (edits per step, one scan
 //                      over the calls)
 //   sharded.cuh        the multi-GPU exchange and merge

@@ -59,8 +59,10 @@ class DeviceGraph:
     def reserve(self, n_nodes: int, n_edges: int):
         _lib.check(self._lib.amira_gmg_reserve(self._h, int(n_nodes), int(n_edges)))
 
-    def build(self, ids, off, k: int, pos_start=None, pos_end=None, on_device: bool = False, wait: bool = True):
-        """amira_gmg_build; ids/off are numpy arrays, torch tensors or raw pointers.
+    def build(self, ids, off, k: int, pos_start=None, pos_end=None, on_device: bool = False, wait: bool = True,
+              n_calls: int | None = None):
+        """amira_gmg_build; ids/off are numpy arrays, torch tensors or raw pointers.  n_calls: the call count off[R] of a
+        device CSR, when the caller knows it (amira_gmg_input_calls): the build then copies nothing back to size itself.
 
         The library only enqueues the build; problems the device finds (a palindromic gene-mer, a table that
         has to grow) surface at the first call that needs a result.  wait=True (default) asks for the early
@@ -75,6 +77,8 @@ class DeviceGraph:
         R = (off.shape[0] if hasattr(off, "shape") else len(off)) - 1
         self._keep = (ids, off, pos_start, pos_end)   # borrowed by the library until the next build
         self.k, self.R, self.has_pos = int(k), int(R), pos_start is not None
+        if on_device and n_calls is not None and R > 0:
+            _lib.check(self._lib.amira_gmg_input_calls(self._h, _ptr(off), R, int(n_calls)))
         _lib.check(self._lib.amira_gmg_build(self._h, _ptr(ids), _ptr(off), R, int(k), _ptr(pos_start), _ptr(pos_end),
                                              int(on_device)))
         if wait:
@@ -205,19 +209,45 @@ class DeviceGraph:
         _lib.check(self._lib.amira_gmg_bubbles(self._h, None, None, *[_ptr(a[f]) for f in BUBBLE_FIELDS]))
         return a
 
-    def correct_bubble_reads(self, replace_with, on_device: bool = False) -> dict:
+    def bubble_counts(self) -> tuple:
+        """(bubbles, branches) of bubbles(), without exporting them"""
+        B, NB = C.c_int64(), C.c_int64()
+        _lib.check(self._lib.amira_gmg_bubbles(self._h, C.byref(B), C.byref(NB), *[None] * 6))
+        return B.value, NB.value
+
+    def bubble_policy(self, spare_ranks=(), want_replace_with: bool = False):
+        """the popping policy over bubbles() (amira_gmg_bubble_policy): per bubble the branch with the largest mean node
+        coverage (then most branch_reads, then the first) replaces every other branch without a node holding one of the
+        genes of spare_ranks (vocabulary ranks).  Returns the number of branches replaced, and with want_replace_with
+        also replace_with (per branch: its replacement, or -1) as a numpy array.  The device keeps replace_with for
+        correct_bubble_reads(None)."""
+        r = np.ascontiguousarray(spare_ranks, np.int32)
+        n = C.c_int64()
+        _lib.check(self._lib.amira_gmg_bubble_policy(self._h, _ptr(r), len(r), C.byref(n), None))
+        if not want_replace_with:
+            return n.value
+        # sized after the call: counting the branches first would compute the bubbles before the policy's reservations
+        rw = np.empty(self.bubble_counts()[1], np.int32)
+        if len(rw):
+            _lib.check(self._lib.amira_gmg_bubble_policy(self._h, _ptr(r), len(r), None, _ptr(rw)))
+        return n.value, rw
+
+    def correct_bubble_reads(self, replace_with=None, on_device: bool = False, flags_on_device: bool = False) -> dict:
         """the reads through the bubbles of bubbles() rewritten along a kept branch (amira_gmg_correct_bubble_reads):
         replace_with[g] = -1 leaves branch g's reads alone, otherwise it is the branch of the same bubble whose genes
-        replace g's calls.  Returns the corrected CSR ids / off / pos_start / pos_end (None without positions) as numpy
-        arrays, or as torch tensors on this handle's device written by the device when on_device; and as numpy arrays
-        changed (per read: 1 when rewritten) and branch_rewritten (per branch: its reads rewritten)"""
-        NB = C.c_int64()
-        _lib.check(self._lib.amira_gmg_bubbles(self._h, None, C.byref(NB), *[None] * 6))
-        rw = np.asarray(replace_with, np.int64).ravel()
-        if len(rw) != NB.value or (len(rw) and (rw.min() < -1 or rw.max() >= NB.value)):
-            raise ValueError("correct_bubble_reads: replace_with must hold -1 or a branch index for each of %d branches"
-                             % NB.value)
-        rw = np.ascontiguousarray(rw, np.int32)
+        replace g's calls; None takes the replace_with of the last bubble_policy().  Returns the corrected CSR ids /
+        off / pos_start / pos_end (None without positions) as numpy arrays, or as torch tensors on this handle's device
+        written by the device when on_device; and changed (per read: 1 when rewritten) and branch_rewritten (per
+        branch: its reads rewritten) as numpy arrays, or with flags_on_device (and on_device) as device tensors of
+        uint8 and int32"""
+        NB = self.bubble_counts()[1]
+        rw = None
+        if replace_with is not None:
+            rw = np.asarray(replace_with, np.int64).ravel()
+            if len(rw) != NB or (len(rw) and (rw.min() < -1 or rw.max() >= NB)):
+                raise ValueError("correct_bubble_reads: replace_with must hold -1 or a branch index for each of %d "
+                                 "branches" % NB)
+            rw = np.ascontiguousarray(rw, np.int32)
         n = C.c_int64()
         _lib.check(self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), C.byref(n), *[None] * 6, 0))
         G, R = n.value, self.R
@@ -229,15 +259,17 @@ class DeviceGraph:
             new = lambda size, dt: np.empty(size, dt)
         a = {"ids": new(G, "int32"), "off": new(R + 1, "int64"),
              "pos_start": new(G, "int32") if self.has_pos else None, "pos_end": new(G, "int32") if self.has_pos else None,
-             "changed": np.empty(R, np.uint8), "branch_rewritten": np.empty(NB.value, np.uint32)}
+             "changed": np.empty(R, np.uint8), "branch_rewritten": np.empty(NB, np.uint32)}
         if on_device:
-            changed, rewritten = new(R, "uint8"), new(NB.value, "int32")     # per branch counts < 2^31, as uint32
+            changed, rewritten = new(R, "uint8"), new(NB, "int32")     # per branch counts < 2^31, as uint32
         else:
             changed, rewritten = a["changed"], a["branch_rewritten"]
         _lib.check(self._lib.amira_gmg_correct_bubble_reads(
             self._h, _ptr(rw), None, _ptr(a["off"]), _ptr(a["ids"]), _ptr(a["pos_start"]), _ptr(a["pos_end"]),
             _ptr(changed), _ptr(rewritten), int(bool(on_device))))
-        if on_device:
+        if on_device and flags_on_device:
+            a["changed"], a["branch_rewritten"] = changed, rewritten
+        elif on_device:
             a["changed"][:] = changed.cpu().numpy()
             a["branch_rewritten"][:] = rewritten.cpu().numpy().view(np.uint32)
         return a

@@ -109,6 +109,14 @@ int amira_gmg_kernel_launches(const amira_gmg *h, int64_t *n);
 int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read_off, int64_t R, int32_t k,
                     const int32_t *pos_start, const int32_t *pos_end, int input_on_device);
 
+/* The call count of the NEXT amira_gmg_build only, for a device CSR (input_on_device) whose read_off[R] the caller
+ * already knows, such as the outputs of amira_gmg_correct_bubble_reads (n_calls).  That build uses n_calls when it
+ * gets the same read_off and R, instead of copying read_off[R] back to the host or trusting a count cached from an
+ * earlier build of an array at the same address (which the caller may have freed and the allocator handed out
+ * again).  The per-read pass still checks the count on the device.  Every build forgets the hint, used or not.
+ * AMIRA_E_ARG for a NULL read_off, R <= 0 or a negative n_calls. */
+int amira_gmg_input_calls(amira_gmg *h, const int64_t *read_off, int64_t R, int64_t n_calls);
+
 /* wait for the handle's stream; returns the deferred status of the last build / filter */
 int amira_gmg_sync(amira_gmg *h);
 
@@ -282,7 +290,10 @@ int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int
  * input CSR (kept or borrowed by amira_gmg_build), the cached read paths and bubbles, and the node keys.
  *
  * replace_with[n_branches] (host): per branch g of amira_gmg_bubbles, -1 leaves g's reads alone; otherwise it is
- * another branch of the same bubble, whose genes replace g's calls.
+ * another branch of the same bubble, whose genes replace g's calls.  NULL: the replace_with the last
+ * amira_gmg_bubble_policy left on the device, used without a host check (it is valid by construction); AMIRA_E_STATE
+ * when there are branches and no policy was computed on the current bubbles (the graph or a device buffer changed
+ * since, or a call with a host replace_with overwrote it).
  * Edit: a read step (amira_gmg_read_unitig_paths) on branch g = unitig b of m nodes in bubble (sigma, tau), with
  * replace_with[g] >= 0, length m, the windows win - 1 and win + m present in its read and live, and their states
  * (2 * node + (dir < 0)) either (sigma, tau) -- the read runs sigma -> b -> tau -- or (tau ^ 1, sigma ^ 1) -- the
@@ -303,13 +314,30 @@ int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int
  * read order (read_off[r] = the output index of the input's call read_off_in[r]); changed[R] = 1 for a read with an
  * edit; branch_rewritten[n_branches] = the edits per branch.  Call with n_calls only to size the outputs, then again
  * for the arrays; every output may be NULL.  out_on_device != 0: the array outputs are device pointers on the handle's
- * device; either way the call returns with the work complete, and the library keeps no pointer.  Leaves the graph,
+ * device; either way the call returns with the work complete, and the library keeps no pointer.  A build from device
+ * outputs can be given n_calls with amira_gmg_input_calls, so that it copies nothing back to size itself.  Leaves the
+ * graph,
  * the cached unitigs / paths / bubbles and the filter masks as they were.  AMIRA_E_ARG when replace_with points out
  * of range, into another bubble or at the branch itself; AMIRA_E_STATE on a sharded handle.  Out of scope: reads that
  * end inside a branch, nested bubbles and superbubbles. */
 int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off,
                                    int32_t *ids, int32_t *pos_start, int32_t *pos_end, uint8_t *changed,
                                    uint32_t *branch_rewritten, int out_on_device);
+
+/* The popping policy of the simple bubbles (no upstream counterpart; GeneMerGraph.pop_compacted_bubbles and
+ * correct_compacted_bubbles use it), over the cached unitigs and bubbles, computed if not cached.  Per bubble the kept
+ * branch has the largest mean node coverage cov_sum / length of its unitig (amira_gmg_unitigs), compared exactly by
+ * cross-multiplying in 128 bits; ties go to the most branch_reads, then to the lowest branch index.  Every other
+ * branch is replaced by the kept one (replace_with[g] = the kept branch), unless one of its nodes holds a gene of
+ * spare_ranks[n_ranks] (vocabulary ranks as amira_gmg_nodes_containing takes them): then, as for the kept branch,
+ * replace_with[g] = -1.
+ *
+ * Outputs: n_replaced = the branches replaced; replace_with[n_branches] (host, may be NULL).  The result stays on the
+ * device, tagged with the bubble cache it belongs to, for amira_gmg_correct_bubble_reads with replace_with == NULL.
+ * One warp per bubble, whatever its branch count.  AMIRA_E_ARG for bad ranks; AMIRA_E_STATE on a sharded handle.
+ * Leaves the graph, the caches and the filter masks as they were. */
+int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_replaced,
+                            int32_t *replace_with);
 
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
