@@ -1183,16 +1183,8 @@ class GeneMerGraph:
             count[c0] = m2
             changed[r] = 1
             rewritten = np.bincount(gt, minlength=NB).astype(np.uint32)
-        idx = np.concatenate([[0], np.cumsum(count)]).astype(np.int64)
-        total = int(idx[-1])
-        out = {"ids": np.empty(total, np.int32), "off": idx[off],
-               "pos_start": None if ps is None else np.empty(total, np.int32),
-               "pos_end": None if pe is None else np.empty(total, np.int32), "changed": changed, "branch_rewritten": rewritten}
-        keep_calls = np.flatnonzero(~touched)
-        out["ids"][idx[keep_calls]] = ids[keep_calls]
-        for f, x in (("pos_start", ps), ("pos_end", pe)):
-            if x is not None:
-                out[f][idx[keep_calls]] = x[keep_calls]
+        out, idx = GeneMerGraph._untouched_calls_over(count, touched, src)
+        out.update(changed=changed, branch_rewritten=rewritten)
         if len(t):
             e = np.repeat(np.arange(len(t)), m2)
             j = np.arange(int(m2.sum())) - np.repeat(np.cumsum(m2) - m2, m2)
@@ -1204,6 +1196,173 @@ class GeneMerGraph:
                 if x is not None:
                     out[f][idx[c0[e]] + j] = x[c0[e] + np.minimum(j, mt[e] - 1)]
         return out
+
+    @staticmethod
+    def _untouched_calls_over(count, touched, src) -> tuple:
+        """the tail of the read corrections over index arrays: count[c] output calls per input call c of the encoded
+        reads src, touched[c] when call c is not copied -> (ids / off / pos_start / pos_end with every untouched call
+        copied to its place and the others left to the caller, the output index idx[c] of every call)"""
+        ids, off = np.asarray(src.ids, np.int32), np.asarray(src.off, np.int64)
+        ps, pe = src.pos_start, src.pos_end
+        idx = np.concatenate([[0], np.cumsum(count)]).astype(np.int64)
+        total = int(idx[-1])
+        out = {"ids": np.empty(total, np.int32), "off": idx[off],
+               "pos_start": None if ps is None else np.empty(total, np.int32),
+               "pos_end": None if pe is None else np.empty(total, np.int32)}
+        keep_calls = np.flatnonzero(~touched)
+        out["ids"][idx[keep_calls]] = ids[keep_calls]
+        for f, x in (("pos_start", ps), ("pos_end", pe)):
+            if x is not None:
+                out[f][idx[keep_calls]] = x[keep_calls]
+        return out, idx
+
+    def compacted_tips(self) -> dict:
+        """the dead-end tips of the compacted graph (include/amira_gmg.h, amira_gmg_tips) as numpy arrays, by unitig of
+        compacted_unitigs(): per tip its unitig, orientation (+1: a walk from the junction into the tip follows the
+        unitig's listed order), attach state (2 * node + side: the junction node's list that holds the edge into the
+        tip) and the read steps on it.  A device graph is served by the device and stays lazy."""
+        if self._on_device():
+            h = self._require_device_state()
+            if hasattr(h, "tips"):
+                return h.tips()
+            a = h.arrays()
+            return self._tips_over(a, a)
+        return self._tips_over(self._unitig_index_arrays(), self._read_index_arrays())
+
+    def _tips_over(self, a, w) -> dict:
+        """amira_gmg_tips over index arrays: the graph `a` (as _unitigs_over) and the windows `w` (as _read_paths_over).
+        Every unitig's two outward end states are tested at once"""
+        out = {"tip_unitig": np.zeros(0, np.int32), "tip_orient": np.zeros(0, np.int8), "tip_attach": np.zeros(0, np.int32),
+               "tip_reads": np.zeros(0, np.uint32)}
+        N, E = len(a["node_cov"]), len(a["edge_src"])
+        if E == 0:                                            # a tip hangs off a junction by one edge
+            return out
+        u = self._unitigs_over(a)
+        tgt, td = np.asarray(a["edge_tgt"], np.int64), np.asarray(a["edge_td"], np.int64)
+        size, one = self._list_sizes(a)
+        nu, uoff = u["node_unitig"].astype(np.int64), u["unitig_off"]
+        unodes = u["unitig_nodes"].astype(np.int64)
+        U = len(uoff) - 1
+        listed = 2 * np.arange(N, dtype=np.int64) + (u["node_orient"] < 0)
+        out1, out0 = listed[unodes[uoff[1:] - 1]], listed[unodes[uoff[:-1]]] ^ 1
+        d0, d1 = size[out0], size[out1]
+        dead1 = d1 == 0
+        e = one[np.where(dead1, out0, out1)]
+        ok = (u["circular"] == 0) & (((d0 == 0) & (d1 == 1)) | ((d1 == 0) & (d0 == 1)))
+        e = np.maximum(e, 0)
+        ok &= nu[tgt[e]] != np.arange(U)
+        b = np.flatnonzero(ok)
+        p = self._read_paths_over(a, w)
+        out.update(tip_unitig=b.astype(np.int32), tip_orient=np.where(dead1[b], 1, -1).astype(np.int8),
+                   tip_attach=((2 * tgt[e[b]] + (td[e[b]] < 0)) ^ 1).astype(np.int32),
+                   tip_reads=np.bincount(np.asarray(p["unitig"], np.int64), minlength=U)[b].astype(np.uint32))
+        return out
+
+    @staticmethod
+    def _tip_clip_flags(tips, u, a, amr, min_length) -> np.ndarray:
+        """the clipping policy of clip_compacted_tips over index arrays: tips as compacted_tips, u as compacted_unitigs,
+        the lists of the graph `a`, amr[n]: node n holds a gene of interest.  Per tip 1 when it has fewer than
+        min_length nodes, no node of interest, and an edge of its attach list leads into another unitig with a strictly
+        larger mean node coverage (cross-multiplied), else 0"""
+        b = np.asarray(tips["tip_unitig"], np.int64)
+        if not len(b):
+            return np.zeros(0, np.uint8)
+        nu = np.asarray(u["node_unitig"], np.int64)
+        ln = np.diff(np.asarray(u["unitig_off"], np.int64))
+        cs = np.asarray(u["cov_sum"], np.int64)
+        att = np.asarray(tips["tip_attach"], np.int64)
+        n, side = att >> 1, att & 1
+        lists = [(np.asarray(a[f + "_off"], np.int64), np.asarray(a[f + "_edges"], np.int64)) for f in ("fw", "bw")]
+        lo = np.where(side == 0, lists[0][0][n], lists[1][0][n])
+        d = np.where(side == 0, lists[0][0][n + 1], lists[1][0][n + 1]) - lo
+        qi = np.repeat(np.arange(len(b)), d)
+        pos = np.repeat(lo - np.cumsum(d) + d, d) + np.arange(int(d.sum()))
+        ent = np.zeros(len(qi), np.int64)
+        for s_, (_, edges) in enumerate(lists):
+            m = side[qi] == s_
+            ent[m] = edges[pos[m]]
+        c, bq = nu[np.asarray(a["edge_tgt"], np.int64)[ent]], b[qi]
+        hit = (c != bq) & (cs[c] * ln[bq] > cs[bq] * ln[c])
+        gene = np.zeros(len(ln), bool)
+        gene[nu[np.flatnonzero(amr)]] = True
+        return ((ln[b] < min_length) & ~gene[b] & (np.bincount(qi[hit], minlength=len(b)) > 0)).astype(np.uint8)
+
+    @staticmethod
+    def _clipped_reads_over(u, p, tips, w, clip, src) -> dict:
+        """amira_gmg_clip_tip_reads over index arrays: u as compacted_unitigs, p as read_unitig_paths, tips as
+        compacted_tips, the windows w (win_off, win_node with -1 for None, win_dir), clip per tip and the encoded reads
+        src.  Every step is tested at once; a clip drops the calls of its step's windows at the read's end"""
+        cf = np.asarray(clip).ravel()
+        Q = len(tips["tip_unitig"])
+        if len(cf) != Q or (Q and not np.isin(cf, (0, 1)).all()):
+            raise ValueError("clip_tip_reads: clip must hold 0 or 1 for each of %d tips" % Q)
+        off = np.asarray(src.off, np.int64)
+        R, G = len(off) - 1, int(off[-1])
+        count = np.ones(G, np.int64)
+        changed = np.zeros(R, np.uint8)
+        clipped = np.zeros(Q, np.uint32)
+        if Q and len(p["unitig"]):
+            unitig_tip = np.full(len(u["unitig_off"]) - 1, -1, np.int64)
+            unitig_tip[np.asarray(tips["tip_unitig"], np.int64)] = np.arange(Q)
+            q = unitig_tip[np.asarray(p["unitig"], np.int64)]
+            read = np.repeat(np.arange(R, dtype=np.int64), np.diff(p["path_off"]))
+            woff = np.asarray(w["win_off"], np.int64)
+            nw = np.diff(woff)[read]
+            i, ln = np.asarray(p["win"], np.int64), np.asarray(p["length"], np.int64)
+            end, start = (i >= 1) & (i + ln == nw), (i == 0) & (ln < nw)
+            flank = woff[read] + np.where(end, i - 1, np.where(start, ln, 0))
+            node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
+            fn = node[np.minimum(flank, max(len(node) - 1, 0))] if len(node) else np.zeros(0, np.int64)
+            state = 2 * fn + (d[np.minimum(flank, max(len(node) - 1, 0))] < 0)
+            att = np.asarray(tips["tip_attach"], np.int64)[np.maximum(q, 0)]
+            on = (q >= 0) & (cf[np.maximum(q, 0)] == 1) & (fn >= 0)
+            t_end = np.flatnonzero(on & end & (state == att))
+            t_start = np.flatnonzero(on & start & (state == (att ^ 1)))
+            t = np.concatenate([t_end, t_start])
+            c0 = np.concatenate([off[read[t_end] + 1] - ln[t_end], off[read[t_start]]])
+            lt = ln[t]
+            count[np.repeat(c0 - np.cumsum(lt) + lt, lt) + np.arange(int(lt.sum()))] = 0
+            changed[read[t]] = 1
+            clipped = np.bincount(q[t], minlength=Q).astype(np.uint32)
+        out, _ = GeneMerGraph._untouched_calls_over(count, count == 0, src)
+        out.update(changed=changed, tip_clipped=clipped)
+        return out
+
+    def clip_compacted_tips(self, min_length, sample_genesOfInterest={}):
+        """the reads clipped at the tips of compacted_tips() that the clipping policy picks, as a new
+        encode.EncodedReads to rebuild from (include/amira_gmg.h, amira_gmg_tip_policy, amira_gmg_clip_tip_reads).  A tip
+        is clipped when it has fewer than min_length nodes, no node holding a gene of sample_genesOfInterest, and a
+        sibling at its junction leads into a unitig with a strictly larger mean node coverage; an error in a read's
+        first or last k calls makes a tip of at most k nodes, so min_length = k + 1 covers single end errors.  A read
+        whose last (first) step runs into a clipped tip from its junction loses the calls only that step holds; every
+        other call is unchanged.  The result shares the vocabulary and read ids of this graph's reads, its dicts are
+        shallow copies with only the changed reads decoded, and it carries `changed` (per read) and `tip_clipped` (per
+        tip of compacted_tips(): the read steps clipped).  The graph and its reads are left as they are.  A device graph
+        is clipped on the device, which writes the new CSR that a rebuild from the result reads without uploading it."""
+        return self._source_encoded().corrected(self._tip_clip(min_length, sample_genesOfInterest), self._device)
+
+    def _tip_clip(self, min_length, sample_genesOfInterest) -> dict:
+        """clip_compacted_tips before it becomes an EncodedReads: the outputs of DeviceGraph.clip_tip_reads.  A device
+        graph whose handle has the policy is clipped on the handle alone; otherwise the numpy implementation runs"""
+        src = self._source_encoded()
+        if self._on_device():
+            h = self._require_device_state()
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            if hasattr(h, "tip_policy"):
+                h.tip_policy(min_length, ranks)
+                return h.clip_tip_reads(None, on_device=True)
+            a = h.arrays()
+            u, tips = self.compacted_unitigs(), self.compacted_tips()
+            amr = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(a["node_cov"]), bool)
+            clip = self._tip_clip_flags(tips, u, a, amr, min_length)
+            if hasattr(h, "clip_tip_reads"):
+                return h.clip_tip_reads(clip, on_device=True)
+            return self._clipped_reads_over(u, self._read_paths_over(a, a), tips, a, clip, src)
+        a, w = self._unitig_index_arrays(), self._read_index_arrays()
+        u, tips = self._unitigs_over(a), self._tips_over(a, w)
+        amr_nodes = self.get_AMR_nodes(sample_genesOfInterest)
+        clip = self._tip_clip_flags(tips, u, a, np.asarray([nh in amr_nodes for nh in self._nodes], bool), min_length)
+        return self._clipped_reads_over(u, self._read_paths_over(a, w), tips, w, clip, src)
 
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
@@ -1611,7 +1770,8 @@ def bind_upstream(upstream_construct_graph):
                    "_read_paths_over", "_list_sizes", "compacted_bubbles", "_bubbles_over", "pop_compacted_bubbles",
                    "_bubble_pop_nodes", "_bubble_winners", "correct_compacted_bubbles", "_source_encoded",
                    "_corrected_reads_over", "_adopt_build", "_bubble_correction", "_handle_correction",
-                   "correct_bubbles_until_stable",
+                   "correct_bubbles_until_stable", "_untouched_calls_over", "compacted_tips", "_tips_over",
+                   "_tip_clip_flags", "_clipped_reads_over", "clip_compacted_tips", "_tip_clip",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

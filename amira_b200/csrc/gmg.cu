@@ -12,6 +12,7 @@
 #include "unitigs.cuh"
 #include "bubbles.cuh"
 #include "correct.cuh"
+#include "tips.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -232,6 +233,17 @@ struct amira_gmg {
         bool policy = false;
         uint64_t policy_version = 0, policy_generation = 0;
     } correct;
+    // the dead-end tips of the compacted graph (tips.cuh), valid under the rule of the unitigs, and the clip flags of
+    // the last amira_gmg_tip_policy (or host flags of amira_gmg_clip_tip_reads), with the tip cache they belong to.
+    // amira_gmg_clip_tip_reads uses the correction's cnt / idx / changed / n_out as scratch.
+    struct {
+        DevBuf flags, n_out, tip_unitig, orient, attach, reads, unitig_tip, clip, spared, clipped;
+        int64_t Q = 0;
+        bool valid = false;
+        uint64_t version = 0, generation = 0;
+        bool policy = false;
+        uint64_t policy_version = 0, policy_generation = 0;
+    } tips;
 };
 
 namespace {
@@ -2445,9 +2457,77 @@ int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig
 }
 
 namespace {
-// the simple bubbles, cached under the rule of unitig_table.  Every buffer and the scan's tile states are reserved
-// before read_path_table (and through it unitig_table) runs, for the reason given at unitig_links_table.  A bubble
-// has two branches or more and a branch is one edge of its list, so E bounds the branches and E / 2 the bubbles.
+// The buffers of the bubble and tip calls are all reserved together, by every one of them, before the cached
+// unitigs, paths, bubbles or tips are looked at: a reservation that grows bumps the buffer generation and would drop
+// those caches and the policy computed on them.  So interleaving bubble and tip calls on one graph loses neither.
+//
+// The bubbles: a bubble has two branches or more and a branch is one edge of its list, so E bounds the branches and
+// E / 2 the bubbles.
+int reserve_bubbles(amira_gmg *h) {
+    auto &q = h->bubbles;
+    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
+    if (E == 0) return AMIRA_OK;  // without an edge there is no branch
+    const size_t e4 = sizeof(int32_t) * (size_t)E;
+    AMIRA_TRY(q.edge_tau.reserve(e4));
+    AMIRA_TRY(q.ebr.reserve(e4));
+    AMIRA_TRY(q.ebub.reserve(e4));
+    AMIRA_TRY(q.ehead.reserve(e4));
+    AMIRA_TRY(q.counts.reserve(sizeof(unsigned long long) * (size_t)S));
+    AMIRA_TRY(q.first.reserve(sizeof(unsigned long long) * (size_t)S));
+    AMIRA_TRY(q.n_out.reserve(sizeof(unsigned long long)));
+    AMIRA_TRY(q.source.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+    AMIRA_TRY(q.sink.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+    AMIRA_TRY(q.branch_off.reserve(sizeof(int64_t) * (size_t)(E / 2 + 1)));
+    AMIRA_TRY(q.branch_unitig.reserve(e4));
+    AMIRA_TRY(q.branch_orient.reserve((size_t)E));
+    AMIRA_TRY(q.branch_reads.reserve(e4));
+    AMIRA_TRY(q.unitig_branch.reserve(sizeof(int32_t) * (size_t)N));
+    return reserve_scan(h, S);
+}
+
+// the policy and correction buffers of the bubbles; cnt / idx / changed / n_out also serve amira_gmg_clip_tip_reads
+int reserve_correct(amira_gmg *h) {
+    auto &c = h->correct;
+    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
+    if (R == 0) return AMIRA_OK;
+    const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
+    AMIRA_TRY(c.replace.reserve(e4));
+    AMIRA_TRY(c.spared.reserve((size_t)std::max<long long>(E, 1)));
+    AMIRA_TRY(c.rewritten.reserve(e4));
+    AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
+    AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
+    AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
+    AMIRA_TRY(c.changed.reserve((size_t)R));
+    AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
+    return reserve_scan(h, G);
+}
+
+// the tips: a unitig is at most one tip, and N bounds the unitigs
+int reserve_tips(amira_gmg *h) {
+    auto &t = h->tips;
+    const long long N = h->n_nodes;
+    if (N == 0) return AMIRA_OK;
+    const size_t n4 = sizeof(int32_t) * (size_t)N;
+    AMIRA_TRY(t.flags.reserve((size_t)N));
+    AMIRA_TRY(t.n_out.reserve(sizeof(unsigned long long)));
+    AMIRA_TRY(t.tip_unitig.reserve(n4));
+    AMIRA_TRY(t.orient.reserve((size_t)N));
+    AMIRA_TRY(t.attach.reserve(n4));
+    AMIRA_TRY(t.reads.reserve(n4));
+    AMIRA_TRY(t.unitig_tip.reserve(n4));
+    AMIRA_TRY(t.clip.reserve((size_t)N));
+    AMIRA_TRY(t.spared.reserve((size_t)N));
+    AMIRA_TRY(t.clipped.reserve(n4));
+    return reserve_scan(h, N);
+}
+
+int reserve_cleaning(amira_gmg *h) {
+    AMIRA_TRY(reserve_bubbles(h));
+    AMIRA_TRY(reserve_correct(h));
+    return reserve_tips(h);
+}
+
+// the simple bubbles, cached under the rule of unitig_table
 int bubble_table(amira_gmg *h) {
     auto &q = h->bubbles;
     if (q.valid && q.version == h->graph_version && q.generation == buffer_generation()) return AMIRA_OK;
@@ -2458,24 +2538,7 @@ int bubble_table(amira_gmg *h) {
         return AMIRA_E_ARG;
     }
     const bool any = E > 0;  // without an edge there is no branch
-    if (any) {
-        const size_t e4 = sizeof(int32_t) * (size_t)E;
-        AMIRA_TRY(q.edge_tau.reserve(e4));
-        AMIRA_TRY(q.ebr.reserve(e4));
-        AMIRA_TRY(q.ebub.reserve(e4));
-        AMIRA_TRY(q.ehead.reserve(e4));
-        AMIRA_TRY(q.counts.reserve(sizeof(unsigned long long) * (size_t)S));
-        AMIRA_TRY(q.first.reserve(sizeof(unsigned long long) * (size_t)S));
-        AMIRA_TRY(q.n_out.reserve(sizeof(unsigned long long)));
-        AMIRA_TRY(q.source.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
-        AMIRA_TRY(q.sink.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
-        AMIRA_TRY(q.branch_off.reserve(sizeof(int64_t) * (size_t)(E / 2 + 1)));
-        AMIRA_TRY(q.branch_unitig.reserve(e4));
-        AMIRA_TRY(q.branch_orient.reserve((size_t)E));
-        AMIRA_TRY(q.branch_reads.reserve(e4));
-        AMIRA_TRY(q.unitig_branch.reserve(sizeof(int32_t) * (size_t)N));
-        AMIRA_TRY(reserve_scan(h, S));
-    }
+    AMIRA_TRY(reserve_cleaning(h));
     AMIRA_TRY(read_path_table(h));
     q.B = q.NB = 0;
     if (any) {
@@ -2561,27 +2624,6 @@ struct CallBuf {
 };
 }  // namespace
 
-namespace {
-// the buffers of amira_gmg_bubble_policy and amira_gmg_correct_bubble_reads, reserved by both before the bubbles: a
-// reservation that grows bumps the buffer generation and would drop them.  Reserving the correction's buffers in the
-// policy too lets a correction that follows the policy find the bubble cache the policy was computed on.
-int reserve_correct(amira_gmg *h) {
-    auto &c = h->correct;
-    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
-    if (R == 0) return AMIRA_OK;
-    const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
-    AMIRA_TRY(c.replace.reserve(e4));
-    AMIRA_TRY(c.spared.reserve((size_t)std::max<long long>(E, 1)));
-    AMIRA_TRY(c.rewritten.reserve(e4));
-    AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
-    AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
-    AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
-    AMIRA_TRY(c.changed.reserve((size_t)R));
-    AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
-    return reserve_scan(h, G);
-}
-}  // namespace
-
 int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_replaced, int32_t *replace_with) {
     AMIRA_TRY(stats_ready(h));
     if (h->world > 1) {
@@ -2595,7 +2637,7 @@ int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_
     auto &c = h->correct;
     c.policy = false;
     // every reservation before the bubbles, the gene flags' (scratch_off, comp_max) included
-    AMIRA_TRY(reserve_correct(h));
+    AMIRA_TRY(reserve_cleaning(h));
     if (n_ranks > 0) AMIRA_TRY(flag_nodes_containing(h, spare_ranks, n_ranks));
     AMIRA_TRY(bubble_table(h));
     const auto &q = h->bubbles;
@@ -2625,79 +2667,49 @@ int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_
     return AMIRA_OK;
 }
 
-int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
-                                   int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
-                                   int out_on_device) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("correct_bubble_reads: not available on a sharded graph");
-        return AMIRA_E_STATE;
+namespace {
+// the outputs of a correction without reads: no call, read_off = {0}
+int corrected_without_reads(amira_gmg *h, int64_t *n_calls, int64_t *read_off, int out_on_device) {
+    if (n_calls) *n_calls = 0;
+    if (read_off) {
+        if (out_on_device) AMIRA_CUDA(cudaMemsetAsync(read_off, 0, sizeof(int64_t), h->stream));
+        else read_off[0] = 0;
     }
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+// before the marks of a correction (R > 0): no read changed, every call untouched
+int clear_correct(amira_gmg *h) {
     auto &c = h->correct;
-    const long long R = h->R, G = R > 0 ? h->G : 0;
-    AMIRA_TRY(reserve_correct(h));
-    AMIRA_TRY(bubble_table(h));
-    const auto &q = h->bubbles;
-    const int64_t B = q.B, NB = q.NB;
+    const long long R = h->R, G = h->G;
     cudaStream_t st = h->stream;
-    // NULL: the replace_with of the last policy, which the device holds, valid by construction
-    const bool held = NB > 0 && !replace_with;
-    if (held && !(c.policy && c.policy_version == q.version && c.policy_generation == q.generation)) {
-        set_error("correct_bubble_reads: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles",
-                  (long long)NB);
-        return AMIRA_E_STATE;
-    }
-    if (NB > 0 && !held) {
-        std::vector<int64_t> boff((size_t)B + 1);
-        AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
-        AMIRA_CUDA(cudaStreamSynchronize(st));
-        for (int64_t b = 0; b < B; ++b)
-            for (int64_t g = boff[b]; g < boff[b + 1]; ++g) {
-                const int64_t x = replace_with[g];
-                if (x != -1 && (x < boff[b] || x >= boff[b + 1] || x == g)) {
-                    set_error("correct_bubble_reads: replace_with[%lld] = %lld is not -1 or another branch of bubble %lld",
-                              (long long)g, (long long)x, (long long)b);
-                    return AMIRA_E_ARG;
-                }
-            }
-    }
-    if (R == 0) {  // no read, no node, no bubble
-        if (n_calls) *n_calls = 0;
-        if (read_off) {
-            if (out_on_device) AMIRA_CUDA(cudaMemsetAsync(read_off, 0, sizeof(int64_t), st));
-            else read_off[0] = 0;
-        }
-        AMIRA_CUDA(cudaStreamSynchronize(st));
-        return AMIRA_OK;
-    }
-    const auto &u = h->unitigs;
-    const auto &p = h->paths;
-    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
-    int64_t *idx = c.idx.as<int64_t>();
-    int32_t *step_new = c.step_new.as<int32_t>(), *replace = c.replace.as<int32_t>();
-    uint8_t *d_changed = c.changed.as<uint8_t>();
-    AMIRA_CUDA(cudaMemsetAsync(d_changed, 0, (size_t)R, st));
-    AMIRA_CUDA(cudaMemsetAsync(idx, 0, sizeof(int64_t), st));  // idx[0] when there is no call
+    AMIRA_CUDA(cudaMemsetAsync(c.changed.p, 0, (size_t)R, st));
+    AMIRA_CUDA(cudaMemsetAsync(c.idx.p, 0, sizeof(int64_t), st));  // idx[0] when there is no call
     h->lib_launches += 2;
     if (G > 0) {
-        AMIRA_CUDA(cudaMemsetAsync(cnt, 0, sizeof(uint32_t) * (size_t)G, st));
+        AMIRA_CUDA(cudaMemsetAsync(c.cnt.p, 0, sizeof(uint32_t) * (size_t)G, st));
         h->lib_launches++;
     }
-    if (NB > 0) {
-        AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
-        h->lib_launches++;
-        if (!held) {
-            c.policy = false;  // the policy's replace_with is overwritten
-            AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
-            h->lib_launches++;
-        }
-        if (p.T > 0)
-            LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
-                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
-                   h->win_dir.as<int8_t>(), h->off, u.off.as<int64_t>(), q.unitig_branch.as<int32_t>(), q.branch_off.as<int64_t>(),
-                   (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(), q.branch_unitig.as<int32_t>(), replace, cnt,
-                   step_new, d_changed, rewritten);
-    }
+    return AMIRA_OK;
+}
+
+// after the marks in the correction's cnt (and, for bubble edits, step_new and the bubbles' replace_with): one scan
+// over the calls gives every call's output index, then the new offsets and calls are written to the caller's device
+// arrays or, through one staging allocation, to its host arrays, with the per read flags and the per item counts
+// d_counts[n_counts].  Tip clips (edits == false) only hold codes 0 and 1, so the fill reads no bubble array.
+int write_corrected(amira_gmg *h, bool edits, int64_t *n_calls, int64_t *read_off, int32_t *ids, int32_t *pos_start,
+                    int32_t *pos_end, uint8_t *changed, uint32_t *counts, const uint32_t *d_counts, int64_t n_counts,
+                    int out_on_device) {
+    auto &c = h->correct;
+    const auto &u = h->unitigs;
+    const auto &p = h->paths;
+    const auto &q = h->bubbles;
+    const long long R = h->R, G = h->G;
+    cudaStream_t st = h->stream;
+    uint32_t *cnt = c.cnt.as<uint32_t>();
+    int64_t *idx = c.idx.as<int64_t>();
+    int32_t *step_new = c.step_new.as<int32_t>();
     long long total = 0;
     if (G > 0) {
         unsigned long long *d_n = c.n_out.as<unsigned long long>();
@@ -2728,16 +2740,17 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
     if (o_off) LAUNCH(h, k_correct_offsets, grid_for(R + 1, 256), 256, h->off, R, idx, o_off);
     if (G > 0 && (o_ids || o_ps || o_pe))
         LAUNCH(h, k_correct_fill, grid_for(G, 256), 256, cnt, idx, G, h->ids, h->ps, h->pe, step_new, p.unitig.as<int32_t>(),
-               p.length.as<int32_t>(), q.unitig_branch.as<int32_t>(), replace, q.branch_unitig.as<int32_t>(),
-               q.branch_orient.as<int8_t>(), u.off.as<int64_t>(), u.nodes.as<int32_t>(), u.node_orient.as<int8_t>(),
-               h->nodes.key.as<int32_t>(), h->k, o_ids, o_ps, o_pe);
+               p.length.as<int32_t>(), edits ? q.unitig_branch.as<int32_t>() : nullptr,
+               edits ? c.replace.as<int32_t>() : nullptr, edits ? q.branch_unitig.as<int32_t>() : nullptr,
+               edits ? q.branch_orient.as<int8_t>() : nullptr, u.off.as<int64_t>(), u.nodes.as<int32_t>(),
+               u.node_orient.as<int8_t>(), h->nodes.key.as<int32_t>(), h->k, o_ids, o_ps, o_pe);
     const cudaMemcpyKind kind = out_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
     struct {
         void *dst;
         const void *src;
         size_t bytes;
-    } jobs[] = {{changed, d_changed, (size_t)R},
-                {branch_rewritten, rewritten, sizeof(uint32_t) * (size_t)NB},
+    } jobs[] = {{changed, c.changed.p, (size_t)R},
+                {counts, d_counts, sizeof(uint32_t) * (size_t)n_counts},
                 {out_on_device ? nullptr : read_off, o_off, sizeof(int64_t) * (size_t)(R + 1)},
                 {out_on_device ? nullptr : ids, o_ids, sizeof(int32_t) * (size_t)total},
                 {out_on_device ? nullptr : o_ps ? pos_start : nullptr, o_ps, sizeof(int32_t) * (size_t)total},
@@ -2749,6 +2762,230 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
         }
     AMIRA_CUDA(cudaStreamSynchronize(st));
     return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
+                                   int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
+                                   int out_on_device) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("correct_bubble_reads: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    auto &c = h->correct;
+    const long long R = h->R;
+    AMIRA_TRY(reserve_cleaning(h));
+    AMIRA_TRY(bubble_table(h));
+    const auto &q = h->bubbles;
+    const int64_t B = q.B, NB = q.NB;
+    cudaStream_t st = h->stream;
+    // NULL: the replace_with of the last policy, which the device holds, valid by construction
+    const bool held = NB > 0 && !replace_with;
+    if (held && !(c.policy && c.policy_version == q.version && c.policy_generation == q.generation)) {
+        set_error("correct_bubble_reads: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles",
+                  (long long)NB);
+        return AMIRA_E_STATE;
+    }
+    if (NB > 0 && !held) {
+        std::vector<int64_t> boff((size_t)B + 1);
+        AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        for (int64_t b = 0; b < B; ++b)
+            for (int64_t g = boff[b]; g < boff[b + 1]; ++g) {
+                const int64_t x = replace_with[g];
+                if (x != -1 && (x < boff[b] || x >= boff[b + 1] || x == g)) {
+                    set_error("correct_bubble_reads: replace_with[%lld] = %lld is not -1 or another branch of bubble %lld",
+                              (long long)g, (long long)x, (long long)b);
+                    return AMIRA_E_ARG;
+                }
+            }
+    }
+    if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no bubble
+    const auto &p = h->paths;
+    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
+    int32_t *replace = c.replace.as<int32_t>();
+    AMIRA_TRY(clear_correct(h));
+    if (NB > 0) {
+        AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
+        h->lib_launches++;
+        if (!held) {
+            c.policy = false;  // the policy's replace_with is overwritten
+            AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
+            h->lib_launches++;
+        }
+        if (p.T > 0)
+            LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
+                   h->win_dir.as<int8_t>(), h->off, h->unitigs.off.as<int64_t>(), q.unitig_branch.as<int32_t>(),
+                   q.branch_off.as<int64_t>(), (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(),
+                   q.branch_unitig.as<int32_t>(), replace, cnt, c.step_new.as<int32_t>(), c.changed.as<uint8_t>(), rewritten);
+    }
+    return write_corrected(h, true, n_calls, read_off, ids, pos_start, pos_end, changed, branch_rewritten, rewritten, NB,
+                           out_on_device);
+}
+
+namespace {
+// the tips, cached under the rule of unitig_table; every buffer reserved ahead (reserve_cleaning)
+int tip_table(amira_gmg *h) {
+    auto &t = h->tips;
+    if (t.valid && t.version == h->graph_version && t.generation == buffer_generation()) return AMIRA_OK;
+    t.valid = false;
+    const long long N = h->n_nodes;
+    if (2 * N >= (1ll << 31)) {
+        set_error("tips: %lld nodes, the states 2 * node + side must fit in 31 bits", N);
+        return AMIRA_E_ARG;
+    }
+    AMIRA_TRY(reserve_cleaning(h));
+    AMIRA_TRY(read_path_table(h));
+    t.Q = 0;
+    const auto &u = h->unitigs;
+    const auto &p = h->paths;
+    const long long U = u.U;
+    if (U > 0) {
+        cudaStream_t st = h->stream;
+        const int64_t *adj_off = h->adj_off.as<int64_t>();
+        const uint32_t *adj_edges = h->adj_edges.as<uint32_t>();
+        const int32_t *e_tgt = h->edges.tgt.as<int32_t>();
+        unsigned long long *d_n = t.n_out.as<unsigned long long>();
+        LAUNCH(h, k_tip_flags, grid_for(U, 256), 256, adj_off, adj_edges, N, e_tgt, u.node_unitig.as<int32_t>(),
+               u.node_orient.as<int8_t>(), u.off.as<int64_t>(), u.nodes.as<int32_t>(), u.circular.as<uint8_t>(), U,
+               t.flags.as<uint8_t>());
+        AMIRA_TRY(run_scan(h, TipLoad{t.flags.as<uint8_t>()}, TipStore{t.tip_unitig.as<int32_t>(), U, d_n}, nullptr, 1, U, U));
+        unsigned long long Q = 0;
+        AMIRA_TRY(d2h(h, &Q, d_n, sizeof(Q)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        if (Q > 0) {
+            int32_t *unitig_tip = t.unitig_tip.as<int32_t>();
+            uint32_t *reads = t.reads.as<uint32_t>();
+            AMIRA_CUDA(cudaMemsetAsync(unitig_tip, 0xff, sizeof(int32_t) * (size_t)U, st));
+            AMIRA_CUDA(cudaMemsetAsync(reads, 0, sizeof(uint32_t) * (size_t)Q, st));
+            h->lib_launches += 2;
+            LAUNCH(h, k_tip_fill, grid_for((int64_t)Q, 256), 256, t.tip_unitig.as<int32_t>(), (long long)Q, adj_off, adj_edges, N,
+                   e_tgt, h->edges.td.as<int8_t>(), u.node_unitig.as<int32_t>(), u.node_orient.as<int8_t>(), u.off.as<int64_t>(),
+                   u.nodes.as<int32_t>(), t.orient.as<int8_t>(), t.attach.as<int32_t>(), unitig_tip);
+            if (p.T > 0)
+                LAUNCH(h, k_tip_reads, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), (long long)p.T, unitig_tip, reads);
+        }
+        t.Q = (int64_t)Q;
+    }
+    t.version = h->graph_version;
+    t.generation = buffer_generation();
+    t.valid = true;
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_tips(amira_gmg *h, int64_t *n_tips, int32_t *tip_unitig, int8_t *tip_orient, int32_t *tip_attach,
+                   uint32_t *tip_reads) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("tips: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    AMIRA_TRY(tip_table(h));
+    const auto &t = h->tips;
+    const int64_t Q = t.Q;
+    if (n_tips) *n_tips = Q;
+    if (Q == 0) return AMIRA_OK;
+    AMIRA_TRY(d2h(h, tip_unitig, t.tip_unitig.p, sizeof(int32_t) * Q));
+    AMIRA_TRY(d2h(h, tip_orient, t.orient.p, (size_t)Q));
+    AMIRA_TRY(d2h(h, tip_attach, t.attach.p, sizeof(int32_t) * Q));
+    AMIRA_TRY(d2h(h, tip_reads, t.reads.p, sizeof(uint32_t) * Q));
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
+}
+
+int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_clipped,
+                         uint8_t *clip) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("tip_policy: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    if (n_ranks < 0 || (n_ranks > 0 && !spare_ranks)) {
+        set_error("tip_policy: bad gene ranks (n = %d)", n_ranks);
+        return AMIRA_E_ARG;
+    }
+    auto &t = h->tips;
+    t.policy = false;
+    // every reservation before the tips, the gene flags' (scratch_off, comp_max) included
+    AMIRA_TRY(reserve_cleaning(h));
+    if (n_ranks > 0) AMIRA_TRY(flag_nodes_containing(h, spare_ranks, n_ranks));
+    AMIRA_TRY(tip_table(h));
+    const int64_t Q = t.Q, N = h->n_nodes;
+    cudaStream_t st = h->stream;
+    unsigned long long total = 0;
+    if (Q > 0) {
+        uint8_t *spared = t.spared.as<uint8_t>();
+        unsigned long long *d_n = t.n_out.as<unsigned long long>();
+        AMIRA_CUDA(cudaMemsetAsync(spared, 0, (size_t)Q, st));
+        AMIRA_CUDA(cudaMemsetAsync(d_n, 0, sizeof(unsigned long long), st));
+        h->lib_launches += 2;
+        if (n_ranks > 0)
+            LAUNCH(h, k_bubble_spare, grid_for(N, 256), 256, h->scratch_off.as<uint8_t>(), (long long)N,
+                   h->unitigs.node_unitig.as<int32_t>(), t.unitig_tip.as<int32_t>(), spared);
+        LAUNCH(h, k_tip_policy, grid_for(Q * 32, 256), 256, t.tip_unitig.as<int32_t>(), t.attach.as<int32_t>(), (long long)Q,
+               h->adj_off.as<int64_t>(), h->adj_edges.as<uint32_t>(), (long long)N, h->edges.tgt.as<int32_t>(),
+               h->unitigs.node_unitig.as<int32_t>(), h->unitigs.off.as<int64_t>(), h->unitigs.cov_sum.as<unsigned long long>(),
+               spared, (long long)min_length, t.clip.as<uint8_t>(), d_n);
+        AMIRA_TRY(d2h(h, &total, d_n, sizeof(total)));
+        AMIRA_TRY(d2h(h, clip, t.clip.p, (size_t)Q));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+    }
+    if (n_clipped) *n_clipped = (int64_t)total;
+    t.policy = true;
+    t.policy_version = t.version;
+    t.policy_generation = t.generation;
+    return AMIRA_OK;
+}
+
+int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
+                             int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped, int out_on_device) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("clip_tip_reads: not available on a sharded graph");
+        return AMIRA_E_STATE;
+    }
+    auto &t = h->tips;
+    auto &c = h->correct;
+    const long long R = h->R;
+    AMIRA_TRY(reserve_cleaning(h));
+    AMIRA_TRY(tip_table(h));
+    const int64_t Q = t.Q;
+    cudaStream_t st = h->stream;
+    // NULL: the clip flags of the last policy, which the device holds
+    const bool held = Q > 0 && !clip;
+    if (held && !(t.policy && t.policy_version == t.version && t.policy_generation == t.generation)) {
+        set_error("clip_tip_reads: no clip flags for %lld tips, and no amira_gmg_tip_policy on these tips", (long long)Q);
+        return AMIRA_E_STATE;
+    }
+    if (Q > 0 && !held)
+        for (int64_t q = 0; q < Q; ++q)
+            if (clip[q] > 1) {
+                set_error("clip_tip_reads: clip[%lld] = %d is not 0 or 1", (long long)q, (int)clip[q]);
+                return AMIRA_E_ARG;
+            }
+    if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no tip
+    const auto &p = h->paths;
+    uint32_t *clipped = t.clipped.as<uint32_t>();
+    AMIRA_TRY(clear_correct(h));
+    if (Q > 0) {
+        AMIRA_CUDA(cudaMemsetAsync(clipped, 0, sizeof(uint32_t) * (size_t)Q, st));
+        h->lib_launches++;
+        if (!held) {
+            t.policy = false;  // the policy's flags are overwritten
+            AMIRA_CUDA(cudaMemcpyAsync(t.clip.p, clip, (size_t)Q, cudaMemcpyHostToDevice, st));
+            h->lib_launches++;
+        }
+        if (p.T > 0)
+            LAUNCH(h, k_tip_clip, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
+                   h->win_dir.as<int8_t>(), h->off, t.unitig_tip.as<int32_t>(), t.attach.as<int32_t>(), t.clip.as<uint8_t>(),
+                   c.cnt.as<uint32_t>(), c.changed.as<uint8_t>(), clipped);
+    }
+    return write_corrected(h, false, n_calls, read_off, ids, pos_start, pos_end, changed, tip_clipped, clipped, Q,
+                           out_on_device);
 }
 
 int amira_gmg_debug_segsort(amira_gmg *h, uint32_t *data, const int64_t *off, int64_t n_seg, uint32_t *dups,

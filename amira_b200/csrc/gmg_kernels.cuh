@@ -30,7 +30,9 @@
 //                      and the popping policy (one warp per bubble)
 //   correct.cuh        the reads through the bubbles rewritten along a kept branch (edits per step, one scan
 //                      over the calls)
-//   sharded.cuh        the multi-GPU exchange and merge
+//   tips.cuh           the dead-end tips of the compacted graph, the clipping policy (one warp per tip), and the
+//                      reads clipped at them (marks per step into the correction's scan and fill)
+//   sharded.cuh       the multi-GPU exchange and merge
 #pragma once
 
 #include "common.cuh"

@@ -19,6 +19,8 @@ LINK_FIELDS = ("edge", "from_unitig", "from_orient", "to_unitig", "to_orient", "
 PATH_FIELDS = ("path_off", "unitig", "orient", "pos", "win", "length")
 # the arrays of amira_gmg_bubbles, in its argument order
 BUBBLE_FIELDS = ("source", "sink", "branch_off", "branch_unitig", "branch_orient", "branch_reads")
+# the arrays of amira_gmg_tips, in its argument order
+TIP_FIELDS = ("tip_unitig", "tip_orient", "tip_attach", "tip_reads")
 
 
 def _ptr(a):
@@ -248,8 +250,15 @@ class DeviceGraph:
                 raise ValueError("correct_bubble_reads: replace_with must hold -1 or a branch index for each of %d "
                                  "branches" % NB)
             rw = np.ascontiguousarray(rw, np.int32)
+        return self._corrected_csr(lambda *a: self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), *a), NB,
+                                   "branch_rewritten", on_device, flags_on_device)
+
+    def _corrected_csr(self, call, n_items, counts, on_device, flags_on_device) -> dict:
+        """the size pass and the fill pass of a correction call (n_calls, read_off, ids, pos_start, pos_end, changed,
+        per item counts, out_on_device) -> the dict correct_bubble_reads and clip_tip_reads return, the per item counts
+        under the name `counts`"""
         n = C.c_int64()
-        _lib.check(self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), C.byref(n), *[None] * 6, 0))
+        _lib.check(call(C.byref(n), *[None] * 6, 0))
         G, R = n.value, self.R
         if on_device:
             import torch
@@ -259,20 +268,69 @@ class DeviceGraph:
             new = lambda size, dt: np.empty(size, dt)
         a = {"ids": new(G, "int32"), "off": new(R + 1, "int64"),
              "pos_start": new(G, "int32") if self.has_pos else None, "pos_end": new(G, "int32") if self.has_pos else None,
-             "changed": np.empty(R, np.uint8), "branch_rewritten": np.empty(NB, np.uint32)}
+             "changed": np.empty(R, np.uint8), counts: np.empty(n_items, np.uint32)}
         if on_device:
-            changed, rewritten = new(R, "uint8"), new(NB, "int32")     # per branch counts < 2^31, as uint32
+            changed, per_item = new(R, "uint8"), new(n_items, "int32")     # per item counts < 2^31, as uint32
         else:
-            changed, rewritten = a["changed"], a["branch_rewritten"]
-        _lib.check(self._lib.amira_gmg_correct_bubble_reads(
-            self._h, _ptr(rw), None, _ptr(a["off"]), _ptr(a["ids"]), _ptr(a["pos_start"]), _ptr(a["pos_end"]),
-            _ptr(changed), _ptr(rewritten), int(bool(on_device))))
+            changed, per_item = a["changed"], a[counts]
+        _lib.check(call(None, _ptr(a["off"]), _ptr(a["ids"]), _ptr(a["pos_start"]), _ptr(a["pos_end"]), _ptr(changed),
+                        _ptr(per_item), int(bool(on_device))))
         if on_device and flags_on_device:
-            a["changed"], a["branch_rewritten"] = changed, rewritten
+            a["changed"], a[counts] = changed, per_item
         elif on_device:
             a["changed"][:] = changed.cpu().numpy()
-            a["branch_rewritten"][:] = rewritten.cpu().numpy().view(np.uint32)
+            a[counts][:] = per_item.cpu().numpy().view(np.uint32)
         return a
+
+    def tips(self) -> dict:
+        """the dead-end tips of the compacted graph (amira_gmg_tips), by unitig: per tip its unitig, orientation (+1: a
+        walk from the junction into the tip follows the unitig's listed order), attach state (the state of the junction
+        node a walk leaves through into the tip) and the read steps on it"""
+        Q = C.c_int64()
+        _lib.check(self._lib.amira_gmg_tips(self._h, C.byref(Q), *[None] * 4))
+        Q = Q.value
+        a = {"tip_unitig": np.empty(Q, np.int32), "tip_orient": np.empty(Q, np.int8), "tip_attach": np.empty(Q, np.int32),
+             "tip_reads": np.empty(Q, np.uint32)}
+        _lib.check(self._lib.amira_gmg_tips(self._h, None, *[_ptr(a[f]) for f in TIP_FIELDS]))
+        return a
+
+    def tip_count(self) -> int:
+        """the number of tips(), without exporting them"""
+        Q = C.c_int64()
+        _lib.check(self._lib.amira_gmg_tips(self._h, C.byref(Q), *[None] * 4))
+        return Q.value
+
+    def tip_policy(self, min_length: int, ranks=(), want_clip: bool = False):
+        """the clipping policy over tips() (amira_gmg_tip_policy): a tip is clipped when it has fewer than min_length
+        nodes, no node holding a gene of `ranks` (vocabulary ranks), and a sibling at its junction leads into a unitig of
+        strictly larger mean node coverage.  min_length = k + 1 covers single errors in a read's first or last k calls.
+        Returns the number of tips clipped, and with want_clip also clip (per tip: 1 or 0) as a numpy array.  The device
+        keeps the flags for clip_tip_reads(None)."""
+        r = np.ascontiguousarray(ranks, np.int32)
+        n = C.c_int64()
+        _lib.check(self._lib.amira_gmg_tip_policy(self._h, int(min_length), _ptr(r), len(r), C.byref(n), None))
+        if not want_clip:
+            return n.value
+        # sized after the call, as in bubble_policy
+        clip = np.empty(self.tip_count(), np.uint8)
+        if len(clip):
+            _lib.check(self._lib.amira_gmg_tip_policy(self._h, int(min_length), _ptr(r), len(r), None, _ptr(clip)))
+        return n.value, clip
+
+    def clip_tip_reads(self, clip=None, on_device: bool = False, flags_on_device: bool = False) -> dict:
+        """the reads that run into clipped tips, clipped (amira_gmg_clip_tip_reads): clip[q] = 1 clips tip q of tips(),
+        0 leaves it; None takes the flags of the last tip_policy().  An end clip drops the calls a read's last step
+        holds on the tip, a start clip those of its first step.  Returns the clipped CSR and changed as
+        correct_bubble_reads does, with tip_clipped (per tip: the read steps clipped) in place of branch_rewritten"""
+        Q = self.tip_count()
+        cf = None
+        if clip is not None:
+            cf = np.asarray(clip).ravel()
+            if len(cf) != Q or (len(cf) and not np.isin(cf, (0, 1)).all()):
+                raise ValueError("clip_tip_reads: clip must hold 0 or 1 for each of %d tips" % Q)
+            cf = np.ascontiguousarray(cf, np.uint8)
+        return self._corrected_csr(lambda *a: self._lib.amira_gmg_clip_tip_reads(self._h, _ptr(cf), *a), Q, "tip_clipped",
+                                   on_device, flags_on_device)
 
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""

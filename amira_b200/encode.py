@@ -190,7 +190,8 @@ class EncodedReads:
 
     def corrected(self, out: dict, device: int | None = None):
         """a new EncodedReads over the corrected CSR `out` (GeneMerGraph.correct_compacted_bubbles: ids, off,
-        pos_start, pos_end, changed per read, branch_rewritten per branch) of these reads.  It shares the vocabulary
+        pos_start, pos_end, changed per read, branch_rewritten per branch; GeneMerGraph.clip_compacted_tips: the same
+        with tip_clipped per tip in place of branch_rewritten) of these reads.  It shares the vocabulary
         and the read ids; its read / position dicts are shallow copies of these with only the changed reads decoded.
         With torch tensors in `out` (written on GPU `device`) they become its device CSR, and the host CSR is one copy
         of them.  This object is left as it is."""
@@ -202,7 +203,11 @@ class EncodedReads:
             csr = [None if x is None else x.cpu().numpy() for x in csr]
         new.ids, new.off, new.pos_start, new.pos_end = csr
         new.changed = np.asarray(out["changed"], np.uint8)
-        new.branch_rewritten = np.asarray(out["branch_rewritten"], np.uint32)
+        counts = [f for f in ("branch_rewritten", "tip_clipped") if f in out]
+        if not counts:
+            raise KeyError("corrected: no branch_rewritten or tip_clipped")
+        for f in counts:
+            setattr(new, f, np.asarray(out[f], np.uint32))
         new.reads = dict(self.reads)
         new.positions = dict(self.positions) if self.positions is not None else None
         names = self.vocab.names

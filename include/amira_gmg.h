@@ -339,6 +339,75 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
 int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_replaced,
                             int32_t *replace_with);
 
+/* The dead-end tips of the compacted graph (no upstream counterpart): the short chain of wrong gene-mers an error in
+ * the first or last k calls of a read makes, which leaves the true path at a junction and stops at the read's end.
+ * Over the unitigs of amira_gmg_unitigs and the read paths of amira_gmg_read_unitig_paths (reused while cached, not
+ * ranked again).  States, list(s) and cont(e) as for amira_gmg_bubbles; a read window on node n with direction d is in
+ * state 2n + (d < 0).
+ *
+ * Tip: a non-circular unitig b, h0 its first node and h1 its last in listed order (one node for a one-node unitig),
+ * with its two outward end states out1 = 2 * h1 + (node_orient[h1] < 0) (leaving h1 in listed order) and
+ * out0 = (2 * h0 + (node_orient[h0] < 0)) ^ 1 (leaving h0 against it), such that
+ *   1. exactly one of list(out0) and list(out1) is empty (the dead end), and
+ *   2. the other one, list(s_t), holds exactly one edge e', whose target v is not a node of b.
+ * By maximality list(attach) then holds two edges or more.  A unitig with both ends dead (a linear component) or both
+ * ends attached (a possible bubble branch) is no tip.
+ * Per tip, in ascending unitig order: tip_unitig = b; tip_orient = +1 when a walk from v into b follows b's listed
+ * order (the dead end is out1), -1 otherwise (for a one-node tip too: it depends on which state is dead);
+ * tip_attach = cont(e') ^ 1, the state a walk leaves v through into the tip; tip_reads = the read steps on b.
+ *
+ * Every pointer may be NULL.  Call with n_tips only to size the outputs, then again for the arrays: the result is
+ * kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.  Not available on a
+ * sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
+int amira_gmg_tips(amira_gmg *h, int64_t *n_tips, int32_t *tip_unitig, int8_t *tip_orient, int32_t *tip_attach,
+                   uint32_t *tip_reads);
+
+/* The clipping policy of the tips (no upstream counterpart), over the cached tips and unitigs, computed if not cached.
+ * Tip q on unitig b, attached at alpha = tip_attach[q], is clipped (clip[q] = 1, else 0) when
+ *   1. b has fewer than min_length nodes;
+ *   2. no node of b holds a gene of spare_ranks[n_ranks] (vocabulary ranks as amira_gmg_nodes_containing takes them);
+ *   3. some edge of list(alpha) whose target w is not on b leads into a unitig c with a strictly larger mean node
+ *      coverage: cov_sum[c] * len(b) > cov_sum[b] * len(c), compared exactly in 128 bits.  Equal means: not clipped.
+ * Condition 3 matters: the true path's own last unitig is often a dead end on the same junction, and so a tip too; it
+ * stays because its coverage is higher.  An error in the last (or first) k calls of a read makes a tip of at most k
+ * nodes, so min_length = k + 1 covers single end errors.
+ *
+ * Outputs: n_clipped = the tips clipped; clip[n_tips] (host, may be NULL).  The flags stay on the device, tagged with
+ * the tip cache they belong to, for amira_gmg_clip_tip_reads with clip == NULL.  One warp per tip scans list(alpha):
+ * d tips on one list of d edges cost O(d^2) in all.  AMIRA_E_ARG for bad ranks; AMIRA_E_STATE on a sharded handle.
+ * Leaves the graph, the caches and the filter masks as they were. */
+int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_ranks, int32_t n_ranks,
+                         int64_t *n_clipped, uint8_t *clip);
+
+/* The reads that run into clipped tips, clipped (no upstream counterpart): the tip counterpart of
+ * amira_gmg_correct_bubble_reads, from the build's input CSR and the cached read paths and tips.
+ *
+ * clip[n_tips] (host): 1 clips tip q, 0 leaves it; any other value is AMIRA_E_ARG.  NULL: the flags the last
+ * amira_gmg_tip_policy left on the device; AMIRA_E_STATE when there are tips and no policy was computed on the current
+ * tips (the graph or a device buffer changed since, or a call with host flags overwrote them).
+ * Clip: a read step (win = i, length = l) of read r with nw windows on the unitig of a clipped tip attached at alpha:
+ *   end clip:   i >= 1, i + l == nw, window i - 1 live with state alpha: the read's last l calls are dropped;
+ *   start clip: i == 0, l < nw, window l live with state alpha ^ 1: the read's first l calls are dropped.
+ * Window i covers calls [i, i + k), so the dropped calls are exactly those only tip windows hold; positions go with
+ * their calls.  A read may have a start clip and an end clip; they never overlap, and a clipped read keeps at least
+ * one window (k calls or more).  Left alone: a read lying wholly on a tip, a step that does not reach the read's end
+ * (None windows follow it), a flank window whose state does not match (a filter with min_edge_cov > 1 can do that),
+ * short reads, every other call and read.
+ *
+ * Outputs as amira_gmg_correct_bubble_reads: n_calls; read_off[R + 1], ids / pos_start / pos_end [n_calls], the
+ * clipped CSR in read order; changed[R] = 1 for a clipped read; tip_clipped[n_tips] = the steps clipped per tip.  Call
+ * with n_calls only to size the outputs, then again for the arrays; every output may be NULL.  out_on_device != 0: the
+ * array outputs are device pointers on the handle's device; a build from them can be given n_calls with
+ * amira_gmg_input_calls.  Leaves the graph, the caches and the filter masks as they were; AMIRA_E_STATE on a sharded
+ * handle.
+ *
+ * The tip and bubble calls reserve each other's buffers, so that on one graph a call of one family leaves the other's
+ * cache and policy in place (for example bubble_policy, tips, tip_policy, clip_tip_reads, then correct_bubble_reads
+ * with the held policy), as long as a call's gene ranks fit the room the handle holds for them. */
+int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
+                             int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped,
+                             int out_on_device);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
