@@ -32,8 +32,9 @@ void set_error(const char *fmt, ...);
         if (_s != AMIRA_OK) return _s; \
     } while (0)
 
-// Bumped whenever a device buffer is reallocated or two buffers trade places.  A captured CUDA graph holds raw
-// pointers: it may only be replayed while the generation it was captured at is still current.
+// Bumped whenever a device buffer is reallocated or two buffers trade places.  Its one reader is the replay key of a
+// captured build (GraphKey in gmg.cu): a captured CUDA graph holds raw pointers, so it may only be replayed while the
+// generation it was captured at is still current.
 inline std::atomic<uint64_t> &buffer_generation() {
     static std::atomic<uint64_t> g{0};
     return g;

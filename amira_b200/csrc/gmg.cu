@@ -185,64 +185,59 @@ struct amira_gmg {
         x_bm, x_pref, x_sorti2, x_sedge, x_redge, x_medge, x_gedge, x_etab, x_fan, cov_local;
     long long *h_cnt = nullptr;  // pinned, world*world + 4
 
-    // linear walks (paths.cuh): the jump table and the forest ranks of the walk states, valid while the graph they
-    // were computed from is (graph_version: bumped by every build and every filter / removal)
+    // The results derived from the graph after a build: cached tables and held policies.  Each one lives until the
+    // next build, filter or node removal, which all bump graph_version.  A table reads only graph buffers, which only
+    // those calls change, and its own and upstream tables' buffers, which are reserved only when they are recomputed.
     uint64_t graph_version = 0;
-    struct {
+    struct Derived {
+        bool valid = false;  // cleared on entering a recompute, so a failed one leaves no stale result
+        uint64_t version = 0;
+        bool fresh(const amira_gmg *h) const { return valid && version == h->graph_version; }
+        void stamp(const amira_gmg *h) {
+            valid = true;
+            version = h->graph_version;
+        }
+    };
+    // linear walks (paths.cuh): the jump table and the forest ranks of the walk states
+    struct : Derived {
         DevBuf jump, nxt, root[2], dist[2], is_label;
         DevBuf q_states, q_steps, q_len, q_off, q_bad, out;
         int L = 0, fin = 0;  // levels; which root / dist buffer holds the final ranks
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
     } walks;
-    // unitigs (unitigs.cuh): the ranking arrays of the 2N states and the compacted graph, valid under the same rule
-    struct {
+    // unitigs (unitigs.cuh): the ranking arrays of the 2N states and the compacted graph
+    struct : Derived {
         DevBuf succ, ptr[2], dist[2], mn[2], circ, any_cycle, uid, len, n_unitigs;
         DevBuf node_unitig, node_pos, node_orient, off, nodes, circular, cov_sum, cov_min, cov_max, edge_internal;
         int64_t U = 0;
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
     } unitigs;
-    // the junction edges as links between unitig ends, and the reads as steps along unitigs (unitigs.cuh), valid under
-    // the same rule
-    struct {
+    // the junction edges as links between unitig ends, and the reads as steps along unitigs (unitigs.cuh)
+    struct : Derived {
         DevBuf n_links, edge, from_unitig, from_orient, to_unitig, to_orient, cov;
         int64_t L = 0;
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
     } links;
-    struct {
+    struct : Derived {
         DevBuf flags, n_steps, path_off, unitig, orient, pos, win, length;
         int64_t T = 0;
         bool on_device = false;  // path_off was computed (else every read's path is empty)
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
     } paths;
-    // the simple bubbles of the compacted graph (bubbles.cuh), valid under the same rule
-    struct {
+    // the simple bubbles of the compacted graph (bubbles.cuh)
+    struct : Derived {
         DevBuf edge_tau, ebr, ebub, ehead, counts, first, n_out;
         DevBuf source, sink, branch_off, branch_unitig, branch_orient, branch_reads, unitig_branch;
         int64_t B = 0, NB = 0;
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
     } bubbles;
     // the scratch of amira_gmg_correct_bubble_reads (correct.cuh), recomputed by every call, and the replace_with of
-    // the last amira_gmg_bubble_policy, valid for the bubble cache (version, generation) it was computed on
+    // the last amira_gmg_bubble_policy, held while `policy` is fresh
     struct {
         DevBuf replace, spared, cnt, idx, step_new, changed, rewritten, n_out;
-        bool policy = false;
-        uint64_t policy_version = 0, policy_generation = 0;
+        Derived policy;
     } correct;
-    // the dead-end tips of the compacted graph (tips.cuh), valid under the rule of the unitigs, and the clip flags of
-    // the last amira_gmg_tip_policy (or host flags of amira_gmg_clip_tip_reads), with the tip cache they belong to.
-    // amira_gmg_clip_tip_reads uses the correction's cnt / idx / changed / n_out as scratch.
-    struct {
+    // the dead-end tips of the compacted graph (tips.cuh), and the clip flags of the last amira_gmg_tip_policy, held
+    // while `policy` is fresh.  amira_gmg_clip_tip_reads uses the correction's scratch.
+    struct : Derived {
         DevBuf flags, n_out, tip_unitig, orient, attach, reads, unitig_tip, clip, spared, clipped;
         int64_t Q = 0;
-        bool valid = false;
-        uint64_t version = 0, generation = 0;
-        bool policy = false;
-        uint64_t policy_version = 0, policy_generation = 0;
+        Derived policy;
     } tips;
 };
 
@@ -1931,6 +1926,16 @@ int stats_ready(amira_gmg *h) {
     AMIRA_TRY(finish(h, false));
     return h->built ? AMIRA_OK : h->last_status;
 }
+
+// stats_ready for the walks and the compacted graph, which need the whole graph's reads on one GPU
+int unsharded_ready(amira_gmg *h, const char *call) {
+    AMIRA_TRY(stats_ready(h));
+    if (h->world > 1) {
+        set_error("%s: not available on a sharded graph", call);
+        return AMIRA_E_STATE;
+    }
+    return AMIRA_OK;
+}
 }  // namespace
 
 int amira_gmg_read_length_coverages(amira_gmg *h, const int32_t *min_len, int32_t n, int64_t *sums) {
@@ -2084,12 +2089,11 @@ int amira_gmg_linear_steps(amira_gmg *h, uint32_t *degree, int32_t *fw_next, int
 }
 
 namespace {
-// jump table and forest ranks of the 2N walk states (paths.cuh), reused while neither the graph nor any device buffer
-// has changed since they were computed
+// jump table and forest ranks of the 2N walk states (paths.cuh), reused while the graph stays the same
 int walk_table(amira_gmg *h, WalkTable &T) {
     auto &w = h->walks;
     const long long S = 2 * h->n_nodes;
-    if (!(w.valid && w.version == h->graph_version && w.generation == buffer_generation())) {
+    if (!w.fresh(h)) {
         w.valid = false;
         int L = 1;
         while ((1ll << L) <= S) ++L;
@@ -2117,9 +2121,7 @@ int walk_table(amira_gmg *h, WalkTable &T) {
         for (int l = 0; l < L; ++l) LAUNCH(h, k_walk_rank_round, grid, 256, r[l & 1], d[l & 1], r[(l + 1) & 1], d[(l + 1) & 1], S);
         w.L = L;
         w.fin = L & 1;
-        w.version = h->graph_version;
-        w.generation = buffer_generation();
-        w.valid = true;
+        w.stamp(h);
     }
     T.J = w.jump.as<int32_t>();
     T.nxt = w.nxt.as<int32_t>();
@@ -2133,11 +2135,7 @@ int walk_table(amira_gmg *h, WalkTable &T) {
 
 int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int want_branched, int64_t *walk_off,
                            int32_t *walk_nodes) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("linear_walks: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "linear_walks"));
     if (n < 0 || (n > 0 && !states) || !walk_off) {
         set_error("linear_walks: bad arguments (n = %lld)", (long long)n);
         return AMIRA_E_ARG;
@@ -2194,11 +2192,11 @@ int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int w
 }
 
 namespace {
-// the compacted graph (unitigs.cuh), reused while neither the graph nor any device buffer has changed since it was
-// computed
+// the compacted graph (unitigs.cuh), reused while the graph stays the same; every table of the compacted graph starts
+// here, so this is where the states are checked to fit
 int unitig_table(amira_gmg *h) {
     auto &u = h->unitigs;
-    if (u.valid && u.version == h->graph_version && u.generation == buffer_generation()) return AMIRA_OK;
+    if (u.fresh(h)) return AMIRA_OK;
     u.valid = false;
     const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
     if (S >= (1ll << 31)) {
@@ -2273,9 +2271,7 @@ int unitig_table(amira_gmg *h) {
         AMIRA_CUDA(cudaStreamSynchronize(st));
         u.U = U;
     }
-    u.version = h->graph_version;
-    u.generation = buffer_generation();
-    u.valid = true;
+    u.stamp(h);
     return AMIRA_OK;
 }
 }  // namespace
@@ -2283,11 +2279,7 @@ int unitig_table(amira_gmg *h) {
 int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, int32_t *node_pos, int8_t *node_orient,
                       int64_t *unitig_off, int32_t *unitig_nodes, uint8_t *circular, int64_t *cov_sum, uint32_t *cov_min,
                       uint32_t *cov_max, uint8_t *edge_internal) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("unitigs: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "unitigs"));
     AMIRA_TRY(unitig_table(h));
     const auto &u = h->unitigs;
     const int64_t N = h->n_nodes, E = h->n_edges, U = u.U;
@@ -2311,18 +2303,14 @@ int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, in
 }
 
 namespace {
-// the scan tile states of a scan over n items, reserved ahead (a buffer that grows bumps the buffer generation)
-int reserve_scan(amira_gmg *h, int64_t n) {
-    return h->scan_state[0].reserve(sizeof(unsigned long long) * (size_t)scan_tiles(n));
-}
-
-// the links of the compacted graph, cached under the rule of unitig_table.  Every buffer is reserved before
-// unitig_table runs: a reservation that grows bumps the buffer generation and would drop the unitigs just computed.
+// the links of the compacted graph, cached under the rule of unitig_table
 int unitig_links_table(amira_gmg *h) {
     auto &l = h->links;
-    if (l.valid && l.version == h->graph_version && l.generation == buffer_generation()) return AMIRA_OK;
+    if (l.fresh(h)) return AMIRA_OK;
     l.valid = false;
+    AMIRA_TRY(unitig_table(h));
     const long long E = h->n_edges;
+    l.L = 0;
     if (E > 0) {
         const size_t e4 = sizeof(int32_t) * (size_t)E;
         AMIRA_TRY(l.n_links.reserve(sizeof(long long)));
@@ -2332,11 +2320,6 @@ int unitig_links_table(amira_gmg *h) {
         AMIRA_TRY(l.to_unitig.reserve(e4));
         AMIRA_TRY(l.to_orient.reserve((size_t)E));
         AMIRA_TRY(l.cov.reserve(e4));
-        AMIRA_TRY(reserve_scan(h, E));
-    }
-    AMIRA_TRY(unitig_table(h));
-    l.L = 0;
-    if (E > 0) {
         const auto &u = h->unitigs;
         cudaStream_t st = h->stream;
         long long *d_L = l.n_links.as<long long>();
@@ -2352,21 +2335,21 @@ int unitig_links_table(amira_gmg *h) {
                    l.to_unitig.as<int32_t>(), l.to_orient.as<int8_t>(), l.cov.as<uint32_t>());
         l.L = L;
     }
-    l.version = h->graph_version;
-    l.generation = buffer_generation();
-    l.valid = true;
+    l.stamp(h);
     return AMIRA_OK;
 }
 
-// the reads as steps along the unitigs, cached under the same rule; reserved ahead for the same reason, with W as
-// the bound on the number of steps
+// the reads as steps along the unitigs, cached under the same rule, with W as the bound on the number of steps
 int read_path_table(amira_gmg *h) {
     auto &p = h->paths;
-    if (p.valid && p.version == h->graph_version && p.generation == buffer_generation()) return AMIRA_OK;
+    if (p.fresh(h)) return AMIRA_OK;
     p.valid = false;
+    AMIRA_TRY(unitig_table(h));
     const long long R = h->R, W = h->W, N = h->n_nodes;
     // without a node every window is None, and without a window every read is short: all paths are empty
     const bool steps = W > 0 && N > 0;
+    p.T = 0;
+    p.on_device = steps;
     if (steps) {
         const size_t w4 = sizeof(int32_t) * (size_t)W;
         AMIRA_TRY(p.flags.reserve((size_t)W));
@@ -2377,12 +2360,6 @@ int read_path_table(amira_gmg *h) {
         AMIRA_TRY(p.pos.reserve(w4));
         AMIRA_TRY(p.win.reserve(w4));
         AMIRA_TRY(p.length.reserve(w4));
-        AMIRA_TRY(reserve_scan(h, W));
-    }
-    AMIRA_TRY(unitig_table(h));
-    p.T = 0;
-    p.on_device = steps;
-    if (steps) {
         const auto &u = h->unitigs;
         cudaStream_t st = h->stream;
         const int32_t *win_node = h->win_node.as<int32_t>(), *win_read = h->win_read.as<int32_t>();
@@ -2402,20 +2379,14 @@ int read_path_table(amira_gmg *h) {
         if (T > 0) LAUNCH(h, k_read_step_lengths, grid_for(T, 256), 256, p.win.as<int32_t>(), T, p.length.as<int32_t>());
         p.T = T;
     }
-    p.version = h->graph_version;
-    p.generation = buffer_generation();
-    p.valid = true;
+    p.stamp(h);
     return AMIRA_OK;
 }
 }  // namespace
 
 int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_t *from_unitig, int8_t *from_orient,
                            int32_t *to_unitig, int8_t *to_orient, uint32_t *cov) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("unitig_links: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "unitig_links"));
     AMIRA_TRY(unitig_links_table(h));
     const auto &l = h->links;
     const int64_t L = l.L;
@@ -2433,11 +2404,7 @@ int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_
 
 int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig, int8_t *orient, int32_t *pos,
                                 int32_t *win, int32_t *length) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("read_unitig_paths: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "read_unitig_paths"));
     AMIRA_TRY(read_path_table(h));
     const auto &p = h->paths;
     const int64_t R = h->R, T = p.T;
@@ -2457,91 +2424,31 @@ int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig
 }
 
 namespace {
-// The buffers of the bubble and tip calls are all reserved together, by every one of them, before the cached
-// unitigs, paths, bubbles or tips are looked at: a reservation that grows bumps the buffer generation and would drop
-// those caches and the policy computed on them.  So interleaving bubble and tip calls on one graph loses neither.
-//
-// The bubbles: a bubble has two branches or more and a branch is one edge of its list, so E bounds the branches and
-// E / 2 the bubbles.
-int reserve_bubbles(amira_gmg *h) {
-    auto &q = h->bubbles;
-    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
-    if (E == 0) return AMIRA_OK;  // without an edge there is no branch
-    const size_t e4 = sizeof(int32_t) * (size_t)E;
-    AMIRA_TRY(q.edge_tau.reserve(e4));
-    AMIRA_TRY(q.ebr.reserve(e4));
-    AMIRA_TRY(q.ebub.reserve(e4));
-    AMIRA_TRY(q.ehead.reserve(e4));
-    AMIRA_TRY(q.counts.reserve(sizeof(unsigned long long) * (size_t)S));
-    AMIRA_TRY(q.first.reserve(sizeof(unsigned long long) * (size_t)S));
-    AMIRA_TRY(q.n_out.reserve(sizeof(unsigned long long)));
-    AMIRA_TRY(q.source.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
-    AMIRA_TRY(q.sink.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
-    AMIRA_TRY(q.branch_off.reserve(sizeof(int64_t) * (size_t)(E / 2 + 1)));
-    AMIRA_TRY(q.branch_unitig.reserve(e4));
-    AMIRA_TRY(q.branch_orient.reserve((size_t)E));
-    AMIRA_TRY(q.branch_reads.reserve(e4));
-    AMIRA_TRY(q.unitig_branch.reserve(sizeof(int32_t) * (size_t)N));
-    return reserve_scan(h, S);
-}
-
-// the policy and correction buffers of the bubbles; cnt / idx / changed / n_out also serve amira_gmg_clip_tip_reads
-int reserve_correct(amira_gmg *h) {
-    auto &c = h->correct;
-    const long long R = h->R, G = R > 0 ? h->G : 0, E = h->n_edges, W = h->W;
-    if (R == 0) return AMIRA_OK;
-    const size_t e4 = sizeof(int32_t) * (size_t)std::max<long long>(E, 1);
-    AMIRA_TRY(c.replace.reserve(e4));
-    AMIRA_TRY(c.spared.reserve((size_t)std::max<long long>(E, 1)));
-    AMIRA_TRY(c.rewritten.reserve(e4));
-    AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
-    AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
-    AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
-    AMIRA_TRY(c.changed.reserve((size_t)R));
-    AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
-    return reserve_scan(h, G);
-}
-
-// the tips: a unitig is at most one tip, and N bounds the unitigs
-int reserve_tips(amira_gmg *h) {
-    auto &t = h->tips;
-    const long long N = h->n_nodes;
-    if (N == 0) return AMIRA_OK;
-    const size_t n4 = sizeof(int32_t) * (size_t)N;
-    AMIRA_TRY(t.flags.reserve((size_t)N));
-    AMIRA_TRY(t.n_out.reserve(sizeof(unsigned long long)));
-    AMIRA_TRY(t.tip_unitig.reserve(n4));
-    AMIRA_TRY(t.orient.reserve((size_t)N));
-    AMIRA_TRY(t.attach.reserve(n4));
-    AMIRA_TRY(t.reads.reserve(n4));
-    AMIRA_TRY(t.unitig_tip.reserve(n4));
-    AMIRA_TRY(t.clip.reserve((size_t)N));
-    AMIRA_TRY(t.spared.reserve((size_t)N));
-    AMIRA_TRY(t.clipped.reserve(n4));
-    return reserve_scan(h, N);
-}
-
-int reserve_cleaning(amira_gmg *h) {
-    AMIRA_TRY(reserve_bubbles(h));
-    AMIRA_TRY(reserve_correct(h));
-    return reserve_tips(h);
-}
-
-// the simple bubbles, cached under the rule of unitig_table
+// the simple bubbles, cached under the rule of unitig_table.  A bubble has two branches or more and a branch is one
+// edge of its list, so E bounds the branches and E / 2 the bubbles.
 int bubble_table(amira_gmg *h) {
     auto &q = h->bubbles;
-    if (q.valid && q.version == h->graph_version && q.generation == buffer_generation()) return AMIRA_OK;
+    if (q.fresh(h)) return AMIRA_OK;
     q.valid = false;
-    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
-    if (S >= (1ll << 31)) {
-        set_error("bubbles: %lld nodes, the states 2 * node + side must fit in 31 bits", N);
-        return AMIRA_E_ARG;
-    }
-    const bool any = E > 0;  // without an edge there is no branch
-    AMIRA_TRY(reserve_cleaning(h));
     AMIRA_TRY(read_path_table(h));
+    const long long N = h->n_nodes, E = h->n_edges, S = 2 * N;
     q.B = q.NB = 0;
-    if (any) {
+    if (E > 0) {  // without an edge there is no branch
+        const size_t e4 = sizeof(int32_t) * (size_t)E;
+        AMIRA_TRY(q.edge_tau.reserve(e4));
+        AMIRA_TRY(q.ebr.reserve(e4));
+        AMIRA_TRY(q.ebub.reserve(e4));
+        AMIRA_TRY(q.ehead.reserve(e4));
+        AMIRA_TRY(q.counts.reserve(sizeof(unsigned long long) * (size_t)S));
+        AMIRA_TRY(q.first.reserve(sizeof(unsigned long long) * (size_t)S));
+        AMIRA_TRY(q.n_out.reserve(sizeof(unsigned long long)));
+        AMIRA_TRY(q.source.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.sink.reserve(sizeof(int32_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.branch_off.reserve(sizeof(int64_t) * (size_t)(E / 2 + 1)));
+        AMIRA_TRY(q.branch_unitig.reserve(e4));
+        AMIRA_TRY(q.branch_orient.reserve((size_t)E));
+        AMIRA_TRY(q.branch_reads.reserve(e4));
+        AMIRA_TRY(q.unitig_branch.reserve(sizeof(int32_t) * (size_t)N));
         const auto &u = h->unitigs;
         const auto &p = h->paths;
         cudaStream_t st = h->stream;
@@ -2579,20 +2486,14 @@ int bubble_table(amira_gmg *h) {
                        unitig_branch, u.off.as<int64_t>(), branch_reads);
         }
     }
-    q.version = h->graph_version;
-    q.generation = buffer_generation();
-    q.valid = true;
+    q.stamp(h);
     return AMIRA_OK;
 }
 }  // namespace
 
 int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int32_t *source, int32_t *sink,
                       int64_t *branch_off, int32_t *branch_unitig, int8_t *branch_orient, uint32_t *branch_reads) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("bubbles: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "bubbles"));
     AMIRA_TRY(bubble_table(h));
     const auto &q = h->bubbles;
     const int64_t B = q.B, NB = q.NB;
@@ -2613,8 +2514,8 @@ int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int
 }
 
 namespace {
-// a device allocation for the length of one call (the staging of host outputs).  It is not a handle buffer, so it
-// leaves the buffer generation, and with it the cached unitigs, read paths and bubbles, alone.
+// a device allocation for the length of one call (the staging of host outputs): the handle holds no memory for it
+// between calls
 struct CallBuf {
     void *p = nullptr;
     cudaStream_t st = nullptr;
@@ -2625,26 +2526,23 @@ struct CallBuf {
 }  // namespace
 
 int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_replaced, int32_t *replace_with) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("bubble_policy: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "bubble_policy"));
     if (n_ranks < 0 || (n_ranks > 0 && !spare_ranks)) {
         set_error("bubble_policy: bad gene ranks (n = %d)", n_ranks);
         return AMIRA_E_ARG;
     }
     auto &c = h->correct;
-    c.policy = false;
-    // every reservation before the bubbles, the gene flags' (scratch_off, comp_max) included
-    AMIRA_TRY(reserve_cleaning(h));
+    c.policy.valid = false;
     if (n_ranks > 0) AMIRA_TRY(flag_nodes_containing(h, spare_ranks, n_ranks));
     AMIRA_TRY(bubble_table(h));
     const auto &q = h->bubbles;
-    const int64_t B = q.B, NB = q.NB, N = h->n_nodes;
+    const int64_t B = q.B, NB = q.NB, N = h->n_nodes, E = h->n_edges;
     cudaStream_t st = h->stream;
     unsigned long long total = 0;
     if (NB > 0) {
+        AMIRA_TRY(c.replace.reserve(sizeof(int32_t) * (size_t)E));
+        AMIRA_TRY(c.spared.reserve((size_t)E));
+        AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
         uint8_t *spared = c.spared.as<uint8_t>();
         unsigned long long *d_n = c.n_out.as<unsigned long long>();
         AMIRA_CUDA(cudaMemsetAsync(spared, 0, (size_t)NB, st));
@@ -2661,9 +2559,7 @@ int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_
         AMIRA_CUDA(cudaStreamSynchronize(st));
     }
     if (n_replaced) *n_replaced = (int64_t)total;
-    c.policy = true;
-    c.policy_version = q.version;
-    c.policy_generation = q.generation;
+    c.policy.stamp(h);
     return AMIRA_OK;
 }
 
@@ -2679,11 +2575,17 @@ int corrected_without_reads(amira_gmg *h, int64_t *n_calls, int64_t *read_off, i
     return AMIRA_OK;
 }
 
-// before the marks of a correction (R > 0): no read changed, every call untouched
+// the scratch of a correction (R > 0) before its marks: no read changed, every call untouched
 int clear_correct(amira_gmg *h) {
     auto &c = h->correct;
-    const long long R = h->R, G = h->G;
+    const long long R = h->R, G = h->G, E = h->n_edges, W = h->W;
     cudaStream_t st = h->stream;
+    AMIRA_TRY(c.rewritten.reserve(sizeof(int32_t) * (size_t)std::max<long long>(E, 1)));
+    AMIRA_TRY(c.cnt.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(G, 1)));
+    AMIRA_TRY(c.idx.reserve(sizeof(int64_t) * (size_t)(G + 1)));
+    AMIRA_TRY(c.step_new.reserve(sizeof(int32_t) * (size_t)std::max<long long>(W, 1)));
+    AMIRA_TRY(c.changed.reserve((size_t)R));
+    AMIRA_TRY(c.n_out.reserve(sizeof(unsigned long long)));
     AMIRA_CUDA(cudaMemsetAsync(c.changed.p, 0, (size_t)R, st));
     AMIRA_CUDA(cudaMemsetAsync(c.idx.p, 0, sizeof(int64_t), st));  // idx[0] when there is no call
     h->lib_launches += 2;
@@ -2768,21 +2670,16 @@ int write_corrected(amira_gmg *h, bool edits, int64_t *n_calls, int64_t *read_of
 int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                                    int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
                                    int out_on_device) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("correct_bubble_reads: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "correct_bubble_reads"));
     auto &c = h->correct;
     const long long R = h->R;
-    AMIRA_TRY(reserve_cleaning(h));
     AMIRA_TRY(bubble_table(h));
     const auto &q = h->bubbles;
     const int64_t B = q.B, NB = q.NB;
     cudaStream_t st = h->stream;
     // NULL: the replace_with of the last policy, which the device holds, valid by construction
     const bool held = NB > 0 && !replace_with;
-    if (held && !(c.policy && c.policy_version == q.version && c.policy_generation == q.generation)) {
+    if (held && !c.policy.fresh(h)) {
         set_error("correct_bubble_reads: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles",
                   (long long)NB);
         return AMIRA_E_STATE;
@@ -2803,15 +2700,15 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
     }
     if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no bubble
     const auto &p = h->paths;
-    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
-    int32_t *replace = c.replace.as<int32_t>();
     AMIRA_TRY(clear_correct(h));
+    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
     if (NB > 0) {
         AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
         h->lib_launches++;
         if (!held) {
-            c.policy = false;  // the policy's replace_with is overwritten
-            AMIRA_CUDA(cudaMemcpyAsync(replace, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
+            c.policy.valid = false;  // the policy's replace_with is overwritten
+            AMIRA_TRY(c.replace.reserve(sizeof(int32_t) * (size_t)h->n_edges));
+            AMIRA_CUDA(cudaMemcpyAsync(c.replace.p, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
             h->lib_launches++;
         }
         if (p.T > 0)
@@ -2819,30 +2716,33 @@ int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, in
                    (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
                    h->win_dir.as<int8_t>(), h->off, h->unitigs.off.as<int64_t>(), q.unitig_branch.as<int32_t>(),
                    q.branch_off.as<int64_t>(), (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(),
-                   q.branch_unitig.as<int32_t>(), replace, cnt, c.step_new.as<int32_t>(), c.changed.as<uint8_t>(), rewritten);
+                   q.branch_unitig.as<int32_t>(), c.replace.as<int32_t>(), cnt, c.step_new.as<int32_t>(), c.changed.as<uint8_t>(),
+                   rewritten);
     }
     return write_corrected(h, true, n_calls, read_off, ids, pos_start, pos_end, changed, branch_rewritten, rewritten, NB,
                            out_on_device);
 }
 
 namespace {
-// the tips, cached under the rule of unitig_table; every buffer reserved ahead (reserve_cleaning)
+// the tips, cached under the rule of unitig_table.  A unitig is at most one tip, and N bounds the unitigs.
 int tip_table(amira_gmg *h) {
     auto &t = h->tips;
-    if (t.valid && t.version == h->graph_version && t.generation == buffer_generation()) return AMIRA_OK;
+    if (t.fresh(h)) return AMIRA_OK;
     t.valid = false;
-    const long long N = h->n_nodes;
-    if (2 * N >= (1ll << 31)) {
-        set_error("tips: %lld nodes, the states 2 * node + side must fit in 31 bits", N);
-        return AMIRA_E_ARG;
-    }
-    AMIRA_TRY(reserve_cleaning(h));
     AMIRA_TRY(read_path_table(h));
     t.Q = 0;
     const auto &u = h->unitigs;
     const auto &p = h->paths;
-    const long long U = u.U;
+    const long long N = h->n_nodes, U = u.U;
     if (U > 0) {
+        const size_t n4 = sizeof(int32_t) * (size_t)N;
+        AMIRA_TRY(t.flags.reserve((size_t)N));
+        AMIRA_TRY(t.n_out.reserve(sizeof(unsigned long long)));
+        AMIRA_TRY(t.tip_unitig.reserve(n4));
+        AMIRA_TRY(t.orient.reserve((size_t)N));
+        AMIRA_TRY(t.attach.reserve(n4));
+        AMIRA_TRY(t.reads.reserve(n4));
+        AMIRA_TRY(t.unitig_tip.reserve(n4));
         cudaStream_t st = h->stream;
         const int64_t *adj_off = h->adj_off.as<int64_t>();
         const uint32_t *adj_edges = h->adj_edges.as<uint32_t>();
@@ -2869,20 +2769,14 @@ int tip_table(amira_gmg *h) {
         }
         t.Q = (int64_t)Q;
     }
-    t.version = h->graph_version;
-    t.generation = buffer_generation();
-    t.valid = true;
+    t.stamp(h);
     return AMIRA_OK;
 }
 }  // namespace
 
 int amira_gmg_tips(amira_gmg *h, int64_t *n_tips, int32_t *tip_unitig, int8_t *tip_orient, int32_t *tip_attach,
                    uint32_t *tip_reads) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("tips: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "tips"));
     AMIRA_TRY(tip_table(h));
     const auto &t = h->tips;
     const int64_t Q = t.Q;
@@ -2898,25 +2792,21 @@ int amira_gmg_tips(amira_gmg *h, int64_t *n_tips, int32_t *tip_unitig, int8_t *t
 
 int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_ranks, int32_t n_ranks, int64_t *n_clipped,
                          uint8_t *clip) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("tip_policy: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "tip_policy"));
     if (n_ranks < 0 || (n_ranks > 0 && !spare_ranks)) {
         set_error("tip_policy: bad gene ranks (n = %d)", n_ranks);
         return AMIRA_E_ARG;
     }
     auto &t = h->tips;
-    t.policy = false;
-    // every reservation before the tips, the gene flags' (scratch_off, comp_max) included
-    AMIRA_TRY(reserve_cleaning(h));
+    t.policy.valid = false;
     if (n_ranks > 0) AMIRA_TRY(flag_nodes_containing(h, spare_ranks, n_ranks));
     AMIRA_TRY(tip_table(h));
     const int64_t Q = t.Q, N = h->n_nodes;
     cudaStream_t st = h->stream;
     unsigned long long total = 0;
     if (Q > 0) {
+        AMIRA_TRY(t.clip.reserve((size_t)N));
+        AMIRA_TRY(t.spared.reserve((size_t)N));
         uint8_t *spared = t.spared.as<uint8_t>();
         unsigned long long *d_n = t.n_out.as<unsigned long long>();
         AMIRA_CUDA(cudaMemsetAsync(spared, 0, (size_t)Q, st));
@@ -2934,29 +2824,22 @@ int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_
         AMIRA_CUDA(cudaStreamSynchronize(st));
     }
     if (n_clipped) *n_clipped = (int64_t)total;
-    t.policy = true;
-    t.policy_version = t.version;
-    t.policy_generation = t.generation;
+    t.policy.stamp(h);
     return AMIRA_OK;
 }
 
 int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                              int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped, int out_on_device) {
-    AMIRA_TRY(stats_ready(h));
-    if (h->world > 1) {
-        set_error("clip_tip_reads: not available on a sharded graph");
-        return AMIRA_E_STATE;
-    }
+    AMIRA_TRY(unsharded_ready(h, "clip_tip_reads"));
     auto &t = h->tips;
     auto &c = h->correct;
-    const long long R = h->R;
-    AMIRA_TRY(reserve_cleaning(h));
+    const long long R = h->R, N = h->n_nodes;
     AMIRA_TRY(tip_table(h));
     const int64_t Q = t.Q;
     cudaStream_t st = h->stream;
     // NULL: the clip flags of the last policy, which the device holds
     const bool held = Q > 0 && !clip;
-    if (held && !(t.policy && t.policy_version == t.version && t.policy_generation == t.generation)) {
+    if (held && !t.policy.fresh(h)) {
         set_error("clip_tip_reads: no clip flags for %lld tips, and no amira_gmg_tip_policy on these tips", (long long)Q);
         return AMIRA_E_STATE;
     }
@@ -2968,13 +2851,14 @@ int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls
             }
     if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no tip
     const auto &p = h->paths;
-    uint32_t *clipped = t.clipped.as<uint32_t>();
     AMIRA_TRY(clear_correct(h));
     if (Q > 0) {
-        AMIRA_CUDA(cudaMemsetAsync(clipped, 0, sizeof(uint32_t) * (size_t)Q, st));
+        AMIRA_TRY(t.clipped.reserve(sizeof(int32_t) * (size_t)N));
+        AMIRA_CUDA(cudaMemsetAsync(t.clipped.p, 0, sizeof(uint32_t) * (size_t)Q, st));
         h->lib_launches++;
         if (!held) {
-            t.policy = false;  // the policy's flags are overwritten
+            t.policy.valid = false;  // the policy's flags are overwritten
+            AMIRA_TRY(t.clip.reserve((size_t)N));
             AMIRA_CUDA(cudaMemcpyAsync(t.clip.p, clip, (size_t)Q, cudaMemcpyHostToDevice, st));
             h->lib_launches++;
         }
@@ -2982,10 +2866,10 @@ int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls
             LAUNCH(h, k_tip_clip, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
                    (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
                    h->win_dir.as<int8_t>(), h->off, t.unitig_tip.as<int32_t>(), t.attach.as<int32_t>(), t.clip.as<uint8_t>(),
-                   c.cnt.as<uint32_t>(), c.changed.as<uint8_t>(), clipped);
+                   c.cnt.as<uint32_t>(), c.changed.as<uint8_t>(), t.clipped.as<uint32_t>());
     }
-    return write_corrected(h, false, n_calls, read_off, ids, pos_start, pos_end, changed, tip_clipped, clipped, Q,
-                           out_on_device);
+    return write_corrected(h, false, n_calls, read_off, ids, pos_start, pos_end, changed, tip_clipped,
+                           t.clipped.as<uint32_t>(), Q, out_on_device);
 }
 
 int amira_gmg_debug_segsort(amira_gmg *h, uint32_t *data, const int64_t *off, int64_t n_seg, uint32_t *dups,

@@ -228,7 +228,6 @@ class DeviceGraph:
         _lib.check(self._lib.amira_gmg_bubble_policy(self._h, _ptr(r), len(r), C.byref(n), None))
         if not want_replace_with:
             return n.value
-        # sized after the call: counting the branches first would compute the bubbles before the policy's reservations
         rw = np.empty(self.bubble_counts()[1], np.int32)
         if len(rw):
             _lib.check(self._lib.amira_gmg_bubble_policy(self._h, _ptr(r), len(r), None, _ptr(rw)))
@@ -311,7 +310,6 @@ class DeviceGraph:
         _lib.check(self._lib.amira_gmg_tip_policy(self._h, int(min_length), _ptr(r), len(r), C.byref(n), None))
         if not want_clip:
             return n.value
-        # sized after the call, as in bubble_policy
         clip = np.empty(self.tip_count(), np.uint8)
         if len(clip):
             _lib.check(self._lib.amira_gmg_tip_policy(self._h, int(min_length), _ptr(r), len(r), None, _ptr(clip)))

@@ -208,7 +208,7 @@ int amira_gmg_linear_walks(amira_gmg *h, const int32_t *states, int64_t n, int w
  *   per directed edge [E]: edge_internal = 1 when the edge joins consecutive nodes of one unitig (in either
  *     direction); the others are the junctions.  There are 2 * (N - linear unitigs) internal edges.
  * Every pointer may be NULL.  Call with n_unitigs only to size the per-unitig arrays, then again for the arrays: the
- * result is kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.
+ * result is kept on the device until the next build, filter or node removal.  Leaves the filter masks alone.
  * Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
 int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, int32_t *node_pos, int8_t *node_orient,
                       int64_t *unitig_off, int32_t *unitig_nodes, uint8_t *circular, int64_t *cov_sum, uint32_t *cov_min,
@@ -238,8 +238,8 @@ int amira_gmg_unitigs(amira_gmg *h, int64_t *n_unitigs, int32_t *node_unitig, in
  *   windows are all None have empty paths.
  *
  * Both calls: every pointer may be NULL.  Call with n_links only, or path_off only, to size the outputs, then again
- * for the arrays: the results are kept on the device until the graph or a device buffer changes.  Leave the filter
- * masks alone.  Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
+ * for the arrays: the results are kept on the device until the next build, filter or node removal.  Leave the
+ * filter masks alone.  Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
 int amira_gmg_unitig_links(amira_gmg *h, int64_t *n_links, int32_t *edge, int32_t *from_unitig, int8_t *from_orient,
                            int32_t *to_unitig, int8_t *to_orient, uint32_t *cov);
 int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig, int8_t *orient, int32_t *pos,
@@ -279,8 +279,8 @@ int amira_gmg_read_unitig_paths(amira_gmg *h, int64_t *path_off, int32_t *unitig
  * branches without a node (an edge joining the two junction nodes directly, as a deletion makes at k = 1).
  *
  * Every pointer may be NULL.  Call with n_bubbles / n_branches only to size the outputs, then again for the arrays:
- * the result is kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.  Not
- * available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31.  Grouping a list of d edges takes
+ * the result is kept on the device until the next build, filter or node removal.  Leaves the filter masks alone.
+ * Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31.  Grouping a list of d edges takes
  * O(d^2 / 32) warp steps. */
 int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int32_t *source, int32_t *sink,
                       int64_t *branch_off, int32_t *branch_unitig, int8_t *branch_orient, uint32_t *branch_reads);
@@ -292,7 +292,7 @@ int amira_gmg_bubbles(amira_gmg *h, int64_t *n_bubbles, int64_t *n_branches, int
  * replace_with[n_branches] (host): per branch g of amira_gmg_bubbles, -1 leaves g's reads alone; otherwise it is
  * another branch of the same bubble, whose genes replace g's calls.  NULL: the replace_with the last
  * amira_gmg_bubble_policy left on the device, used without a host check (it is valid by construction); AMIRA_E_STATE
- * when there are branches and no policy was computed on the current bubbles (the graph or a device buffer changed
+ * when there are branches and no policy was computed on the current bubbles (a build, filter or node removal came
  * since, or a call with a host replace_with overwrote it).
  * Edit: a read step (amira_gmg_read_unitig_paths) on branch g = unitig b of m nodes in bubble (sigma, tau), with
  * replace_with[g] >= 0, length m, the windows win - 1 and win + m present in its read and live, and their states
@@ -357,7 +357,7 @@ int amira_gmg_bubble_policy(amira_gmg *h, const int32_t *spare_ranks, int32_t n_
  * tip_attach = cont(e') ^ 1, the state a walk leaves v through into the tip; tip_reads = the read steps on b.
  *
  * Every pointer may be NULL.  Call with n_tips only to size the outputs, then again for the arrays: the result is
- * kept on the device until the graph or a device buffer changes.  Leaves the filter masks alone.  Not available on a
+ * kept on the device until the next build, filter or node removal.  Leaves the filter masks alone.  Not available on a
  * sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for 2N >= 2^31. */
 int amira_gmg_tips(amira_gmg *h, int64_t *n_tips, int32_t *tip_unitig, int8_t *tip_orient, int32_t *tip_attach,
                    uint32_t *tip_reads);
@@ -384,7 +384,7 @@ int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_
  *
  * clip[n_tips] (host): 1 clips tip q, 0 leaves it; any other value is AMIRA_E_ARG.  NULL: the flags the last
  * amira_gmg_tip_policy left on the device; AMIRA_E_STATE when there are tips and no policy was computed on the current
- * tips (the graph or a device buffer changed since, or a call with host flags overwrote them).
+ * tips (a build, filter or node removal came since, or a call with host flags overwrote them).
  * Clip: a read step (win = i, length = l) of read r with nw windows on the unitig of a clipped tip attached at alpha:
  *   end clip:   i >= 1, i + l == nw, window i - 1 live with state alpha: the read's last l calls are dropped;
  *   start clip: i == 0, l < nw, window l live with state alpha ^ 1: the read's first l calls are dropped.
@@ -399,11 +399,7 @@ int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_
  * with n_calls only to size the outputs, then again for the arrays; every output may be NULL.  out_on_device != 0: the
  * array outputs are device pointers on the handle's device; a build from them can be given n_calls with
  * amira_gmg_input_calls.  Leaves the graph, the caches and the filter masks as they were; AMIRA_E_STATE on a sharded
- * handle.
- *
- * The tip and bubble calls reserve each other's buffers, so that on one graph a call of one family leaves the other's
- * cache and policy in place (for example bubble_policy, tips, tip_policy, clip_tip_reads, then correct_bubble_reads
- * with the held policy), as long as a call's gene ranks fit the room the handle holds for them. */
+ * handle. */
 int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                              int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped,
                              int out_on_device);
