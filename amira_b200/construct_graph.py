@@ -1071,20 +1071,31 @@ class GeneMerGraph:
 
         Rounds after the first run on the device handle alone: the policy, the correction and the rebuild stay on the
         GPU and only counts come back; the corrected reads are copied to the host and decoded once, at the end."""
-        src = self._source_encoded()
-        k = int(self._kmerSize)
-        filt = None if filter_graph is None else (max(int(filter_graph[0]), 0), max(int(filter_graph[1]), 0))
-        rounds, out, last, changed, filtered, h = [], None, None, None, False, None
-        for r in range(max_rounds):
-            if r == 0:
+        def correct(h, ranks):
+            if h is None:
                 x, n_bubbles, n_replaced = self._bubble_correction(sample_genesOfInterest, flags_on_device=True)
             else:
                 x, n_bubbles, n_replaced = self._handle_correction(h, ranks, True)
-            steps = int(x["branch_rewritten"].sum())
-            rounds.append({"bubbles": n_bubbles, "branches": len(x["branch_rewritten"]), "replaced": n_replaced,
-                           "steps": steps, "reads": int(x["changed"].sum()), "calls": len(x["ids"])})
+            return x, {"bubbles": n_bubbles, "branches": len(x["branch_rewritten"]), "replaced": n_replaced}
+        return self._rounds_until_stable(correct, {"branch_rewritten": "steps"}, max_rounds, sample_genesOfInterest,
+                                         filter_graph)
+
+    def _rounds_until_stable(self, correct, counts, max_rounds, sample_genesOfInterest, filter_graph):
+        """the rounds of correct_bubbles_until_stable and clean_until_stable.  correct(h, ranks) corrects this graph
+        (h None) or the graph the device handle h holds (ranks: the vocabulary ranks of sample_genesOfInterest) and
+        returns (the outputs of a DeviceGraph correction call, with its flags on the device for a device graph; the
+        round's own counts).  counts maps every per item count array of those outputs to the name of its sum in the
+        round's entry; the rounds stop at the first that sums all of them to 0"""
+        src = self._source_encoded()
+        k = int(self._kmerSize)
+        filt = None if filter_graph is None else (max(int(filter_graph[0]), 0), max(int(filter_graph[1]), 0))
+        rounds, out, last, changed, filtered, h, ranks = [], None, None, None, False, None, None
+        for r in range(max_rounds):
+            x, info = correct(h, ranks)
+            steps = {name: int(x[f].sum()) for f, name in counts.items()}
+            rounds.append({**info, **steps, "reads": int(x["changed"].sum()), "calls": len(x["ids"])})
             last = x
-            if steps == 0:
+            if not any(steps.values()):
                 break
             out = x                      # the previous CSR is dropped only now, after this round's correction
             changed = x["changed"] if changed is None else _union(changed, x["changed"])
@@ -1102,11 +1113,10 @@ class GeneMerGraph:
             R = len(src.read_ids)
             reads = src.corrected({"ids": src.ids, "off": src.off, "pos_start": src.pos_start, "pos_end": src.pos_end,
                                    "changed": np.zeros(R, np.uint8),
-                                   "branch_rewritten": _host(last["branch_rewritten"]) if last else np.zeros(0, np.uint32)})
+                                   **{f: _host(last[f]) if last else np.zeros(0, np.uint32) for f in counts}})
             reads.rounds = rounds
             return self, reads
-        reads = src.corrected({**out, "changed": _host(changed), "branch_rewritten": _host(out["branch_rewritten"])},
-                              self._device)
+        reads = src.corrected({**out, "changed": _host(changed), **{f: _host(out[f]) for f in counts}}, self._device)
         reads.rounds = rounds
         g = type(self)({}, self._kmerSize, device=self._device)
         g._encoded, g._reads, g._genePositions = reads, reads.reads, reads.positions
@@ -1117,6 +1127,77 @@ class GeneMerGraph:
             if filtered:
                 g._device_ops = (("filter_graph", filt),)
         return g, reads
+
+    def clean_compacted_reads(self, min_tip_length, sample_genesOfInterest={}):
+        """the reads cleaned of bubbles and tips in one pass, as a new encode.EncodedReads to rebuild from
+        (include/amira_gmg.h, amira_gmg_clean_reads): the edits of correct_compacted_bubbles(sample_genesOfInterest)
+        and the clips of clip_compacted_tips(min_tip_length, sample_genesOfInterest), both decided on this graph and
+        applied together (no call is both edited and clipped).  It carries `changed` (per read: edited or clipped),
+        `branch_rewritten` (per branch of compacted_bubbles()) and `tip_clipped` (per tip of compacted_tips()).  The
+        graph and its reads are left as they are.  A device graph is cleaned on the device and stays lazy."""
+        return self._source_encoded().corrected(self._clean(min_tip_length, sample_genesOfInterest)[0], self._device)
+
+    def _clean(self, min_tip_length, sample_genesOfInterest, flags_on_device=False) -> tuple:
+        """clean_compacted_reads before it becomes an EncodedReads: (the outputs of DeviceGraph.clean_reads, the
+        round's counts: bubbles, branches, branches replaced, tips, tips clipped).  A device graph whose handle has
+        clean_reads is cleaned on the handle alone; otherwise the numpy implementation runs"""
+        src = self._source_encoded()
+        if self._on_device():
+            h = self._require_device_state()
+            ranks = self._gene_ranks(list(sample_genesOfInterest))
+            if hasattr(h, "clean_reads"):
+                return self._handle_clean(h, ranks, min_tip_length, flags_on_device)
+            a = w = h.arrays()
+            u, bub, tips = self.compacted_unitigs(), self.compacted_bubbles(), self.compacted_tips()
+            (key,) = self._arrays("node_key")
+            amr = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(key), bool)
+        else:
+            a, w = self._unitig_index_arrays(), self._read_index_arrays()
+            u, bub, tips = self._unitigs_over(a), self._bubbles_over(a, w), self._tips_over(a, w)
+            amr_nodes = self.get_AMR_nodes(sample_genesOfInterest)
+            amr = np.asarray([nh in amr_nodes for nh in self._nodes], bool)
+            rank = {n: i + 1 for i, n in enumerate(src.vocab.names)}
+            key = np.asarray([[g.get_strand() * rank[g.get_name()] for g in n.get_canonical_geneMer()]
+                              for n in self._nodes.values()], np.int64).reshape(len(self._nodes), int(self._kmerSize))
+        rw = self._bubble_winners(bub, u, amr)
+        clip = self._tip_clip_flags(tips, u, a, amr, min_tip_length)
+        out = self._cleaned_reads_over(u, self._read_paths_over(a, w), bub, tips, w, key, rw, clip, src)
+        return out, {"bubbles": len(bub["source"]), "branches": len(rw), "replaced": int((rw >= 0).sum()),
+                     "tips": len(clip), "tips_clipped": int(clip.sum())}
+
+    @staticmethod
+    def _handle_clean(h, ranks, min_tip_length, flags_on_device) -> tuple:
+        """one cleaning of the graph the handle holds, with the device's two policies: (the cleaned CSR written on the
+        device, the round's counts as _clean gives them)"""
+        n_replaced = h.bubble_policy(ranks)
+        n_clipped = h.tip_policy(min_tip_length, ranks)
+        out = h.clean_reads(None, None, on_device=True, flags_on_device=flags_on_device)
+        return out, {"bubbles": h.bubble_counts()[0], "branches": len(out["branch_rewritten"]), "replaced": n_replaced,
+                     "tips": len(out["tip_clipped"]), "tips_clipped": n_clipped}
+
+    def clean_until_stable(self, min_tip_length, max_rounds=30, sample_genesOfInterest={}, filter_graph=None):
+        """rounds of clean_compacted_reads and a rebuild from the cleaned reads, until a round rewrites and clips no
+        read step or max_rounds rounds have run -> (graph, reads).  It gives exactly what this loop gives:
+
+            cur, e = self, reads of self
+            for _ in range(max_rounds):
+                e2 = cur.clean_compacted_reads(min_tip_length, sample_genesOfInterest)
+                if not (e2.branch_rewritten.any() or e2.tip_clipped.any()): break
+                e = e2; cur = GeneMerGraph(e, k); filter_graph and cur.filter_graph(*filter_graph)
+            return cur, e
+
+        As correct_bubbles_until_stable, with the cleaning in place of the bubble correction: `reads` carries
+        `changed` (the union over the rounds), `branch_rewritten` and `tip_clipped` (those of the last round that
+        changed a read), and `rounds`, per round run (the last one included) its bubbles, branches, branches replaced
+        (`replaced`), tips, tips clipped (`tips_clipped`), steps rewritten (`steps`), steps clipped (`steps_clipped`),
+        reads changed (`reads`) and the call count after it (`calls`).  Round 1 runs on this graph as it is; later rounds
+        run on the device handle alone, and only counts come back until the final CSR is copied and decoded once."""
+        def clean(h, ranks):
+            if h is None:
+                return self._clean(min_tip_length, sample_genesOfInterest, flags_on_device=True)
+            return self._handle_clean(h, ranks, min_tip_length, True)
+        return self._rounds_until_stable(clean, {"branch_rewritten": "steps", "tip_clipped": "steps_clipped"},
+                                         max_rounds, sample_genesOfInterest, filter_graph)
 
     def _source_encoded(self):
         """this graph's reads as an encode.EncodedReads: the one it was built from, or the reads encoded as the build
@@ -1132,11 +1213,30 @@ class GeneMerGraph:
     def _corrected_reads_over(u, p, bub, w, key, replace_with, src) -> dict:
         """amira_gmg_correct_bubble_reads over index arrays: u as compacted_unitigs, p as read_unitig_paths, bub as
         compacted_bubbles, the windows w (win_off, win_node with -1 for None, win_dir), node keys key[N, k], and the
-        encoded reads src (ids, off, pos_start, pos_end).  Every step is tested at once; the edits (which never
-        overlap) set per call its number of output calls, whose prefix sums place every call"""
+        encoded reads src (ids, off, pos_start, pos_end): the marks of _bubble_marks_over, the shared tail and the fill
+        of the edits"""
+        count, touched, changed = GeneMerGraph._unmarked(src)
+        rewritten, edits = GeneMerGraph._bubble_marks_over(u, p, bub, w, replace_with, src, count, touched, changed)
+        out, idx = GeneMerGraph._untouched_calls_over(count, touched, src)
+        out.update(changed=changed, branch_rewritten=rewritten)
+        GeneMerGraph._fill_edits(out, idx, edits, u, bub, key, src)
+        return out
+
+    @staticmethod
+    def _unmarked(src) -> tuple:
+        """the marks of a read correction before any edit or clip: (count, touched, changed) with every call copied
+        once and no read changed"""
+        G, R = len(src.ids), len(src.off) - 1
+        return np.ones(G, np.int64), np.zeros(G, bool), np.zeros(R, np.uint8)
+
+    @staticmethod
+    def _bubble_marks_over(u, p, bub, w, replace_with, src, count, touched, changed) -> tuple:
+        """the bubble edits over index arrays (as _corrected_reads_over) marked in count (output calls per input call),
+        touched (the calls not copied) and changed (per read).  Every step is tested at once; the edits never overlap.
+        -> (branch_rewritten, the edits for _fill_edits: None, or their first calls, lengths, kept branches and
+        directions of travel)"""
         rw = np.asarray(replace_with, np.int64)
-        ids, off = np.asarray(src.ids, np.int32), np.asarray(src.off, np.int64)
-        ps, pe = src.pos_start, src.pos_end
+        off = np.asarray(src.off, np.int64)
         R, NB = len(off) - 1, len(rw)
         if NB:
             boff = np.asarray(bub["branch_off"], np.int64)
@@ -1167,35 +1267,37 @@ class GeneMerGraph:
             fwd = (sp == sigma) & (sn == tau)
             ok = (node[before] >= 0) & (node[after] >= 0) & (fwd | ((sp == tau ^ 1) & (sn == sigma ^ 1)))
             t, fwd = t[ok], fwd[ok]
-        changed = np.zeros(R, np.uint8)
-        rewritten = np.zeros(NB, np.uint32)
-        count = np.ones(len(ids), np.int64)
-        touched = np.zeros(len(ids), bool)
-        if len(t):
-            r, gt, mt = read[t], g[t], m[t]
-            keep = rw[gt]
-            kb = bu[keep]
-            m2 = ulen[kb]
-            c0 = off[r] + win[t]
-            rep = np.repeat(c0 - np.cumsum(mt) + mt, mt) + np.arange(int(mt.sum()))
-            touched[rep] = True
-            count[rep] = 0
-            count[c0] = m2
-            changed[r] = 1
-            rewritten = np.bincount(gt, minlength=NB).astype(np.uint32)
-        out, idx = GeneMerGraph._untouched_calls_over(count, touched, src)
-        out.update(changed=changed, branch_rewritten=rewritten)
-        if len(t):
-            e = np.repeat(np.arange(len(t)), m2)
-            j = np.arange(int(m2.sum())) - np.repeat(np.cumsum(m2) - m2, m2)
-            walk = np.where(fwd, 1, -1)[e] * np.asarray(bub["branch_orient"], np.int64)[keep[e]]
-            n = np.asarray(u["unitig_nodes"], np.int64)[np.where(walk > 0, uoff[kb[e]] + j, uoff[kb[e]] + m2[e] - 1 - j)]
-            key = np.asarray(key, np.int64)
-            out["ids"][idx[c0[e]] + j] = np.where(walk * np.asarray(u["node_orient"], np.int64)[n] > 0, key[n, 0], -key[n, -1])
-            for f, x in (("pos_start", ps), ("pos_end", pe)):
-                if x is not None:
-                    out[f][idx[c0[e]] + j] = x[c0[e] + np.minimum(j, mt[e] - 1)]
-        return out
+        if not len(t):
+            return np.zeros(NB, np.uint32), None
+        r, gt, mt = read[t], g[t], m[t]
+        keep = rw[gt]
+        c0 = off[r] + win[t]
+        rep = np.repeat(c0 - np.cumsum(mt) + mt, mt) + np.arange(int(mt.sum()))
+        touched[rep] = True
+        count[rep] = 0
+        count[c0] = ulen[bu[keep]]
+        changed[r] = 1
+        return np.bincount(gt, minlength=NB).astype(np.uint32), (c0, mt, keep, fwd)
+
+    @staticmethod
+    def _fill_edits(out, idx, edits, u, bub, key, src):
+        """the calls of the edits of _bubble_marks_over written to their places idx[c] in the output CSR `out`: the
+        first genes of the kept branch's nodes in the direction of travel, with the positions of the replaced calls"""
+        if edits is None:
+            return
+        c0, mt, keep, fwd = edits
+        uoff = np.asarray(u["unitig_off"], np.int64)
+        kb = np.asarray(bub["branch_unitig"], np.int64)[keep]
+        m2 = np.diff(uoff)[kb]
+        e = np.repeat(np.arange(len(c0)), m2)
+        j = np.arange(int(m2.sum())) - np.repeat(np.cumsum(m2) - m2, m2)
+        walk = np.where(fwd, 1, -1)[e] * np.asarray(bub["branch_orient"], np.int64)[keep[e]]
+        n = np.asarray(u["unitig_nodes"], np.int64)[np.where(walk > 0, uoff[kb[e]] + j, uoff[kb[e]] + m2[e] - 1 - j)]
+        key = np.asarray(key, np.int64)
+        out["ids"][idx[c0[e]] + j] = np.where(walk * np.asarray(u["node_orient"], np.int64)[n] > 0, key[n, 0], -key[n, -1])
+        for f, x in (("pos_start", src.pos_start), ("pos_end", src.pos_end)):
+            if x is not None:
+                out[f][idx[c0[e]] + j] = x[c0[e] + np.minimum(j, mt[e] - 1)]
 
     @staticmethod
     def _untouched_calls_over(count, touched, src) -> tuple:
@@ -1291,41 +1393,62 @@ class GeneMerGraph:
     def _clipped_reads_over(u, p, tips, w, clip, src) -> dict:
         """amira_gmg_clip_tip_reads over index arrays: u as compacted_unitigs, p as read_unitig_paths, tips as
         compacted_tips, the windows w (win_off, win_node with -1 for None, win_dir), clip per tip and the encoded reads
-        src.  Every step is tested at once; a clip drops the calls of its step's windows at the read's end"""
+        src: the marks of _tip_marks_over and the shared tail"""
+        count, touched, changed = GeneMerGraph._unmarked(src)
+        clipped = GeneMerGraph._tip_marks_over(u, p, tips, w, clip, src, count, touched, changed)
+        out, _ = GeneMerGraph._untouched_calls_over(count, touched, src)
+        out.update(changed=changed, tip_clipped=clipped)
+        return out
+
+    @staticmethod
+    def _tip_marks_over(u, p, tips, w, clip, src, count, touched, changed) -> np.ndarray:
+        """the tip clips over index arrays (as _clipped_reads_over) marked in count, touched and changed as
+        _bubble_marks_over marks its edits.  Every step is tested at once; a clip drops the calls of its step's windows
+        at the read's end -> tip_clipped"""
         cf = np.asarray(clip).ravel()
         Q = len(tips["tip_unitig"])
         if len(cf) != Q or (Q and not np.isin(cf, (0, 1)).all()):
             raise ValueError("clip_tip_reads: clip must hold 0 or 1 for each of %d tips" % Q)
         off = np.asarray(src.off, np.int64)
-        R, G = len(off) - 1, int(off[-1])
-        count = np.ones(G, np.int64)
-        changed = np.zeros(R, np.uint8)
-        clipped = np.zeros(Q, np.uint32)
-        if Q and len(p["unitig"]):
-            unitig_tip = np.full(len(u["unitig_off"]) - 1, -1, np.int64)
-            unitig_tip[np.asarray(tips["tip_unitig"], np.int64)] = np.arange(Q)
-            q = unitig_tip[np.asarray(p["unitig"], np.int64)]
-            read = np.repeat(np.arange(R, dtype=np.int64), np.diff(p["path_off"]))
-            woff = np.asarray(w["win_off"], np.int64)
-            nw = np.diff(woff)[read]
-            i, ln = np.asarray(p["win"], np.int64), np.asarray(p["length"], np.int64)
-            end, start = (i >= 1) & (i + ln == nw), (i == 0) & (ln < nw)
-            flank = woff[read] + np.where(end, i - 1, np.where(start, ln, 0))
-            node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
-            fn = node[np.minimum(flank, max(len(node) - 1, 0))] if len(node) else np.zeros(0, np.int64)
-            state = 2 * fn + (d[np.minimum(flank, max(len(node) - 1, 0))] < 0)
-            att = np.asarray(tips["tip_attach"], np.int64)[np.maximum(q, 0)]
-            on = (q >= 0) & (cf[np.maximum(q, 0)] == 1) & (fn >= 0)
-            t_end = np.flatnonzero(on & end & (state == att))
-            t_start = np.flatnonzero(on & start & (state == (att ^ 1)))
-            t = np.concatenate([t_end, t_start])
-            c0 = np.concatenate([off[read[t_end] + 1] - ln[t_end], off[read[t_start]]])
-            lt = ln[t]
-            count[np.repeat(c0 - np.cumsum(lt) + lt, lt) + np.arange(int(lt.sum()))] = 0
-            changed[read[t]] = 1
-            clipped = np.bincount(q[t], minlength=Q).astype(np.uint32)
-        out, _ = GeneMerGraph._untouched_calls_over(count, count == 0, src)
-        out.update(changed=changed, tip_clipped=clipped)
+        R = len(off) - 1
+        if not (Q and len(p["unitig"])):
+            return np.zeros(Q, np.uint32)
+        unitig_tip = np.full(len(u["unitig_off"]) - 1, -1, np.int64)
+        unitig_tip[np.asarray(tips["tip_unitig"], np.int64)] = np.arange(Q)
+        q = unitig_tip[np.asarray(p["unitig"], np.int64)]
+        read = np.repeat(np.arange(R, dtype=np.int64), np.diff(p["path_off"]))
+        woff = np.asarray(w["win_off"], np.int64)
+        nw = np.diff(woff)[read]
+        i, ln = np.asarray(p["win"], np.int64), np.asarray(p["length"], np.int64)
+        end, start = (i >= 1) & (i + ln == nw), (i == 0) & (ln < nw)
+        flank = woff[read] + np.where(end, i - 1, np.where(start, ln, 0))
+        node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
+        fn = node[np.minimum(flank, max(len(node) - 1, 0))] if len(node) else np.zeros(0, np.int64)
+        state = 2 * fn + (d[np.minimum(flank, max(len(node) - 1, 0))] < 0)
+        att = np.asarray(tips["tip_attach"], np.int64)[np.maximum(q, 0)]
+        on = (q >= 0) & (cf[np.maximum(q, 0)] == 1) & (fn >= 0)
+        t_end = np.flatnonzero(on & end & (state == att))
+        t_start = np.flatnonzero(on & start & (state == (att ^ 1)))
+        t = np.concatenate([t_end, t_start])
+        c0 = np.concatenate([off[read[t_end] + 1] - ln[t_end], off[read[t_start]]])
+        lt = ln[t]
+        drop = np.repeat(c0 - np.cumsum(lt) + lt, lt) + np.arange(int(lt.sum()))
+        count[drop] = 0
+        touched[drop] = True
+        changed[read[t]] = 1
+        return np.bincount(q[t], minlength=Q).astype(np.uint32)
+
+    @staticmethod
+    def _cleaned_reads_over(u, p, bub, tips, w, key, replace_with, clip, src) -> dict:
+        """amira_gmg_clean_reads over index arrays (as _corrected_reads_over and _clipped_reads_over): the marks of
+        both into the same arrays (no call is both edited and clipped), then the shared tail and the fill of the edits
+        once"""
+        count, touched, changed = GeneMerGraph._unmarked(src)
+        rewritten, edits = GeneMerGraph._bubble_marks_over(u, p, bub, w, replace_with, src, count, touched, changed)
+        clipped = GeneMerGraph._tip_marks_over(u, p, tips, w, clip, src, count, touched, changed)
+        out, idx = GeneMerGraph._untouched_calls_over(count, touched, src)
+        out.update(changed=changed, branch_rewritten=rewritten, tip_clipped=clipped)
+        GeneMerGraph._fill_edits(out, idx, edits, u, bub, key, src)
         return out
 
     def clip_compacted_tips(self, min_length, sample_genesOfInterest={}):
@@ -1772,6 +1895,8 @@ def bind_upstream(upstream_construct_graph):
                    "_corrected_reads_over", "_adopt_build", "_bubble_correction", "_handle_correction",
                    "correct_bubbles_until_stable", "_untouched_calls_over", "compacted_tips", "_tips_over",
                    "_tip_clip_flags", "_clipped_reads_over", "clip_compacted_tips", "_tip_clip",
+                   "_unmarked", "_bubble_marks_over", "_fill_edits", "_tip_marks_over", "_cleaned_reads_over",
+                   "_rounds_until_stable", "clean_compacted_reads", "_clean", "_handle_clean", "clean_until_stable",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

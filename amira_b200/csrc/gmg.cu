@@ -98,8 +98,8 @@ struct amira_gmg {
     int k = 0;
     bool has_pos = false;
     bool input_on_device = false;
-    // device-resident input: the call count read_off[R] of the last build, reused while the same offsets
-    // array is passed again (the per-read kernel verifies it on the device: ST_STALE)
+    // device-resident input: the call count read_off[R] of the last build, reused by the next build only, when it
+    // gets the same offsets array again (the per-read kernel verifies it on the device: ST_STALE)
     const int64_t *cache_off = nullptr;
     int64_t cache_R = -1, cache_G = 0;
     // the call count the caller gave for the next build from a device CSR (amira_gmg_input_calls), used by that build
@@ -1578,6 +1578,11 @@ int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read
     AMIRA_TRY(check_handle(h));
     const int64_t *hint_off = h->hint_off, hint_R = h->hint_R, hint_G = h->hint_G;
     h->hint_off = nullptr;  // for this build only
+    // the call count cached by the previous build, for the device read_off that build borrowed: the caller keeps that
+    // array valid until this build, so an array passed here at the same address is still it.  Only this build may
+    // reuse the count; a later one could meet the address again in an array allocated after that one was freed.
+    const int64_t *cache_off = h->cache_off;
+    h->cache_off = nullptr;
     // a previous build nobody looked at: keep what it learned (table sizes, id width) if it has finished
     if (h->pending && h->pending_is_build && h->world == 1 && cudaEventQuery(h->ev_done) == cudaSuccess) finish(h, false);
     cudaGetLastError();
@@ -1607,18 +1612,15 @@ int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read
         if (input_on_device) {
             if (read_off == hint_off && R == hint_R) {
                 G = hint_G;  // the caller's count, verified on the device like a cached one
-                h->cache_off = read_off;
-                h->cache_R = R;
-                h->cache_G = G;
-            } else if (read_off == h->cache_off && R == h->cache_R) {
+            } else if (read_off == cache_off && R == h->cache_R) {
                 G = h->cache_G;  // verified on the device by the per-read pass (ST_STALE)
             } else {
                 AMIRA_CUDA(cudaMemcpyAsync(&G, read_off + R, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
                 AMIRA_CUDA(cudaStreamSynchronize(st));
-                h->cache_off = read_off;
-                h->cache_R = R;
-                h->cache_G = G;
             }
+            h->cache_off = read_off;
+            h->cache_R = R;
+            h->cache_G = G;
         } else {
             G = read_off[R];
         }
@@ -2598,11 +2600,16 @@ int clear_correct(amira_gmg *h) {
 
 // after the marks in the correction's cnt (and, for bubble edits, step_new and the bubbles' replace_with): one scan
 // over the calls gives every call's output index, then the new offsets and calls are written to the caller's device
-// arrays or, through one staging allocation, to its host arrays, with the per read flags and the per item counts
-// d_counts[n_counts].  Tip clips (edits == false) only hold codes 0 and 1, so the fill reads no bubble array.
+// arrays or, through one staging allocation, to its host arrays, with the per read flags and the per item counts a
+// and b (b.n = 0 when a call has one kind).  Without bubble edits (edits == false) the codes are 0 and 1 only, so the fill
+// reads no bubble array.
+struct ItemCounts {
+    uint32_t *out;          // the caller's array (may be NULL)
+    const uint32_t *dev;    // the counts on the device
+    int64_t n;
+};
 int write_corrected(amira_gmg *h, bool edits, int64_t *n_calls, int64_t *read_off, int32_t *ids, int32_t *pos_start,
-                    int32_t *pos_end, uint8_t *changed, uint32_t *counts, const uint32_t *d_counts, int64_t n_counts,
-                    int out_on_device) {
+                    int32_t *pos_end, uint8_t *changed, ItemCounts a, ItemCounts b, int out_on_device) {
     auto &c = h->correct;
     const auto &u = h->unitigs;
     const auto &p = h->paths;
@@ -2652,7 +2659,8 @@ int write_corrected(amira_gmg *h, bool edits, int64_t *n_calls, int64_t *read_of
         const void *src;
         size_t bytes;
     } jobs[] = {{changed, c.changed.p, (size_t)R},
-                {counts, d_counts, sizeof(uint32_t) * (size_t)n_counts},
+                {a.out, a.dev, sizeof(uint32_t) * (size_t)a.n},
+                {b.out, b.dev, sizeof(uint32_t) * (size_t)b.n},
                 {out_on_device ? nullptr : read_off, o_off, sizeof(int64_t) * (size_t)(R + 1)},
                 {out_on_device ? nullptr : ids, o_ids, sizeof(int32_t) * (size_t)total},
                 {out_on_device ? nullptr : o_ps ? pos_start : nullptr, o_ps, sizeof(int32_t) * (size_t)total},
@@ -2665,62 +2673,75 @@ int write_corrected(amira_gmg *h, bool edits, int64_t *n_calls, int64_t *read_of
     AMIRA_CUDA(cudaStreamSynchronize(st));
     return AMIRA_OK;
 }
+
+// replace_with (host) against the cached bubbles: every entry -1 or another branch of the same bubble.  NULL stands
+// for the replace_with of the last policy, which the device holds, valid by construction: AMIRA_E_STATE when there
+// are branches and that policy was not computed on the current bubbles.
+int check_replace_with(amira_gmg *h, const char *name, const int32_t *replace_with) {
+    const auto &q = h->bubbles;
+    const int64_t B = q.B, NB = q.NB;
+    if (NB == 0) return AMIRA_OK;
+    if (!replace_with) {
+        if (h->correct.policy.fresh(h)) return AMIRA_OK;
+        set_error("%s: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles", name,
+                  (long long)NB);
+        return AMIRA_E_STATE;
+    }
+    std::vector<int64_t> boff((size_t)B + 1);
+    AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    for (int64_t b = 0; b < B; ++b)
+        for (int64_t g = boff[b]; g < boff[b + 1]; ++g) {
+            const int64_t x = replace_with[g];
+            if (x != -1 && (x < boff[b] || x >= boff[b + 1] || x == g)) {
+                set_error("%s: replace_with[%lld] = %lld is not -1 or another branch of bubble %lld", name, (long long)g,
+                          (long long)x, (long long)b);
+                return AMIRA_E_ARG;
+            }
+        }
+    return AMIRA_OK;
+}
+
+// the bubble edits into the correction's scratch, after clear_correct and check_replace_with: host replace_with
+// overwrites the held policy, NULL uses it.  rewritten[g] counts the steps rewritten per branch.
+int mark_bubble_edits(amira_gmg *h, const int32_t *replace_with) {
+    auto &c = h->correct;
+    const auto &q = h->bubbles;
+    const auto &p = h->paths;
+    const int64_t B = q.B, NB = q.NB;
+    if (NB == 0) return AMIRA_OK;
+    cudaStream_t st = h->stream;
+    uint32_t *rewritten = c.rewritten.as<uint32_t>();
+    AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
+    h->lib_launches++;
+    if (replace_with) {
+        c.policy.valid = false;  // the policy's replace_with is overwritten
+        AMIRA_TRY(c.replace.reserve(sizeof(int32_t) * (size_t)h->n_edges));
+        AMIRA_CUDA(cudaMemcpyAsync(c.replace.p, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
+        h->lib_launches++;
+    }
+    if (p.T > 0)
+        LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+               (long long)p.T, p.path_off.as<int64_t>(), (long long)h->R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
+               h->win_dir.as<int8_t>(), h->off, h->unitigs.off.as<int64_t>(), q.unitig_branch.as<int32_t>(),
+               q.branch_off.as<int64_t>(), (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(),
+               q.branch_unitig.as<int32_t>(), c.replace.as<int32_t>(), c.cnt.as<uint32_t>(), c.step_new.as<int32_t>(),
+               c.changed.as<uint8_t>(), rewritten);
+    return AMIRA_OK;
+}
 }  // namespace
 
 int amira_gmg_correct_bubble_reads(amira_gmg *h, const int32_t *replace_with, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                                    int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
                                    int out_on_device) {
     AMIRA_TRY(unsharded_ready(h, "correct_bubble_reads"));
-    auto &c = h->correct;
-    const long long R = h->R;
     AMIRA_TRY(bubble_table(h));
-    const auto &q = h->bubbles;
-    const int64_t B = q.B, NB = q.NB;
-    cudaStream_t st = h->stream;
-    // NULL: the replace_with of the last policy, which the device holds, valid by construction
-    const bool held = NB > 0 && !replace_with;
-    if (held && !c.policy.fresh(h)) {
-        set_error("correct_bubble_reads: no replace_with for %lld branches, and no amira_gmg_bubble_policy on these bubbles",
-                  (long long)NB);
-        return AMIRA_E_STATE;
-    }
-    if (NB > 0 && !held) {
-        std::vector<int64_t> boff((size_t)B + 1);
-        AMIRA_TRY(d2h(h, boff.data(), q.branch_off.p, sizeof(int64_t) * (size_t)(B + 1)));
-        AMIRA_CUDA(cudaStreamSynchronize(st));
-        for (int64_t b = 0; b < B; ++b)
-            for (int64_t g = boff[b]; g < boff[b + 1]; ++g) {
-                const int64_t x = replace_with[g];
-                if (x != -1 && (x < boff[b] || x >= boff[b + 1] || x == g)) {
-                    set_error("correct_bubble_reads: replace_with[%lld] = %lld is not -1 or another branch of bubble %lld",
-                              (long long)g, (long long)x, (long long)b);
-                    return AMIRA_E_ARG;
-                }
-            }
-    }
-    if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no bubble
-    const auto &p = h->paths;
+    AMIRA_TRY(check_replace_with(h, "correct_bubble_reads", replace_with));
+    if (h->R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no bubble
     AMIRA_TRY(clear_correct(h));
-    uint32_t *cnt = c.cnt.as<uint32_t>(), *rewritten = c.rewritten.as<uint32_t>();
-    if (NB > 0) {
-        AMIRA_CUDA(cudaMemsetAsync(rewritten, 0, sizeof(uint32_t) * (size_t)NB, st));
-        h->lib_launches++;
-        if (!held) {
-            c.policy.valid = false;  // the policy's replace_with is overwritten
-            AMIRA_TRY(c.replace.reserve(sizeof(int32_t) * (size_t)h->n_edges));
-            AMIRA_CUDA(cudaMemcpyAsync(c.replace.p, replace_with, sizeof(int32_t) * (size_t)NB, cudaMemcpyHostToDevice, st));
-            h->lib_launches++;
-        }
-        if (p.T > 0)
-            LAUNCH(h, k_correct_mark, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
-                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
-                   h->win_dir.as<int8_t>(), h->off, h->unitigs.off.as<int64_t>(), q.unitig_branch.as<int32_t>(),
-                   q.branch_off.as<int64_t>(), (long long)B, q.source.as<int32_t>(), q.sink.as<int32_t>(),
-                   q.branch_unitig.as<int32_t>(), c.replace.as<int32_t>(), cnt, c.step_new.as<int32_t>(), c.changed.as<uint8_t>(),
-                   rewritten);
-    }
-    return write_corrected(h, true, n_calls, read_off, ids, pos_start, pos_end, changed, branch_rewritten, rewritten, NB,
-                           out_on_device);
+    AMIRA_TRY(mark_bubble_edits(h, replace_with));
+    return write_corrected(h, true, n_calls, read_off, ids, pos_start, pos_end, changed,
+                           {branch_rewritten, h->correct.rewritten.as<uint32_t>(), h->bubbles.NB}, {}, out_on_device);
 }
 
 namespace {
@@ -2828,48 +2849,80 @@ int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_
     return AMIRA_OK;
 }
 
+namespace {
+// clip (host) against the cached tips: every flag 0 or 1.  NULL stands for the flags of the last policy, which the
+// device holds: AMIRA_E_STATE when there are tips and that policy was not computed on the current tips.
+int check_clip(amira_gmg *h, const char *name, const uint8_t *clip) {
+    const int64_t Q = h->tips.Q;
+    if (Q == 0) return AMIRA_OK;
+    if (!clip) {
+        if (h->tips.policy.fresh(h)) return AMIRA_OK;
+        set_error("%s: no clip flags for %lld tips, and no amira_gmg_tip_policy on these tips", name, (long long)Q);
+        return AMIRA_E_STATE;
+    }
+    for (int64_t q = 0; q < Q; ++q)
+        if (clip[q] > 1) {
+            set_error("%s: clip[%lld] = %d is not 0 or 1", name, (long long)q, (int)clip[q]);
+            return AMIRA_E_ARG;
+        }
+    return AMIRA_OK;
+}
+
+// the tip clips into the correction's scratch, after clear_correct and check_clip: host flags overwrite the held
+// policy, NULL uses it.  tips.clipped[q] counts the steps clipped per tip.
+int mark_tip_clips(amira_gmg *h, const uint8_t *clip) {
+    auto &t = h->tips;
+    auto &c = h->correct;
+    const auto &p = h->paths;
+    const int64_t Q = t.Q, N = h->n_nodes;
+    if (Q == 0) return AMIRA_OK;
+    cudaStream_t st = h->stream;
+    AMIRA_TRY(t.clipped.reserve(sizeof(int32_t) * (size_t)N));
+    AMIRA_CUDA(cudaMemsetAsync(t.clipped.p, 0, sizeof(uint32_t) * (size_t)Q, st));
+    h->lib_launches++;
+    if (clip) {
+        t.policy.valid = false;  // the policy's flags are overwritten
+        AMIRA_TRY(t.clip.reserve((size_t)N));
+        AMIRA_CUDA(cudaMemcpyAsync(t.clip.p, clip, (size_t)Q, cudaMemcpyHostToDevice, st));
+        h->lib_launches++;
+    }
+    if (p.T > 0)
+        LAUNCH(h, k_tip_clip, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
+               (long long)p.T, p.path_off.as<int64_t>(), (long long)h->R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
+               h->win_dir.as<int8_t>(), h->off, t.unitig_tip.as<int32_t>(), t.attach.as<int32_t>(), t.clip.as<uint8_t>(),
+               c.cnt.as<uint32_t>(), c.changed.as<uint8_t>(), t.clipped.as<uint32_t>());
+    return AMIRA_OK;
+}
+}  // namespace
+
 int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                              int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped, int out_on_device) {
     AMIRA_TRY(unsharded_ready(h, "clip_tip_reads"));
-    auto &t = h->tips;
-    auto &c = h->correct;
-    const long long R = h->R, N = h->n_nodes;
     AMIRA_TRY(tip_table(h));
-    const int64_t Q = t.Q;
-    cudaStream_t st = h->stream;
-    // NULL: the clip flags of the last policy, which the device holds
-    const bool held = Q > 0 && !clip;
-    if (held && !t.policy.fresh(h)) {
-        set_error("clip_tip_reads: no clip flags for %lld tips, and no amira_gmg_tip_policy on these tips", (long long)Q);
-        return AMIRA_E_STATE;
-    }
-    if (Q > 0 && !held)
-        for (int64_t q = 0; q < Q; ++q)
-            if (clip[q] > 1) {
-                set_error("clip_tip_reads: clip[%lld] = %d is not 0 or 1", (long long)q, (int)clip[q]);
-                return AMIRA_E_ARG;
-            }
-    if (R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no tip
-    const auto &p = h->paths;
+    AMIRA_TRY(check_clip(h, "clip_tip_reads", clip));
+    if (h->R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node, no tip
     AMIRA_TRY(clear_correct(h));
-    if (Q > 0) {
-        AMIRA_TRY(t.clipped.reserve(sizeof(int32_t) * (size_t)N));
-        AMIRA_CUDA(cudaMemsetAsync(t.clipped.p, 0, sizeof(uint32_t) * (size_t)Q, st));
-        h->lib_launches++;
-        if (!held) {
-            t.policy.valid = false;  // the policy's flags are overwritten
-            AMIRA_TRY(t.clip.reserve((size_t)N));
-            AMIRA_CUDA(cudaMemcpyAsync(t.clip.p, clip, (size_t)Q, cudaMemcpyHostToDevice, st));
-            h->lib_launches++;
-        }
-        if (p.T > 0)
-            LAUNCH(h, k_tip_clip, grid_for(p.T, 256), 256, p.unitig.as<int32_t>(), p.win.as<int32_t>(), p.length.as<int32_t>(),
-                   (long long)p.T, p.path_off.as<int64_t>(), R, h->win_off.as<int64_t>(), h->win_node.as<int32_t>(),
-                   h->win_dir.as<int8_t>(), h->off, t.unitig_tip.as<int32_t>(), t.attach.as<int32_t>(), t.clip.as<uint8_t>(),
-                   c.cnt.as<uint32_t>(), c.changed.as<uint8_t>(), t.clipped.as<uint32_t>());
-    }
-    return write_corrected(h, false, n_calls, read_off, ids, pos_start, pos_end, changed, tip_clipped,
-                           t.clipped.as<uint32_t>(), Q, out_on_device);
+    AMIRA_TRY(mark_tip_clips(h, clip));
+    return write_corrected(h, false, n_calls, read_off, ids, pos_start, pos_end, changed,
+                           {tip_clipped, h->tips.clipped.as<uint32_t>(), h->tips.Q}, {}, out_on_device);
+}
+
+int amira_gmg_clean_reads(amira_gmg *h, const int32_t *replace_with, const uint8_t *clip, int64_t *n_calls, int64_t *read_off,
+                          int32_t *ids, int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *branch_rewritten,
+                          uint32_t *tip_clipped, int out_on_device) {
+    AMIRA_TRY(unsharded_ready(h, "clean_reads"));
+    AMIRA_TRY(bubble_table(h));
+    AMIRA_TRY(tip_table(h));
+    AMIRA_TRY(check_replace_with(h, "clean_reads", replace_with));
+    AMIRA_TRY(check_clip(h, "clean_reads", clip));
+    if (h->R == 0) return corrected_without_reads(h, n_calls, read_off, out_on_device);  // no read, no node
+    // no call is both edited and clipped (include/amira_gmg.h), so both marks share the one code per call
+    AMIRA_TRY(clear_correct(h));
+    AMIRA_TRY(mark_bubble_edits(h, replace_with));
+    AMIRA_TRY(mark_tip_clips(h, clip));
+    return write_corrected(h, h->bubbles.NB > 0, n_calls, read_off, ids, pos_start, pos_end, changed,
+                           {branch_rewritten, h->correct.rewritten.as<uint32_t>(), h->bubbles.NB},
+                           {tip_clipped, h->tips.clipped.as<uint32_t>(), h->tips.Q}, out_on_device);
 }
 
 int amira_gmg_debug_segsort(amira_gmg *h, uint32_t *data, const int64_t *off, int64_t n_seg, uint32_t *dups,

@@ -88,9 +88,10 @@ class DeviceGraph:
         return self
 
     def build_resident(self, encoded, k: int, device: int | None = None):
-        """build from an encode.EncodedReads whose CSR stays on the GPU between builds (k sweeps, rebuilds)"""
+        """build from an encode.EncodedReads whose CSR stays on the GPU between builds (k sweeps, rebuilds); its host
+        CSR gives the call count, so the build copies nothing back to size itself"""
         ids, off, ps, pe = encoded.device_csr(self.device if device is None else device)
-        return self.build(ids, off, k, ps, pe, on_device=True)
+        return self.build(ids, off, k, ps, pe, on_device=True, n_calls=len(encoded.ids))
 
     def sync(self):
         _lib.check(self._lib.amira_gmg_sync(self._h))
@@ -242,22 +243,36 @@ class DeviceGraph:
         branch: its reads rewritten) as numpy arrays, or with flags_on_device (and on_device) as device tensors of
         uint8 and int32"""
         NB = self.bubble_counts()[1]
-        rw = None
-        if replace_with is not None:
-            rw = np.asarray(replace_with, np.int64).ravel()
-            if len(rw) != NB or (len(rw) and (rw.min() < -1 or rw.max() >= NB)):
-                raise ValueError("correct_bubble_reads: replace_with must hold -1 or a branch index for each of %d "
-                                 "branches" % NB)
-            rw = np.ascontiguousarray(rw, np.int32)
-        return self._corrected_csr(lambda *a: self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), *a), NB,
-                                   "branch_rewritten", on_device, flags_on_device)
+        rw = self._replace_with_arg(replace_with, NB, "correct_bubble_reads")
+        return self._corrected_csr(lambda *a: self._lib.amira_gmg_correct_bubble_reads(self._h, _ptr(rw), *a),
+                                   {"branch_rewritten": NB}, on_device, flags_on_device)
 
-    def _corrected_csr(self, call, n_items, counts, on_device, flags_on_device) -> dict:
+    @staticmethod
+    def _replace_with_arg(replace_with, NB, name):
+        """replace_with as the C ABI takes it (None stays None), checked for its length and range"""
+        if replace_with is None:
+            return None
+        rw = np.asarray(replace_with, np.int64).ravel()
+        if len(rw) != NB or (len(rw) and (rw.min() < -1 or rw.max() >= NB)):
+            raise ValueError("%s: replace_with must hold -1 or a branch index for each of %d branches" % (name, NB))
+        return np.ascontiguousarray(rw, np.int32)
+
+    @staticmethod
+    def _clip_arg(clip, Q, name):
+        """clip flags as the C ABI takes them (None stays None), checked for their length and values"""
+        if clip is None:
+            return None
+        cf = np.asarray(clip).ravel()
+        if len(cf) != Q or (len(cf) and not np.isin(cf, (0, 1)).all()):
+            raise ValueError("%s: clip must hold 0 or 1 for each of %d tips" % (name, Q))
+        return np.ascontiguousarray(cf, np.uint8)
+
+    def _corrected_csr(self, call, counts, on_device, flags_on_device) -> dict:
         """the size pass and the fill pass of a correction call (n_calls, read_off, ids, pos_start, pos_end, changed,
-        per item counts, out_on_device) -> the dict correct_bubble_reads and clip_tip_reads return, the per item counts
-        under the name `counts`"""
+        one array per entry of `counts`, out_on_device) -> the dict correct_bubble_reads, clip_tip_reads and
+        clean_reads return, with the per item counts under the names of `counts` ({name: number of items})"""
         n = C.c_int64()
-        _lib.check(call(C.byref(n), *[None] * 6, 0))
+        _lib.check(call(C.byref(n), *[None] * (5 + len(counts)), 0))
         G, R = n.value, self.R
         if on_device:
             import torch
@@ -267,18 +282,20 @@ class DeviceGraph:
             new = lambda size, dt: np.empty(size, dt)
         a = {"ids": new(G, "int32"), "off": new(R + 1, "int64"),
              "pos_start": new(G, "int32") if self.has_pos else None, "pos_end": new(G, "int32") if self.has_pos else None,
-             "changed": np.empty(R, np.uint8), counts: np.empty(n_items, np.uint32)}
-        if on_device:
-            changed, per_item = new(R, "uint8"), new(n_items, "int32")     # per item counts < 2^31, as uint32
+             "changed": np.empty(R, np.uint8), **{f: np.empty(m, np.uint32) for f, m in counts.items()}}
+        if on_device:                                                        # per item counts < 2^31, as uint32
+            changed, per_item = new(R, "uint8"), {f: new(m, "int32") for f, m in counts.items()}
         else:
-            changed, per_item = a["changed"], a[counts]
+            changed, per_item = a["changed"], {f: a[f] for f in counts}
         _lib.check(call(None, _ptr(a["off"]), _ptr(a["ids"]), _ptr(a["pos_start"]), _ptr(a["pos_end"]), _ptr(changed),
-                        _ptr(per_item), int(bool(on_device))))
+                        *[_ptr(per_item[f]) for f in counts], int(bool(on_device))))
         if on_device and flags_on_device:
-            a["changed"], a[counts] = changed, per_item
+            a["changed"] = changed
+            a.update(per_item)
         elif on_device:
             a["changed"][:] = changed.cpu().numpy()
-            a[counts][:] = per_item.cpu().numpy().view(np.uint32)
+            for f in counts:
+                a[f][:] = per_item[f].cpu().numpy().view(np.uint32)
         return a
 
     def tips(self) -> dict:
@@ -321,14 +338,21 @@ class DeviceGraph:
         holds on the tip, a start clip those of its first step.  Returns the clipped CSR and changed as
         correct_bubble_reads does, with tip_clipped (per tip: the read steps clipped) in place of branch_rewritten"""
         Q = self.tip_count()
-        cf = None
-        if clip is not None:
-            cf = np.asarray(clip).ravel()
-            if len(cf) != Q or (len(cf) and not np.isin(cf, (0, 1)).all()):
-                raise ValueError("clip_tip_reads: clip must hold 0 or 1 for each of %d tips" % Q)
-            cf = np.ascontiguousarray(cf, np.uint8)
-        return self._corrected_csr(lambda *a: self._lib.amira_gmg_clip_tip_reads(self._h, _ptr(cf), *a), Q, "tip_clipped",
-                                   on_device, flags_on_device)
+        cf = self._clip_arg(clip, Q, "clip_tip_reads")
+        return self._corrected_csr(lambda *a: self._lib.amira_gmg_clip_tip_reads(self._h, _ptr(cf), *a),
+                                   {"tip_clipped": Q}, on_device, flags_on_device)
+
+    def clean_reads(self, replace_with=None, clip=None, on_device: bool = False, flags_on_device: bool = False) -> dict:
+        """the reads cleaned of bubbles and tips in one pass (amira_gmg_clean_reads): the edits of
+        correct_bubble_reads(replace_with) and the clips of clip_tip_reads(clip) on this graph, written as one CSR (no
+        call is both edited and clipped).  None takes the held replace_with of the last bubble_policy() or the held
+        flags of the last tip_policy().  Returns the CSR and changed as correct_bubble_reads does, with both
+        branch_rewritten and tip_clipped"""
+        NB, Q = self.bubble_counts()[1], self.tip_count()
+        rw = self._replace_with_arg(replace_with, NB, "clean_reads")
+        cf = self._clip_arg(clip, Q, "clean_reads")
+        return self._corrected_csr(lambda *a: self._lib.amira_gmg_clean_reads(self._h, _ptr(rw), _ptr(cf), *a),
+                                   {"branch_rewritten": NB, "tip_clipped": Q}, on_device, flags_on_device)
 
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""

@@ -103,7 +103,9 @@ int amira_gmg_kernel_launches(const amira_gmg *h, int64_t *n);
 /* The build: GeneMerGraph.__init__ (construct_graph.py:45-102) for R reads in CSR form.
  * signed_ids[read_off[R]], read_off[R+1]; pos_start/pos_end (nullable) are per-call read
  * coordinates (gene_positions, construct_read.py:46-52).  input_on_device != 0: the pointers are
- * device pointers valid on the handle's stream (they are borrowed until the next build/destroy).
+ * device pointers valid on the handle's stream (they are borrowed until the next build/destroy).  A device build
+ * remembers read_off[R] for the next build only: that build reuses it when it gets the same read_off and R, which
+ * the borrow makes the same array; any other build copies read_off[R] back unless amira_gmg_input_calls gave it.
  * Asynchronous with respect to the host unless a capacity retry is needed; errors detected on the
  * device (AMIRA_E_PALINDROME) are reported by amira_gmg_sync / amira_gmg_sizes / the exports. */
 int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read_off, int64_t R, int32_t k,
@@ -111,9 +113,8 @@ int amira_gmg_build(amira_gmg *h, const int32_t *signed_ids, const int64_t *read
 
 /* The call count of the NEXT amira_gmg_build only, for a device CSR (input_on_device) whose read_off[R] the caller
  * already knows, such as the outputs of amira_gmg_correct_bubble_reads (n_calls).  That build uses n_calls when it
- * gets the same read_off and R, instead of copying read_off[R] back to the host or trusting a count cached from an
- * earlier build of an array at the same address (which the caller may have freed and the allocator handed out
- * again).  The per-read pass still checks the count on the device.  Every build forgets the hint, used or not.
+ * gets the same read_off and R, instead of copying read_off[R] back to the host.  The per-read pass still checks the
+ * count on the device.  Every build forgets the hint, used or not.
  * AMIRA_E_ARG for a NULL read_off, R <= 0 or a negative n_calls. */
 int amira_gmg_input_calls(amira_gmg *h, const int64_t *read_off, int64_t R, int64_t n_calls);
 
@@ -403,6 +404,28 @@ int amira_gmg_tip_policy(amira_gmg *h, int32_t min_length, const int32_t *spare_
 int amira_gmg_clip_tip_reads(amira_gmg *h, const uint8_t *clip, int64_t *n_calls, int64_t *read_off, int32_t *ids,
                              int32_t *pos_start, int32_t *pos_end, uint8_t *changed, uint32_t *tip_clipped,
                              int out_on_device);
+
+/* The reads cleaned of bubbles and tips in one pass (no upstream counterpart; one iteration of the read corrections of
+ * upstream's iterative_bubble_popping, graph_utils.py:127-181): the edits of amira_gmg_correct_bubble_reads and the
+ * clips of amira_gmg_clip_tip_reads, applied to the same graph and written as one CSR.
+ *
+ * The two never touch the same call.  An edit rewrites calls [win, win + m) strictly inside a read, on the windows of
+ * a branch, and its flanking windows win - 1 and win + m are live windows on the bubble's junction nodes.  A clip
+ * drops the calls only tip windows hold, at a read's first or last step.  A branch unitig has one-edge lists at both
+ * ends; a tip unitig has a dead end, and its attach node has a list of two edges or more, so it lies on no branch.  No
+ * unitig is both a branch and a tip, so no window is, and the dropped calls of a clip (held by tip windows alone) are
+ * no call of an edit, whose windows lie on a branch or are its flanks on junction nodes.
+ *
+ * replace_with[n_branches] and clip[n_tips] (host) as the two calls take them, checked the same way (AMIRA_E_ARG),
+ * and overwriting the held policy the same way; NULL takes the held policy, AMIRA_E_STATE when there are branches
+ * (tips) and no bubble (tip) policy was computed on the current bubbles (tips).  Both are checked before any device
+ * work.  Outputs as the two calls: n_calls; read_off[R + 1], ids / pos_start / pos_end [n_calls]; changed[R] = 1 for a
+ * read edited or clipped; branch_rewritten[n_branches] and tip_clipped[n_tips].  Every output may be NULL; out_on_device
+ * and amira_gmg_input_calls as for the two calls.  Leaves the graph, the caches, both held policies and the filter
+ * masks as they were; AMIRA_E_STATE on a sharded handle. */
+int amira_gmg_clean_reads(amira_gmg *h, const int32_t *replace_with, const uint8_t *clip, int64_t *n_calls,
+                          int64_t *read_off, int32_t *ids, int32_t *pos_start, int32_t *pos_end, uint8_t *changed,
+                          uint32_t *branch_rewritten, uint32_t *tip_clipped, int out_on_device);
 
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
