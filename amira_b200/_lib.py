@@ -24,7 +24,7 @@ EXPORTED = (
     "amira_gmg_remove_nodes", "amira_gmg_remove_nodes_without_reads_of", "amira_gmg_linear_steps", "amira_gmg_linear_walks",
     "amira_gmg_unitigs", "amira_gmg_unitig_links", "amira_gmg_read_unitig_paths", "amira_gmg_bubbles",
     "amira_gmg_correct_bubble_reads", "amira_gmg_bubble_policy", "amira_gmg_input_calls", "amira_gmg_tips",
-    "amira_gmg_tip_policy", "amira_gmg_clip_tip_reads", "amira_gmg_clean_reads",
+    "amira_gmg_tip_policy", "amira_gmg_clip_tip_reads", "amira_gmg_clean_reads", "amira_gmg_gene_paths",
 )
 
 _lib = None
@@ -87,6 +87,7 @@ def load():
     lib.amira_gmg_tip_policy.argtypes = [vp, i32, vp, i32, vp, vp]
     lib.amira_gmg_clip_tip_reads.argtypes = [vp] * 9 + [C.c_int]
     lib.amira_gmg_clean_reads.argtypes = [vp] * 11 + [C.c_int]
+    lib.amira_gmg_gene_paths.argtypes = [vp, vp, i32] + [vp] * 15
     lib.amira_gmg_debug_layout.argtypes = [vp, C.c_int]
     lib.amira_gmg_debug_segsort.argtypes = [vp, vp, vp, i64, vp, C.POINTER(i64), C.c_int, i64]
     lib.amira_gmg_atomic_peak.argtypes = [vp, i64, i64] + [C.POINTER(C.c_double)] * 3

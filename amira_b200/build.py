@@ -10,7 +10,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libamira_gmg.so")
 SOURCES = ["gmg.cu", "comm.cu", "vocab_encode.cpp", "host_keys.cpp"]
-HEADERS = ["common.cuh", "gmg_kernels.cuh", "post_kernels.cuh", "scan.cuh", "segsort.cuh", "incidence.cuh", "stats.cuh", "paths.cuh", "unitigs.cuh", "bubbles.cuh", "correct.cuh", "tips.cuh", "sharded.cuh", os.path.join("..", "..", "include", "amira_gmg.h")]
+HEADERS = ["common.cuh", "gmg_kernels.cuh", "post_kernels.cuh", "scan.cuh", "segsort.cuh", "incidence.cuh", "stats.cuh", "paths.cuh", "unitigs.cuh", "bubbles.cuh", "correct.cuh", "tips.cuh", "gene_paths.cuh", "sharded.cuh", os.path.join("..", "..", "include", "amira_gmg.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "--use_fast_math",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-shared"]

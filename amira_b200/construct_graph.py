@@ -1487,6 +1487,105 @@ class GeneMerGraph:
         clip = self._tip_clip_flags(tips, u, a, np.asarray([nh in amr_nodes for nh in self._nodes], bool), min_length)
         return self._clipped_reads_over(u, self._read_paths_over(a, w), tips, w, clip, src)
 
+    def gene_paths(self, genesOfInterest) -> dict:
+        """the reads grouped by their path through the genes of interest (include/amira_gmg.h, amira_gmg_gene_paths), as
+        numpy arrays.  An occurrence is a maximal run of a read's live windows on nodes holding one of the genes: per
+        occurrence occ_read (index in get_reads()), occ_win (index in _readNodes[read]), occ_length (windows),
+        occ_flanks (1: a live window before it, 2: one after it), occ_orient and occ_cluster.  The occurrences with
+        both flanks (complete) are grouped by the canonical state sequence of their span (the run and its flanks); each
+        cluster, numbered by its first occurrence, is one genomic context: key_state[key_off[c]:key_off[c + 1]],
+        n_complete[c], and its members members[member_off[c]:member_off[c + 1]] (ascending occurrence indices),
+        which add the partial occurrences contained in its key and in no other (-1: in none, -2: in several).  Names
+        not in the graph's vocabulary are ignored.  A device graph is served by the device and stays lazy."""
+        genes = list(genesOfInterest)
+        for g in genes:
+            assert not (g[0] == "+" or g[0] == "-"), "Strand information cannot be present for any specified genes"
+        if self._on_device():
+            h = self._require_device_state()
+            ranks = sorted(set(self._gene_ranks(genes)))
+            if hasattr(h, "gene_paths"):
+                return h.gene_paths(ranks)
+            a = h.arrays()
+            marked = np.asarray(h.nodes_containing(ranks), bool) if ranks else np.zeros(len(a["node_cov"]), bool)
+            return self._gene_paths_over(a, marked)
+        amr_nodes = self.get_AMR_nodes(genes)
+        return self._gene_paths_over(self._read_index_arrays(), np.asarray([nh in amr_nodes for nh in self._nodes], bool))
+
+    @staticmethod
+    def _gene_paths_over(w, marked) -> dict:
+        """amira_gmg_gene_paths over index arrays: the windows w (win_off, win_node with -1 for None, win_dir) and
+        marked[n], node n holds a gene of interest.  The runs and flanks are found for every window at once; the
+        canonical sequences are grouped in a dict, and a partial occurrence is matched through the (cluster, position)
+        entries of the node of its first state"""
+        woff = np.asarray(w["win_off"], np.int64)
+        node, d = np.asarray(w["win_node"], np.int64), np.asarray(w["win_dir"], np.int64)
+        marked = np.asarray(marked, bool)
+        R, W = len(woff) - 1, len(node)
+        nw = np.diff(woff)
+        live = node >= 0
+        on = np.zeros(W, bool)
+        on[live] = marked[node[live]]
+        first, last = np.zeros(W, bool), np.zeros(W, bool)
+        first[woff[:-1][nw > 0]] = True
+        last[woff[1:][nw > 0] - 1] = True
+        before, after = np.zeros(W, bool), np.zeros(W, bool)
+        before[1:], after[:-1] = on[:-1], on[1:]
+        start = np.flatnonzero(on & ~(before & ~first))
+        end = np.flatnonzero(on & ~(after & ~last))
+        read = np.repeat(np.arange(R, dtype=np.int64), nw)[start]
+        left = (start > woff[read]) & live[np.maximum(start - 1, 0)]
+        right = (end + 1 < woff[read + 1]) & live[np.minimum(end + 1, max(W - 1, 0))]
+        s0, s1 = (start - left).tolist(), (end + right).tolist()
+        state = np.where(live, 2 * node + (d < 0), -1).tolist()
+        O = len(start)
+        orient = np.ones(O, np.int8)
+        spans, canon = [], []
+        for o in range(O):
+            S = tuple(state[s0[o]:s1[o] + 1])
+            RS = tuple(x ^ 1 for x in reversed(S))
+            spans.append((S, RS))
+            canon.append(S if S <= RS else RS)
+            orient[o] = 1 if S <= RS else -1
+        complete = left & right
+        cluster = np.full(O, -1, np.int64)
+        keys = {}
+        for o in np.flatnonzero(complete).tolist():
+            cluster[o] = keys.setdefault(canon[o], len(keys))
+        key_list = list(keys)                                     # insertion order: by first occurrence
+        entries = {}
+        for c, key in enumerate(key_list):
+            for j, s in enumerate(key):
+                entries.setdefault(s >> 1, []).append((c, j))
+        for o in np.flatnonzero(~complete).tolist():
+            S, RS = spans[o]
+            L = len(S)
+            found, fwd = set(), set()
+            for c, j in entries.get(S[0] >> 1, ()):
+                key = key_list[c]
+                if key[j] == S[0]:
+                    if key[j:j + L] == S:
+                        found.add(c)
+                        fwd.add(c)
+                elif j >= L - 1 and key[j - L + 1:j + 1] == RS:
+                    found.add(c)
+            if len(found) == 1:
+                cluster[o] = c = found.pop()
+                orient[o] = 1 if c in fwd else -1
+            elif found:
+                cluster[o] = -2
+        C = len(key_list)
+        mem = np.flatnonzero(cluster >= 0)
+        lengths = np.asarray([len(k) for k in key_list], np.int64)
+        return {"occ_read": read.astype(np.int32), "occ_win": (start - woff[read]).astype(np.int32),
+                "occ_length": (end - start + 1).astype(np.int32),
+                "occ_flanks": (left.astype(np.uint8) | (right.astype(np.uint8) << 1)).astype(np.uint8),
+                "occ_orient": orient, "occ_cluster": cluster.astype(np.int32),
+                "key_off": np.concatenate([[0], np.cumsum(lengths)]).astype(np.int64),
+                "key_state": np.asarray([s for k in key_list for s in k], np.int32),
+                "n_complete": np.bincount(cluster[complete], minlength=C).astype(np.uint32),
+                "member_off": np.concatenate([[0], np.cumsum(np.bincount(cluster[mem], minlength=C))]).astype(np.int64),
+                "members": mem[np.argsort(cluster[mem], kind="stable")].astype(np.int32)}
+
     def _on_device(self) -> bool:
         """the device copy still is this graph (no host-side mutation since the build / last device operation)"""
         return bool(self._device_synced) and len(self._reads) > 0
@@ -1897,6 +1996,7 @@ def bind_upstream(upstream_construct_graph):
                    "_tip_clip_flags", "_clipped_reads_over", "clip_compacted_tips", "_tip_clip",
                    "_unmarked", "_bubble_marks_over", "_fill_edits", "_tip_marks_over", "_cleaned_reads_over",
                    "_rounds_until_stable", "clean_compacted_reads", "_clean", "_handle_clean", "clean_until_stable",
+                   "gene_paths", "_gene_paths_over",
                    "_gml_from_arrays", "generate_gml") + _LAZY_ATTRS
     ns = {name: ours.__dict__[name] for name in gpu_methods}
     ns["_cls"] = _Up

@@ -13,6 +13,7 @@
 #include "bubbles.cuh"
 #include "correct.cuh"
 #include "tips.cuh"
+#include "gene_paths.cuh"
 #include "sharded.cuh"
 
 namespace amira {
@@ -82,7 +83,7 @@ struct amira_gmg {
     int n_pieces = 0;
     int n_sm = 148;
     int insert_ctas_per_sm = 1;
-    int force_layout = 0;        // test hook (amira_gmg_debug_layout): 1 = no 16-byte node slots, 2 = no 16-byte edge slots, 4 = no packed keys, 8 = the 16384-bucket shape of the partition pass, 16 = units share buckets pairwise
+    int force_layout = 0;        // test hook (amira_gmg_debug_layout): 1 = no 16-byte node slots, 2 = no 16-byte edge slots, 4 = no packed keys, 8 = the 16384-bucket shape of the partition pass, 16 = units share buckets pairwise, 32 = 3-bit gene path key hashes
     int id_bits = 0;             // bits a signed gene id takes in a packed key (from the largest |id| seen); 0 = unknown
     bool n16 = false, e16 = false;  // 16-byte node / edge slots in the current build
     NodeView nview;
@@ -239,6 +240,16 @@ struct amira_gmg {
         int64_t Q = 0;
         Derived policy;
     } tips;
+    // the reads grouped by their path through the genes of interest (gene_paths.cuh), for the ranks and key hash width
+    // they were computed with
+    struct : Derived {
+        DevBuf flags, counts, occ_read, occ_win, occ_length, occ_flanks, occ_orient, occ_cluster, span_w, span_len, occ_hash,
+            occ_slot, slot_occ, slot_first, cluster_first, key_len, key_off, key_state, node_cnt, node_off, ent_cluster,
+            ent_pos, n_complete, member_cnt, member_off, cursor, members, sort_tmp;
+        std::vector<int32_t> ranks;
+        int hash_bits = 64;
+        int64_t O = 0, C = 0, KS = 0, M = 0;
+    } gene_paths;
 };
 
 namespace {
@@ -2923,6 +2934,181 @@ int amira_gmg_clean_reads(amira_gmg *h, const int32_t *replace_with, const uint8
     return write_corrected(h, h->bubbles.NB > 0, n_calls, read_off, ids, pos_start, pos_end, changed,
                            {branch_rewritten, h->correct.rewritten.as<uint32_t>(), h->bubbles.NB},
                            {tip_clipped, h->tips.clipped.as<uint32_t>(), h->tips.Q}, out_on_device);
+}
+
+namespace {
+// the gene paths for ranks[n], cached under the rule of unitig_table and, beyond it, for the same ranks and hash width
+int gene_path_table(amira_gmg *h, const int32_t *ranks, int32_t n) {
+    auto &g = h->gene_paths;
+    const int hash_bits = (h->force_layout & 32) ? 3 : 64;
+    if (g.fresh(h) && g.hash_bits == hash_bits && g.ranks == std::vector<int32_t>(ranks, ranks + n)) return AMIRA_OK;
+    g.valid = false;
+    g.O = g.C = g.KS = g.M = 0;
+    const long long W = h->W, N = h->n_nodes;
+    cudaStream_t st = h->stream;
+    if (W > 0 && N > 0 && n > 0) {
+        AMIRA_TRY(flag_nodes_containing(h, ranks, n));
+        const uint8_t *marked = h->scratch_off.as<uint8_t>();
+        const int32_t *win_node = h->win_node.as<int32_t>(), *win_read = h->win_read.as<int32_t>();
+        const int8_t *win_dir = h->win_dir.as<int8_t>();
+        const int64_t *win_off = h->win_off.as<int64_t>();
+        AMIRA_TRY(g.flags.reserve((size_t)W));
+        AMIRA_TRY(g.counts.reserve(sizeof(unsigned long long) * 2));
+        uint8_t *flags = g.flags.as<uint8_t>();
+        unsigned long long *d_cnt = g.counts.as<unsigned long long>();
+        LAUNCH(h, k_gp_flags, grid_for(W, 256), 256, win_node, win_read, W, marked, flags);
+        // count, size the per-occurrence arrays, then number them
+        AMIRA_TRY(run_scan(h, GpOccLoad{flags}, GpOccStore{flags, win_read, win_off, W, nullptr, nullptr, nullptr, d_cnt}, nullptr, 1,
+                           W, W));
+        unsigned long long O = 0;
+        AMIRA_TRY(d2h(h, &O, d_cnt, sizeof(O)));
+        AMIRA_CUDA(cudaStreamSynchronize(st));
+        if (O > 0x7FFFFFFFull) {
+            set_error("gene_paths: %llu occurrences, more than 2^31 - 1", O);
+            return AMIRA_E_ARG;
+        }
+        if (O > 0) {
+            const size_t o4 = sizeof(int32_t) * (size_t)O;
+            for (DevBuf *b : {&g.occ_read, &g.occ_win, &g.occ_length, &g.occ_cluster, &g.span_len, &g.occ_slot, &g.cluster_first,
+                              &g.key_len})
+                AMIRA_TRY(b->reserve(o4));
+            AMIRA_TRY(g.occ_flanks.reserve((size_t)O));
+            AMIRA_TRY(g.occ_orient.reserve((size_t)O));
+            AMIRA_TRY(g.span_w.reserve(sizeof(int64_t) * (size_t)O));
+            AMIRA_TRY(g.occ_hash.reserve(sizeof(unsigned long long) * (size_t)O));
+            int32_t *occ_read = g.occ_read.as<int32_t>(), *occ_win = g.occ_win.as<int32_t>(), *occ_length = g.occ_length.as<int32_t>();
+            int32_t *occ_cluster = g.occ_cluster.as<int32_t>(), *span_len = g.span_len.as<int32_t>();
+            uint8_t *occ_flanks = g.occ_flanks.as<uint8_t>();
+            int8_t *occ_orient = g.occ_orient.as<int8_t>();
+            int64_t *span_w = g.span_w.as<int64_t>();
+            unsigned long long *occ_hash = g.occ_hash.as<unsigned long long>();
+            AMIRA_TRY(run_scan(h, GpOccLoad{flags}, GpOccStore{flags, win_read, win_off, W, occ_read, occ_win, occ_length, d_cnt},
+                               nullptr, 1, W, W));
+            LAUNCH(h, k_gp_span, grid_for(O, 256), 256, occ_read, occ_win, occ_length, (long long)O, win_off, win_node, win_dir,
+                   hash_bits, occ_flanks, occ_orient, span_w, span_len, occ_hash);
+            const GpSpans sp{span_w, span_len, occ_orient, win_node, win_dir};
+
+            // clusters of the complete occurrences; the table holds at least twice as many slots as there are occurrences
+            uint64_t cap = 2;
+            while (cap < 2 * (uint64_t)O) cap <<= 1;
+            AMIRA_TRY(g.slot_occ.reserve(sizeof(uint32_t) * cap));
+            AMIRA_TRY(g.slot_first.reserve(sizeof(uint32_t) * cap));
+            uint32_t *slot_first = g.slot_first.as<uint32_t>(), *occ_slot = g.occ_slot.as<uint32_t>();
+            AMIRA_CUDA(cudaMemsetAsync(g.slot_occ.p, 0xff, sizeof(uint32_t) * cap, st));
+            AMIRA_CUDA(cudaMemsetAsync(slot_first, 0xff, sizeof(uint32_t) * cap, st));
+            h->lib_launches += 2;
+            LAUNCH(h, k_gp_group, grid_for(O, 256), 256, occ_flanks, occ_hash, (long long)O, sp, (unsigned long long)(cap - 1),
+                   g.slot_occ.as<uint32_t>(), slot_first, occ_slot);
+            uint32_t *cluster_first = g.cluster_first.as<uint32_t>(), *key_len = g.key_len.as<uint32_t>();
+            AMIRA_TRY(run_scan(h, GpFirstLoad{occ_flanks, occ_slot, slot_first},
+                               GpClusterStore{(long long)O, span_len, occ_cluster, cluster_first, key_len, d_cnt}, nullptr, 1, O, O));
+            unsigned long long C = 0;
+            AMIRA_TRY(d2h(h, &C, d_cnt, sizeof(C)));
+            AMIRA_CUDA(cudaStreamSynchronize(st));
+            LAUNCH(h, k_gp_cluster, grid_for(O, 256), 256, occ_flanks, occ_slot, slot_first, (long long)O, occ_cluster);
+
+            // the keys, and the containment index over the nodes (no cluster: no entry, every partial unassigned)
+            AMIRA_TRY(g.key_off.reserve(sizeof(int64_t) * (size_t)(C + 1)));
+            AMIRA_TRY(g.node_off.reserve(sizeof(int64_t) * (size_t)(N + 1)));
+            AMIRA_TRY(g.node_cnt.reserve(sizeof(unsigned long long) * (size_t)(N + 1)));
+            AMIRA_TRY(g.cursor.reserve(sizeof(unsigned long long) * (size_t)(std::max<long long>(N, (long long)C) + 1)));
+            int64_t *key_off = g.key_off.as<int64_t>(), *node_off = g.node_off.as<int64_t>();
+            unsigned long long *node_cnt = g.node_cnt.as<unsigned long long>(), *cursor = g.cursor.as<unsigned long long>();
+            AMIRA_CUDA(cudaMemsetAsync(node_cnt, 0, sizeof(unsigned long long) * (size_t)N, st));
+            h->lib_launches++;
+            long long KS = 0;
+            if (C > 0) {
+                AMIRA_TRY(run_scan(h, UnitigLenLoad{key_len}, GpOffStore{key_off, nullptr}, nullptr, 1, C, C));
+                AMIRA_TRY(d2h(h, &KS, key_off + C, sizeof(KS)));
+                AMIRA_CUDA(cudaStreamSynchronize(st));
+                AMIRA_TRY(g.key_state.reserve(sizeof(int32_t) * (size_t)KS));
+                AMIRA_TRY(g.ent_cluster.reserve(sizeof(int32_t) * (size_t)KS));
+                AMIRA_TRY(g.ent_pos.reserve(sizeof(int32_t) * (size_t)KS));
+                LAUNCH(h, k_gp_key_fill, grid_for(C, 256), 256, cluster_first, (long long)C, key_off, sp, g.key_state.as<int32_t>(),
+                       node_cnt);
+            }
+            AMIRA_TRY(run_scan(h, DegLoad{node_cnt}, GpOffStore{node_off, cursor}, nullptr, 1, N, N));
+            if (C > 0)
+                LAUNCH(h, k_gp_key_place, grid_for(C, 256), 256, (long long)C, key_off, g.key_state.as<int32_t>(), cursor,
+                       g.ent_cluster.as<int32_t>(), g.ent_pos.as<int32_t>());
+            LAUNCH(h, k_gp_match, grid_for(O, 256), 256, occ_flanks, (long long)O, span_w, span_len, win_node, win_dir, node_off,
+                   g.ent_cluster.as<int32_t>(), g.ent_pos.as<int32_t>(), key_off, g.key_state.as<int32_t>(), occ_cluster, occ_orient);
+
+            // members, ascending per cluster
+            if (C > 0) {
+                AMIRA_TRY(g.member_cnt.reserve(sizeof(uint32_t) * (size_t)C));
+                AMIRA_TRY(g.n_complete.reserve(sizeof(uint32_t) * (size_t)C));
+                AMIRA_TRY(g.member_off.reserve(sizeof(int64_t) * (size_t)(C + 1)));
+                uint32_t *member_cnt = g.member_cnt.as<uint32_t>();
+                int64_t *member_off = g.member_off.as<int64_t>();
+                AMIRA_CUDA(cudaMemsetAsync(member_cnt, 0, sizeof(uint32_t) * (size_t)C, st));
+                AMIRA_CUDA(cudaMemsetAsync(g.n_complete.p, 0, sizeof(uint32_t) * (size_t)C, st));
+                h->lib_launches += 2;
+                LAUNCH(h, k_gp_member_count, grid_for(O, 256), 256, occ_cluster, occ_flanks, (long long)O, member_cnt,
+                       g.n_complete.as<uint32_t>());
+                AMIRA_TRY(run_scan(h, UnitigLenLoad{member_cnt}, GpOffStore{member_off, cursor}, nullptr, 1, C, C));
+                long long M = 0;
+                AMIRA_TRY(d2h(h, &M, member_off + C, sizeof(M)));
+                AMIRA_CUDA(cudaStreamSynchronize(st));
+                AMIRA_TRY(g.members.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(M, 1)));
+                AMIRA_TRY(g.sort_tmp.reserve(sizeof(uint32_t) * (size_t)std::max<long long>(M, 1)));
+                LAUNCH(h, k_gp_member_place, grid_for(O, 256), 256, occ_cluster, (long long)O, cursor, g.members.as<uint32_t>());
+                const long long n_seg = (long long)C;
+                AMIRA_CUDA(cudaMemcpyAsync(d_cnt + 1, &n_seg, sizeof(n_seg), cudaMemcpyHostToDevice, st));
+                h->lib_launches++;
+                AMIRA_TRY(run_segsort(h, g.members.as<uint32_t>(), g.sort_tmp.as<uint32_t>(), member_off, nullptr, false,
+                                      reinterpret_cast<const long long *>(d_cnt + 1), 1, (int64_t)C, M, (int64_t)O, nullptr,
+                                      nullptr));
+                g.M = M;
+            }
+            g.O = (int64_t)O;
+            g.C = (int64_t)C;
+            g.KS = KS;
+        }
+    }
+    g.ranks.assign(ranks, ranks + n);
+    g.hash_bits = hash_bits;
+    g.stamp(h);
+    return AMIRA_OK;
+}
+}  // namespace
+
+int amira_gmg_gene_paths(amira_gmg *h, const int32_t *ranks, int32_t n_ranks, int64_t *n_occurrences, int64_t *n_clusters,
+                         int64_t *n_key_states, int64_t *n_members, int32_t *occ_read, int32_t *occ_win, int32_t *occ_length,
+                         uint8_t *occ_flanks, int8_t *occ_orient, int32_t *occ_cluster, int64_t *key_off, int32_t *key_state,
+                         uint32_t *n_complete, int64_t *member_off, int32_t *members) {
+    AMIRA_TRY(unsharded_ready(h, "gene_paths"));
+    if (n_ranks < 0 || (n_ranks > 0 && !ranks)) {
+        set_error("gene_paths: bad gene ranks (n = %d)", n_ranks);
+        return AMIRA_E_ARG;
+    }
+    AMIRA_TRY(gene_path_table(h, ranks, n_ranks));
+    const auto &g = h->gene_paths;
+    const int64_t O = g.O, Cn = g.C, KS = g.KS, M = g.M;
+    if (n_occurrences) *n_occurrences = O;
+    if (n_clusters) *n_clusters = Cn;
+    if (n_key_states) *n_key_states = KS;
+    if (n_members) *n_members = M;
+    if (Cn == 0) {
+        if (key_off) key_off[0] = 0;
+        if (member_off) member_off[0] = 0;
+    }
+    if (O == 0) return AMIRA_OK;
+    AMIRA_TRY(d2h(h, occ_read, g.occ_read.p, sizeof(int32_t) * O));
+    AMIRA_TRY(d2h(h, occ_win, g.occ_win.p, sizeof(int32_t) * O));
+    AMIRA_TRY(d2h(h, occ_length, g.occ_length.p, sizeof(int32_t) * O));
+    AMIRA_TRY(d2h(h, occ_flanks, g.occ_flanks.p, (size_t)O));
+    AMIRA_TRY(d2h(h, occ_orient, g.occ_orient.p, (size_t)O));
+    AMIRA_TRY(d2h(h, occ_cluster, g.occ_cluster.p, sizeof(int32_t) * O));
+    if (Cn > 0) {
+        AMIRA_TRY(d2h(h, key_off, g.key_off.p, sizeof(int64_t) * (Cn + 1)));
+        AMIRA_TRY(d2h(h, key_state, g.key_state.p, sizeof(int32_t) * KS));
+        AMIRA_TRY(d2h(h, n_complete, g.n_complete.p, sizeof(uint32_t) * Cn));
+        AMIRA_TRY(d2h(h, member_off, g.member_off.p, sizeof(int64_t) * (Cn + 1)));
+        AMIRA_TRY(d2h(h, members, g.members.p, sizeof(uint32_t) * M));
+    }
+    AMIRA_CUDA(cudaStreamSynchronize(h->stream));
+    return AMIRA_OK;
 }
 
 int amira_gmg_debug_segsort(amira_gmg *h, uint32_t *data, const int64_t *off, int64_t n_seg, uint32_t *dups,

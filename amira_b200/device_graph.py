@@ -21,6 +21,10 @@ PATH_FIELDS = ("path_off", "unitig", "orient", "pos", "win", "length")
 BUBBLE_FIELDS = ("source", "sink", "branch_off", "branch_unitig", "branch_orient", "branch_reads")
 # the arrays of amira_gmg_tips, in its argument order
 TIP_FIELDS = ("tip_unitig", "tip_orient", "tip_attach", "tip_reads")
+# the arrays of amira_gmg_gene_paths, in its argument order, with their types
+GENE_PATH_FIELDS = (("occ_read", np.int32), ("occ_win", np.int32), ("occ_length", np.int32), ("occ_flanks", np.uint8),
+                    ("occ_orient", np.int8), ("occ_cluster", np.int32), ("key_off", np.int64), ("key_state", np.int32),
+                    ("n_complete", np.uint32), ("member_off", np.int64), ("members", np.int32))
 
 
 def _ptr(a):
@@ -354,6 +358,22 @@ class DeviceGraph:
         return self._corrected_csr(lambda *a: self._lib.amira_gmg_clean_reads(self._h, _ptr(rw), _ptr(cf), *a),
                                    {"branch_rewritten": NB, "tip_clipped": Q}, on_device, flags_on_device)
 
+    def gene_paths(self, ranks) -> dict:
+        """the reads grouped by their path through the genes of `ranks` (vocabulary ranks; amira_gmg_gene_paths): per
+        occurrence (a maximal run of a read's windows on nodes holding one of the genes) its read, first window, length
+        in windows, flanks (1 left, 2 right), orientation and cluster (-1 unassigned, -2 ambiguous); per cluster of
+        complete occurrences its key key_state[key_off[c]:key_off[c + 1]], its complete occurrences n_complete[c] and
+        its members members[member_off[c]:member_off[c + 1]] (occurrence indices, ascending)"""
+        r = np.ascontiguousarray(ranks, np.int32)
+        n = [C.c_int64() for _ in range(4)]
+        _lib.check(self._lib.amira_gmg_gene_paths(self._h, _ptr(r), len(r), *[C.byref(x) for x in n], *[None] * 11))
+        O, Cn, KS, M = (x.value for x in n)
+        size = {"key_off": Cn + 1, "key_state": KS, "n_complete": Cn, "member_off": Cn + 1, "members": M}
+        a = {f: np.zeros(size.get(f, O), t) for f, t in GENE_PATH_FIELDS}
+        _lib.check(self._lib.amira_gmg_gene_paths(self._h, _ptr(r), len(r), None, None, None, None,
+                                                  *[_ptr(a[f]) for f, _ in GENE_PATH_FIELDS]))
+        return a
+
     def filter_masks(self):
         """keep flags of the last filter / component removal, indexed by the pre-filter node / edge order"""
         a, b = C.c_int64(), C.c_int64()
@@ -389,7 +409,8 @@ class DeviceGraph:
         return n.value
 
     def debug_layout(self, mask: int):
-        """test hook: 1 = no 16-byte node slots, 2 = no 16-byte edge slots, 4 = no packed keys"""
+        """test hook: 1 = no 16-byte node slots, 2 = no 16-byte edge slots, 4 = no packed keys, 32 = gene_paths with a
+        3-bit key hash (include/amira_gmg.h)"""
         _lib.check(self._lib.amira_gmg_debug_layout(self._h, int(mask)))
 
     def debug_segsort(self, data, off, out_of_place=False, max_value=None):

@@ -84,6 +84,8 @@ class _Pool:
         backbone = rng.permutation(V)[: n_blocks * blk].astype(np.int32) + 1
         backbone *= rng.choice(np.array([-1, 1], np.int32), size=backbone.size)
         amr = rng.choice(V, size=cfg.n_amr, replace=False).astype(np.int32) + 1
+        self.amr = amr                                     # the AMR genes' ranks, and their loci over all genomes
+        self.amr_loci = np.zeros(cfg.n_amr, np.int64)
         seqs, genome_of, weight = [], [], []
         for g in range(cfg.n_genomes):
             chrom = backbone.copy().reshape(n_blocks, blk)
@@ -104,8 +106,9 @@ class _Pool:
                 p *= rng.choice(np.array([-1, 1], np.int32), size=p.size)
                 reps.append(p)
             # multi-copy AMR contexts: each AMR gene dropped into several loci of this genome
-            for a in amr:
+            for ai, a in enumerate(amr):
                 n_copy = int(rng.integers(cfg.amr_copies[0], cfg.amr_copies[1] + 1))
+                self.amr_loci[ai] += n_copy
                 for _ in range(n_copy):
                     ri = int(rng.integers(0, len(reps)))
                     at = int(rng.integers(0, len(reps[ri]) + 1))

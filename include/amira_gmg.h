@@ -427,6 +427,42 @@ int amira_gmg_clean_reads(amira_gmg *h, const int32_t *replace_with, const uint8
                           int64_t *read_off, int32_t *ids, int32_t *pos_start, int32_t *pos_end, uint8_t *changed,
                           uint32_t *branch_rewritten, uint32_t *tip_clipped, int out_on_device);
 
+/* The reads grouped by their path through the genes of interest (no upstream counterpart as one call; the nearest
+ * relative is assign_reads_to_genes with get_AMR_anchors and get_full_paths, construct_graph.py:2629-2691, 2725-2782,
+ * 2880-2939).  Over the per-read windows of the graph as it stands (built, filtered, nodes removed: amira_gmg_export_reads),
+ * not the compacted graph.
+ *
+ * Marked node: one that holds a gene of ranks[n_ranks] (vocabulary ranks, checked as amira_gmg_nodes_containing checks
+ * them).  A window of read r (index i in 0..nw-1) is live when its node is >= 0; its state is 2 * node + (dir < 0).
+ * Occurrence: a maximal run of windows i..j of one read, all live and on marked nodes; occurrences are numbered in
+ * global window order (read, then window).  It has a left flank when i >= 1 and window i - 1 is live (unmarked, by
+ * maximality), a right flank when j + 1 < nw and window j + 1 is live; with both it is complete, else partial.
+ * Span S: the states of windows i - 1 (with a left flank) .. j + 1 (with a right flank), in read order.  R(S) is S
+ * reversed with every state ^ 1; the canonical sequence is the lexicographically smaller of S and R(S) (int32
+ * sequences); occ_orient = +1 when S <= R(S), -1 otherwise.
+ * Clusters: the complete occurrences grouped by canonical sequence, numbered by their first occurrence; key(c) is that
+ * sequence.  A partial occurrence whose S or R(S) is a contiguous subsequence of the key of exactly one cluster c gets
+ * occ_cluster = c and occ_orient = +1 when S itself occurs in key(c), else -1; of no cluster -1, of two or more -2
+ * (ambiguous), both keeping the orientation of their own canonical sequence.  A complete occurrence's occ_cluster is
+ * its cluster.  Members of c: its complete occurrences and the partial ones assigned to it, ascending.
+ *
+ * Outputs, in an order that does not depend on thread timing or on the key hash:
+ *   per occurrence [n_occurrences]: occ_read, occ_win (its first window's index within the read, as in _readNodes),
+ *     occ_length (windows), occ_flanks (1 left, 2 right), occ_orient, occ_cluster;
+ *   per cluster [n_clusters]: key_off[C + 1] into key_state[n_key_states], n_complete (its complete occurrences),
+ *     member_off[C + 1] into members[n_members] (occurrence indices).
+ * Every pointer may be NULL.  Call with the counts only to size the outputs, then again for the arrays: the result is
+ * kept on the device, with the ranks it was computed for, until the next build, filter or node removal; a call with the
+ * same ranks launches nothing.  Leaves the graph, the filter masks, the other caches and both held policies as they were.
+ * Not available on a sharded handle (AMIRA_E_STATE); AMIRA_E_ARG for bad ranks and for more than 2^31 - 1 occurrences.
+ * Matching a partial occurrence walks the key entries of the node of its first state: O(partials x entries of that
+ * node x span length).  Out of scope: clusters that differ by a call error (clean the reads first, or threshold on the
+ * member counts), context beyond one flank window, one cluster set per gene (call once per gene). */
+int amira_gmg_gene_paths(amira_gmg *h, const int32_t *ranks, int32_t n_ranks, int64_t *n_occurrences, int64_t *n_clusters,
+                         int64_t *n_key_states, int64_t *n_members, int32_t *occ_read, int32_t *occ_win, int32_t *occ_length,
+                         uint8_t *occ_flanks, int8_t *occ_orient, int32_t *occ_cluster, int64_t *key_off, int32_t *key_state,
+                         uint32_t *n_complete, int64_t *member_off, int32_t *members);
+
 /* Multi-GPU (one process per GPU; no upstream counterpart -- upstream's joblib fan-out,
  * graph_utils.py:105-124, is disabled at every call site).  The globally ordered read set is
  * sharded contiguously over ranks in rank order; canonical gene-mers and edges are owned by hash
@@ -442,7 +478,8 @@ int amira_gmg_comm_init(amira_gmg *h, const void *nccl_unique_id, int rank, int 
 /* Test hook: forbid table layouts the library would otherwise choose from the input, so that the
  * rarely taken ones are exercised at small sizes.  mask bits: 1 = no 16-byte node slots, 2 = no
  * 16-byte edge slots, 4 = no packed keys (gene-mers compared through the ids array), 8 = the 16384-bucket
- * shape of the partition pass, 16 = units of the node -> reads transpose share buckets. */
+ * shape of the partition pass, 16 = units of the node -> reads transpose share buckets, 32 = amira_gmg_gene_paths
+ * cuts its key hash to 3 bits (every probe of its table then compares sequences; the outputs do not change). */
 int amira_gmg_debug_layout(amira_gmg *h, int mask);
 
 /* Test hook: the segmented sort behind the node -> reads and node -> edges lists, on host arrays:
